@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- path evaluations / second of the B200 hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Default workload (N=1): BASELINE config 4 -- MAACO, 4096 ants on a 512x512 synthetic block map
 (`blocks(512, 0.20, seed=4000)`), parameters of main.py:34-38.  One *step* = one colony pass
@@ -11,6 +11,10 @@ N>1 (torchrun): one process per GPU, the colony is sharded with 4096 ants per GP
 buffer of move codes + tau slices per pass; the same run also reports the fixed 4096-ant colony (strong scaling)
 and BASELINE config 5 (independent maps sharded over the ranks, no collective) under "extra", and checks that the
 sharded colony reproduces a single-GPU replay bit for bit ("parity_check").
+
+`--dump-outputs DIR` writes what the last timed pass handed its caller to DIR/<name>.npy (finite float64: -1 stands for
+the length of a failed tour; 64 MiB at most), so that two builds can be compared output for output: the inputs depend
+only on the arguments.
 
 `--impl reference` times the UNMODIFIED Python reference (baseline/_ref, copied there by build(); one single-threaded
 interpreter per host core) on bounded samples of the same workload, and reports the CPU oracle port
@@ -248,6 +252,52 @@ def time_colony(solver, K, W, flush, sync_all, it0=0):
     return ev, it
 
 
+# --dump-outputs: bytes each array may take (64 MiB in all); a larger one is written as a seeded sample of its rows
+DUMP_BUDGETS = {"ant_n_cells": 2 << 20, "ant_length": 2 << 20, "ant_turns": 2 << 20, "ant_tours": 32 << 20,
+                "pheromone": 24 << 20, "best": 1 << 10, "best_path": 1 << 20}
+
+
+def last_pass_outputs(solver):
+    """What the last colony pass handed a caller of MAACO.run_iteration: every ant's record and tour (last_tours; a
+    tour is -1 past its last cell; with N>1 GPUs the tours of this rank's ants), the pheromone field and the best
+    length / turns / cell count / path so far.  A length is -1 where the caller receives inf (no tour reached the
+    target), as the turns already are, so that every value written is finite.  Collective when the colony is sharded
+    (the best path lives on the rank whose ant found it)."""
+    import numpy as np
+    nc, ln, tn, cells = solver.last_tours()
+    cells[np.arange(cells.shape[1])[None, :] >= nc[:, None]] = -1
+    ln[~np.isfinite(ln)] = -1.0
+    st = solver._read_state()
+    if not np.isfinite(st.best_len):
+        st.best_len = -1.0
+    n_best = min(st.best_n_cells, solver._best_cells.numel())
+    if solver.world > 1 and n_best > 0:
+        import torch.distributed as dist
+        owner = dist.get_global_rank(solver.group, st.best_ant // solver.n_local)
+        dist.broadcast(solver._best_cells, src=owner, group=solver.group)
+    return {"ant_n_cells": nc, "ant_length": ln, "ant_turns": tn, "ant_tours": cells,
+            "pheromone": solver.pheromone_matrix, "best": [st.best_len, st.best_turns, st.best_n_cells],
+            "best_path": solver._best_cells[:n_best].cpu().numpy()}
+
+
+def save_outputs(out_dir, arrays, budgets):
+    """arrays[name] -> out_dir/<name>.npy in float64.  An array above budgets[name] bytes is replaced by the rows (first
+    axis) of a fixed, seeded sample that fits, and their indices go to <name>_rows.npy.  Every value must be finite."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if not np.isfinite(a).all():
+            raise ValueError(f"--dump-outputs: {name} has values that are not finite")
+        row_bytes = 8 * (a.size // max(1, a.shape[0]))
+        if row_bytes * a.shape[0] > budgets[name]:
+            k = budgets[name] // (row_bytes + 8)
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], k, replace=False))
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
 def run_gpu(args):
     import numpy as np
     import torch
@@ -305,6 +355,10 @@ def run_gpu(args):
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
     nc_last, _, _ = solver.last_results()
     path_cells = int(nc_last[nc_last > 0].sum())                   # cells that receive a deposit in one pass
+    if args.dump_outputs:                                          # before the e2e passes below move the colony on
+        outputs = last_pass_outputs(solver)
+        if rank == 0:
+            save_outputs(args.dump_outputs, outputs, DUMP_BUDGETS)
 
     # ---- e2e: the colony pass through the host-buffer entry point (MAACO.run_iteration_host -> C ABI
     #      mpp_maaco_pass_host): pinned host pheromone field in; per-ant records, best path, updated field out ----
@@ -668,7 +722,13 @@ def main():
     ap.add_argument("--batch-wave", type=int, default=128)
     ap.add_argument("--mpa-batch-maps", type=int, default=16, help="maps per GPU in the MPA part of config 5 (bounded sample)")
     ap.add_argument("--mpa-batch-iters", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed pass computed to DIR/<name>.npy (float64, at most 64 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)
