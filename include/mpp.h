@@ -255,6 +255,10 @@ typedef struct {
  * with libm on the host.  0 <= msd <= 180 (u16 classes).  Cached in the map for one msd at a time; called
  * implicitly by the stats entry points. */
 int mpp_map_safety_table(mpp_map *map, double min_safe_distance, void *stream);
+/* the same tables for every map of a batch (one launch, grid.y = map): [n_maps][rows*cols] classes and one LUT shared
+ * by all maps (it depends on msd only).  Cached in the batch for one msd at a time; called implicitly by
+ * mpp_astar_batch_maps.  Not for the view mpp_map_as_batch returns (its map has its own table). */
+int mpp_map_batch_safety_table(mpp_map_batch *maps, double min_safe_distance, void *stream);
 
 /* replaces helper.calculate_path_stats (helper.py:98-113; count_turns :58-65, safety :67-80, diagonal
  * penalty :82-96) and MPA._calculate_path_stats (MPA.py:215-229) for n_paths paths, one warp each.
@@ -280,6 +284,26 @@ int mpp_astar_batch(mpp_map *map, int variant, const int32_t *src_dev, const int
                     const uint32_t *avoid_bits_dev, int n, int allow_diagonal, int restrict_corner,
                     int32_t *cells_dev, int max_cells, int32_t *n_cells_dev, double *g_dev, void *scratch_dev,
                     size_t scratch_bytes, int n_slots, int heap_cap, unsigned long long *counters_dev, void *stream);
+
+/* search slots of a batch that are resident at once (mpp_astar_max_slots for a batch); the scratch of
+ * mpp_astar_batch_maps is 256 + n_slots * mpp_astar_slot_bytes(rows, cols, heap_cap) bytes, zero-filled once. */
+int mpp_map_batch_max_slots(const mpp_map_batch *maps);
+
+/* replaces one AStarSolver(grid).solve() (astar.py:33-101) / DijkstraSolver(grid).solve() (dijkstra.py:32-97) per map
+ * of a sweep over independent maps, statistics (helper.py:98-113) included: mpp_astar_batch over a batch of same-shape
+ * maps in one launch.  Query i runs on map map_dev[i] (any number of queries per map, each with its own endpoints and
+ * avoid set); a query whose map index or endpoint lies outside the batch / map gets n_cells = 0 without a search.
+ * Result conventions, avoid_bits_dev and counters_dev as mpp_astar_batch.  stats_policy (nullable): the lane group
+ * computes the statistics of its own path right after the search into stats_dev (n x 5, as mpp_path_stats; mode 0
+ * uses that map's safety table, mpp_map_batch_safety_table); a query with n_cells <= 0 or > max_cells gets the empty
+ * path's (inf, 0, 0, 0, inf).  order_dev: optional permutation of 0..n-1 = the order in which free slots take the
+ * queries (start the long ones first); results stay indexed by query.  n_slots <= mpp_map_batch_max_slots is useful. */
+int mpp_astar_batch_maps(mpp_map_batch *maps, int variant, const int32_t *map_dev, const int32_t *src_dev,
+                         const int32_t *dst_dev, const uint32_t *avoid_bits_dev, int n, int allow_diagonal,
+                         int restrict_corner, const mpp_policy *stats_policy, int32_t *cells_dev, int max_cells,
+                         int32_t *n_cells_dev, double *g_dev, double *stats_dev, void *scratch_dev, size_t scratch_bytes,
+                         int n_slots, int heap_cap, unsigned long long *counters_dev, const int32_t *order_dev,
+                         void *stream);
 
 /* replaces PSOSolver._reconstruct_path_from_position (pso.py:56-94, after rounding/clamping) /
  * GASolver._reconstruct_path_from_chromosome (ga_solver.py:58-93) followed by

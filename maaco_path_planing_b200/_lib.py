@@ -89,6 +89,11 @@ _SIGS = {
     "mpp_path_stats": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, C.POINTER(Policy), c_void_p, c_void_p]),
     "mpp_astar_scratch_bytes": (C.c_size_t, [c_void_p, c_int, c_int]),
     "mpp_astar_max_slots": (c_int, [c_void_p]),
+    "mpp_map_batch_safety_table": (c_int, [c_void_p, c_double, c_void_p]),
+    "mpp_map_batch_max_slots": (c_int, [c_void_p]),
+    "mpp_astar_batch_maps": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                                     C.POINTER(Policy), c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
+                                     C.c_size_t, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "mpp_astar_batch": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int,
                                 c_void_p, c_void_p, c_void_p, C.c_size_t, c_int, c_int, c_void_p, c_void_p]),
     "mpp_waypoint_fitness": (c_int, [c_void_p, c_void_p, c_int, c_int, C.POINTER(Policy), c_void_p, c_int, c_void_p,

@@ -405,3 +405,220 @@ def solve_mpa_batch(grids, num_predators, num_iterations, params, seeds=None, wa
             b.close()
     out.sort(key=lambda r: r[0])
     return out
+
+
+# ---- A* / Dijkstra over a batch of maps (astar.py, dijkstra.py) ------------------------------------------------------
+# algorithm -> (connector variant, the reference's errors for a map without start / target)
+_SEARCH_ALGORITHMS = {
+    "astar": (0, "AStar: Start node not found in grid.", "AStar: Target node not found in grid."),      # astar.py:19-20
+    "dijkstra": (2, "Dijkstra: Start node not found.", "Dijkstra: Target node not found."),           # dijkstra.py:19-20
+}
+
+
+def _search_algorithm(algorithm):
+    if algorithm not in _SEARCH_ALGORITHMS:
+        raise ValueError(f"algorithm must be 'astar' or 'dijkstra', not {algorithm!r}")
+    return _SEARCH_ALGORITHMS[algorithm]
+
+
+def _check_endpoints(flat, algorithm):
+    """Raises the reference constructor's ValueError for the first map (a row of `flat`, cell codes) that has no start
+    or no target -- what a loop of AStarSolver / DijkstraSolver constructors over the maps would raise."""
+    _, no_start, no_target = _search_algorithm(algorithm)
+    flat = np.asarray(flat)
+    has_s = (flat == START_NODE_VAL).any(axis=1)
+    has_t = (flat == TARGET_NODE_VAL).any(axis=1)
+    bad = np.flatnonzero(~(has_s & has_t))
+    if bad.size:
+        raise ValueError(no_start if not has_s[bad[0]] else no_target)
+
+
+def _valid_queries(map_index, src, dst, n_maps, n_cells):
+    """Bool tensor: query i names a map of the batch and both its endpoints are cells of that map.  The others get the
+    empty result without a search (astar.py:37-39)."""
+    if not (map_index.dim() == src.dim() == dst.dim() == 1):
+        raise ValueError("map_index, src and dst must be 1-D")
+    if not (map_index.numel() == src.numel() == dst.numel()):
+        raise ValueError(f"map_index, src and dst differ in length ({map_index.numel()}, {src.numel()}, {dst.numel()})")
+    return (map_index >= 0) & (map_index < n_maps) & (src >= 0) & (src < n_cells) & (dst >= 0) & (dst < n_cells)
+
+
+def _shape_waves(grids, lo, hi, wave=None):
+    """Maps lo..hi-1 grouped by shape (one mpp_map_batch each), `wave` maps per group at most (None: all of them)."""
+    shapes = {}
+    for i in range(lo, hi):
+        shapes.setdefault(np.asarray(grids[i]).shape, []).append(i)
+    out = []
+    for idx in shapes.values():
+        step = wave or len(idx)
+        out += [idx[w0:w0 + step] for w0 in range(0, len(idx), step)]
+    return out
+
+
+class SearchBatch:
+    """M same-shape maps for the deterministic baselines: `search` runs any number of A* / Dijkstra queries, each on
+    its own map with its own endpoints and avoid set, in one launch with the statistics of every path fused in
+    (mpp_astar_batch_maps); `solve` is AStarSolver(grid).solve() / DijkstraSolver(grid).solve() for every map at once.
+    Same parameters and defaults as AStarSolver (astar.py:11-14); start and target may differ from map to map."""
+
+    def __init__(self, grids, turn_penalty_factor=0.1, safety_penalty_factor=0.05, min_safe_distance=1.5,
+                 allow_diagonal_moves=True, restrict_diagonal_near_obstacle_policy=True,
+                 diagonal_obstacle_penalty_value=1000.0, *, device=None, max_cells=None, heap_cap=None, n_slots=None):
+        import torch
+        from .engine import make_policy
+        L = _lib.lib()
+        self._grids8 = _grids_u8(grids)
+        self.n_maps, self.rows, self.cols = self._grids8.shape
+        _lib.require_device()
+        self.device_index = torch.cuda.current_device() if device is None else int(device)
+        self.device = torch.device("cuda", self.device_index)
+        h = C.c_void_p()
+        _lib.check(L.mpp_map_batch_create(self._grids8.ctypes.data_as(C.c_void_p), self.n_maps, self.rows, self.cols,
+                                          self.device_index, C.byref(h)), "mpp_map_batch_create")
+        self._maps = h
+        self.allow_diagonal_moves = bool(allow_diagonal_moves)
+        self.restrict_corners = bool(restrict_diagonal_near_obstacle_policy)   # astar_strictly_restricts_corners
+        self.policy = make_policy(turn_penalty_factor, safety_penalty_factor, min_safe_distance,
+                                  diagonal_obstacle_penalty_value, restrict_diagonal_near_obstacle_policy,
+                                  allow_diagonal_moves, mode=0)
+        self.n = self.rows * self.cols
+        self.words = (self.n + 31) // 32
+        self.heap_cap = int(heap_cap or min(8 * self.n, max(4096, self.n // 4)))        # SearchEngine's sizes
+        self.max_cells = int(max_cells or min(self.n, max(4096, 16 * (self.rows + self.cols))))
+        self.max_slots = L.mpp_map_batch_max_slots(h)
+        self.n_slots = int(n_slots or self.max_slots)
+        self.counters = torch.zeros(4, dtype=torch.int64, device=self.device)  # expansions, relaxations, ring / heap pushes
+        self.launches = 0
+        self._scratch, self._scratch_key = None, None
+
+    def close(self):
+        h, self._maps = getattr(self, "_maps", None), None
+        if h:
+            _lib.lib().mpp_map_batch_destroy(h)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def expansions(self):
+        return int(self.counters[0].item())
+
+    def _i32(self, a):
+        import torch
+        if isinstance(a, torch.Tensor):
+            return a.to(device=self.device, dtype=torch.int32).contiguous()
+        return torch.as_tensor(np.ascontiguousarray(a, dtype=np.int32), device=self.device)
+
+    def _launch(self, variant, mi, src, dst, avoid, longest_first):
+        """One mpp_astar_batch_maps launch over the given (valid) queries with the current sizes."""
+        import torch as t
+        n, mc = mi.numel(), self.max_cells
+        slots = max(1, min(self.n_slots, n))
+        if self._scratch_key != (slots, self.heap_cap):                   # zero-filled once: search stamps live in it
+            nbytes = 256 + slots * _lib.lib().mpp_astar_slot_bytes(self.rows, self.cols, self.heap_cap)
+            self._scratch = t.zeros(nbytes, dtype=t.uint8, device=self.device)
+            self._scratch_key = (slots, self.heap_cap)
+        order = None
+        if longest_first and n > slots:
+            # a search costs roughly the square of its endpoint distance; the launch ends with its slowest query
+            dr = t.div(src, self.cols, rounding_mode="floor") - t.div(dst, self.cols, rounding_mode="floor")
+            dc = src % self.cols - dst % self.cols
+            order = t.argsort(dr.long() ** 2 + dc.long() ** 2, descending=True).to(t.int32).contiguous()
+        cells = t.empty((n, mc), dtype=t.int32, device=self.device)
+        ncell = t.empty(n, dtype=t.int32, device=self.device)
+        g = t.empty(n, dtype=t.float64, device=self.device)
+        stats = t.empty((n, 5), dtype=t.float64, device=self.device)
+        stream = C.c_void_p(t.cuda.current_stream(self.device).cuda_stream)
+        _lib.check(_lib.lib().mpp_astar_batch_maps(
+            self._maps, int(variant), _lib.ptr(mi), _lib.ptr(src), _lib.ptr(dst), _lib.ptr(avoid), n,
+            int(self.allow_diagonal_moves), int(self.restrict_corners), C.byref(self.policy), _lib.ptr(cells), mc,
+            _lib.ptr(ncell), _lib.ptr(g), _lib.ptr(stats), _lib.ptr(self._scratch), self._scratch.numel(), slots,
+            self.heap_cap, _lib.ptr(self.counters), _lib.ptr(order), stream), "mpp_astar_batch_maps")
+        self.launches += 1
+        return cells, ncell, g, stats
+
+    def search(self, variant, map_index, src, dst, avoid_bits=None, *, longest_first=True):
+        """Query i: connector `variant` (0 = astar.py, 1 = MPA.py's private A*, 2 = dijkstra.py) from cell src[i] to
+        cell dst[i] of map map_index[i], avoiding the cells set in avoid_bits[i] (n x ceil(rows*cols/32) bitmap words,
+        or None).  Returns device tensors (cells [n, max_cells] int32, n_cells [n] int32, g [n] float64 = g of the
+        popped target, stats [n, 5] float64 = (length, turns, safety, diag, fitness) of the path).  n_cells = 0: no
+        path, or an endpoint / map index outside the batch (not searched).  A heap overflow or a truncated path grows
+        the buffers and repeats only those queries (the searches are deterministic)."""
+        import torch as t
+        from .engine import SearchEngine
+        mi, src, dst = self._i32(map_index), self._i32(src), self._i32(dst)
+        valid = _valid_queries(mi, src, dst, self.n_maps, self.n)
+        n = mi.numel()
+        avoid = None
+        if avoid_bits is not None:
+            if isinstance(avoid_bits, np.ndarray):
+                avoid_bits = np.ascontiguousarray(avoid_bits).view(np.int32)
+            avoid = t.as_tensor(avoid_bits, device=self.device).contiguous().view(t.int32)   # (uint32 words as int32)
+            if avoid.numel() != n * self.words:
+                raise ValueError(f"avoid_bits must hold {n} x {self.words} words, not {avoid.numel()}")
+            avoid = avoid.reshape(n, self.words).contiguous()
+        cells = t.zeros((n, self.max_cells), dtype=t.int32, device=self.device)
+        ncell = t.zeros(n, dtype=t.int32, device=self.device)
+        g = t.full((n,), INF, dtype=t.float64, device=self.device)
+        stats = t.tensor([INF, 0.0, 0.0, 0.0, INF], dtype=t.float64, device=self.device).repeat(n, 1)   # helper.py:104-105
+        idx = valid.nonzero().squeeze(1)
+        while idx.numel():
+            sub = lambda x: None if x is None else x.index_select(0, idx).contiguous()
+            c, nc, gg, st = self._launch(variant, sub(mi), sub(src), sub(dst), sub(avoid), longest_first)
+            if c.shape[1] > cells.shape[1]:                                  # max_cells grew: widen the earlier rows
+                wide = t.zeros((n, c.shape[1]), dtype=t.int32, device=self.device)
+                wide[:, :cells.shape[1]] = cells
+                cells = wide
+            cells[idx, :c.shape[1]] = c
+            ncell[idx], g[idx], stats[idx] = nc, gg, st
+            bad = (nc < 0) | (nc > c.shape[1])
+            if not SearchEngine._grow_from(self, int(nc.min().item()), int(nc.max().item())):
+                break
+            idx = idx[bad]
+        return cells, ncell, g, stats
+
+    def solve(self, algorithm="astar"):
+        """One start -> target query per map.  Returns, per map, what AStarSolver(grid, ...).solve() (algorithm
+        "astar") or DijkstraSolver(grid, ...).solve() ("dijkstra") returns -- (path, length, turns, safety_p, diag_p,
+        fitness) -- followed by the value that solver appends to its convergence_curve (g, or None when the path has
+        at most one cell)."""
+        variant = _search_algorithm(algorithm)[0]
+        flat = self._grids8.reshape(self.n_maps, -1)
+        _check_endpoints(flat, algorithm)
+        src = (flat == START_NODE_VAL).argmax(axis=1)                      # first row-major 2 / 3 (astar.py:17-18)
+        dst = (flat == TARGET_NODE_VAL).argmax(axis=1)
+        cells, ncell, g, stats = self.search(variant, np.arange(self.n_maps), src, dst)
+        cells, ncell, g, stats = cells.cpu().numpy(), ncell.cpu().numpy(), g.cpu().numpy(), stats.cpu().numpy()
+        out = []
+        for k in range(self.n_maps):
+            n = int(ncell[k])
+            if n == 0:
+                out.append(([], INF, 0, 0.0, 0.0, INF, None))               # helper.py:104-105
+                continue
+            r, c = np.divmod(cells[k, :n], self.cols)
+            path = list(zip(r.tolist(), c.tolist()))
+            st = stats[k]
+            out.append((path, float(st[0]) if n > 1 else 0, int(st[1]), float(st[2]), float(st[3]), float(st[4]),
+                        float(g[k]) if n > 1 else None))                      # astar.py:70 (path and len(path) > 1)
+        return out
+
+
+def solve_search_batch(grids, algorithm, params, wave=None, group=None, device=None):
+    """A* or Dijkstra (algorithm "astar" / "dijkstra") start -> target on every grid of `grids` (this rank's shard when
+    `group` is given), grouped by shape, `wave` maps per launch (None: all of a shape).  `params` = SearchBatch's keyword
+    arguments.  Returns (map_index, path, length, turns, safety_p, diag_p, fitness, g) per map of this rank, g being the
+    convergence-curve value (None for a path of at most one cell)."""
+    _search_algorithm(algorithm)
+    lo, hi = shard_maps(len(grids), group)
+    for i in range(lo, hi):                                                  # before any device work
+        _check_endpoints(np.asarray(grids[i]).reshape(1, -1), algorithm)
+    out = []
+    for idx in _shape_waves(grids, lo, hi, wave):
+        b = SearchBatch(np.stack([np.asarray(grids[i]) for i in idx]), device=device, **params)
+        for i, r in zip(idx, b.solve(algorithm)):
+            out.append((i,) + tuple(r))
+        b.close()
+    out.sort(key=lambda r: r[0])
+    return out

@@ -2,6 +2,7 @@
 // Reference semantics: astar.py:33-101, MPA.py:106-151, helper.py:58-113, MPA.py:176-229,
 // pso.py:56-94, ga_solver.py:58-93.
 #include <cmath>
+#include <type_traits>
 #include <vector>
 
 #include "mpp_astar.cuh"
@@ -18,10 +19,12 @@
 // Only obstacles nearer than msd contribute (helper.py:76), and those lie inside the stencil.
 // Out-of-bounds is NOT an obstacle here (obstacle_nodes = argwhere(grid == 1), helper.py:125).
 // ---------------------------------------------------------------------------------------------
-__global__ void mpp_safety_kernel(const uint32_t *__restrict__ occ, int pitch, int R, int C, int radius,
+__global__ void mpp_safety_kernel(const uint32_t *__restrict__ occ, int occ_words, int pitch, int R, int C, int radius,
                                   uint16_t *__restrict__ cls) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= R * C) return;
+    occ += (size_t)blockIdx.y * occ_words;                     // blockIdx.y = map of a batch
+    cls += (size_t)blockIdx.y * R * C;
     const int r = i / C, c = i % C;
     int best = 1 << 30;
     for (int dr = -radius; dr <= radius; ++dr) {
@@ -40,35 +43,49 @@ __global__ void mpp_safety_kernel(const uint32_t *__restrict__ occ, int pitch, i
     cls[i] = (best == (1 << 30)) ? 0 : (uint16_t)best;          // best <= 2*radius^2 < 65536 (radius <= 180)
 }
 
+int mpp_build_safety(int device, const uint32_t *occ, int occ_words, int pitch_words, int rows, int cols, int n_maps,
+                     double msd, cudaStream_t s, double *cached_msd, uint16_t **d2, double **lut, int *lut_n) {
+    if (*cached_msd == msd && *d2) return MPP_OK;
+    MPP_CUDA(cudaSetDevice(device));
+    const int n = rows * cols;
+    const int radius = (int)msd;                               // an obstacle nearer than msd has |dr|, |dc| <= floor(msd)
+    const int need = 2 * radius * radius + 2;
+    if (!*d2) MPP_CUDA(cudaMalloc(d2, (size_t)n * n_maps * sizeof(uint16_t)));
+    if (*lut_n < need) {
+        MPP_CUDA(cudaStreamSynchronize(s));                     // a kernel of an earlier call may still read the old table
+        if (*lut) MPP_CUDA(cudaFree(*lut));
+        *lut = nullptr;
+        MPP_CUDA(cudaMalloc(lut, (size_t)need * sizeof(double)));
+        *lut_n = need;
+    }
+    std::vector<double> h((size_t)need, 0.0);
+    for (int k = 1; k < need; ++k) {
+        const double d = std::sqrt((double)k);
+        h[k] = (d < msd) ? std::pow(msd - d, 2.0) : 0.0;        // helper.py:77-78 (float ** 2 -> libm pow)
+    }
+    MPP_CUDA(cudaMemcpyAsync(*lut, h.data(), (size_t)need * sizeof(double), cudaMemcpyHostToDevice, s));
+    MPP_CUDA(cudaStreamSynchronize(s));
+    mpp_safety_kernel<<<dim3((n + 255) / 256, n_maps), 256, 0, s>>>(occ, occ_words, pitch_words, rows, cols, radius, *d2);
+    MPP_CUDA(cudaGetLastError());
+    *cached_msd = msd;
+    return MPP_OK;
+}
+
 extern "C" int mpp_map_safety_table(mpp_map *map, double msd, void *stream) {
     MPP_REQUIRE(map, "mpp_map_safety_table: null map");
     MPP_REQUIRE(msd >= 0.0 && msd <= 180.0, "mpp_map_safety_table: min_safe_distance %g unsupported (0 <= msd <= 180)", msd);
-    if (map->safety_msd == msd && map->safety_d2_dev) return MPP_OK;
-    MPP_CUDA(cudaSetDevice(map->device));
-    const int n = map->rows * map->cols;
-    const int radius = (int)msd;                               // an obstacle nearer than msd has |dr|, |dc| <= floor(msd)
-    const int lut_n = 2 * radius * radius + 2;
-    cudaStream_t s = (cudaStream_t)stream;
-    if (!map->safety_d2_dev) MPP_CUDA(cudaMalloc(&map->safety_d2_dev, (size_t)n * sizeof(uint16_t)));
-    if (map->safety_lut_n < lut_n) {
-        MPP_CUDA(cudaStreamSynchronize(s));                     // a kernel of an earlier call may still read the old table
-        if (map->safety_lut_dev) MPP_CUDA(cudaFree(map->safety_lut_dev));
-        map->safety_lut_dev = nullptr;
-        MPP_CUDA(cudaMalloc(&map->safety_lut_dev, (size_t)lut_n * sizeof(double)));
-        map->safety_lut_n = lut_n;
-    }
-    std::vector<double> lut((size_t)lut_n, 0.0);
-    for (int d2 = 1; d2 < lut_n; ++d2) {
-        const double d = std::sqrt((double)d2);
-        lut[d2] = (d < msd) ? std::pow(msd - d, 2.0) : 0.0;     // helper.py:77-78 (float ** 2 -> libm pow)
-    }
-    MPP_CUDA(cudaMemcpyAsync(map->safety_lut_dev, lut.data(), (size_t)lut_n * sizeof(double), cudaMemcpyHostToDevice, s));
-    MPP_CUDA(cudaStreamSynchronize(s));
-    mpp_safety_kernel<<<(n + 255) / 256, 256, 0, s>>>(map->occ_dev, map->pitch_words, map->rows, map->cols, radius,
-                                                      map->safety_d2_dev);
-    MPP_CUDA(cudaGetLastError());
-    map->safety_msd = msd;
-    return MPP_OK;
+    return mpp_build_safety(map->device, map->occ_dev, map->occ_words, map->pitch_words, map->rows, map->cols, 1, msd,
+                            (cudaStream_t)stream, &map->safety_msd, &map->safety_d2_dev, &map->safety_lut_dev,
+                            &map->safety_lut_n);
+}
+
+extern "C" int mpp_map_batch_safety_table(mpp_map_batch *maps, double msd, void *stream) {
+    MPP_REQUIRE(maps, "mpp_map_batch_safety_table: null batch");
+    MPP_REQUIRE(maps->owns, "mpp_map_batch_safety_table: a single map's batch view has no tables of its own (use mpp_map_safety_table)");
+    MPP_REQUIRE(msd >= 0.0 && msd <= 180.0, "mpp_map_batch_safety_table: min_safe_distance %g unsupported (0 <= msd <= 180)", msd);
+    return mpp_build_safety(maps->device, maps->occ_dev, maps->occ_words, maps->pitch_words, maps->rows, maps->cols,
+                            maps->n_maps, msd, (cudaStream_t)stream, &maps->safety_msd, &maps->safety_d2_dev,
+                            &maps->safety_lut_dev, &maps->safety_lut_n);
 }
 
 __global__ void __launch_bounds__(MPP_AS_THREADS)
@@ -124,6 +141,7 @@ extern "C" size_t mpp_astar_slot_bytes(int rows, int cols, int heap_cap) {
 
 // search slots (lane groups) that are resident at once: three CTAs of MPP_AS_GROUPS groups per SM
 extern "C" int mpp_astar_max_slots(const mpp_map *map) { return map ? map->sm_count * 3 * MPP_AS_GROUPS : 0; }
+extern "C" int mpp_map_batch_max_slots(const mpp_map_batch *maps) { return maps ? maps->sm_count * 3 * MPP_AS_GROUPS : 0; }
 
 struct BatchArgs {
     AStarGrid G;
@@ -141,8 +159,21 @@ struct BatchArgs {
     unsigned long long *counters;
 };
 
-template <bool OCC_SMEM>
-__global__ void __launch_bounds__(MPP_AS_THREADS, 3) mpp_astar_batch_kernel(BatchArgs A) {
+// queries over a batch of maps: query i runs on map map[i] of the [n_maps][occ_words] occupancy
+struct BatchMapsArgs : BatchArgs {
+    const int32_t *map;
+    int n_maps;
+    const int32_t *order;   // optional processing order of the queries (null: index order)
+    StatsCtx X;             // statistics of each found path (X.cls: [n_maps][R*C] safety classes or null)
+    double *stats;          // n x 5, or null: no statistics
+};
+
+// BatchArgs:     every query on the one map (G.occ, staged in shared memory when OCC_SMEM).
+// BatchMapsArgs: query i on map A.map[i], read through that map's slice of global memory (L2), and -- with A.stats --
+//                the statistics of its path computed by the same lane group right after the search.
+template <bool OCC_SMEM, class Args>
+__global__ void __launch_bounds__(MPP_AS_THREADS, 3) mpp_astar_batch_kernel(Args A) {
+    constexpr bool MAPS = std::is_same<Args, BatchMapsArgs>::value;
     extern __shared__ __align__(16) uint32_t s_occ[];
     __shared__ __align__(8) uint64_t s_bar;
     __shared__ __align__(16) uint8_t s_cnt[MPP_AS_GROUPS][MPP_PQ_NB];
@@ -165,9 +196,29 @@ __global__ void __launch_bounds__(MPP_AS_THREADS, 3) mpp_astar_batch_kernel(Batc
         i = grp_shfl(L, i, 0);
         if (i >= A.n) break;
         double g;
-        const int len = astar_search(L, G, S, A.variant, A.src[i], A.dst[i], A.avoid ? A.avoid + (size_t)i * A.words : nullptr,
-                                     A.cells + (size_t)i * A.max_cells, A.max_cells, &g, A.counters);
-        if (lane == 0) { A.n_cells[i] = len; if (A.g) A.g[i] = g; }
+        if constexpr (!MAPS) {
+            const int len = astar_search(L, G, S, A.variant, A.src[i], A.dst[i], A.avoid ? A.avoid + (size_t)i * A.words : nullptr,
+                                         A.cells + (size_t)i * A.max_cells, A.max_cells, &g, A.counters);
+            if (lane == 0) { A.n_cells[i] = len; if (A.g) A.g[i] = g; }
+        } else {
+            if (A.order) i = A.order[i];                               // longest queries first (see mpp_astar_batch_maps)
+            const int m = A.map[i], src = A.src[i], dst = A.dst[i];
+            int32_t *path = A.cells + (size_t)i * A.max_cells;
+            int len = 0;
+            g = __longlong_as_double(MPP_INF_BITS);
+            AStarGrid Gm = G;
+            Gm.occ = A.G.occ + (size_t)m * A.occ_words;
+            if ((unsigned)m < (unsigned)A.n_maps && (unsigned)src < (unsigned)rc && (unsigned)dst < (unsigned)rc)
+                len = astar_search(L, Gm, S, A.variant, src, dst, A.avoid ? A.avoid + (size_t)i * A.words : nullptr, path,
+                                   A.max_cells, &g, A.counters);
+            if (lane == 0) { A.n_cells[i] = len; if (A.g) A.g[i] = g; }
+            if (A.stats) {                                             // helper.py:98-113 on the path just found
+                StatsCtx X = A.X;
+                X.occ = Gm.occ;
+                if (X.cls) X.cls += (size_t)m * rc;
+                path_stats_warp(L, X, path, (len > 0 && len <= A.max_cells) ? len : 0, A.stats + (size_t)i * 5);
+            }
+        }
     }
 }
 
@@ -204,13 +255,57 @@ extern "C" int mpp_astar_batch(mpp_map *map, int variant, const int32_t *src_dev
     const size_t smem = (size_t)map->occ_words * 4;
     const int blocks = (n_slots + MPP_AS_GROUPS - 1) / MPP_AS_GROUPS;
     if (smem <= 32 * 1024) {
-        mpp_astar_batch_kernel<true><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
+        mpp_astar_batch_kernel<true, BatchArgs><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
     } else if (smem <= 40 * 1024) {
-        MPP_CUDA(cudaFuncSetAttribute(mpp_astar_batch_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        mpp_astar_batch_kernel<true><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
+        MPP_CUDA(cudaFuncSetAttribute(mpp_astar_batch_kernel<true, BatchArgs>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        mpp_astar_batch_kernel<true, BatchArgs><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
     } else {
-        mpp_astar_batch_kernel<false><<<blocks, MPP_AS_THREADS, 0, s>>>(A);
+        mpp_astar_batch_kernel<false, BatchArgs><<<blocks, MPP_AS_THREADS, 0, s>>>(A);
     }
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
+
+// Queries over a batch of same-shape maps (query i on map map_dev[i]), the statistics of each path fused in.
+extern "C" int mpp_astar_batch_maps(mpp_map_batch *maps, int variant, const int32_t *map_dev, const int32_t *src_dev,
+                                    const int32_t *dst_dev, const uint32_t *avoid_bits_dev, int n, int allow_diagonal,
+                                    int restrict_corner, const mpp_policy *stats_policy, int32_t *cells_dev, int max_cells,
+                                    int32_t *n_cells_dev, double *g_dev, double *stats_dev, void *scratch_dev,
+                                    size_t scratch_bytes, int n_slots, int heap_cap, unsigned long long *counters_dev,
+                                    const int32_t *order_dev, void *stream) {
+    MPP_REQUIRE(maps && map_dev && src_dev && dst_dev && cells_dev && n_cells_dev && scratch_dev,
+                "mpp_astar_batch_maps: null argument");
+    MPP_REQUIRE(!stats_policy || stats_dev, "mpp_astar_batch_maps: stats_policy without stats_dev");
+    MPP_REQUIRE(variant >= 0 && variant <= 2, "mpp_astar_batch_maps: variant must be 0 (astar.py), 1 (MPA.py) or 2 (dijkstra.py)");
+    MPP_REQUIRE(n > 0 && max_cells > 0, "mpp_astar_batch_maps: bad sizes");
+    MPP_REQUIRE(maps->rows < 32768 && maps->cols < 65536,
+                "A*: map %dx%d exceeds the packed-node limit (rows < 32768, cols < 65536)", maps->rows, maps->cols);
+    MPP_REQUIRE(n_slots > 0 && heap_cap >= 64, "A*: n_slots=%d heap_cap=%d", n_slots, heap_cap);
+    const size_t need = 256 + (size_t)n_slots * astar_slot_bytes(maps->rows * maps->cols, heap_cap);
+    MPP_REQUIRE(scratch_bytes >= need, "A*: scratch too small (%zu < %zu)", scratch_bytes, need);
+    MPP_CUDA(cudaSetDevice(maps->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    BatchMapsArgs A;
+    memset(&A, 0, sizeof(A));
+    if (stats_policy) {
+        A.X.occ = maps->occ_dev; A.X.pitch = maps->pitch_words; A.X.R = maps->rows; A.X.C = maps->cols;
+        A.X.pol = *stats_policy;
+        if (stats_policy->mode == 0 && maps->n_obstacles > 0) {  // an obstacle-free map's classes are all 0 (penalty 0.0)
+            const int rc = mpp_map_batch_safety_table(maps, stats_policy->min_safe_distance, stream);
+            if (rc) return rc;
+            A.X.cls = maps->safety_d2_dev; A.X.lut = maps->safety_lut_dev;
+        }
+        A.stats = stats_dev;
+    }
+    MPP_CUDA(cudaMemsetAsync(scratch_dev, 0, 256, s));
+    A.G.occ = maps->occ_dev; A.G.pitch = maps->pitch_words; A.G.R = maps->rows; A.G.C = maps->cols;
+    A.G.allow_diag = allow_diagonal; A.G.restrict_corner = restrict_corner;
+    A.occ_words = maps->occ_words; A.variant = variant; A.src = src_dev; A.dst = dst_dev; A.avoid = avoid_bits_dev;
+    A.n = n; A.words = (maps->rows * maps->cols + 31) / 32; A.cells = cells_dev; A.max_cells = max_cells;
+    A.n_cells = n_cells_dev; A.g = g_dev; A.scratch = (char *)scratch_dev; A.n_slots = n_slots; A.heap_cap = heap_cap;
+    A.counters = counters_dev; A.map = map_dev; A.n_maps = maps->n_maps; A.order = order_dev;
+    const int blocks = (n_slots + MPP_AS_GROUPS - 1) / MPP_AS_GROUPS;
+    mpp_astar_batch_kernel<false, BatchMapsArgs><<<blocks, MPP_AS_THREADS, 0, s>>>(A);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }

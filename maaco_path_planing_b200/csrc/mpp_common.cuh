@@ -58,6 +58,12 @@ struct mpp_map_batch {
     MppMapMeta *meta_host;  // [n_maps]
     uint8_t *grid_host;     // [n_maps][rows*cols] (host copy for host-side table builds), may be null for views
     int owns;               // 1 = buffers are freed by mpp_map_batch_destroy
+    long long n_obstacles;  // over all maps (0 = no map needs a safety table)
+    // safety-class cache of every map (helper.py:67-80, see mpp_map below); built by mpp_map_batch_safety_table
+    double safety_msd;      // msd the tables were built for (<0 = none)
+    uint16_t *safety_d2_dev; // [n_maps][rows*cols]
+    double *safety_lut_dev; // safety_lut_n doubles, shared by every map (the LUT depends on msd only)
+    int safety_lut_n;
 };
 
 struct mpp_map {
@@ -79,6 +85,12 @@ struct mpp_map {
 };
 
 int mpp_check_device(int device);
+
+// Builds the safety-class tables of n_maps maps whose occupancy is laid out [n_maps][occ_words] (mpp_astar.cu): one
+// kernel launch (grid.y = map) into *d2 ([n_maps][rows*cols] u16) and one LUT for msd into *lut, (re)allocating both
+// as needed and recording msd in *cached_msd.  Shared by mpp_map_safety_table and mpp_map_batch_safety_table.
+int mpp_build_safety(int device, const uint32_t *occ, int occ_words, int pitch_words, int rows, int cols, int n_maps,
+                     double msd, cudaStream_t s, double *cached_msd, uint16_t **d2, double **lut, int *lut_n);
 
 // ---------------------------------------------------------------------------------------------
 // Philox4x32-10 streams (RNG contract)

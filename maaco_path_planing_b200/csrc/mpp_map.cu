@@ -133,6 +133,7 @@ extern "C" int mpp_map_create(const uint8_t *grid_host, int rows, int cols, int 
     B.n_maps = 1; B.rows = rows; B.cols = cols; B.device = device; B.sm_count = m->sm_count;
     B.pitch_words = m->pitch_words; B.occ_words = m->occ_words;
     B.occ_dev = m->occ_dev; B.svalid_dev = m->svalid_dev; B.grid_host = m->grid_host; B.owns = 0;
+    B.n_obstacles = m->n_obstacles; B.safety_msd = -1.0;
     B.meta_host = (MppMapMeta *)malloc(sizeof(MppMapMeta));
     *B.meta_host = mpp_make_meta(rows, cols, m->start, m->target);
     MPP_CUDA(cudaMalloc(&B.meta_dev, sizeof(MppMapMeta)));
@@ -186,6 +187,7 @@ extern "C" int mpp_map_batch_create(const uint8_t *grids_host, int n_maps, int r
     mpp_map_batch *B = (mpp_map_batch *)calloc(1, sizeof(mpp_map_batch));
     if (!B) { mpp_set_error("out of host memory"); return MPP_ENOMEM; }
     B->n_maps = n_maps; B->rows = rows; B->cols = cols; B->device = device; B->owns = 1;
+    B->safety_msd = -1.0;
     const size_t n = (size_t)rows * cols;
     B->grid_host = (uint8_t *)malloc(n * n_maps);
     B->meta_host = (MppMapMeta *)malloc(sizeof(MppMapMeta) * n_maps);
@@ -197,6 +199,7 @@ extern "C" int mpp_map_batch_create(const uint8_t *grids_host, int n_maps, int r
         for (size_t i = 0; i < n; ++i) {
             if (g[i] == 2 && start < 0) start = (int)i;             // first row-major hit, MAACO.py:32-41
             if (g[i] == 3 && target < 0) target = (int)i;
+            if (g[i] == 1) B->n_obstacles++;
         }
         B->meta_host[k] = mpp_make_meta(rows, cols, start, target);
     }
@@ -228,6 +231,8 @@ extern "C" void mpp_map_batch_destroy(mpp_map_batch *B) {
     if (B->occ_dev) cudaFree(B->occ_dev);
     if (B->svalid_dev) cudaFree(B->svalid_dev);
     if (B->meta_dev) cudaFree(B->meta_dev);
+    if (B->safety_d2_dev) cudaFree(B->safety_d2_dev);
+    if (B->safety_lut_dev) cudaFree(B->safety_lut_dev);
     free(B->grid_host);
     free(B->meta_host);
     free(B);
