@@ -29,6 +29,12 @@ def shard_maps(n_maps, group=None):
     return min(n_maps, rank * per), min(n_maps, (rank + 1) * per)
 
 
+def default_max_cells(rows, cols):
+    """Per-ant path capacity of MAACO and MAACOBatch when `max_cells` is not given: tours are a few (rows + cols) cells
+    long (MAACO.py:278-302 never backtracks); a best path that does not fit makes the solve repeat with rows * cols."""
+    return min(rows * cols, max(1024, 8 * (rows + cols)))
+
+
 def _grids_u8(grids):
     """[n_maps, rows, cols] cell codes as uint8 (what mpp_map_batch_create takes): values clipped to 0..255 like
     np.clip(int grid), written straight into the byte array (an int64 wave of 128 256x256 maps is 67 MB: the
@@ -47,7 +53,9 @@ def _grids_u8(grids):
 
 class MAACOBatch:
     """M same-shape maps that share start and target, one colony of `num_ants` ants per map, solved together.
-    Same parameters as MAACO (MAACO.py:11-14); `seeds` = one Philox seed per map."""
+    Same parameters as MAACO (MAACO.py:11-14); `seeds` = one Philox seed per map.  `max_cells` works as in MAACO: left
+    at its default, solve() repeats the whole wave with rows*cols cells of path capacity when a best path did not fit;
+    given explicitly, such a wave raises MppError."""
 
     def __init__(self, grids, num_ants, num_iterations, alpha, beta, rho, Q, a_turn_coef, wh_max, wh_min, k_h_adaptive,
                  q0_initial, C0_initial_pheromone=0.1, *, seeds=None, device=None, max_cells=None, ants_per_warp=0,
@@ -75,13 +83,18 @@ class MAACOBatch:
         M, R, Cc, N = self.n_maps, self.rows, self.cols, self.num_ants
         n = R * Cc
         TR = (R + 31) // 32
+        self._auto_cells = max_cells is None
         if max_cells is None:
-            max_cells = min(n, max(1024, 8 * (R + Cc)))
+            max_cells = default_max_cells(R, Cc)
         self.max_cells = int(max_cells)
         self._apw = int(ants_per_warp)
         if seeds is None:
             seeds = [int.from_bytes(np.random.bytes(8), "little") for _ in range(M)]
         self.seeds = [int(s) & (2 ** 64 - 1) for s in seeds]
+        self._ctor = dict(grids=g8, num_ants=num_ants, num_iterations=num_iterations, alpha=alpha, beta=beta, rho=rho, Q=Q,
+                          a_turn_coef=a_turn_coef, wh_max=wh_max, wh_min=wh_min, k_h_adaptive=k_h_adaptive,
+                          q0_initial=q0_initial, C0_initial_pheromone=C0_initial_pheromone, seeds=self.seeds,
+                          device=self.device_index, ants_per_warp=ants_per_warp)
         dev = self.device
         f64, i32, i64, u8 = torch.float64, torch.int32, torch.int64, torch.uint8
         K = max(1, self.num_iterations)
@@ -170,7 +183,16 @@ class MAACOBatch:
             [("best_len", "<f8"), ("best_turns", "<i4"), ("best_n_cells", "<i4"), ("best_iter", "<i4"), ("best_ant", "<i4"),
              ("iter_best_len", "<f8"), ("iter_best_turns", "<i4"), ("iter_best_ant", "<i4")]))
         if (st["best_n_cells"] - 1 > self.max_cells).any():
-            raise _lib.MppError(f"a best path outgrew max_cells={self.max_cells}; re-run with a larger max_cells")
+            if not self._auto_cells or self.max_cells >= self.rows * self.cols:
+                raise _lib.MppError(f"a tour outgrew max_cells={self.max_cells} (best path: "
+                                    f"{int(st['best_n_cells'].max())} cells); re-run with a larger max_cells")
+            # the solve is a deterministic function of (grids, parameters, seeds): repeat the wave with full path capacity
+            again = type(self)(max_cells=self.rows * self.cols, **self._ctor)
+            again.kernel_launches = self.kernel_launches
+            self.close()
+            self.__dict__.update(again.__dict__)
+            again._maps = None                                                # the map handle is ours now
+            return self.solve()
         best = self._best_cells.cpu().numpy()
         log = self._log.cpu().numpy()[:, :K]
         out = []

@@ -22,6 +22,7 @@ import numpy as np
 
 from . import _lib
 from . import dist as dist_mod
+from .batch import default_max_cells
 from .dist import padded_tile_rows
 from .gridmap import GridMap, START_NODE_VAL, TARGET_NODE_VAL
 
@@ -109,7 +110,7 @@ class MAACO:
         # solve_path_planning() re-runs the (deterministic) solve with full capacity if the best path was cut
         self._auto_cells = max_cells is None
         if max_cells is None:
-            max_cells = min(n, max(1024, 8 * (R + Cc)))
+            max_cells = default_max_cells(R, Cc)
         self.max_cells = int(max_cells)
         self.max_cells_hint = self.max_cells
         dev = self.device

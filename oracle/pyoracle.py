@@ -166,9 +166,12 @@ class AStarOracle:
         self.out = np.zeros(self.R * self.C, np.int32)
 
     def __del__(self):
-        if getattr(self, "ctx", None):
-            lib().orc_astar_ctx_free(self.ctx)
-            self.ctx = None
+        ctx, self.ctx = getattr(self, "ctx", None), None
+        try:
+            if ctx and _lib is not None:
+                _lib.orc_astar_ctx_free(ctx)
+        except Exception:                             # at interpreter exit the module's globals may be gone already
+            pass
 
     def solve(self, variant, src, dst, avoid_bits=None):
         """Returns (cells int32 array, popped_g, expansions, relaxations)."""
