@@ -319,6 +319,20 @@ int mpp_waypoint_fitness(mpp_map *map, const int32_t *waypoints_dev, int n_indiv
                          int n_slots, int heap_cap, unsigned long long *counters_dev, const int32_t *order_dev,
                          void *stream);
 
+/* replaces one PSOSolver / GASolver fitness evaluation per (map, individual) of a sweep over independent maps:
+ * _reconstruct_path_from_position (pso.py:56-94) / _reconstruct_path_from_chromosome (ga_solver.py:58-93) followed by
+ * helper.calculate_path_stats (helper.py:98-113) -- mpp_waypoint_fitness over a batch of same-shape maps in one launch.
+ * Individual i runs on map map_dev[i] from that map's start, through its waypoints, to that map's target; mode 0 uses
+ * that map's safety table (mpp_map_batch_safety_table).  An individual whose map index lies outside the batch (or whose
+ * map has no start / target) gets n_cells = 0 without a search.  visited_dev: n_slots x ceil(rows*cols/32) words of
+ * scratch (one bitmap per search slot).  Scratch as mpp_astar_batch_maps; result conventions and order_dev as
+ * mpp_waypoint_fitness. */
+int mpp_waypoint_fitness_maps(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *waypoints_dev,
+                              int n_individuals, int n_waypoints, const mpp_policy *policy, int32_t *cells_dev,
+                              int max_cells, int32_t *n_cells_dev, double *stats_dev, uint32_t *visited_dev,
+                              void *scratch_dev, size_t scratch_bytes, int n_slots, int heap_cap,
+                              unsigned long long *counters_dev, const int32_t *order_dev, void *stream);
+
 /* ---- PSO / GA population updates (pso.py, ga_solver.py) ------------------------------------------- */
 
 /* replaces the velocity/position update of the particle loop (pso.py:183-206) for particles
@@ -404,6 +418,36 @@ int mpp_pso_init(const mpp_map *map, int n_attempts, int attempt_offset, int n_w
  * Stream (seed, GA_INIT, 0, attempt). */
 int mpp_ga_init(const mpp_map *map, int n_attempts, int attempt_offset, int n_waypoints, uint64_t seed, int32_t *chrom_dev,
                 void *stream);
+
+/* ---- PSO / GA over a batch of independent same-shape maps (one launch per step for every map) -------------------
+ * The same kernels as the single-map entry points above, with grid.y = map: map m's arrays are row m of
+ * [n_maps][...] buffers, and it draws from the streams of seeds_dev[m] -- exactly what a per-map solver with
+ * rng_seed = seeds[m] draws.  Replace a Python loop `for grid in grids: PSOSolver(grid, ...).solve()` /
+ * `GASolver(grid, ...).solve()`.
+ * mpp_pso_init_batch: pso.py:97-105, :50-51, :61, :69-70 -- attempts [off[m], off[m] + n_attempts) of every map with
+ *   attempt_offset_dev[m] >= 0 (a negative offset: the map is done, its rows are not written).  pos / vel: [n_maps]
+ *   [n_attempts][W][2], waypoint cells [n_maps][n_attempts][W].
+ * mpp_ga_init_batch: ga_solver.py:48-56, :95-104 -- the same for chromosomes [n_maps][n_attempts][W].
+ * mpp_pso_update_batch: pso.py:183-206 -- particles [start_dev[m], n_particles) of map m (start = n_particles: the map
+ *   is idle; the particles below start are not touched).  pos / vel / pbest: [n_maps][n_particles][W][2], gbest
+ *   [n_maps][W][2], waypoint cells [n_maps][n_particles][W].
+ * mpp_ga_select_batch: ga_solver.py:136-142 over fitness [n_maps][n] -> parents [n_maps][n].
+ * mpp_ga_breed_batch: ga_solver.py:144-160, :186-194 over chromosomes / children [n_maps][n][W]; mutated genes are
+ *   free cells of the map's own grid. */
+int mpp_pso_init_batch(const mpp_map_batch *maps, int n_attempts, const int32_t *attempt_offset_dev, int n_waypoints,
+                       double max_vel, const uint64_t *seeds_dev, double *pos_dev, double *vel_dev,
+                       int32_t *waypoint_cells_dev, void *stream);
+int mpp_ga_init_batch(const mpp_map_batch *maps, int n_attempts, const int32_t *attempt_offset_dev, int n_waypoints,
+                      const uint64_t *seeds_dev, int32_t *chrom_dev, void *stream);
+int mpp_pso_update_batch(const mpp_map_batch *maps, double *pos_dev, double *vel_dev, const double *pbest_pos_dev,
+                         const double *gbest_pos_dev, int n_particles, const int32_t *start_dev, int n_waypoints,
+                         double w, double c1, double c2, double max_vel, const uint64_t *seeds_dev, int iteration,
+                         int32_t *waypoint_cells_dev, void *stream);
+int mpp_ga_select_batch(const mpp_map_batch *maps, const double *fitness_dev, int n, int tournament_size,
+                        const uint64_t *seeds_dev, int generation, int32_t *parents_dev, void *stream);
+int mpp_ga_breed_batch(const mpp_map_batch *maps, const int32_t *chrom_dev, const int32_t *parents_dev, int n,
+                       int n_waypoints, double crossover_rate, double mutation_rate, const uint64_t *seeds_dev,
+                       int generation, int32_t *children_dev, void *stream);
 
 #ifdef __cplusplus
 }

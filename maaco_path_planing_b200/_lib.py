@@ -114,6 +114,17 @@ _SIGS = {
                                         c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "mpp_pso_init": (c_int, [c_void_p, c_int, c_int, c_int, c_double, c_u64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "mpp_ga_init": (c_int, [c_void_p, c_int, c_int, c_int, c_u64, c_void_p, c_void_p]),
+    "mpp_waypoint_fitness_maps": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, C.POINTER(Policy), c_void_p, c_int,
+                                          c_void_p, c_void_p, c_void_p, c_void_p, C.c_size_t, c_int, c_int, c_void_p,
+                                          c_void_p, c_void_p]),
+    "mpp_pso_init_batch": (c_int, [c_void_p, c_int, c_void_p, c_int, c_double, c_void_p, c_void_p, c_void_p, c_void_p,
+                                   c_void_p]),
+    "mpp_ga_init_batch": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
+    "mpp_pso_update_batch": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_double,
+                                     c_double, c_double, c_double, c_void_p, c_int, c_void_p, c_void_p]),
+    "mpp_ga_select_batch": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p]),
+    "mpp_ga_breed_batch": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_double, c_double, c_void_p, c_int,
+                                   c_void_p, c_void_p]),
     "mpp_mpa_iteration": (c_int, [c_void_p, C.POINTER(Policy), c_int, c_int, c_int, c_int, c_int, c_double, c_double, c_double,
                                   c_double, c_double, c_u64, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p,
                                   c_void_p, c_void_p, c_void_p, c_void_p, C.c_size_t, c_int, c_int, c_void_p, c_void_p,

@@ -443,10 +443,19 @@ def _search_algorithm(algorithm):
     return _SEARCH_ALGORITHMS[algorithm]
 
 
+# planner -> the reference constructor's errors for a map without start / target
+_ENDPOINT_ERRORS = {name: msgs for name, (_, *msgs) in _SEARCH_ALGORITHMS.items()}
+_ENDPOINT_ERRORS.update(pso=("PSO: Start node not found.", "PSO: Target node not found."),              # pso.py:19-20
+                        ga=("GA: Start node not found.", "GA: Target node not found."))                 # ga_solver.py:19-20
+
+
 def _check_endpoints(flat, algorithm):
     """Raises the reference constructor's ValueError for the first map (a row of `flat`, cell codes) that has no start
-    or no target -- what a loop of AStarSolver / DijkstraSolver constructors over the maps would raise."""
-    _, no_start, no_target = _search_algorithm(algorithm)
+    or no target -- what a loop of AStarSolver / DijkstraSolver / PSOSolver / GASolver constructors over the maps would
+    raise."""
+    if algorithm not in _ENDPOINT_ERRORS:
+        _search_algorithm(algorithm)
+    no_start, no_target = _ENDPOINT_ERRORS[algorithm]
     flat = np.asarray(flat)
     has_s = (flat == START_NODE_VAL).any(axis=1)
     has_t = (flat == TARGET_NODE_VAL).any(axis=1)
@@ -511,7 +520,10 @@ class SearchBatch:
         self.n_slots = int(n_slots or self.max_slots)
         self.counters = torch.zeros(4, dtype=torch.int64, device=self.device)  # expansions, relaxations, ring / heap pushes
         self.launches = 0
-        self._scratch, self._scratch_key = None, None
+        self._scratch, self._scratch_key, self._visited = None, None, None
+        flat = self._grids8.reshape(self.n_maps, -1)                       # first row-major 2 / 3, -1 = none
+        ends = [np.where((flat == v).any(axis=1), (flat == v).argmax(axis=1), -1) for v in (START_NODE_VAL, TARGET_NODE_VAL)]
+        self._start_dev, self._target_dev = (torch.as_tensor(e.astype(np.int32), device=self.device) for e in ends)
 
     def close(self):
         h, self._maps = getattr(self, "_maps", None), None
@@ -533,15 +545,21 @@ class SearchBatch:
             return a.to(device=self.device, dtype=torch.int32).contiguous()
         return torch.as_tensor(np.ascontiguousarray(a, dtype=np.int32), device=self.device)
 
-    def _launch(self, variant, mi, src, dst, avoid, longest_first):
-        """One mpp_astar_batch_maps launch over the given (valid) queries with the current sizes."""
+    def _scratch_for(self, n):
+        """(scratch, search slots) for a launch over n queries / individuals with the current heap_cap."""
         import torch as t
-        n, mc = mi.numel(), self.max_cells
         slots = max(1, min(self.n_slots, n))
         if self._scratch_key != (slots, self.heap_cap):                   # zero-filled once: search stamps live in it
             nbytes = 256 + slots * _lib.lib().mpp_astar_slot_bytes(self.rows, self.cols, self.heap_cap)
             self._scratch = t.zeros(nbytes, dtype=t.uint8, device=self.device)
             self._scratch_key = (slots, self.heap_cap)
+        return self._scratch, slots
+
+    def _launch(self, variant, mi, src, dst, avoid, longest_first):
+        """One mpp_astar_batch_maps launch over the given (valid) queries with the current sizes."""
+        import torch as t
+        n, mc = mi.numel(), self.max_cells
+        _, slots = self._scratch_for(n)
         order = None
         if longest_first and n > slots:
             # a search costs roughly the square of its endpoint distance; the launch ends with its slowest query
@@ -560,6 +578,64 @@ class SearchBatch:
             self.heap_cap, _lib.ptr(self.counters), _lib.ptr(order), stream), "mpp_astar_batch_maps")
         self.launches += 1
         return cells, ncell, g, stats
+
+    def _chain_launch(self, mi, wps):
+        """One mpp_waypoint_fitness_maps launch over individuals mi [n] (map index, -1 = not searched), wps [n, W] with the
+        current sizes, longest chains first."""
+        import torch as t
+        n, W = wps.shape
+        mc = self.max_cells
+        scratch, slots = self._scratch_for(n)
+        if self._visited is None or self._visited.shape[0] < slots:
+            self._visited = t.empty((slots, self.words), dtype=t.int32, device=self.device)
+        order = None
+        if n > slots // 2:
+            # a chain costs roughly the sum of its squared hop lengths; the launch ends with its slowest individual
+            ok = (mi >= 0) & (mi < self.n_maps)
+            m = mi.clamp(0, self.n_maps - 1).long()
+            chain = t.cat([self._start_dev[m][:, None], wps, self._target_dev[m][:, None]], dim=1).to(t.float64)
+            r, c = t.div(chain, self.cols, rounding_mode="floor"), chain % self.cols
+            d = ((r[:, 1:] - r[:, :-1]) ** 2 + (c[:, 1:] - c[:, :-1]) ** 2).sqrt().sum(dim=1)
+            order = t.argsort(t.where(ok, d, -1.0), descending=True).to(t.int32).contiguous()
+        cells = t.empty((n, mc), dtype=t.int32, device=self.device)
+        ncell = t.empty(n, dtype=t.int32, device=self.device)
+        stats = t.empty((n, 5), dtype=t.float64, device=self.device)
+        stream = C.c_void_p(t.cuda.current_stream(self.device).cuda_stream)
+        _lib.check(_lib.lib().mpp_waypoint_fitness_maps(
+            self._maps, _lib.ptr(mi), _lib.ptr(wps), n, W, C.byref(self.policy), _lib.ptr(cells), mc, _lib.ptr(ncell),
+            _lib.ptr(stats), _lib.ptr(self._visited), _lib.ptr(scratch), scratch.numel(), slots, self.heap_cap,
+            _lib.ptr(self.counters), _lib.ptr(order), stream), "mpp_waypoint_fitness_maps")
+        self.launches += 1
+        return cells, ncell, stats
+
+    def _chain_repeat(self, mi, wps, cells, ncell, stats):
+        """After _grow_from enlarged the buffers: repeats the individuals whose heap overflowed or whose path was truncated
+        (the searches are deterministic) until none is; returns the patched (cells, n_cells, stats)."""
+        import torch as t
+        from .engine import SearchEngine
+        while True:
+            bad = ((ncell < 0) | (ncell > cells.shape[1])).nonzero().squeeze(1)
+            c, nc, st = self._chain_launch(mi.index_select(0, bad).contiguous(), wps.index_select(0, bad).contiguous())
+            if c.shape[1] > cells.shape[1]:                                  # max_cells grew: widen the earlier rows
+                cells = t.nn.functional.pad(cells, (0, c.shape[1] - cells.shape[1]))
+            cells[bad, :c.shape[1]] = c
+            ncell[bad], stats[bad] = nc, st
+            if not SearchEngine._grow_from(self, *t.stack([nc.min(), nc.max()]).tolist()):
+                return cells, ncell, stats
+
+    def chains(self, map_index, waypoints):
+        """Waypoint-chain fitness (pso.py:56-94 / ga_solver.py:58-93 + helper.py:98-113): individual i runs on map
+        map_index[i] from that map's start through the W cells waypoints[i] to its target.  Returns device tensors
+        (cells [n, max_cells] int32, n_cells [n] int32, stats [n, 5] float64).  n_cells = 0: an invalid chain, or a map
+        index outside the batch (not searched).  A heap overflow or a truncated path grows the buffers and repeats only
+        those individuals."""
+        from .engine import SearchEngine
+        import torch as t
+        mi, wps = self._i32(map_index), self._i32(waypoints)
+        cells, ncell, stats = self._chain_launch(mi, wps)
+        if SearchEngine._grow_from(self, *t.stack([ncell.min(), ncell.max()]).tolist()):
+            cells, ncell, stats = self._chain_repeat(mi, wps, cells, ncell, stats)
+        return cells, ncell, stats
 
     def search(self, variant, map_index, src, dst, avoid_bits=None, *, longest_first=True):
         """Query i: connector `variant` (0 = astar.py, 1 = MPA.py's private A*, 2 = dijkstra.py) from cell src[i] to
@@ -644,3 +720,405 @@ def solve_search_batch(grids, algorithm, params, wave=None, group=None, device=N
         b.close()
     out.sort(key=lambda r: r[0])
     return out
+
+
+# ---- PSO / GA over a batch of maps (pso.py, ga_solver.py) -------------------------------------------------------------
+def default_pop_wave(rows, cols, population):
+    """Maps per wave of solve_pso_batch / solve_ga_batch: one [maps, population, max_cells] int32 array of paths (the
+    population's evaluation; GA keeps a second one, the sorted population) stays near 1 GiB.  At 256x256 max_cells is
+    8192 (32 KB per individual): 32 maps of 1024 individuals."""
+    n = rows * cols
+    max_cells = min(n, max(4096, 16 * (rows + cols)))                      # SearchBatch's default
+    return max(1, (1 << 30) // (population * max_cells * 4))
+
+
+class _WaypointBatch:
+    """What PSOBatch and GABatch share: M same-shape maps (start and target may differ from map to map) behind one
+    SearchBatch (map batch, policy, buffer sizes and their growth), one Philox seed per map, and the population
+    initialisation of pso.py:97-161 / ga_solver.py:95-133 for every map at once."""
+    _planner = None        # "pso" / "ga"
+    _pad_class = None      # RNG class of the padding draws
+
+    def __init__(self, grids, num_waypoints, policy, seeds, device, max_cells, heap_cap, n_slots):
+        import torch
+        g8 = _grids_u8(grids)
+        self.n_maps, self.rows, self.cols = g8.shape
+        _check_endpoints(g8.reshape(self.n_maps, -1), self._planner)
+        if seeds is None:
+            seeds = [int.from_bytes(np.random.bytes(8), "little") for _ in range(self.n_maps)]
+        if len(seeds) != self.n_maps:
+            raise ValueError(f"seeds holds {len(seeds)} values for {self.n_maps} maps")
+        self.seeds = [int(s) & (2 ** 64 - 1) for s in seeds]
+        self.num_waypoints = int(num_waypoints)
+        self._search = SearchBatch(g8, device=device, max_cells=max_cells, heap_cap=heap_cap, n_slots=n_slots, **policy)
+        self.device = self._search.device
+        self._seeds = torch.from_numpy(np.array(self.seeds, np.uint64).view(np.int64)).to(self.device)
+        self.fitness_evaluations = [0] * self.n_maps
+        self.init_attempts = [0] * self.n_maps
+        self.kernel_launches = 0
+
+    def close(self):
+        self._search.close()
+
+    @property
+    def launches(self):
+        """Kernel launches so far: population kernels and fitness / connector searches."""
+        return self.kernel_launches + self._search.launches
+
+    def _stream(self):
+        import torch
+        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _solve_direct(self):
+        """num_waypoints == 0 (pso.py:165-170, ga_solver.py:163-168): one start -> target connector per map and the
+        statistics of its path; the curve holds that fitness."""
+        return [r[:6] + ([r[5]],) for r in self._search.solve("astar")]
+
+    def _initialize(self, generate, n):
+        """pso.py:97-161 / ga_solver.py:95-133 for every map.  Each round generates one block of attempts for every map
+        that still needs individuals -- generate(offsets [M] device int32, B) enqueues attempts [offsets[m],
+        offsets[m] + B) of every map with offsets[m] >= 0 and returns (tensors [M, B, ...] an individual keeps,
+        waypoint cells [M, B, W]) -- and evaluates them in one launch; each map accepts valid attempts in attempt
+        order until it has n or has used 20 n.  A map without any valid chain gets its direct start -> target path
+        (pso.py:128-145, ga_solver.py:111-117).  Returns (n_acc [M] before padding, direct [M] bool, kept [M, n, ...]
+        tensors, stats [M, n, 5], cells [M, n, mc], n_cells [M, n]) with every map's rows padded to n (pso.py:159-160,
+        ga_solver.py:129-130)."""
+        import torch as t
+        from . import rng
+        M, W, dev = self.n_maps, self.num_waypoints, self.device
+        max_total = 20 * n
+        n_acc, attempts = np.zeros(M, np.int64), np.zeros(M, np.int64)
+        kept = stats = cells = ncell = None
+        rows = t.arange(M, device=dev)
+        while True:
+            need = (n_acc < n) & (attempts < max_total)
+            if not need.any():
+                break
+            block = np.where(need, np.minimum(max_total - attempts, np.maximum(32, (1.25 * (n - n_acc)).astype(np.int64) + 8)),
+                             0)
+            B = int(block.max())
+            offs = t.as_tensor(np.where(need, attempts, -1).astype(np.int32), device=dev)
+            k_r, wp = generate(offs, B)
+            self.kernel_launches += 1
+            mi = t.where(t.arange(B, device=dev)[None, :] < t.as_tensor(block, device=dev)[:, None], rows[:, None], -1)
+            c_r, nc_r, st_r = self._search.chains(mi.reshape(-1), wp.reshape(M * B, W))
+            valid = (nc_r > 0).reshape(M, B).cpu().numpy()
+            src, dst = [], []
+            for m in np.flatnonzero(need):
+                take = np.flatnonzero(valid[m, :block[m]])
+                room = n - n_acc[m]
+                if take.size >= room:
+                    take = take[:room]
+                    attempts[m] += int(take[-1]) + 1                         # the loop stops right after the n-th accept
+                else:
+                    attempts[m] += block[m]
+                self.fitness_evaluations[m] += int(block[m])
+                src.append(m * B + take)
+                dst.append(m * n + n_acc[m] + np.arange(take.size))
+                n_acc[m] += take.size
+            if kept is None:
+                kept = [t.zeros((M * n,) + x.shape[2:], dtype=x.dtype, device=dev) for x in k_r]
+                stats = t.zeros((M * n, 5), dtype=t.float64, device=dev)
+                cells = t.zeros((M * n, c_r.shape[1]), dtype=t.int32, device=dev)
+                ncell = t.zeros(M * n, dtype=t.int32, device=dev)
+            if c_r.shape[1] > cells.shape[1]:
+                cells = t.nn.functional.pad(cells, (0, c_r.shape[1] - cells.shape[1]))
+            si = t.as_tensor(np.concatenate(src), device=dev)
+            di = t.as_tensor(np.concatenate(dst), device=dev)
+            for buf, x in zip(kept, k_r):
+                buf[di] = x.reshape((M * B,) + x.shape[2:])[si]
+            stats[di], ncell[di] = st_r[si], nc_r[si]
+            cells[di, :c_r.shape[1]] = c_r[si]
+        self.init_attempts = attempts.tolist()
+        direct = np.zeros(M, bool)
+        lost = np.flatnonzero(n_acc == 0)
+        if lost.size:                                                        # the direct path as the one individual
+            s, g = self._search._start_dev[lost], self._search._target_dev[lost]
+            c_d, nc_d, _, st_d = self._search.search(0, lost, s, g)
+            found = (nc_d > 0).cpu().numpy()
+            if found.any():
+                if c_d.shape[1] > cells.shape[1]:
+                    cells = t.nn.functional.pad(cells, (0, c_d.shape[1] - cells.shape[1]))
+                fi = t.as_tensor(np.flatnonzero(found), device=dev)
+                di = t.as_tensor(lost[found] * n, device=dev)
+                stats[di], ncell[di] = st_d[fi], nc_d[fi]
+                cells[di, :c_d.shape[1]] = c_d[fi, :cells.shape[1]]
+                for buf in kept:
+                    buf[di] = 0                                              # position = velocity = [[0.0, 0.0]] * W
+                direct[lost[found]] = True
+        # padding: random.choice(population).copy() with draws from (seed, PAD, 0, len(population))
+        have = np.where(direct, 1, n_acc)
+        idx = np.tile(np.arange(n), (M, 1))
+        for m in np.flatnonzero((have > 0) & (have < n)):
+            k0 = int(have[m])
+            u = rng.stream_block(self.seeds[m], self._pad_class, 0, np.arange(k0, n), 1)[:, 0]
+            for j, k in enumerate(range(k0, n)):
+                idx[m, k] = idx[m, min(int(u[j] * k), k - 1)]
+        flat = t.as_tensor((idx + np.arange(M)[:, None] * n).reshape(-1), device=dev)
+        view = lambda x: x[flat].reshape((M, n) + x.shape[1:])
+        return n_acc, direct, [view(b) for b in kept], view(stats), view(cells), view(ncell)
+
+    def _result(self, n, cells, stats, curve):
+        """One map's (path, length, turns, safety_p, diag_p, fitness, convergence_curve) from its best individual."""
+        r, c = np.divmod(cells[:n], self.cols)
+        return (list(zip(r.tolist(), c.tolist())), float(stats[0]), int(stats[1]), float(stats[2]), float(stats[3]),
+                float(stats[4]), curve)
+
+
+_FAILED = ([], INF, 0, 0.0, 0.0, INF, [])                                    # pso.py:147-157 / ga_solver.py:120-126
+
+
+class PSOBatch(_WaypointBatch):
+    """M same-shape maps, one PSO swarm per map, solved together: PSOSolver (pso.py:8-240) for every map with the same
+    arguments and defaults, `grids` [M, rows, cols] in place of `grid` and `seeds` = one Philox seed per map (row m
+    draws what PSOSolver(grid, ..., rng_seed=seeds[m]) draws).  Start and target may differ from map to map.  An
+    iteration is the speculative repair of PSOSolver._iterate for all maps at once: every map's active suffix is
+    updated and evaluated in one update launch and one fitness launch (mpp_pso_update_batch, mpp_waypoint_fitness_maps),
+    each map's first global-best improver is found on the device, and only the rest of that map's swarm is restored
+    and re-run in the next round; one host synchronise per round."""
+    _planner = "pso"
+
+    def __init__(self, grids, num_iterations, num_particles, num_waypoints_per_particle, w, c1, c2,
+                 turn_penalty_factor=0.1, safety_penalty_factor=0.05, min_safe_distance=1.5, allow_diagonal_moves=True,
+                 restrict_diagonal_near_obstacle_policy=True, diagonal_obstacle_penalty_value=1000.0, *, seeds=None,
+                 device=None, max_cells=None, heap_cap=None, n_slots=None):
+        from . import rng
+        self._pad_class = rng.CLS_PSO_PAD
+        policy = dict(turn_penalty_factor=turn_penalty_factor, safety_penalty_factor=safety_penalty_factor,
+                      min_safe_distance=min_safe_distance, allow_diagonal_moves=allow_diagonal_moves,
+                      restrict_diagonal_near_obstacle_policy=restrict_diagonal_near_obstacle_policy,
+                      diagonal_obstacle_penalty_value=diagonal_obstacle_penalty_value)
+        super().__init__(grids, num_waypoints_per_particle, policy, seeds, device, max_cells, heap_cap, n_slots)
+        self.num_iterations, self.num_particles = int(num_iterations), int(num_particles)
+        self.w, self.c1, self.c2 = w, c1, c2
+        self.max_vel = max(1.0, 0.15 * max(self.rows, self.cols))            # pso.py:34
+        self.pos = self.vel = self.pbest_fit = None
+
+    def _generate(self, offs, B):
+        import torch as t
+        M, W = self.n_maps, self.num_waypoints
+        pos = t.empty((M, B, W, 2), dtype=t.float64, device=self.device)
+        vel = t.empty((M, B, W, 2), dtype=t.float64, device=self.device)
+        wp = t.empty((M, B, W), dtype=t.int32, device=self.device)
+        _lib.check(_lib.lib().mpp_pso_init_batch(self._search._maps, B, _lib.ptr(offs), W, self.max_vel, _lib.ptr(self._seeds),
+                                                 _lib.ptr(pos), _lib.ptr(vel), _lib.ptr(wp), self._stream()),
+                   "mpp_pso_init_batch")
+        return (pos, vel), wp
+
+    def solve(self):
+        """Returns, per map, what PSOSolver(grid, ..., rng_seed=seeds[m]).solve() returns followed by that solver's
+        convergence_curve.  After it, pos / vel / pbest_fit hold every swarm's final state ([M, N, W, 2], [M, N])."""
+        import torch as t
+        if self.num_waypoints == 0:
+            return self._solve_direct()
+        M, N, W, K, dev = self.n_maps, self.num_particles, self.num_waypoints, self.num_iterations, self.device
+        n_acc, direct, (pos, vel), stats, cells, ncell = self._initialize(self._generate, N)
+        live = t.as_tensor((n_acc > 0) | direct, device=dev)
+        fit = stats[..., 4]
+        rows, ar = t.arange(M, device=dev), t.arange(N, device=dev)
+        gi = (fit == fit.min(dim=1, keepdim=True).values).int().argmax(dim=1)   # first strictly-best, pso.py:121
+        g_pos, g_stats, g_cells, g_n = pos[rows, gi], stats[rows, gi], cells[rows, gi], ncell[rows, gi]
+        pbest_pos, pbest_fit = pos.clone(), fit.clone()
+        curve = t.empty((K + 1, M), dtype=t.float64, device=dev)
+        curve[0] = g_stats[:, 4]
+        L = _lib.lib()
+        idle = np.where(live.cpu().numpy(), 0, N)
+        for it in range(K):
+            pos0, vel0 = pos.clone(), vel.clone()
+            start = idle.copy()
+            while (start < N).any():
+                st_d = t.as_tensor(start.astype(np.int32), device=dev)
+                wp = t.empty((M, N, W), dtype=t.int32, device=dev)
+                _lib.check(L.mpp_pso_update_batch(self._search._maps, _lib.ptr(pos), _lib.ptr(vel), _lib.ptr(pbest_pos),
+                                                  _lib.ptr(g_pos), N, _lib.ptr(st_d), W, self.w, self.c1, self.c2,
+                                                  self.max_vel, _lib.ptr(self._seeds), it, _lib.ptr(wp), self._stream()),
+                           "mpp_pso_update_batch")
+                self.kernel_launches += 1
+                act = ar[None, :] >= st_d[:, None]
+                mi = t.where(act, rows[:, None], -1).to(t.int32).reshape(-1)
+                wp = wp.reshape(M * N, W)
+                c_r, nc_r, s_r = self._search._chain_launch(mi, wp)
+                for m in np.flatnonzero(start < N):
+                    self.fitness_evaluations[m] += N - int(start[m])
+                while True:
+                    nc = nc_r.reshape(M, N)
+                    f = s_r[:, 4].reshape(M, N)
+                    imp_p = act & (nc > 0) & (f < pbest_fit)                  # pso.py:216
+                    imp_g = imp_p & (f < g_stats[:, 4:5])                     # pso.py:222
+                    hit = imp_g.any(dim=1)
+                    q = t.where(hit, imp_g.int().argmax(dim=1), N - 1)       # the last particle final this round
+                    nxt = t.where(hit, q + 1, N)
+                    # the round's one host synchronise: buffer growth flags and the next round's start of every map
+                    flags = t.cat([t.stack([nc_r.min(), nc_r.max()]).to(t.int64), nxt.to(t.int64)]).tolist()
+                    from .engine import SearchEngine
+                    if not SearchEngine._grow_from(self._search, flags[0], flags[1]):
+                        break
+                    c_r, nc_r, s_r = self._search._chain_repeat(mi, wp, c_r, nc_r, s_r)
+                upd = imp_p & (ar[None, :] <= q[:, None])                     # pso.py:217-220 for the final particles
+                pbest_fit = t.where(upd, f, pbest_fit)
+                pbest_pos = t.where(upd[..., None, None], pos, pbest_pos)
+                if c_r.shape[1] > g_cells.shape[1]:
+                    g_cells = t.nn.functional.pad(g_cells, (0, c_r.shape[1] - g_cells.shape[1]))
+                fq = rows * N + q                                             # pso.py:223-229
+                g_pos = t.where(hit[:, None, None], pos[rows, q], g_pos)
+                g_stats = t.where(hit[:, None], s_r[fq], g_stats)
+                g_cells[hit, :c_r.shape[1]] = c_r[fq][hit]
+                g_n = t.where(hit, nc_r[fq], g_n)
+                rest = (ar[None, :] > q[:, None]) & hit[:, None]             # speculated with the old gbest: re-run
+                pos = t.where(rest[..., None, None], pos0, pos).contiguous()
+                vel = t.where(rest[..., None, None], vel0, vel).contiguous()
+                pbest_pos = pbest_pos.contiguous()
+                start = np.array(flags[2:], np.int64)
+            curve[it + 1] = g_stats[:, 4]
+        self.pos, self.vel, self.pbest_fit = pos, vel, pbest_fit
+        g_stats, g_cells, g_n, curve = g_stats.cpu().numpy(), g_cells.cpu().numpy(), g_n.cpu().numpy(), curve.cpu().numpy()
+        return [self._result(int(g_n[m]), g_cells[m], g_stats[m], [float(v) for v in curve[:, m]]) if idle[m] == 0
+                else _FAILED[:6] + ([],) for m in range(M)]
+
+
+class GABatch(_WaypointBatch):
+    """M same-shape maps, one GA population per map, solved together: GASolver (ga_solver.py:8-223) for every map with
+    the same arguments and defaults, `grids` [M, rows, cols] in place of `grid` and `seeds` = one Philox seed per map
+    (row m draws what GASolver(grid, ..., rng_seed=seeds[m]) draws).  Start and target may differ from map to map.  A
+    generation is one selection, one breeding and one fitness launch for every map (mpp_ga_select_batch,
+    mpp_ga_breed_batch, mpp_waypoint_fitness_maps); the invalid-child replacement (:204-205), the stable sort
+    (:208-209) and the best-so-far update (:211-213) are torch operations over all maps."""
+    _planner = "ga"
+
+    def __init__(self, grids, num_generations, population_size, num_waypoints_per_chromosome, mutation_rate,
+                 crossover_rate, tournament_size=3, turn_penalty_factor=0.1, safety_penalty_factor=0.05,
+                 min_safe_distance=1.5, allow_diagonal_moves=True, restrict_diagonal_near_obstacle_policy=True,
+                 diagonal_obstacle_penalty_value=1000.0, *, seeds=None, device=None, max_cells=None, heap_cap=None,
+                 n_slots=None):
+        from . import rng
+        self._pad_class = rng.CLS_GA_PAD
+        policy = dict(turn_penalty_factor=turn_penalty_factor, safety_penalty_factor=safety_penalty_factor,
+                      min_safe_distance=min_safe_distance, allow_diagonal_moves=allow_diagonal_moves,
+                      restrict_diagonal_near_obstacle_policy=restrict_diagonal_near_obstacle_policy,
+                      diagonal_obstacle_penalty_value=diagonal_obstacle_penalty_value)
+        super().__init__(grids, num_waypoints_per_chromosome, policy, seeds, device, max_cells, heap_cap, n_slots)
+        self.num_generations, self.population_size = int(num_generations), int(population_size)
+        self.mutation_rate, self.crossover_rate, self.tournament_size = mutation_rate, crossover_rate, tournament_size
+        self.chrom = self.fitness = None
+
+    def _generate(self, offs, B):
+        import torch as t
+        chrom = t.empty((self.n_maps, B, self.num_waypoints), dtype=t.int32, device=self.device)
+        _lib.check(_lib.lib().mpp_ga_init_batch(self._search._maps, B, _lib.ptr(offs), self.num_waypoints,
+                                                _lib.ptr(self._seeds), _lib.ptr(chrom), self._stream()), "mpp_ga_init_batch")
+        return (chrom,), chrom
+
+    def solve(self):
+        """Returns, per map, what GASolver(grid, ..., rng_seed=seeds[m]).solve() returns followed by that solver's
+        convergence_curve.  After it, chrom / fitness hold every map's final population in sorted order ([M, N, W],
+        [M, N]; meaningful for maps whose initialisation found a valid chain)."""
+        import torch as t
+        from .engine import SearchEngine
+        if self.num_waypoints == 0:
+            return self._solve_direct()
+        M, N, W, K, dev = self.n_maps, self.population_size, self.num_waypoints, self.num_generations, self.device
+        n_acc, direct, (chrom,), stats, cells, ncell = self._initialize(self._generate, N)
+        evolving = n_acc > 0                       # a direct-path population is a fixed point (ga_solver.py:144-160)
+        live = t.as_tensor(evolving, device=dev)
+        rows = t.arange(M, device=dev)
+
+        def sort(chrom, stats, cells, ncell):                                 # list.sort is stable (:132, :208-209)
+            o = t.sort(stats[..., 4], dim=1, stable=True).indices
+            return chrom[rows[:, None], o], stats[rows[:, None], o], cells[rows[:, None], o], ncell[rows[:, None], o]
+
+        chrom, stats, cells, ncell = sort(chrom, stats, cells, ncell)
+        b_stats, b_cells, b_n = stats[:, 0].clone(), cells[:, 0].clone(), ncell[:, 0].clone()
+        curve = t.empty((K + 1, M), dtype=t.float64, device=dev)
+        curve[0] = b_stats[:, 4]
+        L = _lib.lib()
+        mi = t.where(live[:, None], rows[:, None], -1).expand(M, N).to(t.int32).reshape(-1).contiguous()
+        for gen in range(K if evolving.any() else 0):
+            parents = t.empty((M, N), dtype=t.int32, device=dev)
+            fit = stats[..., 4].contiguous()
+            _lib.check(L.mpp_ga_select_batch(self._search._maps, _lib.ptr(fit), N, self.tournament_size,
+                                             _lib.ptr(self._seeds), gen, _lib.ptr(parents), self._stream()),
+                       "mpp_ga_select_batch")
+            children = t.empty((M, N, W), dtype=t.int32, device=dev)
+            _lib.check(L.mpp_ga_breed_batch(self._search._maps, _lib.ptr(chrom.contiguous()), _lib.ptr(parents), N, W,
+                                            self.crossover_rate, self.mutation_rate, _lib.ptr(self._seeds), gen,
+                                            _lib.ptr(children), self._stream()), "mpp_ga_breed_batch")
+            self.kernel_launches += 2
+            c_c, c_n, c_s = self._search.chains(mi, children.reshape(M * N, W))
+            for m in np.flatnonzero(evolving):
+                self.fitness_evaluations[m] += N
+            # an invalid child is replaced by its parent object (:204-205): child slot s of a map has parent parents[s]
+            if c_c.shape[1] > cells.shape[2]:
+                cells = t.nn.functional.pad(cells, (0, c_c.shape[1] - cells.shape[2]))
+                b_cells = t.nn.functional.pad(b_cells, (0, c_c.shape[1] - b_cells.shape[1]))
+            pi = (rows[:, None] * N + parents.long()).reshape(-1)
+            bad = (c_n <= 0).nonzero().squeeze(1)
+            src = pi[bad]
+            children = children.reshape(M * N, W)
+            children[bad] = chrom.reshape(M * N, W)[src]
+            c_s[bad] = stats.reshape(M * N, 5)[src]
+            c_c[bad] = cells.reshape(M * N, -1)[src]
+            c_n[bad] = ncell.reshape(M * N)[src]
+            chrom, stats, cells, ncell = sort(children.reshape(M, N, W), c_s.reshape(M, N, 5), c_c.reshape(M, N, -1),
+                                              c_n.reshape(M, N))
+            better = live & (stats[:, 0, 4] < b_stats[:, 4])                 # :211-213
+            b_stats = t.where(better[:, None], stats[:, 0], b_stats)
+            b_cells = t.where(better[:, None], cells[:, 0], b_cells)
+            b_n = t.where(better, ncell[:, 0], b_n)
+            curve[gen + 1] = b_stats[:, 4]
+        self.chrom, self.fitness = chrom, stats[..., 4]
+        b_stats, b_cells, b_n = b_stats.cpu().numpy(), b_cells.cpu().numpy(), b_n.cpu().numpy()
+        curve = curve.cpu().numpy()
+        out = []
+        for m in range(M):
+            if evolving[m]:
+                out.append(self._result(int(b_n[m]), b_cells[m], b_stats[m], [float(v) for v in curve[:, m]]))
+            elif direct[m]:                      # every generation reproduces the direct-path individual (:111-117)
+                r = self._result(int(b_n[m]), b_cells[m], b_stats[m], None)
+                out.append(r[:6] + ([r[5]] * (K + 1),))
+            else:
+                out.append(_FAILED[:6] + ([],))
+        return out
+
+
+def _pop_waves(grids, lo, hi, population, wave=None):
+    """Maps lo..hi-1 grouped by shape, `wave` maps per wave at most (None: default_pop_wave of the shape)."""
+    out = []
+    for idx in _shape_waves(grids, lo, hi):
+        step = wave or default_pop_wave(*np.asarray(grids[idx[0]]).shape, population)
+        out += [idx[w0:w0 + step] for w0 in range(0, len(idx), step)]
+    return out
+
+
+def _pop_sweep(cls, grids, sizes, params, seeds, wave, group, device):
+    lo, hi = shard_maps(len(grids), group)
+    for i in range(lo, hi):                                                  # before any device work
+        _check_endpoints(np.asarray(grids[i]).reshape(1, -1), cls._planner)
+    out = []
+    for idx in _pop_waves(grids, lo, hi, sizes[1], wave):
+        b = cls(np.stack([np.asarray(grids[i]) for i in idx]), *sizes,
+                seeds=None if seeds is None else [seeds[i] for i in idx], device=device, **params)
+        for i, r in zip(idx, b.solve()):
+            out.append((i,) + tuple(r))
+        b.close()
+    out.sort(key=lambda r: r[0])
+    return out
+
+
+def solve_pso_batch(grids, num_iterations, num_particles, num_waypoints_per_particle, params, seeds=None, wave=None,
+                    group=None, device=None):
+    """PSO on every grid of `grids` (this rank's shard when `group` is given), grouped by shape, `wave` maps per
+    PSOBatch (None: default_pop_wave, about 1 GiB of population paths per wave -- 32 maps of 1024 particles at
+    256x256).  `params` = PSOBatch's other arguments (w, c1, c2, the policy, max_cells / heap_cap / n_slots).  Returns
+    (map_index, path, length, turns, safety_p, diag_p, fitness, convergence_curve) per map of this rank, sorted by map
+    index; identical to PSOSolver(grid, ..., rng_seed=seeds[i]).solve() per map."""
+    return _pop_sweep(PSOBatch, grids, (num_iterations, num_particles, num_waypoints_per_particle), params, seeds, wave,
+                      group, device)
+
+
+def solve_ga_batch(grids, num_generations, population_size, num_waypoints_per_chromosome, params, seeds=None, wave=None,
+                   group=None, device=None):
+    """GA on every grid of `grids` (this rank's shard when `group` is given), like solve_pso_batch.  A wave keeps two
+    [maps, population, max_cells] int32 path arrays (the population and its children): about 2 GiB with the default
+    wave.  `params` = GABatch's other arguments (mutation_rate, crossover_rate, tournament_size, the policy, ...)."""
+    return _pop_sweep(GABatch, grids, (num_generations, population_size, num_waypoints_per_chromosome), params, seeds,
+                      wave, group, device)

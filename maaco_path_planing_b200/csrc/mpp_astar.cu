@@ -334,8 +334,19 @@ struct ChainArgs {
     const int32_t *order;  // optional processing order of the individuals (null: index order)
 };
 
-template <bool OCC_SMEM>
-__global__ void __launch_bounds__(MPP_AS_THREADS, 3) mpp_waypoint_fitness_kernel(ChainArgs A) {
+// individuals over a batch of maps: individual i runs on map map[i] of the [n_maps][occ_words] occupancy
+struct ChainMapsArgs : ChainArgs {
+    const int32_t *map;
+    int n_maps;
+    const MppMapMeta *meta;  // [n_maps]: start and target of every map
+};
+
+// ChainArgs:     every individual on the one map (G.occ, staged in shared memory when OCC_SMEM), visited: N x words.
+// ChainMapsArgs: individual i on map A.map[i] from that map's start to its target, read through that map's slice of
+//                global memory (L2), its statistics from that map's safety classes; visited: n_slots x words.
+template <bool OCC_SMEM, class Args>
+__global__ void __launch_bounds__(MPP_AS_THREADS, 3) mpp_waypoint_fitness_kernel(Args A) {
+    constexpr bool MAPS = std::is_same<Args, ChainMapsArgs>::value;
     extern __shared__ __align__(16) uint32_t s_occ[];
     __shared__ __align__(8) uint64_t s_bar;
     __shared__ __align__(16) uint8_t s_cnt[MPP_AS_GROUPS][MPP_PQ_NB];
@@ -360,18 +371,34 @@ __global__ void __launch_bounds__(MPP_AS_THREADS, 3) mpp_waypoint_fitness_kernel
         i = grp_shfl(L, i, 0);
         if (i >= A.N) break;
         if (A.order) i = A.order[i];                                   // longest chains first (see mpp_waypoint_fitness)
-        uint32_t *vis = A.visited + (size_t)i * A.words;
+        int start = 0, target = 0;                                     // (MAPS: the endpoints of the individual's map)
+        AStarGrid Gm = G;
+        StatsCtx Xm = X;
+        if constexpr (MAPS) {
+            const int m = A.map[i];
+            if ((unsigned)m < (unsigned)A.n_maps) { start = A.meta[m].start; target = A.meta[m].target; }
+            if ((unsigned)m >= (unsigned)A.n_maps || start < 0 || target < 0) {    // outside the batch: not searched
+                if (lane == 0) A.n_cells[i] = 0;
+                path_stats_warp(L, X, A.cells + (size_t)i * A.max_cells, 0, A.stats + (size_t)i * 5);
+                continue;
+            }
+            Gm.occ = A.G.occ + (size_t)m * A.occ_words;
+            Xm.occ = Gm.occ;
+            if (Xm.cls) Xm.cls += (size_t)m * rc;
+        }
+        uint32_t *vis = A.visited + (size_t)(MAPS ? slot : i) * A.words;   // MAPS: a slot runs one chain at a time
         int32_t *path = A.cells + (size_t)i * A.max_cells;
         for (int w = lane; w < A.words; w += MPP_GL) vis[w] = 0u;
         grp_sync(L);
-        int n = 1, cur = A.start, status = 1;
-        if (lane == 0) { path[0] = A.start; vis[A.start >> 5] |= 1u << (A.start & 31); }   // pso.py:63-65
+        const int s0 = MAPS ? start : A.start;
+        int n = 1, cur = s0, status = 1;
+        if (lane == 0) { path[0] = s0; vis[s0 >> 5] |= 1u << (s0 & 31); }       // pso.py:63-65
         grp_sync(L);
         for (int k = 0; k <= A.W; ++k) {
-            const int goal = (k < A.W) ? A.wps[(size_t)i * A.W + k] : A.target;
+            const int goal = (k < A.W) ? A.wps[(size_t)i * A.W + k] : (MAPS ? target : A.target);
             // the segment is written over the tail cell of the path (segment[0] == current_start)
             const int cap = A.max_cells - (n - 1);
-            const int sl = astar_search(L, G, S, 0, cur, goal, vis, path + (n - 1), cap, nullptr, A.counters);
+            const int sl = astar_search(L, Gm, S, 0, cur, goal, vis, path + (n - 1), cap, nullptr, A.counters);
             if (sl < 0) { status = -1; break; }
             if (sl == 0 || (sl == 1 && cur != goal)) { status = 0; break; }          // pso.py:77,87 -> []
             if (sl > cap) { status = 2; n += sl - 1; break; }                        // truncated
@@ -386,7 +413,7 @@ __global__ void __launch_bounds__(MPP_AS_THREADS, 3) mpp_waypoint_fitness_kernel
         // (consecutive duplicates cannot occur: a segment never repeats its first cell; pso.py:91-93 is a no-op)
         int n_out = status == 1 ? n : (status == 2 ? n : status);
         if (lane == 0) A.n_cells[i] = n_out;
-        path_stats_warp(L, X, path, status == 1 ? n : 0, A.stats + (size_t)i * 5);
+        path_stats_warp(L, Xm, path, status == 1 ? n : 0, A.stats + (size_t)i * 5);
     }
 }
 
@@ -418,13 +445,54 @@ extern "C" int mpp_waypoint_fitness(mpp_map *map, const int32_t *waypoints_dev, 
     const size_t smem = (size_t)map->occ_words * 4;
     const int blocks = (n_slots + MPP_AS_GROUPS - 1) / MPP_AS_GROUPS;
     if (smem <= 32 * 1024) {
-        mpp_waypoint_fitness_kernel<true><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
+        mpp_waypoint_fitness_kernel<true, ChainArgs><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
     } else if (smem <= 40 * 1024) {
-        MPP_CUDA(cudaFuncSetAttribute(mpp_waypoint_fitness_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        mpp_waypoint_fitness_kernel<true><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
+        MPP_CUDA(cudaFuncSetAttribute(mpp_waypoint_fitness_kernel<true, ChainArgs>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)smem));
+        mpp_waypoint_fitness_kernel<true, ChainArgs><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
     } else {
-        mpp_waypoint_fitness_kernel<false><<<blocks, MPP_AS_THREADS, 0, s>>>(A);
+        mpp_waypoint_fitness_kernel<false, ChainArgs><<<blocks, MPP_AS_THREADS, 0, s>>>(A);
     }
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
+
+// Waypoint chains over a batch of same-shape maps (individual i on map map_dev[i], from that map's start to its target).
+extern "C" int mpp_waypoint_fitness_maps(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *waypoints_dev,
+                                         int n_individuals, int n_waypoints, const mpp_policy *policy, int32_t *cells_dev,
+                                         int max_cells, int32_t *n_cells_dev, double *stats_dev, uint32_t *visited_dev,
+                                         void *scratch_dev, size_t scratch_bytes, int n_slots, int heap_cap,
+                                         unsigned long long *counters_dev, const int32_t *order_dev, void *stream) {
+    MPP_REQUIRE(maps && map_dev && policy && cells_dev && n_cells_dev && stats_dev && visited_dev && scratch_dev,
+                "mpp_waypoint_fitness_maps: null argument");
+    MPP_REQUIRE(n_individuals > 0 && n_waypoints >= 0 && max_cells > 1, "mpp_waypoint_fitness_maps: bad sizes");
+    MPP_REQUIRE(n_waypoints == 0 || waypoints_dev, "mpp_waypoint_fitness_maps: null waypoints");
+    MPP_REQUIRE(maps->rows < 32768 && maps->cols < 65536,
+                "A*: map %dx%d exceeds the packed-node limit (rows < 32768, cols < 65536)", maps->rows, maps->cols);
+    MPP_REQUIRE(n_slots > 0 && heap_cap >= 64, "A*: n_slots=%d heap_cap=%d", n_slots, heap_cap);
+    const size_t need = 256 + (size_t)n_slots * astar_slot_bytes(maps->rows * maps->cols, heap_cap);
+    MPP_REQUIRE(scratch_bytes >= need, "A*: scratch too small (%zu < %zu)", scratch_bytes, need);
+    MPP_CUDA(cudaSetDevice(maps->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    ChainMapsArgs A;
+    memset(&A, 0, sizeof(A));
+    A.X.occ = maps->occ_dev; A.X.pitch = maps->pitch_words; A.X.R = maps->rows; A.X.C = maps->cols;
+    A.X.pol = *policy;
+    if (policy->mode == 0 && maps->n_obstacles > 0) {             // an obstacle-free map's classes are all 0 (penalty 0.0)
+        const int rc = mpp_map_batch_safety_table(maps, policy->min_safe_distance, stream);
+        if (rc) return rc;
+        A.X.cls = maps->safety_d2_dev; A.X.lut = maps->safety_lut_dev;
+    }
+    MPP_CUDA(cudaMemsetAsync(scratch_dev, 0, 256, s));
+    A.G.occ = maps->occ_dev; A.G.pitch = maps->pitch_words; A.G.R = maps->rows; A.G.C = maps->cols;
+    A.G.allow_diag = policy->allow_diagonal; A.G.restrict_corner = policy->restrict_policy;
+    A.occ_words = maps->occ_words; A.start = -1; A.target = -1;
+    A.wps = waypoints_dev; A.N = n_individuals; A.W = n_waypoints; A.words = (maps->rows * maps->cols + 31) / 32;
+    A.cells = cells_dev; A.max_cells = max_cells; A.n_cells = n_cells_dev; A.stats = stats_dev; A.visited = visited_dev;
+    A.scratch = (char *)scratch_dev; A.n_slots = n_slots; A.heap_cap = heap_cap; A.counters = counters_dev;
+    A.order = order_dev; A.map = map_dev; A.n_maps = maps->n_maps; A.meta = maps->meta_dev;
+    const int blocks = (n_slots + MPP_AS_GROUPS - 1) / MPP_AS_GROUPS;
+    mpp_waypoint_fitness_kernel<false, ChainMapsArgs><<<blocks, MPP_AS_THREADS, 0, s>>>(A);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }

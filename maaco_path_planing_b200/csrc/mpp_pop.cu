@@ -2,7 +2,19 @@
 // GA tournament selection / crossover / mutation (ga_solver.py:136-160).  One thread per
 // (particle, waypoint) / tournament / parent pair; every uniform comes from the Philox stream of the
 // RNG contract, so any rank can regenerate any individual's draws.
+// Every kernel runs over a batch of maps with grid.y = map: map m's arrays are row m of [n_maps][...] buffers and
+// its seed is seeds[m] (the same streams as a single-map solver with that seed).  A single map is the one-map case
+// (seeds = null: the scalar key k0, k1).
 #include "mpp_common.cuh"
+
+#define MPP_POP_MAX_MAPS 65535                                 // grid.y
+
+__device__ __forceinline__ void pop_key(const uint64_t *seeds, uint32_t &k0, uint32_t &k1) {
+    if (seeds) {
+        const uint64_t sd = seeds[blockIdx.y];
+        k0 = (uint32_t)sd; k1 = (uint32_t)(sd >> 32);
+    }
+}
 
 // ---------------------------------------------------------------------------------------------
 // K8: PSO update.  v = ((w*v) + ((c1*r1)*(pbest-x))) + ((c2*r2)*(gbest-x)); clip; x = clip(x+v).
@@ -10,13 +22,21 @@
 // => draws 4*dim+{0,1,2,3} of stream (seed, PSO_UPDATE, iteration, particle).
 // Also emits the integer waypoint pso.py:61,69-70: int(round(x)) (half-even) clamped to the grid.
 // ---------------------------------------------------------------------------------------------
+// Batch: particles [start[m], n) of map m (pid = particle index); start = null: all n, pid = particle_offset + p.
 __global__ void mpp_pso_update_kernel(double *__restrict__ pos, double *__restrict__ vel,
                                       const double *__restrict__ pbest, const double *__restrict__ gbest, int n, int W,
-                                      int particle_offset, double w, double c1, double c2, double max_vel, int R, int C,
-                                      uint32_t k0, uint32_t k1, uint32_t iteration, int32_t *__restrict__ wp_cells) {
+                                      int particle_offset, const int32_t *__restrict__ start, double w, double c1,
+                                      double c2, double max_vel, int R, int C, uint32_t k0, uint32_t k1,
+                                      const uint64_t *__restrict__ seeds, uint32_t iteration,
+                                      int32_t *__restrict__ wp_cells) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n * W) return;
     const int p = t / W, dim = t % W;
+    if (start && p < start[blockIdx.y]) return;
+    pop_key(seeds, k0, k1);
+    const size_t row = (size_t)blockIdx.y * n * W;             // map m's particles
+    pos += 2 * row; vel += 2 * row; pbest += 2 * row; wp_cells += row;
+    gbest += (size_t)blockIdx.y * W * 2;
     const uint32_t pid = (uint32_t)(particle_offset + p);
     const mpp_u4 a = mpp_philox(2u * dim, pid, iteration, MPP_CLS_PSO_UPDATE, k0, k1);
     const mpp_u4 b = mpp_philox(2u * dim + 1u, pid, iteration, MPP_CLS_PSO_UPDATE, k0, k1);
@@ -46,8 +66,26 @@ extern "C" int mpp_pso_update(const mpp_map *map, double *pos_dev, double *vel_d
     MPP_CUDA(cudaSetDevice(map->device));
     const int total = n_particles * n_waypoints;
     mpp_pso_update_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
-        pos_dev, vel_dev, pbest_pos_dev, gbest_pos_dev, n_particles, n_waypoints, particle_offset, w, c1, c2, max_vel,
-        map->rows, map->cols, (uint32_t)seed, (uint32_t)(seed >> 32), (uint32_t)iteration, waypoint_cells_dev);
+        pos_dev, vel_dev, pbest_pos_dev, gbest_pos_dev, n_particles, n_waypoints, particle_offset, nullptr, w, c1, c2,
+        max_vel, map->rows, map->cols, (uint32_t)seed, (uint32_t)(seed >> 32), nullptr, (uint32_t)iteration,
+        waypoint_cells_dev);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
+
+extern "C" int mpp_pso_update_batch(const mpp_map_batch *maps, double *pos_dev, double *vel_dev,
+                                    const double *pbest_pos_dev, const double *gbest_pos_dev, int n_particles,
+                                    const int32_t *start_dev, int n_waypoints, double w, double c1, double c2,
+                                    double max_vel, const uint64_t *seeds_dev, int iteration,
+                                    int32_t *waypoint_cells_dev, void *stream) {
+    MPP_REQUIRE(maps && pos_dev && vel_dev && pbest_pos_dev && gbest_pos_dev && start_dev && seeds_dev &&
+                waypoint_cells_dev, "mpp_pso_update_batch: null argument");
+    MPP_REQUIRE(n_particles > 0 && n_waypoints > 0 && maps->n_maps <= MPP_POP_MAX_MAPS, "mpp_pso_update_batch: bad sizes");
+    MPP_CUDA(cudaSetDevice(maps->device));
+    const int total = n_particles * n_waypoints;
+    mpp_pso_update_kernel<<<dim3((total + 255) / 256, maps->n_maps), 256, 0, (cudaStream_t)stream>>>(
+        pos_dev, vel_dev, pbest_pos_dev, gbest_pos_dev, n_particles, n_waypoints, 0, start_dev, w, c1, c2, max_vel,
+        maps->rows, maps->cols, 0u, 0u, seeds_dev, (uint32_t)iteration, waypoint_cells_dev);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }
@@ -79,9 +117,13 @@ extern "C" int mpp_pso_round(const mpp_map *map, const double *pos_dev, int n_pa
 // ---------------------------------------------------------------------------------------------
 #define MPP_GA_MAX_K 16
 __global__ void mpp_ga_select_kernel(const double *__restrict__ fitness, int n, int k, uint32_t k0, uint32_t k1,
-                                     uint32_t generation, int32_t *__restrict__ parents) {
+                                     const uint64_t *__restrict__ seeds, uint32_t generation,
+                                     int32_t *__restrict__ parents) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n) return;
+    pop_key(seeds, k0, k1);
+    fitness += (size_t)blockIdx.y * n;
+    parents += (size_t)blockIdx.y * n;
     mpp_stream_rng rng;
     rng.init(((uint64_t)k1 << 32) | k0, MPP_CLS_GA_SELECT, generation, (uint32_t)t);
     int setsize = 21;
@@ -120,17 +162,28 @@ __global__ void mpp_ga_select_kernel(const double *__restrict__ fitness, int n, 
     parents[t] = best;
 }
 
-extern "C" int mpp_ga_select(const double *fitness_dev, int n, int tournament_size, uint64_t seed, int generation,
-                             int32_t *parents_dev, void *stream) {
+static int ga_select(int n_maps, const double *fitness_dev, int n, int tournament_size, uint64_t seed,
+                     const uint64_t *seeds_dev, int generation, int32_t *parents_dev, void *stream) {
     MPP_REQUIRE(fitness_dev && parents_dev && n > 0, "mpp_ga_select: bad argument");
     int k = tournament_size < n ? tournament_size : n;  // min(tournament_size, len(population))
     MPP_REQUIRE(k >= 1 && k <= MPP_GA_MAX_K, "mpp_ga_select: tournament size %d unsupported (1..%d)", k, MPP_GA_MAX_K);
     MPP_REQUIRE(k <= 5 || n > 21 + 64, "mpp_ga_select: tiny population with large tournament unsupported");
-    mpp_ga_select_kernel<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(fitness_dev, n, k, (uint32_t)seed,
-                                                                           (uint32_t)(seed >> 32), (uint32_t)generation,
-                                                                           parents_dev);
+    mpp_ga_select_kernel<<<dim3((n + 127) / 128, n_maps), 128, 0, (cudaStream_t)stream>>>(
+        fitness_dev, n, k, (uint32_t)seed, (uint32_t)(seed >> 32), seeds_dev, (uint32_t)generation, parents_dev);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
+}
+
+extern "C" int mpp_ga_select(const double *fitness_dev, int n, int tournament_size, uint64_t seed, int generation,
+                             int32_t *parents_dev, void *stream) {
+    return ga_select(1, fitness_dev, n, tournament_size, seed, nullptr, generation, parents_dev, stream);
+}
+
+extern "C" int mpp_ga_select_batch(const mpp_map_batch *maps, const double *fitness_dev, int n, int tournament_size,
+                                   const uint64_t *seeds_dev, int generation, int32_t *parents_dev, void *stream) {
+    MPP_REQUIRE(maps && seeds_dev && maps->n_maps <= MPP_POP_MAX_MAPS, "mpp_ga_select_batch: bad argument");
+    MPP_CUDA(cudaSetDevice(maps->device));
+    return ga_select(maps->n_maps, fitness_dev, n, tournament_size, 0, seeds_dev, generation, parents_dev, stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -148,13 +201,19 @@ __device__ __forceinline__ int ga_random_free_cell(mpp_stream_rng &rng, const ui
     }
 }
 
-__global__ void mpp_ga_breed_kernel(const uint32_t *__restrict__ occ, int pitch, int R, int C,
+__global__ void mpp_ga_breed_kernel(const uint32_t *__restrict__ occ, int occ_words, int pitch, int R, int C,
                                     const int32_t *__restrict__ chrom, const int32_t *__restrict__ parents, int n, int W,
-                                    double cx_rate, double mut_rate, uint32_t k0, uint32_t k1, uint32_t generation,
+                                    double cx_rate, double mut_rate, uint32_t k0, uint32_t k1,
+                                    const uint64_t *__restrict__ seeds, uint32_t generation,
                                     int32_t *__restrict__ children) {
     const int pair = blockIdx.x * blockDim.x + threadIdx.x;
     const int n_pairs = (n + 1) / 2;
     if (pair >= n_pairs) return;
+    pop_key(seeds, k0, k1);
+    occ += (size_t)blockIdx.y * occ_words;                     // mutated genes are free cells of the map's own grid
+    chrom += (size_t)blockIdx.y * n * W;
+    parents += (size_t)blockIdx.y * n;
+    children += (size_t)blockIdx.y * n * W;
     mpp_stream_rng rng;
     rng.init(((uint64_t)k1 << 32) | k0, MPP_CLS_GA_BREED, generation, (uint32_t)pair);
     const int32_t *p1 = chrom + (size_t)parents[(2 * pair) % n] * W;
@@ -188,8 +247,27 @@ extern "C" int mpp_ga_breed(const mpp_map *map, const int32_t *chrom_dev, const 
     MPP_CUDA(cudaSetDevice(map->device));
     const int n_pairs = (n + 1) / 2;
     mpp_ga_breed_kernel<<<(n_pairs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        map->occ_dev, map->pitch_words, map->rows, map->cols, chrom_dev, parents_dev, n, n_waypoints, crossover_rate,
-        mutation_rate, (uint32_t)seed, (uint32_t)(seed >> 32), (uint32_t)generation, children_dev);
+        map->occ_dev, map->occ_words, map->pitch_words, map->rows, map->cols, chrom_dev, parents_dev, n, n_waypoints,
+        crossover_rate, mutation_rate, (uint32_t)seed, (uint32_t)(seed >> 32), nullptr, (uint32_t)generation,
+        children_dev);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
+
+extern "C" int mpp_ga_breed_batch(const mpp_map_batch *maps, const int32_t *chrom_dev, const int32_t *parents_dev, int n,
+                                  int n_waypoints, double crossover_rate, double mutation_rate, const uint64_t *seeds_dev,
+                                  int generation, int32_t *children_dev, void *stream) {
+    MPP_REQUIRE(maps && chrom_dev && parents_dev && seeds_dev && children_dev && n > 0 && maps->n_maps <= MPP_POP_MAX_MAPS,
+                "mpp_ga_breed_batch: bad argument");
+    MPP_REQUIRE(n_waypoints >= 1 && n_waypoints <= MPP_GA_MAX_W, "mpp_ga_breed_batch: %d waypoints unsupported (1..%d)",
+                n_waypoints, MPP_GA_MAX_W);
+    for (int k = 0; k < maps->n_maps; ++k)                             // the start cell is free: mutation terminates
+        MPP_REQUIRE(maps->meta_host[k].start >= 0, "mpp_ga_breed_batch: map %d has no start", k);
+    MPP_CUDA(cudaSetDevice(maps->device));
+    const int n_pairs = (n + 1) / 2;
+    mpp_ga_breed_kernel<<<dim3((n_pairs + 127) / 128, maps->n_maps), 128, 0, (cudaStream_t)stream>>>(
+        maps->occ_dev, maps->occ_words, maps->pitch_words, maps->rows, maps->cols, chrom_dev, parents_dev, n, n_waypoints,
+        crossover_rate, mutation_rate, 0u, 0u, seeds_dev, (uint32_t)generation, children_dev);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }
@@ -201,10 +279,16 @@ extern "C" int mpp_ga_breed(const mpp_map *map, const int32_t *chrom_dev, const 
 // ---------------------------------------------------------------------------------------------
 // PSO attempt: W waypoints [uniform(0, R-1), uniform(0, C-1)] (pso.py:50-51, draws 0..2W-1), then W velocities
 // [uniform(-max_vel/5, max_vel/5)] x 2 (pso.py:105, draws 2W..4W-1); also the rounded, clamped cells (pso.py:61,69-70).
-__global__ void mpp_pso_init_kernel(int n, int W, int attempt0, int R, int C, double max_vel, uint32_t k0, uint32_t k1,
+// Batch: attempts [offsets[m], offsets[m] + n) of map m (offsets[m] < 0: the map is done, nothing is written).
+__global__ void mpp_pso_init_kernel(int n, int W, int attempt0, const int32_t *__restrict__ offsets, int R, int C,
+                                    double max_vel, uint32_t k0, uint32_t k1, const uint64_t *__restrict__ seeds,
                                     double *__restrict__ pos, double *__restrict__ vel, int32_t *__restrict__ wp_cells) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n * W) return;
+    if (offsets && (attempt0 = offsets[blockIdx.y]) < 0) return;
+    pop_key(seeds, k0, k1);
+    const size_t row = (size_t)blockIdx.y * n * W;
+    pos += 2 * row; vel += 2 * row; wp_cells += row;
     const int p = t / W, dim = t % W;
     const uint32_t att = (uint32_t)(attempt0 + p);
     // draws 2*dim, 2*dim+1 = block dim; draws 2W + 2*dim, +1 = block W + dim
@@ -229,17 +313,36 @@ extern "C" int mpp_pso_init(const mpp_map *map, int n_attempts, int attempt_offs
     MPP_CUDA(cudaSetDevice(map->device));
     const int total = n_attempts * n_waypoints;
     mpp_pso_init_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
-        n_attempts, n_waypoints, attempt_offset, map->rows, map->cols, max_vel, (uint32_t)seed, (uint32_t)(seed >> 32),
-        pos_dev, vel_dev, waypoint_cells_dev);
+        n_attempts, n_waypoints, attempt_offset, nullptr, map->rows, map->cols, max_vel, (uint32_t)seed,
+        (uint32_t)(seed >> 32), nullptr, pos_dev, vel_dev, waypoint_cells_dev);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
+
+extern "C" int mpp_pso_init_batch(const mpp_map_batch *maps, int n_attempts, const int32_t *attempt_offset_dev,
+                                  int n_waypoints, double max_vel, const uint64_t *seeds_dev, double *pos_dev,
+                                  double *vel_dev, int32_t *waypoint_cells_dev, void *stream) {
+    MPP_REQUIRE(maps && attempt_offset_dev && seeds_dev && pos_dev && vel_dev && waypoint_cells_dev && n_attempts > 0 &&
+                n_waypoints > 0 && maps->n_maps <= MPP_POP_MAX_MAPS, "mpp_pso_init_batch: bad argument");
+    MPP_CUDA(cudaSetDevice(maps->device));
+    const int total = n_attempts * n_waypoints;
+    mpp_pso_init_kernel<<<dim3((total + 255) / 256, maps->n_maps), 256, 0, (cudaStream_t)stream>>>(
+        n_attempts, n_waypoints, 0, attempt_offset_dev, maps->rows, maps->cols, max_vel, 0u, 0u, seeds_dev, pos_dev,
+        vel_dev, waypoint_cells_dev);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }
 
 // GA attempt: W genes, each (randint(0, R-1), randint(0, C-1)) redrawn until the cell is free (ga_solver.py:48-56)
-__global__ void mpp_ga_init_kernel(const uint32_t *__restrict__ occ, int pitch, int R, int C, int n, int W, int attempt0,
-                                   uint32_t k0, uint32_t k1, int32_t *__restrict__ chrom) {
+__global__ void mpp_ga_init_kernel(const uint32_t *__restrict__ occ, int occ_words, int pitch, int R, int C, int n, int W,
+                                   int attempt0, const int32_t *__restrict__ offsets, uint32_t k0, uint32_t k1,
+                                   const uint64_t *__restrict__ seeds, int32_t *__restrict__ chrom) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n) return;
+    if (offsets && (attempt0 = offsets[blockIdx.y]) < 0) return;   // the map is done
+    pop_key(seeds, k0, k1);
+    occ += (size_t)blockIdx.y * occ_words;
+    chrom += (size_t)blockIdx.y * n * W;
     mpp_stream_rng rng;
     rng.init(((uint64_t)k1 << 32) | k0, MPP_CLS_GA_INIT, 0u, (uint32_t)(attempt0 + p));
     for (int k = 0; k < W; ++k) chrom[(size_t)p * W + k] = ga_random_free_cell(rng, occ, pitch, R, C);
@@ -251,8 +354,22 @@ extern "C" int mpp_ga_init(const mpp_map *map, int n_attempts, int attempt_offse
     MPP_REQUIRE(map->n_obstacles < map->rows * map->cols, "mpp_ga_init: map has no free cell");
     MPP_CUDA(cudaSetDevice(map->device));
     mpp_ga_init_kernel<<<(n_attempts + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        map->occ_dev, map->pitch_words, map->rows, map->cols, n_attempts, n_waypoints, attempt_offset, (uint32_t)seed,
-        (uint32_t)(seed >> 32), chrom_dev);
+        map->occ_dev, map->occ_words, map->pitch_words, map->rows, map->cols, n_attempts, n_waypoints, attempt_offset,
+        nullptr, (uint32_t)seed, (uint32_t)(seed >> 32), nullptr, chrom_dev);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
+
+extern "C" int mpp_ga_init_batch(const mpp_map_batch *maps, int n_attempts, const int32_t *attempt_offset_dev,
+                                 int n_waypoints, const uint64_t *seeds_dev, int32_t *chrom_dev, void *stream) {
+    MPP_REQUIRE(maps && attempt_offset_dev && seeds_dev && chrom_dev && n_attempts > 0 && n_waypoints > 0 &&
+                maps->n_maps <= MPP_POP_MAX_MAPS, "mpp_ga_init_batch: bad argument");
+    for (int k = 0; k < maps->n_maps; ++k)                             // the start cell is free: mutation terminates
+        MPP_REQUIRE(maps->meta_host[k].start >= 0, "mpp_ga_init_batch: map %d has no start", k);
+    MPP_CUDA(cudaSetDevice(maps->device));
+    mpp_ga_init_kernel<<<dim3((n_attempts + 127) / 128, maps->n_maps), 128, 0, (cudaStream_t)stream>>>(
+        maps->occ_dev, maps->occ_words, maps->pitch_words, maps->rows, maps->cols, n_attempts, n_waypoints, 0,
+        attempt_offset_dev, 0u, 0u, seeds_dev, chrom_dev);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }
