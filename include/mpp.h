@@ -81,6 +81,19 @@ int mpp_map_batch_size(const mpp_map_batch *maps);
 int mpp_map_batch_start(const mpp_map_batch *maps, int k);  /* cell id of map k's start or -1 */
 int mpp_map_batch_target(const mpp_map_batch *maps, int k);
 const mpp_map_batch *mpp_map_as_batch(const mpp_map *map);
+/* The same batch from grids already in device memory of `device`: grids_dev = n_maps x rows x cols contiguous cells of
+ * elem_bytes bytes each (1 = uint8, 4 = int32, 8 = int64).  Cells are compared raw: 1 obstacle, 2 start candidate,
+ * 3 target candidate, any other value free -- the classification the uint8 path gives after clipping to 0..255.
+ * Everything runs on `stream` (the grids may have been written by work enqueued on it just before); the grids never
+ * leave the device, only the per-map start / target and the obstacle count are read back.  Synchronous: returns when
+ * the batch is ready. */
+int mpp_map_batch_create_device(const void *grids_dev, int elem_bytes, int n_maps, int rows, int cols, int device,
+                                void *stream, mpp_map_batch **out);
+/* the batch's occupancy, [n_maps][((rows+2) * pitch_words + 3) & ~3] words in mpp_map_occ_bits's layout, its static
+ * move masks [n_maps][rows*cols] (MAACO move order) and its obstacle count over all maps */
+const uint32_t *mpp_map_batch_occ_bits(const mpp_map_batch *maps, int *pitch_words);
+const uint8_t *mpp_map_batch_svalid(const mpp_map_batch *maps);
+long long mpp_map_batch_obstacles(const mpp_map_batch *maps);
 
 /* ---- MAACO (MAACO.py) -------------------------------------------------------------------- */
 typedef struct {

@@ -64,6 +64,10 @@ _SIGS = {
     "mpp_map_batch_start": (c_int, [c_void_p, c_int]),
     "mpp_map_batch_target": (c_int, [c_void_p, c_int]),
     "mpp_map_as_batch": (c_void_p, [c_void_p]),
+    "mpp_map_batch_create_device": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, C.POINTER(c_void_p)]),
+    "mpp_map_batch_occ_bits": (c_void_p, [c_void_p, C.POINTER(c_int)]),
+    "mpp_map_batch_svalid": (c_void_p, [c_void_p]),
+    "mpp_map_batch_obstacles": (C.c_longlong, [c_void_p]),
     "mpp_maaco_tables": (c_int, [c_void_p, C.POINTER(MaacoParams), c_void_p, C.c_longlong, c_void_p, c_void_p, c_void_p]),
     "mpp_maaco_q0": (c_double, [c_int, c_int, c_double]),
     "mpp_maaco_rank_words": (C.c_longlong, [c_int, c_int]),

@@ -6,7 +6,12 @@ without host synchronisation.  Results are identical to solving each map alone w
 
 The eta'**beta / dist-to-target tables depend only on (shape, start, target, parameters), so a wave shares ONE
 table computed on the host with libm (bit-identical to the reference), and tau0 of each map is that shared table
-with the map's obstacles masked on the device (mpp_maaco_tables)."""
+with the map's obstacles masked on the device (mpp_maaco_tables).
+
+Every batch class takes `grids` either on the host ([M, rows, cols] cell codes, anything np.asarray takes) or as an
+[M, rows, cols] CUDA tensor of bool, uint8, int8, int16, int32 or int64 cells; every sweep also takes a sequence of 2-D
+CUDA tensors.  Device grids are packed on the GPU, on torch's current stream (mpp_map_batch_create_device), and never go
+through the host; results are the same as from the same grids on the host."""
 from __future__ import annotations
 
 import ctypes as C
@@ -51,6 +56,111 @@ def _grids_u8(grids):
     return g8
 
 
+_DEVICE_DTYPES = "bool, uint8, int8, int16, int32 or int64"
+
+
+def _on_device(grids):
+    """True for device grids: a CUDA tensor, or a sequence whose first map is one."""
+    import torch
+    if isinstance(grids, torch.Tensor):
+        return grids.is_cuda
+    return (not isinstance(grids, np.ndarray) and len(grids) > 0 and isinstance(grids[0], torch.Tensor)
+            and grids[0].is_cuda)
+
+
+def _device_cells(g):
+    """g (a CUDA tensor of cell codes) with bool / int8 / int16 widened to a width mpp_map_batch_create_device reads
+    (uint8 / int32); floating-point and other dtypes raise TypeError."""
+    import torch
+    widen = {torch.bool: torch.uint8, torch.int8: torch.int32, torch.int16: torch.int32, torch.uint8: None,
+             torch.int32: None, torch.int64: None}
+    if g.dtype not in widen:
+        raise TypeError(f"device grids must hold {_DEVICE_DTYPES} cell codes, not {g.dtype}")
+    return g if widen[g.dtype] is None else g.to(widen[g.dtype])
+
+
+def _first_cells(flat):
+    """First row-major start (2) and target (3) cell of every row of `flat` ([n_maps, rows*cols] cell codes on the host),
+    -1 = none: what the reference constructors look for (MAACO.py:32-41, astar.py:17-18, ...)."""
+    ends = []
+    for v in (START_NODE_VAL, TARGET_NODE_VAL):
+        hit = flat == v
+        ends.append(np.where(hit.any(axis=1), hit.argmax(axis=1), -1))
+    return tuple(ends)
+
+
+class _MapSet:
+    """An mpp_map_batch with what Python reads from it: (n_maps, rows, cols), its device and every map's first
+    row-major start and target cell (-1 = none).  A wave repeated with more buffer room shares its MapSet, so the handle
+    is freed when the last batch object holding it lets go of it (or by close())."""
+
+    def __init__(self, handle, shape, device_index, start, target):
+        self.handle, self.shape, self.device_index = handle, tuple(int(x) for x in shape), int(device_index)
+        self.start, self.target = np.asarray(start, np.int64), np.asarray(target, np.int64)
+
+    def close(self):
+        h, self.handle = self.handle, None
+        if h:
+            _lib.lib().mpp_map_batch_destroy(h)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _map_set(grids, device=None, check=None):
+    """The _MapSet every batch class solves on (a _MapSet is returned as it is).  Host grids ([n_maps, rows, cols] cell
+    codes, anything np.asarray takes) go through _grids_u8 and mpp_map_batch_create; a [n_maps, rows, cols] CUDA tensor
+    goes through mpp_map_batch_create_device on torch's current stream and never leaves the GPU -- it runs on its own
+    device unless `device` names another, which then receives a copy of just these maps.  check(start, target) raises
+    the planner's errors for maps without a start or target: for host grids before any device work, for device grids
+    from the endpoints the ingestion read back, after freeing the handle."""
+    import torch
+    if isinstance(grids, _MapSet):
+        return grids
+    L = _lib.lib()
+    h = C.c_void_p()
+    if isinstance(grids, torch.Tensor) and grids.is_cuda:
+        if grids.dim() != 3:
+            raise ValueError("grids must be [n_maps, rows, cols]")
+        g = grids if device is None else grids.to(torch.device("cuda", int(device)))
+        g = _device_cells(g).contiguous()
+        _lib.require_device()
+        M, R, Cc = g.shape
+        stream = C.c_void_p(torch.cuda.current_stream(g.device).cuda_stream)
+        _lib.check(L.mpp_map_batch_create_device(g.data_ptr(), g.element_size(), M, R, Cc, g.device.index, stream,
+                                                 C.byref(h)), "mpp_map_batch_create_device")
+        maps = _MapSet(h, g.shape, g.device.index, [L.mpp_map_batch_start(h, k) for k in range(M)],
+                       [L.mpp_map_batch_target(h, k) for k in range(M)])
+        if check is not None:
+            try:
+                check(maps.start, maps.target)
+            except ValueError:
+                maps.close()
+                raise
+        return maps
+    g8 = _grids_u8(grids)
+    start, target = _first_cells(g8.reshape(g8.shape[0], -1))
+    if check is not None:
+        check(start, target)
+    _lib.require_device()
+    dev = torch.cuda.current_device() if device is None else int(device)
+    _lib.check(L.mpp_map_batch_create(g8.ctypes.data_as(C.c_void_p), *g8.shape, dev, C.byref(h)), "mpp_map_batch_create")
+    return _MapSet(h, g8.shape, dev, start, target)
+
+
+def _all_endpoints(no_start, no_target):
+    """MAACOBatch's / MPABatch's check: any map without a start raises no_start, else any without a target no_target."""
+    def check(start, target):
+        if (start < 0).any():
+            raise ValueError(no_start)
+        if (target < 0).any():
+            raise ValueError(no_target)
+    return check
+
+
 class MAACOBatch:
     """M same-shape maps that share start and target, one colony of `num_ants` ants per map, solved together.
     Same parameters as MAACO (MAACO.py:11-14); `seeds` = one Philox seed per map.  `max_cells` works as in MAACO: left
@@ -62,20 +172,12 @@ class MAACOBatch:
                  reuse=None):
         import torch
         L = _lib.lib()
-        g8 = _grids_u8(grids)
-        self.n_maps, self.rows, self.cols = g8.shape
-        flat = g8.reshape(self.n_maps, -1)
-        if not (flat == START_NODE_VAL).any(axis=1).all():
-            raise ValueError("MAACO: Start node not found.")                  # MAACO.py:35-36
-        if not (flat == TARGET_NODE_VAL).any(axis=1).all():
-            raise ValueError("MAACO: Target node not found.")                 # MAACO.py:37-38
-        _lib.require_device()
-        self.device_index = torch.cuda.current_device() if device is None else int(device)
+        self._map_set = _map_set(grids, device, _all_endpoints("MAACO: Start node not found.",        # MAACO.py:35-36
+                                                               "MAACO: Target node not found."))      # MAACO.py:37-38
+        self._maps = self._map_set.handle
+        self.n_maps, self.rows, self.cols = self._map_set.shape
+        self.device_index = self._map_set.device_index
         self.device = torch.device("cuda", self.device_index)
-        h = C.c_void_p()
-        _lib.check(L.mpp_map_batch_create(g8.ctypes.data_as(C.c_void_p), self.n_maps, self.rows, self.cols,
-                                          self.device_index, C.byref(h)), "mpp_map_batch_create")
-        self._maps = h
         self.num_ants, self.num_iterations = int(num_ants), int(num_iterations)
         self.alpha, self.rho, self.Q = alpha, rho, Q
         self._params = _lib.MaacoParams(alpha, beta, rho, Q, a_turn_coef, wh_max, wh_min, k_h_adaptive, q0_initial,
@@ -91,10 +193,10 @@ class MAACOBatch:
         if seeds is None:
             seeds = [int.from_bytes(np.random.bytes(8), "little") for _ in range(M)]
         self.seeds = [int(s) & (2 ** 64 - 1) for s in seeds]
-        self._ctor = dict(grids=g8, num_ants=num_ants, num_iterations=num_iterations, alpha=alpha, beta=beta, rho=rho, Q=Q,
+        self._ctor = dict(num_ants=num_ants, num_iterations=num_iterations, alpha=alpha, beta=beta, rho=rho, Q=Q,
                           a_turn_coef=a_turn_coef, wh_max=wh_max, wh_min=wh_min, k_h_adaptive=k_h_adaptive,
                           q0_initial=q0_initial, C0_initial_pheromone=C0_initial_pheromone, seeds=self.seeds,
-                          device=self.device_index, ants_per_warp=ants_per_warp)
+                          ants_per_warp=ants_per_warp)
         dev = self.device
         f64, i32, i64, u8 = torch.float64, torch.int32, torch.int64, torch.uint8
         K = max(1, self.num_iterations)
@@ -136,9 +238,7 @@ class MAACOBatch:
         self.kernel_launches = 0
 
     def close(self):
-        h, self._maps = getattr(self, "_maps", None), None
-        if h:
-            _lib.lib().mpp_map_batch_destroy(h)
+        self._maps = self._map_set = None
 
     def __del__(self):
         try:
@@ -186,12 +286,11 @@ class MAACOBatch:
             if not self._auto_cells or self.max_cells >= self.rows * self.cols:
                 raise _lib.MppError(f"a tour outgrew max_cells={self.max_cells} (best path: "
                                     f"{int(st['best_n_cells'].max())} cells); re-run with a larger max_cells")
-            # the solve is a deterministic function of (grids, parameters, seeds): repeat the wave with full path capacity
-            again = type(self)(max_cells=self.rows * self.cols, **self._ctor)
+            # the solve is a deterministic function of (maps, parameters, seeds): repeat the wave with full path capacity
+            # on the same map batch (not on the caller's grids, which may have changed since)
+            again = type(self)(self._map_set, max_cells=self.rows * self.cols, **self._ctor)
             again.kernel_launches = self.kernel_launches
-            self.close()
             self.__dict__.update(again.__dict__)
-            again._maps = None                                                # the map handle is ours now
             return self.solve()
         best = self._best_cells.cpu().numpy()
         log = self._log.cpu().numpy()[:, :K]
@@ -206,13 +305,76 @@ class MAACOBatch:
         return out
 
 
-def _waves(grids, lo, hi, wave):
-    """Group this rank's maps into waves of same shape / start / target (what one mpp_map_batch needs)."""
+class _HostSweep:
+    """The maps lo..hi-1 of a sweep over host grids: a wave is stacked on the host and uploaded by its batch."""
+
+    def __init__(self, grids, lo, hi):
+        self.grids, self.lo, self.hi = grids, lo, hi
+
+    def wave(self, idx):
+        return np.stack([np.asarray(self.grids[i]) for i in idx])
+
+    def first_cells(self):
+        """(start, target) of maps lo..hi-1: first row-major cell, -1 = none."""
+        ends = [_first_cells(np.asarray(self.grids[i]).reshape(1, -1)) for i in range(self.lo, self.hi)]
+        return tuple(np.array([e[k][0] for e in ends], np.int64) for k in (0, 1))
+
+
+class _DeviceSweep:
+    """The maps lo..hi-1 of a sweep over device grids (a [n_maps, rows, cols] CUDA tensor or a sequence of 2-D CUDA
+    tensors), grouped by shape and stacked on their device once -- the shard of a 3-D tensor is a slice of it -- so a
+    wave is a slice of its group (a gather for MAACO's endpoint groups) and no grid goes through the host."""
+
+    def __init__(self, grids, lo, hi):
+        import torch
+        if isinstance(grids, torch.Tensor):
+            if grids.dim() != 3:
+                raise ValueError("grids must be [n_maps, rows, cols]")
+            self.groups = [(list(range(lo, hi)), grids[lo:hi])] if hi > lo else []
+        else:
+            self.groups = [(idx, torch.stack([grids[i] for i in idx])) for idx in _shape_waves(grids, lo, hi)]
+        for _, g in self.groups:
+            _device_cells(g[:0])                                             # dtype check before any work
+        self._at = {i: (g, k) for idx, g in self.groups for k, i in enumerate(idx)}
+        self.lo, self.hi = lo, hi
+
+    def wave(self, idx):
+        import torch
+        g, k0 = self._at[idx[0]]
+        pos = [self._at[i][1] for i in idx]
+        if pos == list(range(k0, k0 + len(idx))):
+            return g[k0:k0 + len(idx)]
+        return g[torch.as_tensor(pos, device=g.device)]
+
+    def first_cells(self):
+        """(start, target) of maps lo..hi-1: first row-major cell, -1 = none; computed on the device, one read back."""
+        import torch
+        if not self.groups:
+            return np.zeros(0, np.int64), np.zeros(0, np.int64)
+        ends = []
+        for idx, g in self.groups:
+            flat = g.reshape(len(idx), -1)
+            for v in (START_NODE_VAL, TARGET_NODE_VAL):
+                hit = flat == v
+                ends.append(torch.where(hit.any(dim=1), hit.to(torch.uint8).argmax(dim=1), -1).to(self.groups[0][1].device))
+        ends = torch.cat(ends).cpu().numpy()
+        start, target = np.empty(self.hi - self.lo, np.int64), np.empty(self.hi - self.lo, np.int64)
+        o = 0
+        for idx, _ in self.groups:
+            at = np.asarray(idx) - self.lo
+            start[at], target[at] = ends[o:o + len(idx)], ends[o + len(idx):o + 2 * len(idx)]
+            o += 2 * len(idx)
+        return start, target
+
+
+def _sweep_maps(grids, lo, hi):
+    return (_DeviceSweep if _on_device(grids) else _HostSweep)(grids, lo, hi)
+
+
+def _waves(keys, wave):
+    """Group maps into waves of same shape / start / target (what one mpp_map_batch needs); keys: map index -> key."""
     groups = {}
-    for i in range(lo, hi):
-        g = np.asarray(grids[i])
-        s, t = np.argwhere(g == START_NODE_VAL), np.argwhere(g == TARGET_NODE_VAL)
-        key = (g.shape, tuple(s[0]) if len(s) else None, tuple(t[0]) if len(t) else None)
+    for i, key in keys.items():
         groups.setdefault(key, []).append(i)
     for idx in groups.values():
         for w0 in range(0, len(idx), wave):
@@ -221,15 +383,19 @@ def _waves(grids, lo, hi, wave):
 
 def solve_maaco_batch(grids, num_ants, num_iterations, params, seeds=None, wave=256, group=None, device=None,
                       max_cells=None):
-    """Run MAACO on every grid of `grids` (this rank's shard when `group` is given), `wave` maps per launch.
+    """Run MAACO on every grid of `grids` (this rank's shard when `group` is given), `wave` maps per launch.  `grids`:
+    host maps, a [n_maps, rows, cols] CUDA tensor or a sequence of 2-D CUDA tensors (which never leave the GPU).
 
     Returns a list of (map_index, path, length, turns, convergence_curve) for the maps of this rank; results
     are identical to solving each map alone (same seeds => same Philox streams)."""
     lo, hi = shard_maps(len(grids), group)
+    maps = _sweep_maps(grids, lo, hi)
+    start, target = maps.first_cells()
+    keys = {i: (_map_shape(grids[i]), start[i - lo], target[i - lo]) for i in range(lo, hi)}
     out = []
     prev = None
-    for idx in _waves(grids, lo, hi, wave):
-        b = MAACOBatch(np.stack([np.asarray(grids[i]) for i in idx]), num_ants, num_iterations,
+    for idx in _waves(keys, wave):
+        b = MAACOBatch(maps.wave(idx), num_ants, num_iterations,
                        seeds=None if seeds is None else [seeds[i] for i in idx], device=device, max_cells=max_cells,
                        reuse=prev, **params)
         for i, (path, length, turns, curve) in zip(idx, b.solve()):
@@ -253,22 +419,12 @@ class MPABatch:
         import math
         import torch
         from .engine import make_policy
-        L = _lib.lib()
-        g8 = _grids_u8(grids)
-        self.n_maps, self.rows, self.cols = g8.shape
-        flat = g8.reshape(self.n_maps, -1)
-        if not (flat == START_NODE_VAL).any(axis=1).all():
-            raise ValueError("MPA: Start node not found in grid.")            # MPA.py:36-37
-        if not (flat == TARGET_NODE_VAL).any(axis=1).all():
-            raise ValueError("MPA: Target node not found in grid.")           # MPA.py:38-39
-        _lib.require_device()
-        self.device_index = torch.cuda.current_device() if device is None else int(device)
+        self._map_set = _map_set(grids, device, _all_endpoints("MPA: Start node not found in grid.",      # MPA.py:36-37
+                                                               "MPA: Target node not found in grid."))    # MPA.py:38-39
+        self._maps = self._map_set.handle
+        self.n_maps, self.rows, self.cols = self._map_set.shape
+        self.device_index = self._map_set.device_index
         self.device = torch.device("cuda", self.device_index)
-        self._grids8 = g8
-        h = C.c_void_p()
-        _lib.check(L.mpp_map_batch_create(self._grids8.ctypes.data_as(C.c_void_p), self.n_maps, self.rows, self.cols,
-                                          self.device_index, C.byref(h)), "mpp_map_batch_create")
-        self._maps = h
         self.num_predators, self.num_iterations = int(num_predators), int(num_iterations)
         self.FADs_rate, self.P_const, self.levy_beta = FADs_rate, P_const, levy_beta
         self.policy = make_policy(turn_penalty_factor, safety_penalty_factor, min_safe_distance, diagonal_obstacle_penalty,
@@ -289,20 +445,18 @@ class MPABatch:
         sm = torch.cuda.get_device_properties(self.device).multi_processor_count
         # search slots (one warp each): three CTAs of 8 warps per SM in total, split evenly over the maps (at least one CTA each)
         self.warps_per_map = int(warps_per_map or max(8, ((sm * 24) // self.n_maps) // 8 * 8))
-        self._ctor = dict(grids=grids, num_predators=num_predators, num_iterations=num_iterations, FADs_rate=FADs_rate,
+        self._ctor = dict(num_predators=num_predators, num_iterations=num_iterations, FADs_rate=FADs_rate,
                           P_const=P_const, levy_beta=levy_beta, turn_penalty_factor=turn_penalty_factor,
                           safety_penalty_factor=safety_penalty_factor, min_safe_distance=min_safe_distance,
                           allow_diagonal_moves=allow_diagonal_moves,
                           restrict_diagonal_near_obstacle=restrict_diagonal_near_obstacle,
-                          diagonal_obstacle_penalty=diagonal_obstacle_penalty, seeds=self.seeds, device=device,
+                          diagonal_obstacle_penalty=diagonal_obstacle_penalty, seeds=self.seeds,
                           warps_per_map=warps_per_map)
         self.predator_evaluations = 0
         self.kernel_launches = 0
 
     def close(self):
-        h, self._maps = getattr(self, "_maps", None), None
-        if h:
-            _lib.lib().mpp_map_batch_destroy(h)
+        self._maps = self._map_set = None
 
     def __del__(self):
         try:
@@ -391,7 +545,7 @@ class MPABatch:
                 if self.max_cells >= 2 * self.rows * self.cols:
                     raise _lib.MppError("path buffer overflow at maximum capacity")
                 kw.update(max_cells=min(2 * self.rows * self.cols, 2 * self.max_cells), heap_cap=self.heap_cap)
-            again = MPABatch(**kw)
+            again = MPABatch(self._map_set, **kw)                                # the same map batch
             again.predator_evaluations, again.kernel_launches = self.predator_evaluations, self.kernel_launches
             out = again.solve()
             self.predator_evaluations, self.kernel_launches = again.predator_evaluations, again.kernel_launches
@@ -410,21 +564,18 @@ class MPABatch:
 
 
 def solve_mpa_batch(grids, num_predators, num_iterations, params, seeds=None, wave=32, group=None, device=None):
-    """MPA over this rank's shard of the maps, `wave` maps per launch (grouped by shape).  Returns
-    (map_index, path, length, turns, safety_p, diag_p, fitness, convergence_curve) per map of this rank."""
+    """MPA over this rank's shard of the maps (host maps or device grids, as solve_maaco_batch takes), `wave` maps per
+    launch (grouped by shape).  Returns (map_index, path, length, turns, safety_p, diag_p, fitness, convergence_curve)
+    per map of this rank."""
     lo, hi = shard_maps(len(grids), group)
+    maps = _sweep_maps(grids, lo, hi)
     out = []
-    shapes = {}
-    for i in range(lo, hi):
-        shapes.setdefault(np.asarray(grids[i]).shape, []).append(i)
-    for idx_all in shapes.values():
-        for w0 in range(0, len(idx_all), wave):
-            idx = idx_all[w0:w0 + wave]
-            b = MPABatch(np.stack([np.asarray(grids[i]) for i in idx]), num_predators, num_iterations,
-                         seeds=None if seeds is None else [seeds[i] for i in idx], device=device, **params)
-            for i, r in zip(idx, b.solve()):
-                out.append((i,) + tuple(r))
-            b.close()
+    for idx in _shape_waves(grids, lo, hi, wave):
+        b = MPABatch(maps.wave(idx), num_predators, num_iterations,
+                     seeds=None if seeds is None else [seeds[i] for i in idx], device=device, **params)
+        for i, r in zip(idx, b.solve()):
+            out.append((i,) + tuple(r))
+        b.close()
     out.sort(key=lambda r: r[0])
     return out
 
@@ -449,19 +600,24 @@ _ENDPOINT_ERRORS.update(pso=("PSO: Start node not found.", "PSO: Target node not
                         ga=("GA: Start node not found.", "GA: Target node not found."))                 # ga_solver.py:19-20
 
 
-def _check_endpoints(flat, algorithm):
-    """Raises the reference constructor's ValueError for the first map (a row of `flat`, cell codes) that has no start
-    or no target -- what a loop of AStarSolver / DijkstraSolver / PSOSolver / GASolver constructors over the maps would
-    raise."""
+def _endpoint_check(algorithm):
+    """check(start, target) (per-map first start / target cell, -1 = none) raising the reference constructor's
+    ValueError for the first map that has no start or no target -- what a loop of AStarSolver / DijkstraSolver /
+    PSOSolver / GASolver constructors over the maps would raise."""
     if algorithm not in _ENDPOINT_ERRORS:
         _search_algorithm(algorithm)
     no_start, no_target = _ENDPOINT_ERRORS[algorithm]
-    flat = np.asarray(flat)
-    has_s = (flat == START_NODE_VAL).any(axis=1)
-    has_t = (flat == TARGET_NODE_VAL).any(axis=1)
-    bad = np.flatnonzero(~(has_s & has_t))
-    if bad.size:
-        raise ValueError(no_start if not has_s[bad[0]] else no_target)
+
+    def check(start, target):
+        bad = np.flatnonzero((start < 0) | (target < 0))
+        if bad.size:
+            raise ValueError(no_start if start[bad[0]] < 0 else no_target)
+    return check
+
+
+def _check_endpoints(flat, algorithm):
+    """_endpoint_check on host maps, one per row of `flat` (cell codes)."""
+    _endpoint_check(algorithm)(*_first_cells(np.asarray(flat)))
 
 
 def _valid_queries(map_index, src, dst, n_maps, n_cells):
@@ -474,11 +630,15 @@ def _valid_queries(map_index, src, dst, n_maps, n_cells):
     return (map_index >= 0) & (map_index < n_maps) & (src >= 0) & (src < n_cells) & (dst >= 0) & (dst < n_cells)
 
 
+def _map_shape(g):
+    return tuple(g.shape) if hasattr(g, "shape") else np.shape(g)
+
+
 def _shape_waves(grids, lo, hi, wave=None):
     """Maps lo..hi-1 grouped by shape (one mpp_map_batch each), `wave` maps per group at most (None: all of them)."""
     shapes = {}
     for i in range(lo, hi):
-        shapes.setdefault(np.asarray(grids[i]).shape, []).append(i)
+        shapes.setdefault(_map_shape(grids[i]), []).append(i)
     out = []
     for idx in shapes.values():
         step = wave or len(idx)
@@ -498,15 +658,11 @@ class SearchBatch:
         import torch
         from .engine import make_policy
         L = _lib.lib()
-        self._grids8 = _grids_u8(grids)
-        self.n_maps, self.rows, self.cols = self._grids8.shape
-        _lib.require_device()
-        self.device_index = torch.cuda.current_device() if device is None else int(device)
+        self._map_set = _map_set(grids, device)
+        self._maps = self._map_set.handle
+        self.n_maps, self.rows, self.cols = self._map_set.shape
+        self.device_index = self._map_set.device_index
         self.device = torch.device("cuda", self.device_index)
-        h = C.c_void_p()
-        _lib.check(L.mpp_map_batch_create(self._grids8.ctypes.data_as(C.c_void_p), self.n_maps, self.rows, self.cols,
-                                          self.device_index, C.byref(h)), "mpp_map_batch_create")
-        self._maps = h
         self.allow_diagonal_moves = bool(allow_diagonal_moves)
         self.restrict_corners = bool(restrict_diagonal_near_obstacle_policy)   # astar_strictly_restricts_corners
         self.policy = make_policy(turn_penalty_factor, safety_penalty_factor, min_safe_distance,
@@ -516,19 +672,16 @@ class SearchBatch:
         self.words = (self.n + 31) // 32
         self.heap_cap = int(heap_cap or min(8 * self.n, max(4096, self.n // 4)))        # SearchEngine's sizes
         self.max_cells = int(max_cells or min(self.n, max(4096, 16 * (self.rows + self.cols))))
-        self.max_slots = L.mpp_map_batch_max_slots(h)
+        self.max_slots = L.mpp_map_batch_max_slots(self._maps)
         self.n_slots = int(n_slots or self.max_slots)
         self.counters = torch.zeros(4, dtype=torch.int64, device=self.device)  # expansions, relaxations, ring / heap pushes
         self.launches = 0
         self._scratch, self._scratch_key, self._visited = None, None, None
-        flat = self._grids8.reshape(self.n_maps, -1)                       # first row-major 2 / 3, -1 = none
-        ends = [np.where((flat == v).any(axis=1), (flat == v).argmax(axis=1), -1) for v in (START_NODE_VAL, TARGET_NODE_VAL)]
-        self._start_dev, self._target_dev = (torch.as_tensor(e.astype(np.int32), device=self.device) for e in ends)
+        self._start_dev, self._target_dev = (torch.as_tensor(e.astype(np.int32), device=self.device)
+                                             for e in (self._map_set.start, self._map_set.target))
 
     def close(self):
-        h, self._maps = getattr(self, "_maps", None), None
-        if h:
-            _lib.lib().mpp_map_batch_destroy(h)
+        self._maps = self._map_set = None
 
     def __del__(self):
         try:
@@ -683,10 +836,8 @@ class SearchBatch:
         fitness) -- followed by the value that solver appends to its convergence_curve (g, or None when the path has
         at most one cell)."""
         variant = _search_algorithm(algorithm)[0]
-        flat = self._grids8.reshape(self.n_maps, -1)
-        _check_endpoints(flat, algorithm)
-        src = (flat == START_NODE_VAL).argmax(axis=1)                      # first row-major 2 / 3 (astar.py:17-18)
-        dst = (flat == TARGET_NODE_VAL).argmax(axis=1)
+        src, dst = self._map_set.start, self._map_set.target              # first row-major 2 / 3 (astar.py:17-18)
+        _endpoint_check(algorithm)(src, dst)
         cells, ncell, g, stats = self.search(variant, np.arange(self.n_maps), src, dst)
         cells, ncell, g, stats = cells.cpu().numpy(), ncell.cpu().numpy(), g.cpu().numpy(), stats.cpu().numpy()
         out = []
@@ -710,11 +861,11 @@ def solve_search_batch(grids, algorithm, params, wave=None, group=None, device=N
     convergence-curve value (None for a path of at most one cell)."""
     _search_algorithm(algorithm)
     lo, hi = shard_maps(len(grids), group)
-    for i in range(lo, hi):                                                  # before any device work
-        _check_endpoints(np.asarray(grids[i]).reshape(1, -1), algorithm)
+    maps = _sweep_maps(grids, lo, hi)
+    _endpoint_check(algorithm)(*maps.first_cells())                         # before any search
     out = []
     for idx in _shape_waves(grids, lo, hi, wave):
-        b = SearchBatch(np.stack([np.asarray(grids[i]) for i in idx]), device=device, **params)
+        b = SearchBatch(maps.wave(idx), device=device, **params)
         for i, r in zip(idx, b.solve(algorithm)):
             out.append((i,) + tuple(r))
         b.close()
@@ -741,16 +892,19 @@ class _WaypointBatch:
 
     def __init__(self, grids, num_waypoints, policy, seeds, device, max_cells, heap_cap, n_slots):
         import torch
-        g8 = _grids_u8(grids)
-        self.n_maps, self.rows, self.cols = g8.shape
-        _check_endpoints(g8.reshape(self.n_maps, -1), self._planner)
+        endpoints = _endpoint_check(self._planner)
+
+        def check(start, target):                                            # (host grids: before any device work)
+            endpoints(start, target)
+            if seeds is not None and len(seeds) != len(start):
+                raise ValueError(f"seeds holds {len(seeds)} values for {len(start)} maps")
+        maps = _map_set(grids, device, check)
+        self.n_maps, self.rows, self.cols = maps.shape
         if seeds is None:
             seeds = [int.from_bytes(np.random.bytes(8), "little") for _ in range(self.n_maps)]
-        if len(seeds) != self.n_maps:
-            raise ValueError(f"seeds holds {len(seeds)} values for {self.n_maps} maps")
         self.seeds = [int(s) & (2 ** 64 - 1) for s in seeds]
         self.num_waypoints = int(num_waypoints)
-        self._search = SearchBatch(g8, device=device, max_cells=max_cells, heap_cap=heap_cap, n_slots=n_slots, **policy)
+        self._search = SearchBatch(maps, max_cells=max_cells, heap_cap=heap_cap, n_slots=n_slots, **policy)
         self.device = self._search.device
         self._seeds = torch.from_numpy(np.array(self.seeds, np.uint64).view(np.int64)).to(self.device)
         self.fitness_evaluations = [0] * self.n_maps
@@ -1084,18 +1238,18 @@ def _pop_waves(grids, lo, hi, population, wave=None):
     """Maps lo..hi-1 grouped by shape, `wave` maps per wave at most (None: default_pop_wave of the shape)."""
     out = []
     for idx in _shape_waves(grids, lo, hi):
-        step = wave or default_pop_wave(*np.asarray(grids[idx[0]]).shape, population)
+        step = wave or default_pop_wave(*_map_shape(grids[idx[0]]), population)
         out += [idx[w0:w0 + step] for w0 in range(0, len(idx), step)]
     return out
 
 
 def _pop_sweep(cls, grids, sizes, params, seeds, wave, group, device):
     lo, hi = shard_maps(len(grids), group)
-    for i in range(lo, hi):                                                  # before any device work
-        _check_endpoints(np.asarray(grids[i]).reshape(1, -1), cls._planner)
+    maps = _sweep_maps(grids, lo, hi)
+    _endpoint_check(cls._planner)(*maps.first_cells())                      # before any search
     out = []
     for idx in _pop_waves(grids, lo, hi, sizes[1], wave):
-        b = cls(np.stack([np.asarray(grids[i]) for i in idx]), *sizes,
+        b = cls(maps.wave(idx), *sizes,
                 seeds=None if seeds is None else [seeds[i] for i in idx], device=device, **params)
         for i, r in zip(idx, b.solve()):
             out.append((i,) + tuple(r))
