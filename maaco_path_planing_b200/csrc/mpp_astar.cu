@@ -222,6 +222,22 @@ __global__ void __launch_bounds__(MPP_AS_THREADS, 3) mpp_astar_batch_kernel(Args
     }
 }
 
+int mpp_occ_staging(const void *kernel, MppStaging &st, int device, size_t occ_bytes, bool *stage) {
+    *stage = occ_bytes <= MPP_OCC_STAGE_MAX;
+    if (!*stage) return MPP_OK;
+    if (st.static_bytes < 0) {
+        cudaFuncAttributes fa;
+        MPP_CUDA(cudaFuncGetAttributes(&fa, kernel));
+        st.static_bytes = (int)fa.sharedSizeBytes;
+    }
+    const int dv = device & 63;
+    if ((size_t)st.static_bytes + occ_bytes > 48 * 1024 && (int)occ_bytes > st.raised[dv]) {
+        MPP_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)occ_bytes));
+        st.raised[dv] = (int)occ_bytes;
+    }
+    return MPP_OK;
+}
+
 static int check_scratch(const mpp_map *map, size_t scratch_bytes, int n_slots, int heap_cap) {
     // the searches pack a node as (row << 16 | col) in a signed int (same (r, c) order as the reference's tuples)
     MPP_REQUIRE(map->rows < 32768 && map->cols < 65536, "A*: map %dx%d exceeds the packed-node limit (rows < 32768, cols < 65536)",
@@ -254,14 +270,12 @@ extern "C" int mpp_astar_batch(mpp_map *map, int variant, const int32_t *src_dev
     A.counters = counters_dev;
     const size_t smem = (size_t)map->occ_words * 4;
     const int blocks = (n_slots + MPP_AS_GROUPS - 1) / MPP_AS_GROUPS;
-    if (smem <= 32 * 1024) {
-        mpp_astar_batch_kernel<true, BatchArgs><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
-    } else if (smem <= 40 * 1024) {
-        MPP_CUDA(cudaFuncSetAttribute(mpp_astar_batch_kernel<true, BatchArgs>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        mpp_astar_batch_kernel<true, BatchArgs><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
-    } else {
-        mpp_astar_batch_kernel<false, BatchArgs><<<blocks, MPP_AS_THREADS, 0, s>>>(A);
-    }
+    static MppStaging staging = {-1, {0}};
+    bool stage = false;
+    rc = mpp_occ_staging((const void *)mpp_astar_batch_kernel<true, BatchArgs>, staging, map->device, smem, &stage);
+    if (rc) return rc;
+    if (stage) mpp_astar_batch_kernel<true, BatchArgs><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
+    else mpp_astar_batch_kernel<false, BatchArgs><<<blocks, MPP_AS_THREADS, 0, s>>>(A);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }
@@ -444,15 +458,12 @@ extern "C" int mpp_waypoint_fitness(mpp_map *map, const int32_t *waypoints_dev, 
     A.order = order_dev;
     const size_t smem = (size_t)map->occ_words * 4;
     const int blocks = (n_slots + MPP_AS_GROUPS - 1) / MPP_AS_GROUPS;
-    if (smem <= 32 * 1024) {
-        mpp_waypoint_fitness_kernel<true, ChainArgs><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
-    } else if (smem <= 40 * 1024) {
-        MPP_CUDA(cudaFuncSetAttribute(mpp_waypoint_fitness_kernel<true, ChainArgs>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)smem));
-        mpp_waypoint_fitness_kernel<true, ChainArgs><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
-    } else {
-        mpp_waypoint_fitness_kernel<false, ChainArgs><<<blocks, MPP_AS_THREADS, 0, s>>>(A);
-    }
+    static MppStaging staging = {-1, {0}};
+    bool stage = false;
+    rc = mpp_occ_staging((const void *)mpp_waypoint_fitness_kernel<true, ChainArgs>, staging, map->device, smem, &stage);
+    if (rc) return rc;
+    if (stage) mpp_waypoint_fitness_kernel<true, ChainArgs><<<blocks, MPP_AS_THREADS, smem, s>>>(A);
+    else mpp_waypoint_fitness_kernel<false, ChainArgs><<<blocks, MPP_AS_THREADS, 0, s>>>(A);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }

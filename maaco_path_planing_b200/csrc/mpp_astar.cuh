@@ -91,6 +91,20 @@ struct AStarSlot {
     int heap_cap;
 };
 
+// Occupancy staging of the connector, fitness and MPA kernels (the <true> instantiations): a map of up to
+// MPP_OCC_STAGE_MAX bytes of packed occupancy is copied into dynamic shared memory by every block, a larger one is read
+// through L2 by the <false> instantiation.  The kernels also declare ~16 KB of static shared memory (the bucket
+// counts), so a staged launch needs the kernel's dynamic limit raised as soon as static + dynamic exceeds the default
+// 48 KB -- a map of exactly 32 KB (510x510) already does.  One MppStaging per staged kernel caches its static size and,
+// per device, the limit raised so far (the attribute only grows; the call is slow).
+#define MPP_OCC_STAGE_MAX (40 * 1024)
+struct MppStaging {
+    int static_bytes;       // -1: not read yet
+    int raised[64];         // dynamic limit set on device d & 63 (0: the default)
+};
+// *stage = whether `kernel` (a <true> instantiation) stages `occ_bytes`; if it does, the launch may use that much.
+int mpp_occ_staging(const void *kernel, MppStaging &st, int device, size_t occ_bytes, bool *stage);
+
 __host__ __device__ __forceinline__ size_t astar_align256(size_t b) { return (b + 255) & ~(size_t)255; }
 __host__ __device__ __forceinline__ size_t astar_slot_bytes(int rc, int heap_cap) {
     size_t b = 256;                                                    // header

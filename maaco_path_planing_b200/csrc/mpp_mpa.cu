@@ -298,17 +298,15 @@ __global__ void __launch_bounds__(MPP_MPA_THREADS, 3) mpp_mpa_iteration_kernel(M
     }
 }
 
-static int mpa_launch(MpaArgs &A, int n_maps, size_t occ_bytes, cudaStream_t s) {
+static int mpa_launch(MpaArgs &A, int n_maps, int device, size_t occ_bytes, cudaStream_t s) {
     const int blocks = (A.warps_per_map + MPP_MPA_GROUPS - 1) / MPP_MPA_GROUPS;
     const dim3 grid(blocks, n_maps);
-    if (occ_bytes <= 32 * 1024) {
-        mpp_mpa_iteration_kernel<true><<<grid, MPP_MPA_THREADS, occ_bytes, s>>>(A);
-    } else if (occ_bytes <= 40 * 1024) {
-        MPP_CUDA(cudaFuncSetAttribute(mpp_mpa_iteration_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)occ_bytes));
-        mpp_mpa_iteration_kernel<true><<<grid, MPP_MPA_THREADS, occ_bytes, s>>>(A);
-    } else {
-        mpp_mpa_iteration_kernel<false><<<grid, MPP_MPA_THREADS, 0, s>>>(A);
-    }
+    static MppStaging staging = {-1, {0}};
+    bool stage = false;
+    const int rc = mpp_occ_staging((const void *)mpp_mpa_iteration_kernel<true>, staging, device, occ_bytes, &stage);
+    if (rc) return rc;
+    if (stage) mpp_mpa_iteration_kernel<true><<<grid, MPP_MPA_THREADS, occ_bytes, s>>>(A);
+    else mpp_mpa_iteration_kernel<false><<<grid, MPP_MPA_THREADS, 0, s>>>(A);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }
@@ -350,7 +348,7 @@ extern "C" int mpp_mpa_iteration(mpp_map *map, const mpp_policy *policy, int n_p
     A.scratch = (char *)scratch_dev; A.n_slots = n_slots; A.heap_cap = heap_cap; A.status = status_dev;
     A.counters = counters_dev;
     A.meta = nullptr; A.seeds = nullptr; A.order = nullptr; A.queue = (unsigned int *)scratch_dev; A.warps_per_map = n_slots;
-    return mpa_launch(A, 1, (size_t)map->occ_words * 4, s);
+    return mpa_launch(A, 1, map->device, (size_t)map->occ_words * 4, s);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -397,7 +395,7 @@ extern "C" int mpp_mpa_iteration_batch(const mpp_map_batch *maps, const mpp_poli
     A.scratch = (char *)scratch_dev; A.n_slots = warps_per_map * maps->n_maps; A.heap_cap = heap_cap; A.status = status_dev;
     A.counters = counters_dev;
     A.meta = maps->meta_dev; A.seeds = seeds_dev; A.order = order_dev; A.queue = queue_dev; A.warps_per_map = warps_per_map;
-    return mpa_launch(A, maps->n_maps, (size_t)maps->occ_words * 4, s);
+    return mpa_launch(A, maps->n_maps, maps->device, (size_t)maps->occ_words * 4, s);
 }
 
 // The initial population of every map (MPA.py:231-245): N identical runs of the private A* start -> target are ONE
