@@ -196,6 +196,8 @@ int mpp_maaco_tours_p2p(const mpp_map_batch *maps, const mpp_colony *colony, int
                         int n_ants, int ant_offset, int n_ants_total, int ants_per_warp,
                         uint32_t *const *slabs_peers, uint32_t *const *touched_peers,
                         mpp_ant_result *const *result_peers, int n_peers, int tile_rows_per_rank, void *stream);
+/* the largest n_peers mpp_maaco_tours_p2p takes: a group of more ranks exchanges through mpp_maaco_xpack / _xunpack */
+int mpp_maaco_max_peers(void);
 
 /* replaces the order-dependent best tracking MAACO.py:343-358 for one iteration over all n_ants_total results of each
  * map (global ant order) and prepares deposit / okbits (:307-308).  Updates state and appends to log.  colony->moves

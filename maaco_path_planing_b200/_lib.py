@@ -84,6 +84,7 @@ _SIGS = {
     "mpp_maaco_pass": (c_int, [c_void_p, C.POINTER(Colony), C.POINTER(MaacoParams), c_int, c_int, c_int, c_void_p]),
     "mpp_maaco_pass_host": (c_int, [c_void_p, C.POINTER(Colony), C.POINTER(MaacoParams), c_int, c_int, c_int, c_void_p,
                                     c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
+    "mpp_maaco_max_peers": (c_int, []),
     "mpp_maaco_xhdr_bytes": (C.c_longlong, [c_int]),
     "mpp_maaco_xpack": (c_int, [c_void_p, C.POINTER(Colony), c_int, c_int, c_int, c_void_p, c_void_p, C.c_longlong,
                                 c_void_p, c_int, c_int, c_void_p]),

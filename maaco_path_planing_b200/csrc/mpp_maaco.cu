@@ -184,6 +184,7 @@ extern "C" long long mpp_maaco_touched_words(int tile_rows, int cols, int n_ants
 // `apw` lanes of each warp own an ant: fewer ants per warp = more warps to spread over the SMs.
 // ---------------------------------------------------------------------------------------------
 #define MPP_MAX_PEERS 16
+extern "C" int mpp_maaco_max_peers(void) { return MPP_MAX_PEERS; }
 struct TourArgs {
     const MppMapMeta *meta;      // [n_maps]
     const uint32_t *rank;        // [n_maps][rank_stride] ranking buffers (mpp_maaco_rank), layout: rank_layout()

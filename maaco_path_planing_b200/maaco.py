@@ -10,7 +10,8 @@ Keyword-only additions (none changes a result; every combination is bit-identica
   device, group   CUDA device index; torch.distributed group to shard the colony over
   ants_per_warp   form of the tour kernel (one thread per ant): 0 = chosen from the colony size, or 1, 2, 4, ..., 32
   max_cells       capacity of the per-ant tour buffers (default 8*(rows+cols); the solve repeats itself with rows*cols
-                  if the best path did not fit)
+                  if the best path did not fit; a colony sharded over the all-gather exchange grows them instead when
+                  any tour does not fit)
 """
 from __future__ import annotations
 
@@ -27,10 +28,6 @@ from .dist import padded_tile_rows
 from .gridmap import GridMap, START_NODE_VAL, TARGET_NODE_VAL
 
 INF = float("inf")
-
-
-class _PathOverflow(Exception):
-    """a tour did not fit max_cells (internal: solve_path_planning repeats the solve with full capacity)"""
 
 
 def _round64k(x):
@@ -112,12 +109,12 @@ class MAACO:
         if max_cells is None:
             max_cells = default_max_cells(R, Cc)
         self.max_cells = int(max_cells)
-        self.max_cells_hint = self.max_cells
+        self.max_cells_hint = self.max_cells                          # what was asked (max_cells can grow, see _rewind)
         dev = self.device
         f64, i32, i64, u8 = torch.float64, torch.int32, torch.int64, torch.uint8
         nl = self.n_local
         self._p2p = None
-        if self.world > 1 and os.environ.get("MPP_P2P", "1") != "0":
+        if 1 < self.world <= L.mpp_maaco_max_peers() and os.environ.get("MPP_P2P", "1") != "0":
             self._p2p = self._setup_peer_memory(npad)                # NVLink peer memory for the two exchanges (or None)
         if self._p2p is not None:
             self._tau = self._p2p["tau"]
@@ -364,23 +361,33 @@ class MAACO:
             vals = self._ring[slot].tolist()
             totals, latch = vals[:self.world], vals[self.world]
             if latch != 0:
-                self._rewind(latch)
+                self._rewind(latch, totals)
                 continue
             self._enqueued.pop(0)
             self._cap = min(self._cap_max, _round64k(int(1.5 * max(totals)) + 4096))
 
-    def _rewind(self, first_bad):
-        """The exchange of pass `first_bad` did not fit: since then every kernel was a no-op (device latch), so the colony
-        is exactly as pass first_bad - 1 left it.  Make room and enqueue those passes again."""
+    def _rewind(self, first_bad, totals):
+        """The exchange of pass `first_bad` did not fit: a rank's move codes outgrew the capacity of the exchange (`totals`:
+        every rank's code bytes in that pass, from its ring slot) or a tour outgrew max_cells (its codes were cut at the
+        source, so no rank could replay it).  Since then every kernel was a no-op (device latch), so the colony is exactly
+        as pass first_bad - 1 left it.  Make room and enqueue those passes again."""
         import torch
+        import torch.distributed as dist
         torch.cuda.synchronize(self.device)
         redo = [it for it, _ in self._enqueued if it >= first_bad]
         cap_bad = dict(self._enqueued)[first_bad]
-        seg = self._xhdr + cap_bad
-        totals = self._xbuf_all.view(torch.int32).as_strided((self.world,), (seg // 4,), (16 * self.n_local) // 4).tolist()
-        if max(totals) <= cap_bad:                                   # not the capacity: a tour outgrew max_cells
-            raise _PathOverflow()
-        self._cap_max = max(self._cap_max, _round64k(2 * max(totals)))
+        # the longest tour of the bad pass: this rank's own records are still the ones its tour kernel wrote then (the
+        # unpack of the other ranks' records may have stopped at the latch)
+        own = self._result.view(torch.int32).view(self.num_ants, 4)[self.ant_offset:self.ant_offset + self.n_local, 2]
+        longest = (own.max() - 1).reshape(1)
+        dist.all_reduce(longest, op=dist.ReduceOp.MAX, group=self.group)
+        longest = int(longest.item())
+        if max(totals) <= cap_bad and longest <= self.max_cells:
+            raise _lib.MppError(f"sharded colony: the exchange of pass {first_bad} was stopped without an overflow")
+        if longest > self.max_cells:
+            self._grow_moves(min(self.rows * self.cols, max(longest, 2 * self.max_cells)))
+        if max(totals) > cap_bad:
+            self._cap_max = max(self._cap_max, _round64k(2 * max(totals)))
         self._cap = self._cap_max
         if self._xbuf_local.numel() < self._xhdr + self._cap_max:
             self._xbuf_local = torch.zeros(self._xhdr + self._cap_max, dtype=torch.uint8, device=self.device)
@@ -393,6 +400,17 @@ class MAACO:
         self.exchange_rewinds = getattr(self, "exchange_rewinds", 0) + 1
         for it in redo:
             self._enqueue_pass(it)
+
+    def _grow_moves(self, max_cells):
+        """Per-ant move buffers (and the best path) of `max_cells` moves; the best path found so far is kept."""
+        import torch
+        best = self._best_cells
+        self.max_cells = int(max_cells)
+        self._moves = torch.zeros(self.n_local * self.max_cells, dtype=torch.uint8, device=self.device)
+        self._best_cells = torch.zeros(self.max_cells + 1, dtype=torch.int32, device=self.device)
+        self._best_cells[:best.numel()].copy_(best)
+        self._colony.moves, self._colony.best_cells = self._moves.data_ptr(), self._best_cells.data_ptr()
+        self._colony.max_cells = self.max_cells
 
     def _settle(self):
         """Block until everything enqueued has really happened (a sharded colony may have to repeat passes)."""
@@ -408,19 +426,16 @@ class MAACO:
     def solve_path_planning(self):
         import torch
         K = self.num_iterations
-        overflow = False
-        try:
-            for it in range(self._iter_done + 1, K + 1):
-                self._enqueue_iteration(it)
-            self._settle()
-        except _PathOverflow:
-            overflow = True
+        for it in range(self._iter_done + 1, K + 1):
+            self._enqueue_iteration(it)
+        self._settle()
         self._iter_done = K
         st = self._read_state()
-        overflow = overflow or st.best_n_cells - 1 > self.max_cells
-        if overflow:
+        # (an explicit max_cells is a limit on the best path even where the sharded exchange grew the buffers)
+        limit = self.max_cells if self._auto_cells else self.max_cells_hint
+        if st.best_n_cells - 1 > limit:
             if not self._auto_cells or self.max_cells >= self.rows * self.cols:
-                raise _lib.MppError(f"a tour outgrew max_cells={self.max_cells} (best path: {st.best_n_cells} cells); "
+                raise _lib.MppError(f"a tour outgrew max_cells={limit} (best path: {st.best_n_cells} cells); "
                                     "re-run with a larger max_cells")
             # the solve is a deterministic function of (grid, parameters, seed): repeat it with full path capacity
             again = MAACO(max_cells=self.rows * self.cols, **self._ctor)
@@ -492,7 +507,8 @@ class MAACO:
         return st
 
     def last_results(self):
-        """(n_cells, length, turns) of every ant of the colony in the last pass (numpy)."""
+        """(n_cells, length, turns) of every ant of the colony in the last pass (numpy).  A colony sharded over peer memory
+        receives the other ranks' records from their tour kernels: read them before any rank enqueues the next pass."""
         self._settle()
         raw = self._result.cpu().numpy()
         rec = raw.view(np.dtype([("length", "<f8"), ("n_cells", "<i4"), ("turns", "<i4")])).reshape(-1)
