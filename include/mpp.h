@@ -320,6 +320,29 @@ int mpp_astar_batch_maps(mpp_map_batch *maps, int variant, const int32_t *map_de
                          int n_slots, int heap_cap, unsigned long long *counters_dev, const int32_t *order_dev,
                          void *stream);
 
+/* ---- exact Dijkstra distance fields (dijkstra.py) -----------------------------------------------------------------
+ * replaces DijkstraSolver.solve's search (dijkstra.py:32-97, with get_valid_neighbors helper.py:18-53) when one source
+ * serves many targets, or a whole map's costs are wanted: ONE field per map gives every target's popped g and path.
+ * mpp_dijkstra_fields: for every map k of the batch (a single map: mpp_map_as_batch), the complete field from cell
+ *   src_dev[k]: g_dev [n_maps][rows*cols] = the g with which dijkstra.py pops each cell (+inf: obstacle or unreachable),
+ *   parent_dev [n_maps][rows*cols] = the move parent -> cell in the move order of helper.py:30-36 ((0,1), (0,-1), (1,0),
+ *   (-1,0), (1,1), (1,-1), (-1,1), (-1,-1)), 0xFF = none (source, obstacle, unreachable).  Both are bit for bit what the
+ *   reference's search computes for that cell as its target: g*(cell) is the least fixed point of the relaxations
+ *   (fp64 rounding is monotone and every step weighs >= 1), the parent the first strict improvement in (g, r, c) pop
+ *   order.  A source outside the map or on an obstacle gives an all-inf field.  scratch: mpp_dijkstra_field_scratch_bytes
+ *   bytes, no initialisation needed.  One thread-block cluster per map (up to 16 CTAs when the batch has few maps).
+ * mpp_dijkstra_field_paths: query i reads the path from the source of map map_dev[i]'s field to cell dst_dev[i]
+ *   (dijkstra.py:64-70): cells_dev n x max_cells, n_cells_dev[i] = path length (0 = unreachable / obstacle / endpoint or
+ *   map index outside the batch, > max_cells = truncated), g_out_dev[i] = g*(dst) (+inf without a path; nullable), and
+ *   with stats_policy the statistics into stats_dev as mpp_astar_batch_maps computes them.  A target equal to the source
+ *   gives [src] with g = 0.  One lane group (warp) per query. */
+size_t mpp_dijkstra_field_scratch_bytes(const mpp_map_batch *maps);
+int mpp_dijkstra_fields(const mpp_map_batch *maps, const int32_t *src_dev, int allow_diagonal, int restrict_corner,
+                        double *g_dev, uint8_t *parent_dev, void *scratch_dev, size_t scratch_bytes, void *stream);
+int mpp_dijkstra_field_paths(mpp_map_batch *maps, const double *g_dev, const uint8_t *parent_dev, const int32_t *map_dev,
+                             const int32_t *dst_dev, int n, const mpp_policy *stats_policy, int32_t *cells_dev,
+                             int max_cells, int32_t *n_cells_dev, double *g_out_dev, double *stats_dev, void *stream);
+
 /* replaces PSOSolver._reconstruct_path_from_position (pso.py:56-94, after rounding/clamping) /
  * GASolver._reconstruct_path_from_chromosome (ga_solver.py:58-93) followed by
  * BasePathfinder._calculate_stats_for_path (helper.py:138-147) for a whole population: one lane group (a warp)

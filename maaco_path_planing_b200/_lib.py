@@ -104,6 +104,10 @@ _SIGS = {
     "mpp_waypoint_fitness": (c_int, [c_void_p, c_void_p, c_int, c_int, C.POINTER(Policy), c_void_p, c_int, c_void_p,
                                      c_void_p, c_void_p, c_void_p, C.c_size_t, c_int, c_int, c_void_p, c_void_p,
                                      c_void_p]),
+    "mpp_dijkstra_field_scratch_bytes": (C.c_size_t, [c_void_p]),
+    "mpp_dijkstra_fields": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, C.c_size_t, c_void_p]),
+    "mpp_dijkstra_field_paths": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, C.POINTER(Policy),
+                                         c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "mpp_pso_update": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_double,
                                c_double, c_double, c_double, c_u64, c_int, c_void_p, c_void_p]),
     "mpp_pso_round": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),

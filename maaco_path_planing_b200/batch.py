@@ -649,7 +649,8 @@ def _shape_waves(grids, lo, hi, wave=None):
 class SearchBatch:
     """M same-shape maps for the deterministic baselines: `search` runs any number of A* / Dijkstra queries, each on
     its own map with its own endpoints and avoid set, in one launch with the statistics of every path fused in
-    (mpp_astar_batch_maps); `solve` is AStarSolver(grid).solve() / DijkstraSolver(grid).solve() for every map at once.
+    (mpp_astar_batch_maps); `solve` is AStarSolver(grid).solve() / DijkstraSolver(grid).solve() for every map at once;
+    `distance_fields` / `field_paths` give exact Dijkstra fields and the paths read from them (field.py).
     Same parameters and defaults as AStarSolver (astar.py:11-14); start and target may differ from map to map."""
 
     def __init__(self, grids, turn_penalty_factor=0.1, safety_penalty_factor=0.05, min_safe_distance=1.5,
@@ -829,6 +830,31 @@ class SearchBatch:
                 break
             idx = idx[bad]
         return cells, ncell, g, stats
+
+    def _fields(self, src):
+        from .field import dijkstra_fields
+        s = self._start_dev if src is None else self._i32(src)
+        if s.shape != (self.n_maps,):
+            raise ValueError(f"src must hold one cell per map ({self.n_maps}), not shape {tuple(s.shape)}")
+        return dijkstra_fields(self, self._maps, (self.n_maps, self.rows, self.cols), s, self.allow_diagonal_moves,
+                               self.restrict_corners)
+
+    def distance_fields(self, src=None):
+        """[M, rows, cols] float64 CUDA tensor: map k's exact Dijkstra distance field from cell src[k] (None: every map's
+        own start) -- at each cell the g that search(2, ...) from src[k] to that cell returns (+inf at obstacles and
+        unreachable cells; all +inf when the source is outside the map or an obstacle)."""
+        return self._fields(src)[0]
+
+    def field_paths(self, map_index, dst, src=None):
+        """What search(2, map_index, src[map_index], dst) returns -- (cells, n_cells, g, stats) device tensors, bit for
+        bit -- from one distance field per map (from src[k], None: every map's own start) and one path-reading launch.
+        A truncated path grows max_cells and repeats only the truncated queries."""
+        from .field import field_paths
+        mi, dst = self._i32(map_index), self._i32(dst)
+        if not (mi.dim() == dst.dim() == 1) or mi.numel() != dst.numel():
+            raise ValueError(f"map_index and dst must be 1-D and of one length, not {tuple(mi.shape)}, {tuple(dst.shape)}")
+        g, parent = self._fields(src)
+        return field_paths(self, self._maps, g, parent, mi, dst, self.policy)
 
     def solve(self, algorithm="astar"):
         """One start -> target query per map.  Returns, per map, what AStarSolver(grid, ...).solve() (algorithm
