@@ -163,6 +163,21 @@ long long mpp_maaco_touched_words(int tile_rows, int cols, int n_ants);
 int mpp_maaco_tables(const mpp_map_batch *maps, const mpp_maaco_params *p, double *tau0_dev, long long tau_stride,
                      double *E01_dev, double *dist_t_dev, void *stream);
 
+/* The tables of a batch whose maps have their own start and target (colony->E01_stride = 2*rows*cols):
+ * mpp_maaco_e01_host: replaces the per-candidate heuristic eta'**beta (MAACO.py:197-210, :238) for n endpoint pairs
+ *   (start[k], target[k]) of a rows x cols map: out [n][2*rows*cols], interleaved by turn flag, table k bit for bit
+ *   what mpp_maaco_tables writes for a batch with those endpoints (the same host code, libm exp/pow).  Pure host code:
+ *   touches no device, may run on any thread.  threads = 0: at most 16 (one below 65536 cells in all); the work is
+ *   spread over maps and rows.  A cell outside 0..rows*cols-1 or n < 0 is an MPP_EINVAL.  Synchronous.
+ * mpp_maaco_tau0_maps: replaces MAACO._initialize_pheromones_maaco (MAACO.py:58-84) for every map of the batch from
+ *   that map's own start and target, obstacles at 1e-9 (:62-63): one kernel (grid.y = map) whose values are bit for bit
+ *   mpp_maaco_tables' (integer squared distances, correctly rounded sqrt and division, no FMA).  tau0_dev:
+ *   [n_maps][tau_stride].  Asynchronous on `stream`.  No dist_to_target table is produced. */
+int mpp_maaco_e01_host(int rows, int cols, int n, const int32_t *start, const int32_t *target, const mpp_maaco_params *p,
+                       double *out, int threads);
+int mpp_maaco_tau0_maps(const mpp_map_batch *maps, const mpp_maaco_params *p, double *tau0_dev, long long tau_stride,
+                        void *stream);
+
 /* replaces MAACO._calculate_adaptive_q0 (MAACO.py:212-226); pure host function */
 double mpp_maaco_q0(int num_iterations, int iteration, double q0_initial);
 

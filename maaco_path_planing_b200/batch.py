@@ -4,9 +4,12 @@ data-path collective, and on each GPU a WAVE of same-shape maps is one mpp_map_b
 whole wave is four kernel launches (ranking, tours, best tracking, pheromone update with grid.y = map), enqueued
 without host synchronisation.  Results are identical to solving each map alone with the same seed.
 
-The eta'**beta / dist-to-target tables depend only on (shape, start, target, parameters), so a wave shares ONE
-table computed on the host with libm (bit-identical to the reference), and tau0 of each map is that shared table
-with the map's obstacles masked on the device (mpp_maaco_tables).
+The eta'**beta / dist-to-target tables depend only on (shape, start, target, parameters), so by default a MAACO wave
+holds maps of one (start, target) pair and shares ONE table computed on the host with libm (bit-identical to the
+reference), and tau0 of each map is that shared table with the map's obstacles masked on the device
+(mpp_maaco_tables).  With per_map_endpoints=True a wave may mix endpoints: it then holds one eta'**beta table per map,
+still computed on the host with libm (mpp_maaco_e01_host; solve_maaco_batch builds the next wave's tables on a worker
+thread while the GPU runs the current one), and tau0 is computed per map on the device (mpp_maaco_tau0_maps).
 
 Every batch class takes `grids` either on the host ([M, rows, cols] cell codes, anything np.asarray takes) or as an
 [M, rows, cols] CUDA tensor of bool, uint8, int8, int16, int32 or int64 cells; every sweep also takes a sequence of 2-D
@@ -161,15 +164,43 @@ def _all_endpoints(no_start, no_target):
     return check
 
 
+def _maaco_params(num_iterations, alpha, beta, rho, Q, a_turn_coef, wh_max, wh_min, k_h_adaptive, q0_initial,
+                  C0_initial_pheromone=0.1):
+    """mpp_maaco_params of MAACO's parameters (MAACO.py:11-14)."""
+    return _lib.MaacoParams(alpha, beta, rho, Q, a_turn_coef, wh_max, wh_min, k_h_adaptive, q0_initial,
+                            C0_initial_pheromone, num_iterations)
+
+
+def _e01_host(rows, cols, start, target, params, out, threads=0):
+    """eta'**beta tables of the endpoint pairs (start[k], target[k]) of a rows x cols map into `out` (a contiguous
+    float64 host tensor or array of at least len(start) * 2 * rows * cols values): mpp_maaco_e01_host."""
+    s, t = np.ascontiguousarray(start, np.int32), np.ascontiguousarray(target, np.int32)
+    ptr = out.data_ptr() if hasattr(out, "data_ptr") else out.ctypes.data
+    _lib.check(_lib.lib().mpp_maaco_e01_host(rows, cols, len(s), s.ctypes.data_as(C.c_void_p),
+                                             t.ctypes.data_as(C.c_void_p), C.byref(params), C.c_void_p(ptr), threads),
+               "mpp_maaco_e01_host")
+    return out
+
+
 class MAACOBatch:
-    """M same-shape maps that share start and target, one colony of `num_ants` ants per map, solved together.
-    Same parameters as MAACO (MAACO.py:11-14); `seeds` = one Philox seed per map.  `max_cells` works as in MAACO: left
-    at its default, solve() repeats the whole wave with rows*cols cells of path capacity when a best path did not fit;
-    given explicitly, such a wave raises MppError."""
+    """M same-shape maps, one colony of `num_ants` ants per map, solved together.  Same parameters as MAACO
+    (MAACO.py:11-14); `seeds` = one Philox seed per map.  `max_cells` works as in MAACO: left at its default, solve()
+    repeats the whole wave with rows*cols cells of path capacity when a best path did not fit; given explicitly, such a
+    wave raises MppError.
+
+    By default the maps must share start and target: they then share one table built once (mpp_maaco_tables), and
+    maps with other endpoints raise MppError.  With per_map_endpoints=True each map may have its own start and target:
+    the wave then holds one eta'**beta table per map ([M, 2*rows*cols] doubles, 16 B per cell per map, built on the host
+    with mpp_maaco_e01_host and copied without blocking from pinned memory), and tau0 is computed on the device from each
+    map's own endpoints (mpp_maaco_tau0_maps).  A wave whose maps all share their endpoints takes the shared table
+    either way.  Results are those of solo MAACO with the same seed in both modes."""
 
     def __init__(self, grids, num_ants, num_iterations, alpha, beta, rho, Q, a_turn_coef, wh_max, wh_min, k_h_adaptive,
                  q0_initial, C0_initial_pheromone=0.1, *, seeds=None, device=None, max_cells=None, ants_per_warp=0,
-                 reuse=None):
+                 reuse=None, per_map_endpoints=False, _e01=None):
+        # _e01 (solve_maaco_batch and the max_cells repeat): this wave's per-map tables, already built -- a float64
+        # host tensor of at least M * 2 * rows * cols values that the caller keeps unchanged until the copy enqueued here
+        # has run, or an [M, 2 * rows * cols] CUDA tensor on the wave's device, used as it is
         import torch
         L = _lib.lib()
         self._map_set = _map_set(grids, device, _all_endpoints("MAACO: Start node not found.",        # MAACO.py:35-36
@@ -180,9 +211,13 @@ class MAACOBatch:
         self.device = torch.device("cuda", self.device_index)
         self.num_ants, self.num_iterations = int(num_ants), int(num_iterations)
         self.alpha, self.rho, self.Q = alpha, rho, Q
-        self._params = _lib.MaacoParams(alpha, beta, rho, Q, a_turn_coef, wh_max, wh_min, k_h_adaptive, q0_initial,
-                                        C0_initial_pheromone, num_iterations)
+        self._params = _maaco_params(num_iterations, alpha, beta, rho, Q, a_turn_coef, wh_max, wh_min, k_h_adaptive,
+                                     q0_initial, C0_initial_pheromone)
         M, R, Cc, N = self.n_maps, self.rows, self.cols, self.num_ants
+        start, target = self._map_set.start, self._map_set.target
+        # one table per map only where the endpoints differ: a wave that shares them keeps the shared table
+        self.per_map_tables = bool(per_map_endpoints) and M > 0 and not (
+            (start == start[0]).all() and (target == target[0]).all())
         n = R * Cc
         TR = (R + 31) // 32
         self._auto_cells = max_cells is None
@@ -196,11 +231,11 @@ class MAACOBatch:
         self._ctor = dict(num_ants=num_ants, num_iterations=num_iterations, alpha=alpha, beta=beta, rho=rho, Q=Q,
                           a_turn_coef=a_turn_coef, wh_max=wh_max, wh_min=wh_min, k_h_adaptive=k_h_adaptive,
                           q0_initial=q0_initial, C0_initial_pheromone=C0_initial_pheromone, seeds=self.seeds,
-                          ants_per_warp=ants_per_warp)
+                          ants_per_warp=ants_per_warp, per_map_endpoints=per_map_endpoints)
         dev = self.device
         f64, i32, i64, u8 = torch.float64, torch.int32, torch.int64, torch.uint8
         K = max(1, self.num_iterations)
-        key = (M, R, Cc, N, self.max_cells, K, self.device_index)
+        key = (M, R, Cc, N, self.max_cells, K, self.device_index, self.per_map_tables)   # (the E01 layout)
         if reuse is not None and getattr(reuse, "_key", None) == key:
             # the previous wave's device buffers (same shapes): nothing to allocate, only `touched` / counters to clear
             for name in ("_tau", "_E01", "_dist_t", "_rank", "_slabs", "_touched", "_moves", "_result", "_deposit", "_okbits",
@@ -210,8 +245,13 @@ class MAACOBatch:
             self._steps.zero_()
         else:
             self._tau = torch.empty((M, n), dtype=f64, device=dev)
-            self._E01 = torch.empty(2 * n, dtype=f64, device=dev)             # shared by the whole wave
-            self._dist_t = torch.empty(n, dtype=f64, device=dev)
+            if self.per_map_tables:
+                self._E01 = None if isinstance(_e01, torch.Tensor) and _e01.is_cuda else \
+                    torch.empty((M, 2 * n), dtype=f64, device=dev)
+                self._dist_t = None                                           # nothing in the batch reads it
+            else:
+                self._E01 = torch.empty(2 * n, dtype=f64, device=dev)         # shared by the whole wave
+                self._dist_t = torch.empty(n, dtype=f64, device=dev)
             self._rank = torch.empty(M * L.mpp_maaco_rank_words(R, Cc), dtype=i32, device=dev)
             self._slabs = torch.empty(M * L.mpp_maaco_slab_words(TR, Cc, N), dtype=i32, device=dev)
             self._touched = torch.zeros(M * L.mpp_maaco_touched_words(TR, Cc, N), dtype=i32, device=dev)
@@ -224,13 +264,28 @@ class MAACOBatch:
             self._log = torch.zeros((M, K, 4), dtype=f64, device=dev)
         self._key = key
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        _lib.check(L.mpp_maaco_tables(self._maps, C.byref(self._params), _lib.ptr(self._tau), n, _lib.ptr(self._E01),
-                                      _lib.ptr(self._dist_t), stream), "mpp_maaco_tables")
+        if self.per_map_tables:
+            if isinstance(_e01, torch.Tensor) and _e01.is_cuda:
+                if tuple(_e01.shape) != (M, 2 * n) or _e01.device != dev or _e01.dtype != f64:
+                    raise ValueError(f"_e01 must be a float64 [{M}, {2 * n}] tensor on {dev}")
+                self._E01 = _e01
+            else:
+                if _e01 is None:
+                    _e01 = _e01_host(R, Cc, start, target, self._params,
+                                     torch.empty(M * 2 * n, dtype=f64, pin_memory=True))
+                # (a pinned tensor of torch's host allocator is not reused before this copy has run)
+                self._E01.view(-1).copy_(_e01.view(-1)[:M * 2 * n], non_blocking=True)
+            _lib.check(L.mpp_maaco_tau0_maps(self._maps, C.byref(self._params), _lib.ptr(self._tau), n, stream),
+                       "mpp_maaco_tau0_maps")
+        else:
+            _lib.check(L.mpp_maaco_tables(self._maps, C.byref(self._params), _lib.ptr(self._tau), n,
+                                          _lib.ptr(self._E01), _lib.ptr(self._dist_t), stream), "mpp_maaco_tables")
         self._seeds = torch.from_numpy(np.array(self.seeds, np.uint64).view(np.int64)).to(dev)
         st = bytes(_lib.MaacoState(INF, -1, 0, 0, -1, INF, -1, -1))
         self._state = torch.frombuffer(bytearray(st * M), dtype=u8).to(dev)
         self._colony = _lib.Colony(
-            self._tau.data_ptr(), n, self._E01.data_ptr(), 0, self._rank.data_ptr(), self._slabs.data_ptr(),
+            self._tau.data_ptr(), n, self._E01.data_ptr(), 2 * n if self.per_map_tables else 0, self._rank.data_ptr(),
+            self._slabs.data_ptr(),
             self._touched.data_ptr(), self._moves.data_ptr(), self.max_cells, K, self._result.data_ptr(),
             self._deposit.data_ptr(), self._okbits.data_ptr(), self._state.data_ptr(), self._best_cells.data_ptr(),
             self._log.data_ptr(), self._steps.data_ptr(), self._seeds.data_ptr(), None)
@@ -287,8 +342,9 @@ class MAACOBatch:
                 raise _lib.MppError(f"a tour outgrew max_cells={self.max_cells} (best path: "
                                     f"{int(st['best_n_cells'].max())} cells); re-run with a larger max_cells")
             # the solve is a deterministic function of (maps, parameters, seeds): repeat the wave with full path capacity
-            # on the same map batch (not on the caller's grids, which may have changed since)
-            again = type(self)(self._map_set, max_cells=self.rows * self.cols, **self._ctor)
+            # on the same map batch (not on the caller's grids, which may have changed since) and per-map tables
+            again = type(self)(self._map_set, max_cells=self.rows * self.cols,
+                               _e01=self._E01 if self.per_map_tables else None, **self._ctor)
             again.kernel_launches = self.kernel_launches
             self.__dict__.update(again.__dict__)
             return self.solve()
@@ -382,15 +438,24 @@ def _waves(keys, wave):
 
 
 def solve_maaco_batch(grids, num_ants, num_iterations, params, seeds=None, wave=256, group=None, device=None,
-                      max_cells=None):
+                      max_cells=None, per_map_endpoints=False):
     """Run MAACO on every grid of `grids` (this rank's shard when `group` is given), `wave` maps per launch.  `grids`:
     host maps, a [n_maps, rows, cols] CUDA tensor or a sequence of 2-D CUDA tensors (which never leave the GPU).
+
+    By default a wave holds maps of one shape and one (start, target) pair, so a sweep whose maps have their own
+    endpoints runs one small wave per pair.  With per_map_endpoints=True waves are formed by shape only, in index order
+    (MAACOBatch(per_map_endpoints=True)); one worker thread builds the next wave's eta'**beta tables on the host while
+    the GPU runs the current wave, so the host cost is hidden as long as it stays below a wave's GPU time.  A map
+    without a start or target then raises before any wave runs.
 
     Returns a list of (map_index, path, length, turns, convergence_curve) for the maps of this rank; results
     are identical to solving each map alone (same seeds => same Philox streams)."""
     lo, hi = shard_maps(len(grids), group)
     maps = _sweep_maps(grids, lo, hi)
     start, target = maps.first_cells()
+    if per_map_endpoints:
+        return _solve_maaco_per_map(grids, maps, lo, hi, start, target, num_ants, num_iterations, params, seeds, wave,
+                                    group, device, max_cells)
     keys = {i: (_map_shape(grids[i]), start[i - lo], target[i - lo]) for i in range(lo, hi)}
     out = []
     prev = None
@@ -402,6 +467,58 @@ def solve_maaco_batch(grids, num_ants, num_iterations, params, seeds=None, wave=
             out.append((i, path, length, turns, curve))
         b.close()
         prev = b
+    out.sort(key=lambda r: r[0])
+    return out
+
+
+def _solve_maaco_per_map(grids, maps, lo, hi, start, target, num_ants, num_iterations, params, seeds, wave, group,
+                         device, max_cells):
+    """solve_maaco_batch(per_map_endpoints=True): waves by shape in index order.  Wave k+1's tables are built into ONE
+    pinned buffer by a worker thread while wave k runs; the worker first waits for the copy that read wave k's tables
+    out of that buffer, so the buffer is never rewritten before that copy has run."""
+    import os
+    from concurrent.futures import ThreadPoolExecutor
+    import torch
+    _all_endpoints("MAACO: Start node not found.", "MAACO: Target node not found.")(start, target)
+    waves = _shape_waves(grids, lo, hi, wave)
+    p = _maaco_params(num_iterations, **params)
+    threads = 0                                      # ranks that share a host split its cores instead of taking 16 each
+    if group is not None and os.environ.get("LOCAL_WORLD_SIZE"):
+        threads = max(1, (os.cpu_count() or 1) // int(os.environ["LOCAL_WORLD_SIZE"]))
+
+    def ends(idx):
+        at = np.asarray(idx) - lo
+        return start[at], target[at]
+
+    def mixed(idx):                                  # MAACOBatch's choice: one table per map only where endpoints differ
+        s, t = ends(idx)
+        return not ((s == s[0]).all() and (t == t[0]).all())
+
+    size = max([2 * len(idx) * int(np.prod(_map_shape(grids[idx[0]]))) for idx in waves if mixed(idx)], default=0)
+    pinned = torch.empty(size, dtype=torch.float64, pin_memory=True) if size else None
+
+    def build(idx, copied):
+        if copied is not None:
+            copied.synchronize()
+        return _e01_host(*_map_shape(grids[idx[0]]), *ends(idx), p, pinned, threads)
+
+    out, prev, copied = [], None, None
+    with ThreadPoolExecutor(1) as pool:
+        submit = lambda k: pool.submit(build, waves[k], copied) if k < len(waves) and mixed(waves[k]) else None
+        pending = submit(0)
+        for k, idx in enumerate(waves):
+            e01 = pending.result() if pending is not None else None
+            b = MAACOBatch(maps.wave(idx), num_ants, num_iterations,
+                           seeds=None if seeds is None else [seeds[i] for i in idx], device=device, max_cells=max_cells,
+                           reuse=prev, per_map_endpoints=True, _e01=e01, **params)
+            if e01 is not None:
+                copied = torch.cuda.Event()
+                copied.record(torch.cuda.current_stream(b.device))
+            pending = submit(k + 1)
+            for i, (path, length, turns, curve) in zip(idx, b.solve()):
+                out.append((i, path, length, turns, curve))
+            b.close()
+            prev = b
     out.sort(key=lambda r: r[0])
     return out
 

@@ -14,7 +14,9 @@
 //   moves    [ant][max_cells] uint8   the tour as move codes (MAACO.py:98 order): the best path is decoded from them,
 //                                     and they are what a sharded colony exchanges when it has no peer access
 #include <type_traits>
+#include <algorithm>
 #include <cmath>
+#include <exception>
 #include <cstdlib>
 #include <thread>
 #include <vector>
@@ -43,53 +45,100 @@ extern "C" double mpp_maaco_q0(int K, int k, double q0_initial) {  // MAACO.py:2
     return q0 < 0.99 ? q0 : 0.99;
 }
 
-// tau0 (as if no cell were an obstacle), E01 and dist_to_target of an R x C map with the given start / target:
-// functions of (shape, start, target, parameters) only -- a batch of maps that share them shares the tables.
-static void host_tables(int R, int C, int start, int target, const mpp_maaco_params *p, double *tau0, double *E01,
-                        double *dt) {
+// Rows [r_lo, r_hi) of the tables of an R x C map with the given start / target: tau0 (as if no cell were an
+// obstacle), E01 and dist_to_target, each indexed by cell; tau0 / dt may be null.  Functions of (shape, start, target,
+// parameters) only -- a batch of maps that share them shares the tables.
+static void host_table_rows(int C, int start, int target, const mpp_maaco_params *p, int r_lo, int r_hi, double *tau0,
+                            double *E01, double *dt) {
     const int sr = start / C, sc = start % C, tr = target / C, tc = target % C;
     double dsT = hdist(sr, sc, tr, tc);
     if (dsT < 1e-9) dsT = 1e-9;  // MAACO.py:43-45
-    auto work = [&](int r_lo, int r_hi) {
-        for (int r = r_lo; r < r_hi; ++r)
-            for (int c = 0; c < C; ++c) {
-                const size_t i = (size_t)r * C + c;
-                const double diT = hdist(r, c, tr, tc);
-                const double dsi = hdist(sr, sc, r, c);
-                dt[i] = diT;
-                {
-                    const double den = dsi + diT;                // MAACO.py:58-84
-                    double factor;
-                    if (den < 1e-9) factor = (dsi < 1e-6 || diT < 1e-6) ? 1.0 : 0.1;
-                    else factor = dsT / den;
-                    const double v = factor * p->C0_initial_pheromone;
-                    tau0[i] = v < 1e-9 ? 1e-9 : v;
-                }
-                double h;                                        // MAACO.py:197-210
-                if (dsT < 1e-9) h = p->wh_min;
-                else h = p->wh_max - (p->wh_max - p->wh_min) * std::exp(-p->k_h_adaptive * diT / dsT);
-                const double g = 1.0 - h;
-                const double base = g * dsi + h * diT;
-                double d0 = base + p->a_turn_coef * 0.0, d1 = base + p->a_turn_coef * 1.0;
-                d0 = d0 > 1e-9 ? d0 : 1e-9;
-                d1 = d1 > 1e-9 ? d1 : 1e-9;
-                E01[2 * i] = std::pow(1.0 / d0, p->beta);        // turn flag 0
-                E01[2 * i + 1] = std::pow(1.0 / d1, p->beta);    // turn flag 1
+    for (int r = r_lo; r < r_hi; ++r)
+        for (int c = 0; c < C; ++c) {
+            const size_t i = (size_t)r * C + c;
+            const double diT = hdist(r, c, tr, tc);
+            const double dsi = hdist(sr, sc, r, c);
+            if (dt) dt[i] = diT;
+            if (tau0) {
+                const double den = dsi + diT;                // MAACO.py:58-84
+                double factor;
+                if (den < 1e-9) factor = (dsi < 1e-6 || diT < 1e-6) ? 1.0 : 0.1;
+                else factor = dsT / den;
+                const double v = factor * p->C0_initial_pheromone;
+                tau0[i] = v < 1e-9 ? 1e-9 : v;
             }
-    };
+            double h;                                        // MAACO.py:197-210
+            if (dsT < 1e-9) h = p->wh_min;
+            else h = p->wh_max - (p->wh_max - p->wh_min) * std::exp(-p->k_h_adaptive * diT / dsT);
+            const double g = 1.0 - h;
+            const double base = g * dsi + h * diT;
+            double d0 = base + p->a_turn_coef * 0.0, d1 = base + p->a_turn_coef * 1.0;
+            d0 = d0 > 1e-9 ? d0 : 1e-9;
+            d1 = d1 > 1e-9 ? d1 : 1e-9;
+            E01[2 * i] = std::pow(1.0 / d0, p->beta);        // turn flag 0
+            E01[2 * i + 1] = std::pow(1.0 / d1, p->beta);    // turn flag 1
+        }
+}
+
+// run work(lo, hi) over [0, n_items) on up to nt threads (nt <= 1: on the caller's thread)
+template <class F>
+static void host_parallel(long long n_items, unsigned nt, F work) {
+    if (nt > n_items) nt = (unsigned)n_items;
+    if (nt < 2) {
+        work(0ll, n_items);
+        return;
+    }
+    std::vector<std::thread> th;
+    const long long per = (n_items + nt - 1) / nt;
+    for (unsigned t = 0; t < nt; ++t) {
+        const long long lo = (long long)t * per, hi = lo + per > n_items ? n_items : lo + per;
+        if (lo < hi) th.emplace_back(work, lo, hi);
+    }
+    for (auto &t : th) t.join();
+}
+
+// the default thread count of the host table builds: at most 16, one thread below 65536 cells
+static unsigned host_threads(size_t cells) {
     unsigned nt = std::thread::hardware_concurrency();
     if (nt > 16) nt = 16;
-    if (nt < 2 || (size_t)R * C < 65536) {
-        work(0, R);
-    } else {
-        std::vector<std::thread> th;
-        int per = (R + (int)nt - 1) / (int)nt;
-        for (unsigned t = 0; t < nt; ++t) {
-            int lo = (int)t * per, hi = lo + per > R ? R : lo + per;
-            if (lo < hi) th.emplace_back(work, lo, hi);
-        }
-        for (auto &t : th) t.join();
+    return cells < 65536 ? 1u : nt;
+}
+
+static void host_tables(int R, int C, int start, int target, const mpp_maaco_params *p, double *tau0, double *E01,
+                        double *dt) {
+    host_parallel(R, host_threads((size_t)R * C), [&](long long lo, long long hi) {
+        host_table_rows(C, start, target, p, (int)lo, (int)hi, tau0, E01, dt);
+    });
+}
+
+extern "C" int mpp_maaco_e01_host(int rows, int cols, int n, const int32_t *start, const int32_t *target,
+                                  const mpp_maaco_params *p, double *out, int threads) {
+    MPP_REQUIRE(rows > 0 && cols > 0, "mpp_maaco_e01_host: bad shape %d x %d", rows, cols);
+    MPP_REQUIRE(n >= 0, "mpp_maaco_e01_host: n = %d < 0", n);
+    MPP_REQUIRE(threads >= 0, "mpp_maaco_e01_host: threads = %d < 0", threads);
+    if (n == 0) return MPP_OK;
+    MPP_REQUIRE(start && target && p && out, "mpp_maaco_e01_host: null argument");
+    const long long cells = (long long)rows * cols;
+    for (int k = 0; k < n; ++k)
+        MPP_REQUIRE(start[k] >= 0 && start[k] < cells && target[k] >= 0 && target[k] < cells,
+                    "mpp_maaco_e01_host: pair %d (start %d, target %d) is outside the %d x %d map", k, (int)start[k],
+                    (int)target[k], rows, cols);
+    // one work item = one row of one map: a batch spreads over its maps, a single map over its rows
+    const unsigned nt = threads ? (unsigned)threads : host_threads((size_t)cells * n);
+    try {
+        host_parallel((long long)n * rows, nt, [&](long long lo, long long hi) {
+            for (long long w = lo; w < hi;) {
+                const int k = (int)(w / rows), r0 = (int)(w % rows);
+                const int r1 = (int)std::min<long long>(rows, r0 + (hi - w));
+                host_table_rows(cols, start[k], target[k], p, r0, r1, nullptr, out + (size_t)k * 2 * cells, nullptr);
+                w += r1 - r0;
+            }
+        });
+    } catch (const std::exception &e) {
+        mpp_set_error("mpp_maaco_e01_host: %s", e.what());
+        return MPP_ENOMEM;
     }
+    return MPP_OK;
 }
 
 // tau0 of every map of the batch = the shared free-cell table with the map's obstacles at 1e-9 (MAACO.py:62-63)
@@ -129,6 +178,53 @@ extern "C" int mpp_maaco_tables(const mpp_map_batch *maps, const mpp_maaco_param
     MPP_CUDA(cudaGetLastError());
     MPP_CUDA(cudaStreamSynchronize(s));  // buf / tau0_free are released on return
     MPP_CUDA(cudaFree(tau0_free));
+    return MPP_OK;
+}
+
+// tau0 of every map from its OWN start / target (MAACO.py:58-84, dsT floored as :43-45), obstacles at 1e-9 (:62-63):
+// host_table_rows' expression with the same integer dr^2 + dc^2, correctly rounded sqrt and division and no FMA
+// (-fmad=false), so each value is bit for bit what the host writes.
+__global__ void mpp_maaco_tau0_maps_kernel(const MppMapMeta *__restrict__ meta, const uint32_t *__restrict__ occ,
+                                           int occ_words, int pitch, int R, int C, double C0, double *__restrict__ tau,
+                                           long long tau_stride) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= R * C) return;
+    const int k = blockIdx.y;
+    occ += (size_t)k * occ_words;
+    const int r = i / C, c = i % C, pb = c + 1;
+    const int start = meta[k].start, target = meta[k].target;
+    const int sr = start / C, sc = start % C, tr = target / C, tc = target % C;
+    auto dist = [](int r0, int c0, int r1, int c1) {
+        const long long dr = r0 - r1, dc = c0 - c1;
+        return sqrt((double)(dr * dr + dc * dc));
+    };
+    double dsT = dist(sr, sc, tr, tc);
+    if (dsT < 1e-9) dsT = 1e-9;
+    const double diT = dist(r, c, tr, tc), dsi = dist(sr, sc, r, c);
+    const double den = dsi + diT;
+    double factor;
+    if (den < 1e-9) factor = (dsi < 1e-6 || diT < 1e-6) ? 1.0 : 0.1;
+    else factor = dsT / den;
+    const double v = factor * C0;
+    const bool obst = (occ[(r + 1) * pitch + (pb >> 5)] >> (pb & 31)) & 1u;
+    tau[(size_t)k * tau_stride + i] = obst || v < 1e-9 ? 1e-9 : v;
+}
+
+extern "C" int mpp_maaco_tau0_maps(const mpp_map_batch *maps, const mpp_maaco_params *p, double *tau0_dev,
+                                   long long tau_stride, void *stream) {
+    MPP_REQUIRE(maps && p && tau0_dev, "mpp_maaco_tau0_maps: null argument");
+    const int R = maps->rows, C = maps->cols;
+    const long long n = (long long)R * C;
+    MPP_REQUIRE(tau_stride >= n, "mpp_maaco_tau0_maps: tau_stride < rows*cols");
+    for (int k = 0; k < maps->n_maps; ++k)
+        MPP_REQUIRE(maps->meta_host[k].start >= 0 && maps->meta_host[k].target >= 0,
+                    "mpp_maaco_tau0_maps: map %d has no start/target", k);
+    if (maps->n_maps == 0) return MPP_OK;
+    MPP_CUDA(cudaSetDevice(maps->device));
+    mpp_maaco_tau0_maps_kernel<<<dim3((unsigned)((n + 255) / 256), maps->n_maps), 256, 0, (cudaStream_t)stream>>>(
+        maps->meta_dev, maps->occ_dev, maps->occ_words, maps->pitch_words, R, C, p->C0_initial_pheromone, tau0_dev,
+        tau_stride);
+    MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }
 
