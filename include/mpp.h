@@ -172,11 +172,23 @@ int mpp_maaco_tables(const mpp_map_batch *maps, const mpp_maaco_params *p, doubl
  * mpp_maaco_tau0_maps: replaces MAACO._initialize_pheromones_maaco (MAACO.py:58-84) for every map of the batch from
  *   that map's own start and target, obstacles at 1e-9 (:62-63): one kernel (grid.y = map) whose values are bit for bit
  *   mpp_maaco_tables' (integer squared distances, correctly rounded sqrt and division, no FMA).  tau0_dev:
- *   [n_maps][tau_stride].  Asynchronous on `stream`.  No dist_to_target table is produced. */
+ *   [n_maps][tau_stride].  Asynchronous on `stream`.  No dist_to_target table is produced.
+ * mpp_maaco_e01_maps: mpp_maaco_e01_host on the device for every map of the batch from that map's own start and
+ *   target: one thread per cell (grid.y = map), each writing its (E0, E1) pair as one 16-byte store.  exp / pow are
+ *   mpp_exp / mpp_pow (csrc/mpp_libm.cuh), replicas of the x86-64 glibc 2.39 FMA-build functions, so the tables are
+ *   bit for bit mpp_maaco_e01_host's where the host's libm is that build.  E01_dev: [n_maps][E01_stride] doubles,
+ *   16-byte aligned, E01_stride even and >= 2*rows*cols.  A map without start or target is an MPP_EINVAL.
+ *   Asynchronous on `stream`.
+ * mpp_libm_exp_pow: out[2i] = mpp_exp(e[i]), out[2i+1] = mpp_pow(x[i], y[i]) for i < n, on the device (all pointers
+ *   device memory), with the code mpp_maaco_e01_maps runs; what a caller compares with the host's libm before it
+ *   trusts the device tables.  Asynchronous on `stream`. */
 int mpp_maaco_e01_host(int rows, int cols, int n, const int32_t *start, const int32_t *target, const mpp_maaco_params *p,
                        double *out, int threads);
 int mpp_maaco_tau0_maps(const mpp_map_batch *maps, const mpp_maaco_params *p, double *tau0_dev, long long tau_stride,
                         void *stream);
+int mpp_maaco_e01_maps(const mpp_map_batch *maps, const mpp_maaco_params *p, double *E01_dev, long long E01_stride,
+                       void *stream);
+int mpp_libm_exp_pow(int n, const double *e, const double *x, const double *y, double *out, int device, void *stream);
 
 /* replaces MAACO._calculate_adaptive_q0 (MAACO.py:212-226); pure host function */
 double mpp_maaco_q0(int num_iterations, int iteration, double q0_initial);

@@ -8,8 +8,8 @@ The eta'**beta / dist-to-target tables depend only on (shape, start, target, par
 holds maps of one (start, target) pair and shares ONE table computed on the host with libm (bit-identical to the
 reference), and tau0 of each map is that shared table with the map's obstacles masked on the device
 (mpp_maaco_tables).  With per_map_endpoints=True a wave may mix endpoints: it then holds one eta'**beta table per map,
-still computed on the host with libm (mpp_maaco_e01_host; solve_maaco_batch builds the next wave's tables on a worker
-thread while the GPU runs the current one), and tau0 is computed per map on the device (mpp_maaco_tau0_maps).
+built on the device with replicas of the host libm's exp / pow (mpp_maaco_e01_maps, bit for bit mpp_maaco_e01_host's),
+and tau0 is computed per map on the device (mpp_maaco_tau0_maps).
 
 Every batch class takes `grids` either on the host ([M, rows, cols] cell codes, anything np.asarray takes) or as an
 [M, rows, cols] CUDA tensor of bool, uint8, int8, int16, int32 or int64 cells; every sweep also takes a sequence of 2-D
@@ -182,6 +182,48 @@ def _e01_host(rows, cols, start, target, params, out, threads=0):
     return out
 
 
+_DEVICE_E01 = None       # per process: do the device's exp / pow match the host's libm?  None = not probed yet
+
+
+def _libm_probe(device_index):
+    """True when mpp_exp / mpp_pow on the GPU -- what mpp_maaco_e01_maps evaluates -- return the host libm's exp / pow
+    bit for bit on a fixed seeded probe of 2**16 arguments of each from the tables' domain (exp on [-800, 0]; pow with
+    x in [1e-7, 1e9], y in [0, 64], a quarter of the y whole numbers).  The host values come from the C library's exp /
+    pow, the functions mpp_maaco_e01_host calls.  A tripwire, not a proof: it catches a host libm other than the build
+    the replicas reproduce (glibc 2.39, x86-64, FMA), it cannot show that every argument agrees."""
+    import ctypes.util
+    import torch
+    libm = C.CDLL(ctypes.util.find_library("m"))
+    libm.exp.restype, libm.exp.argtypes = C.c_double, [C.c_double]
+    libm.pow.restype, libm.pow.argtypes = C.c_double, [C.c_double, C.c_double]
+    rng = np.random.default_rng(0x6C69626D)
+    n = 1 << 16
+    e = rng.uniform(-800.0, 0.0, n)
+    x = np.exp(rng.uniform(np.log(1e-7), np.log(1e9), n))
+    y = rng.uniform(0.0, 64.0, n)
+    y[: n // 4] = np.floor(y[: n // 4])
+    want = np.empty(2 * n)
+    want[0::2] = [libm.exp(v) for v in e.tolist()]
+    want[1::2] = [libm.pow(a, b) for a, b in zip(x.tolist(), y.tolist())]
+    dev = torch.device("cuda", device_index)
+    args = [torch.from_numpy(a).to(dev) for a in (e, x, y)]
+    got = torch.empty(2 * n, dtype=torch.float64, device=dev)
+    stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+    _lib.check(_lib.lib().mpp_libm_exp_pow(n, *(_lib.ptr(a) for a in args), _lib.ptr(got), device_index, stream),
+               "mpp_libm_exp_pow")
+    return bool((got.cpu().numpy().view(np.uint64) == want.view(np.uint64)).all())
+
+
+def _device_e01(device_index):
+    """Whether this process builds per-map eta'**beta tables on the device (mpp_maaco_e01_maps): _libm_probe, run by the
+    first per-map wave.  Where it fails every per-map table of the process is built on the host (mpp_maaco_e01_host),
+    so the tables stay bit for bit the reference's."""
+    global _DEVICE_E01
+    if _DEVICE_E01 is None:
+        _DEVICE_E01 = _libm_probe(device_index)
+    return _DEVICE_E01
+
+
 class MAACOBatch:
     """M same-shape maps, one colony of `num_ants` ants per map, solved together.  Same parameters as MAACO
     (MAACO.py:11-14); `seeds` = one Philox seed per map.  `max_cells` works as in MAACO: left at its default, solve()
@@ -190,17 +232,17 @@ class MAACOBatch:
 
     By default the maps must share start and target: they then share one table built once (mpp_maaco_tables), and
     maps with other endpoints raise MppError.  With per_map_endpoints=True each map may have its own start and target:
-    the wave then holds one eta'**beta table per map ([M, 2*rows*cols] doubles, 16 B per cell per map, built on the host
-    with mpp_maaco_e01_host and copied without blocking from pinned memory), and tau0 is computed on the device from each
-    map's own endpoints (mpp_maaco_tau0_maps).  A wave whose maps all share their endpoints takes the shared table
+    the wave then holds one eta'**beta table per map ([M, 2*rows*cols] doubles, 16 B per cell per map, built on the
+    device on the wave's stream by mpp_maaco_e01_maps -- or on the host by mpp_maaco_e01_host where _device_e01 says the
+    device's exp / pow do not match the host libm), and tau0 is computed on the device from each map's own endpoints
+    (mpp_maaco_tau0_maps).  A wave whose maps all share their endpoints takes the shared table
     either way.  Results are those of solo MAACO with the same seed in both modes."""
 
     def __init__(self, grids, num_ants, num_iterations, alpha, beta, rho, Q, a_turn_coef, wh_max, wh_min, k_h_adaptive,
                  q0_initial, C0_initial_pheromone=0.1, *, seeds=None, device=None, max_cells=None, ants_per_warp=0,
                  reuse=None, per_map_endpoints=False, _e01=None):
-        # _e01 (solve_maaco_batch and the max_cells repeat): this wave's per-map tables, already built -- a float64
-        # host tensor of at least M * 2 * rows * cols values that the caller keeps unchanged until the copy enqueued here
-        # has run, or an [M, 2 * rows * cols] CUDA tensor on the wave's device, used as it is
+        # _e01 (the max_cells repeat): this wave's per-map tables, already built -- an [M, 2 * rows * cols] CUDA tensor
+        # on the wave's device, used as it is
         import torch
         L = _lib.lib()
         self._map_set = _map_set(grids, device, _all_endpoints("MAACO: Start node not found.",        # MAACO.py:35-36
@@ -246,8 +288,7 @@ class MAACOBatch:
         else:
             self._tau = torch.empty((M, n), dtype=f64, device=dev)
             if self.per_map_tables:
-                self._E01 = None if isinstance(_e01, torch.Tensor) and _e01.is_cuda else \
-                    torch.empty((M, 2 * n), dtype=f64, device=dev)
+                self._E01 = None if _e01 is not None else torch.empty((M, 2 * n), dtype=f64, device=dev)
                 self._dist_t = None                                           # nothing in the batch reads it
             else:
                 self._E01 = torch.empty(2 * n, dtype=f64, device=dev)         # shared by the whole wave
@@ -265,16 +306,17 @@ class MAACOBatch:
         self._key = key
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         if self.per_map_tables:
-            if isinstance(_e01, torch.Tensor) and _e01.is_cuda:
+            if _e01 is not None:
                 if tuple(_e01.shape) != (M, 2 * n) or _e01.device != dev or _e01.dtype != f64:
                     raise ValueError(f"_e01 must be a float64 [{M}, {2 * n}] tensor on {dev}")
                 self._E01 = _e01
+            elif _device_e01(self.device_index):
+                _lib.check(L.mpp_maaco_e01_maps(self._maps, C.byref(self._params), _lib.ptr(self._E01), 2 * n, stream),
+                           "mpp_maaco_e01_maps")
             else:
-                if _e01 is None:
-                    _e01 = _e01_host(R, Cc, start, target, self._params,
-                                     torch.empty(M * 2 * n, dtype=f64, pin_memory=True))
+                host = _e01_host(R, Cc, start, target, self._params, torch.empty(M * 2 * n, dtype=f64, pin_memory=True))
                 # (a pinned tensor of torch's host allocator is not reused before this copy has run)
-                self._E01.view(-1).copy_(_e01.view(-1)[:M * 2 * n], non_blocking=True)
+                self._E01.view(-1).copy_(host, non_blocking=True)
             _lib.check(L.mpp_maaco_tau0_maps(self._maps, C.byref(self._params), _lib.ptr(self._tau), n, stream),
                        "mpp_maaco_tau0_maps")
         else:
@@ -444,9 +486,8 @@ def solve_maaco_batch(grids, num_ants, num_iterations, params, seeds=None, wave=
 
     By default a wave holds maps of one shape and one (start, target) pair, so a sweep whose maps have their own
     endpoints runs one small wave per pair.  With per_map_endpoints=True waves are formed by shape only, in index order
-    (MAACOBatch(per_map_endpoints=True)); one worker thread builds the next wave's eta'**beta tables on the host while
-    the GPU runs the current wave, so the host cost is hidden as long as it stays below a wave's GPU time.  A map
-    without a start or target then raises before any wave runs.
+    (MAACOBatch(per_map_endpoints=True), whose per-map eta'**beta tables are built on the device).  A map without a
+    start or target then raises before any wave runs.
 
     Returns a list of (map_index, path, length, turns, convergence_curve) for the maps of this rank; results
     are identical to solving each map alone (same seeds => same Philox streams)."""
@@ -454,71 +495,20 @@ def solve_maaco_batch(grids, num_ants, num_iterations, params, seeds=None, wave=
     maps = _sweep_maps(grids, lo, hi)
     start, target = maps.first_cells()
     if per_map_endpoints:
-        return _solve_maaco_per_map(grids, maps, lo, hi, start, target, num_ants, num_iterations, params, seeds, wave,
-                                    group, device, max_cells)
-    keys = {i: (_map_shape(grids[i]), start[i - lo], target[i - lo]) for i in range(lo, hi)}
+        _all_endpoints("MAACO: Start node not found.", "MAACO: Target node not found.")(start, target)
+        waves = _shape_waves(grids, lo, hi, wave)
+    else:
+        waves = _waves({i: (_map_shape(grids[i]), start[i - lo], target[i - lo]) for i in range(lo, hi)}, wave)
     out = []
     prev = None
-    for idx in _waves(keys, wave):
+    for idx in waves:
         b = MAACOBatch(maps.wave(idx), num_ants, num_iterations,
                        seeds=None if seeds is None else [seeds[i] for i in idx], device=device, max_cells=max_cells,
-                       reuse=prev, **params)
+                       reuse=prev, per_map_endpoints=per_map_endpoints, **params)
         for i, (path, length, turns, curve) in zip(idx, b.solve()):
             out.append((i, path, length, turns, curve))
         b.close()
         prev = b
-    out.sort(key=lambda r: r[0])
-    return out
-
-
-def _solve_maaco_per_map(grids, maps, lo, hi, start, target, num_ants, num_iterations, params, seeds, wave, group,
-                         device, max_cells):
-    """solve_maaco_batch(per_map_endpoints=True): waves by shape in index order.  Wave k+1's tables are built into ONE
-    pinned buffer by a worker thread while wave k runs; the worker first waits for the copy that read wave k's tables
-    out of that buffer, so the buffer is never rewritten before that copy has run."""
-    import os
-    from concurrent.futures import ThreadPoolExecutor
-    import torch
-    _all_endpoints("MAACO: Start node not found.", "MAACO: Target node not found.")(start, target)
-    waves = _shape_waves(grids, lo, hi, wave)
-    p = _maaco_params(num_iterations, **params)
-    threads = 0                                      # ranks that share a host split its cores instead of taking 16 each
-    if group is not None and os.environ.get("LOCAL_WORLD_SIZE"):
-        threads = max(1, (os.cpu_count() or 1) // int(os.environ["LOCAL_WORLD_SIZE"]))
-
-    def ends(idx):
-        at = np.asarray(idx) - lo
-        return start[at], target[at]
-
-    def mixed(idx):                                  # MAACOBatch's choice: one table per map only where endpoints differ
-        s, t = ends(idx)
-        return not ((s == s[0]).all() and (t == t[0]).all())
-
-    size = max([2 * len(idx) * int(np.prod(_map_shape(grids[idx[0]]))) for idx in waves if mixed(idx)], default=0)
-    pinned = torch.empty(size, dtype=torch.float64, pin_memory=True) if size else None
-
-    def build(idx, copied):
-        if copied is not None:
-            copied.synchronize()
-        return _e01_host(*_map_shape(grids[idx[0]]), *ends(idx), p, pinned, threads)
-
-    out, prev, copied = [], None, None
-    with ThreadPoolExecutor(1) as pool:
-        submit = lambda k: pool.submit(build, waves[k], copied) if k < len(waves) and mixed(waves[k]) else None
-        pending = submit(0)
-        for k, idx in enumerate(waves):
-            e01 = pending.result() if pending is not None else None
-            b = MAACOBatch(maps.wave(idx), num_ants, num_iterations,
-                           seeds=None if seeds is None else [seeds[i] for i in idx], device=device, max_cells=max_cells,
-                           reuse=prev, per_map_endpoints=True, _e01=e01, **params)
-            if e01 is not None:
-                copied = torch.cuda.Event()
-                copied.record(torch.cuda.current_stream(b.device))
-            pending = submit(k + 1)
-            for i, (path, length, turns, curve) in zip(idx, b.solve()):
-                out.append((i, path, length, turns, curve))
-            b.close()
-            prev = b
     out.sort(key=lambda r: r[0])
     return out
 

@@ -22,6 +22,7 @@
 #include <vector>
 
 #include "mpp_common.cuh"
+#include "mpp_libm.cuh"
 
 // ---------------------------------------------------------------------------------------------
 // host: tables (libm exp/pow == what CPython / NumPy call, so the tables are bit-identical)
@@ -224,6 +225,72 @@ extern "C" int mpp_maaco_tau0_maps(const mpp_map_batch *maps, const mpp_maaco_pa
     mpp_maaco_tau0_maps_kernel<<<dim3((unsigned)((n + 255) / 256), maps->n_maps), 256, 0, (cudaStream_t)stream>>>(
         maps->meta_dev, maps->occ_dev, maps->occ_words, maps->pitch_words, R, C, p->C0_initial_pheromone, tau0_dev,
         tau_stride);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
+
+// E01 of every map from its OWN start / target (MAACO.py:197-210, dsT floored as :43-45): host_table_rows' expression
+// in its order -- integer dr^2 + dc^2, correctly rounded sqrt and division, no FMA (-fmad=false) -- with mpp_exp /
+// mpp_pow for libm's exp / pow, so each value is bit for bit what mpp_maaco_e01_host writes.
+__global__ void mpp_maaco_e01_maps_kernel(const MppMapMeta *__restrict__ meta, int R, int C, double beta, double wh_max,
+                                          double wh_min, double k_h, double a_turn, double *__restrict__ E01,
+                                          long long E01_stride) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= R * C) return;
+    const int k = blockIdx.y;
+    const int r = i / C, c = i % C;
+    const int start = meta[k].start, target = meta[k].target;
+    const int sr = start / C, sc = start % C, tr = target / C, tc = target % C;
+    auto dist = [](int r0, int c0, int r1, int c1) {
+        const long long dr = r0 - r1, dc = c0 - c1;
+        return sqrt((double)(dr * dr + dc * dc));
+    };
+    double dsT = dist(sr, sc, tr, tc);
+    if (dsT < 1e-9) dsT = 1e-9;
+    const double diT = dist(r, c, tr, tc), dsi = dist(sr, sc, r, c);
+    const double h = wh_max - (wh_max - wh_min) * mpp_exp(-k_h * diT / dsT);
+    const double g = 1.0 - h;
+    const double base = g * dsi + h * diT;
+    double d0 = base + a_turn * 0.0, d1 = base + a_turn * 1.0;
+    d0 = d0 > 1e-9 ? d0 : 1e-9;
+    d1 = d1 > 1e-9 ? d1 : 1e-9;
+    *(double2 *)(E01 + (size_t)k * E01_stride + 2 * (size_t)i) = make_double2(mpp_pow(1.0 / d0, beta), mpp_pow(1.0 / d1, beta));
+}
+
+extern "C" int mpp_maaco_e01_maps(const mpp_map_batch *maps, const mpp_maaco_params *p, double *E01_dev,
+                                  long long E01_stride, void *stream) {
+    MPP_REQUIRE(maps && p && E01_dev, "mpp_maaco_e01_maps: null argument");
+    const int R = maps->rows, C = maps->cols;
+    const long long n = (long long)R * C;
+    MPP_REQUIRE(E01_stride >= 2 * n && E01_stride % 2 == 0, "mpp_maaco_e01_maps: E01_stride %lld is odd or < 2*rows*cols",
+                E01_stride);
+    MPP_REQUIRE(((uintptr_t)E01_dev & 15) == 0, "mpp_maaco_e01_maps: E01_dev is not 16-byte aligned");
+    for (int k = 0; k < maps->n_maps; ++k)
+        MPP_REQUIRE(maps->meta_host[k].start >= 0 && maps->meta_host[k].target >= 0,
+                    "mpp_maaco_e01_maps: map %d has no start/target", k);
+    if (maps->n_maps == 0) return MPP_OK;
+    MPP_CUDA(cudaSetDevice(maps->device));
+    mpp_maaco_e01_maps_kernel<<<dim3((unsigned)((n + 255) / 256), maps->n_maps), 256, 0, (cudaStream_t)stream>>>(
+        maps->meta_dev, R, C, p->beta, p->wh_max, p->wh_min, p->k_h_adaptive, p->a_turn_coef, E01_dev, E01_stride);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
+
+__global__ void mpp_libm_exp_pow_kernel(int n, const double *__restrict__ e, const double *__restrict__ x,
+                                        const double *__restrict__ y, double *__restrict__ out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    out[2 * (size_t)i] = mpp_exp(e[i]);
+    out[2 * (size_t)i + 1] = mpp_pow(x[i], y[i]);
+}
+
+extern "C" int mpp_libm_exp_pow(int n, const double *e, const double *x, const double *y, double *out, int device,
+                                void *stream) {
+    MPP_REQUIRE(n >= 0, "mpp_libm_exp_pow: n = %d < 0", n);
+    if (n == 0) return MPP_OK;
+    MPP_REQUIRE(e && x && y && out, "mpp_libm_exp_pow: null argument");
+    MPP_CUDA(cudaSetDevice(device));
+    mpp_libm_exp_pow_kernel<<<(n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(n, e, x, y, out);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }

@@ -10,13 +10,19 @@ ants x 10 passes, --wave maps per wave, all from host grids.  Two workloads:
 
 Every arm is timed with the host clock around the sweep (it ends in a device synchronise), --rounds rounds with the arms
 alternated; medians and the spread (min..max) are reported.  For the per-map sweep on random endpoints it also reports,
-per wave: the host table build (host clock around mpp_maaco_e01_host on the worker thread), the GPU time (CUDA events
-from the wave's construction to the end of its solve) and the exposed host time between one wave's solve and the next
-wave's construction (the wait for the tables plus the sweep's own overhead).  Result check: a seeded sample of
---check-sample maps of the per-map sweep against solo MAACO with the same seeds.  Prints one JSON line with the card's
-name and power limit, read in the same run.  Needs a GPU; there is no fallback.
+per wave: the GPU time (CUDA events from the wave's construction to the end of its solve) and the host time between one
+wave's solve and the next wave's construction.  The device table time of one --wave-map wave (CUDA events around
+mpp_maaco_e01_maps alone, --table-reps launches after a warm-up, median) is reported next to the host build of the same
+tables (host clock around mpp_maaco_e01_host, default thread count).  Result check: a seeded sample of --check-sample maps
+of the per-map sweep against solo MAACO with the same seeds.  Prints one JSON line with the card's name and power limit,
+read in the same run.  Needs a GPU; there is no fallback.
+
+--ab TREE compares two builds of the project instead: the random-endpoint per-map sweep from TREE (another checkout
+whose library is built, e.g. the parent commit) and from this tree, --rounds rounds alternated, each run a fresh process
+(`--gpus G`: G ranks under torchrun, maps sharded over them, time = the slowest rank's).
 
     python tools/maaco_endpoints_time.py [--maps 1250] [--wave 128] [--rounds 3] [--grouped-sample 64]
+    python tools/maaco_endpoints_time.py --ab ../parent --maps 1250 [--gpus 8 --maps 10000]
 """
 import argparse
 import json
@@ -58,22 +64,15 @@ def moved(grids, seed):
 
 
 class _Probe:
-    """Per-wave timings of a per-map sweep: patches batch._e01_host and batch.MAACOBatch while active."""
+    """Per-wave timings of a per-map sweep: patches batch.MAACOBatch while active."""
 
     def __init__(self, batch):
-        self.batch, self.table_s, self.gpu_ms, self.exposed_s = batch, [], [], []
+        self.batch, self.gpu_ms, self.exposed_s = batch, [], []
         self._last_end = None
 
     def __enter__(self):
         b, probe = self.batch, self
-        self._orig = (b._e01_host, b.MAACOBatch)
-        host = b._e01_host
-
-        def timed_tables(*a, **kw):
-            t0 = time.perf_counter()
-            out = host(*a, **kw)
-            probe.table_s.append(time.perf_counter() - t0)
-            return out
+        self._orig = b.MAACOBatch
 
         class Timed(b.MAACOBatch):
             def __init__(self, *a, **kw):
@@ -93,12 +92,117 @@ class _Probe:
                 probe._last_end = time.perf_counter()
                 return out
 
-        b._e01_host, b.MAACOBatch = timed_tables, Timed
-        self._last_end = time.perf_counter()                 # the first wave's tables are fully exposed
+        b.MAACOBatch = Timed
         return self
 
     def __exit__(self, *exc):
-        self.batch._e01_host, self.batch.MAACOBatch = self._orig
+        self.batch.MAACOBatch = self._orig
+
+
+def table_times(grids, reps):
+    """(device ms, host ms): mpp_maaco_e01_maps on one wave of `grids` (CUDA events, median of `reps` launches after a
+    warm-up) and mpp_maaco_e01_host on the same maps (host clock, median of 3)."""
+    import ctypes as C
+    from maaco_path_planing_b200 import _lib
+    from maaco_path_planing_b200.batch import _e01_host, _maaco_params, _map_set
+    p = _maaco_params(1, **PARAMS)
+    maps = _map_set(grids)
+    M, n = len(grids), grids[0].size
+    e01 = torch.empty((M, 2 * n), dtype=torch.float64, device="cuda")
+    stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    launch = lambda: _lib.check(_lib.lib().mpp_maaco_e01_maps(maps.handle, C.byref(p), _lib.ptr(e01), 2 * n, stream),
+                                "mpp_maaco_e01_maps")
+    launch()
+    dev = []
+    for _ in range(reps):
+        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a.record()
+        launch()
+        b.record()
+        b.synchronize()
+        dev.append(a.elapsed_time(b))
+    host = []
+    out = torch.empty(M * 2 * n, dtype=torch.float64, pin_memory=True)
+    for _ in range(3):
+        t0 = time.perf_counter()
+        _e01_host(*grids[0].shape, maps.start, maps.target, p, out)
+        host.append(1e3 * (time.perf_counter() - t0))
+    same = out.numpy().tobytes() == e01.cpu().numpy().tobytes()
+    maps.close()
+    return statistics.median(dev), statistics.median(host), same
+
+
+def child(tree, maps, ants, iters, wave):
+    """One per-map sweep over the random-endpoint maps from the project at `tree`; prints {"seconds", "digest"} (rank 0;
+    under torchrun the slowest rank's time)."""
+    sys.path.insert(0, os.path.abspath(tree))
+    import hashlib
+    group = None
+    if int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        import torch.distributed as dist
+        torch.cuda.set_device(int(os.environ["LOCAL_RANK"]))
+        dist.init_process_group("nccl")
+        group = dist.group.WORLD
+    else:
+        torch.cuda.set_device(0)
+    from maaco_path_planing_b200 import blocks_map
+    from maaco_path_planing_b200.batch import shard_maps, solve_maaco_batch
+    lo, hi = shard_maps(maps, group)
+    grids = [None] * maps
+    shard = moved(np.stack([blocks_map(256, 0.20, seed=5000 + i) for i in range(lo, hi)]), 5000 + lo)
+    grids[lo:hi] = list(shard)
+    for i in range(maps):                                     # other ranks' maps: only their shape is read
+        if grids[i] is None:
+            grids[i] = shard[0]
+    solve_maaco_batch(grids[lo:lo + wave] if group is None else grids, ants, 1, PARAMS, seeds=list(range(maps)),
+                      wave=wave, group=group, per_map_endpoints=True)       # warm-up
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    out = solve_maaco_batch(grids, ants, iters, PARAMS, seeds=list(range(maps)), wave=wave, group=group,
+                            per_map_endpoints=True)
+    torch.cuda.synchronize()
+    t = torch.tensor([time.perf_counter() - t0], device="cuda")
+    digest = hashlib.sha256(repr(out).encode()).hexdigest()
+    if group is not None:
+        import torch.distributed as dist
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+        digests = [None] * dist.get_world_size()
+        dist.all_gather_object(digests, digest)
+        digest = hashlib.sha256("".join(digests).encode()).hexdigest()
+        dist.destroy_process_group()
+    if int(os.environ.get("RANK", "0")) == 0:
+        print(json.dumps({"seconds": float(t.item()), "digest": digest}), flush=True)
+
+
+def ab(args):
+    """Alternate child sweeps of the tree at args.ab ("parent") and this tree ("new")."""
+    trees = {"parent": os.path.abspath(args.ab), "new": ROOT}
+    me = os.path.abspath(__file__)
+    times = {k: [] for k in trees}
+    digests = {k: set() for k in trees}
+    for r in range(args.rounds):
+        for k in (("parent", "new") if r % 2 == 0 else ("new", "parent")):
+            cmd = [sys.executable, me]
+            if args.gpus > 1:
+                cmd = [sys.executable, "-m", "torch.distributed.run", "--standalone", f"--nproc_per_node={args.gpus}",
+                       me]
+            cmd += ["--child", trees[k], "--maps", str(args.maps), "--ants", str(args.ants), "--iters", str(args.iters),
+                    "--wave", str(args.wave)]
+            res = subprocess.run(cmd, capture_output=True, text=True, cwd=trees[k])
+            line = [l for l in res.stdout.splitlines() if l.startswith("{")]
+            if res.returncode != 0 or not line:
+                raise SystemExit(f"{k} run failed ({res.returncode}):\n{res.stdout[-2000:]}\n{res.stderr[-4000:]}")
+            d = json.loads(line[-1])
+            times[k].append(d["seconds"])
+            digests[k].add(d["digest"])
+    name, power = card()
+    rate = {k: {"maps_per_s_median": args.maps / statistics.median(v), "maps_per_s_min": args.maps / max(v),
+                "maps_per_s_max": args.maps / min(v), "seconds": v} for k, v in times.items()}
+    print(json.dumps({"tool": "maaco_endpoints_time", "mode": "ab", "card": name, "power_limit_w": power,
+                      "gpus": args.gpus, "maps": args.maps, "ants": args.ants, "passes": args.iters, "wave": args.wave,
+                      "rounds": args.rounds, "host_cpus": os.cpu_count(), "arms": rate,
+                      "speedup_new_vs_parent": rate["new"]["maps_per_s_median"] / rate["parent"]["maps_per_s_median"],
+                      "results_equal": len(digests["parent"] | digests["new"]) == 1}))
 
 
 def main():
@@ -110,7 +214,15 @@ def main():
     ap.add_argument("--rounds", type=int, default=3)
     ap.add_argument("--grouped-sample", type=int, default=64)
     ap.add_argument("--check-sample", type=int, default=8)
+    ap.add_argument("--table-reps", type=int, default=20)
+    ap.add_argument("--ab", default=None)
+    ap.add_argument("--gpus", type=int, default=1)
+    ap.add_argument("--child", default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.child:
+        return child(args.child, args.maps, args.ants, args.iters, args.wave)
+    if args.ab:
+        return ab(args)
     if not torch.cuda.is_available():
         raise SystemExit("maaco_endpoints_time.py measures the GPU: no CUDA device visible")
     torch.cuda.set_device(0)
@@ -137,6 +249,7 @@ def main():
         "corners_default": lambda: sweep(corners, seeds, False),
         "corners_per_map": lambda: sweep(corners, seeds, True),
     }
+    table_dev_ms, table_host_ms, tables_equal = table_times(rand[:W], args.table_reps)
     # warm-up: every arm's launch shapes (a full wave, 1-map waves, the table builder) once
     sweep(rand[:W], seeds[:W], True)
     sweep(rand_sample[:2], seeds[:2], False)
@@ -179,8 +292,9 @@ def main():
         "arms": rate,
         "speedup_random_per_map_vs_grouped": rate["random_per_map"]["maps_per_s_median"] /
         rate["random_grouped_sample"]["maps_per_s_median"],
+        "tables_one_wave": {"maps": min(W, M), "device_ms_median": table_dev_ms, "host_ms_median": table_host_ms,
+                            "host_threads": min(16, os.cpu_count() or 1), "device_equals_host": tables_equal},
         "per_wave": {"waves": waves,
-                     "host_table_ms_median": 1e3 * med([t for p in probes for t in p.table_s]),
                      "gpu_ms_median": med([t for p in probes for t in p.gpu_ms]),
                      "exposed_host_ms_median": 1e3 * med([t for p in probes for t in p.exposed_s]),
                      "exposed_host_ms_total_per_sweep": [1e3 * sum(p.exposed_s) for p in probes]},
