@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MPP_ABI_VERSION 2
+#define MPP_ABI_VERSION 3
 
 #define MPP_OK 0
 #define MPP_EINVAL (-1)
@@ -47,40 +47,24 @@ extern "C" {
 #define MPP_CLS_MPA_PHASE 9
 #define MPP_CLS_MPA_FADS 10
 
-typedef struct mpp_map mpp_map; /* opaque: bit-packed occupancy grid + per-map tables on one device */
-
 int mpp_abi_version(void);
 const char *mpp_last_error(void);
 /* number of sm_100 devices visible (0 => every compute entry point fails) */
 int mpp_device_count(void);
 
-/* ---- grid map: env.py grid convention (0 free, 1 obstacle, 2 start, 3 target) ------------
+/* ---- maps: env.py grid convention (0 free, 1 obstacle, 2 start, 3 target) -------------------------------------------
+ * A batch of independent same-shape maps (BASELINE config 5: "batched sweep over independent maps") on one device; every
+ * compute entry point takes a batch, and a single map is a batch of one (n_maps = 1).
  * replaces: np.array(grid) + argwhere(grid==2/3) in every constructor
- * (MAACO.py:15-41, helper.py:121-125, astar.py:17-22, pso.py:17-22, ga_solver.py:17-22, MPA.py:20-43).
- * grid_host: rows*cols bytes, row-major.  Start/target = first row-major 2 / 3.  Synchronous. */
-int mpp_map_create(const uint8_t *grid_host, int rows, int cols, int device, mpp_map **out);
-void mpp_map_destroy(mpp_map *map);
-int mpp_map_rows(const mpp_map *map);
-int mpp_map_cols(const mpp_map *map);
-int mpp_map_start(const mpp_map *map);  /* cell id or -1 */
-int mpp_map_target(const mpp_map *map); /* cell id or -1 */
-int mpp_map_device(const mpp_map *map);
-/* device pointer to the border-padded bit-packed occupancy grid ((rows+2) x pitch_words uint32,
- * bit (r+1, c+1); the border is marked occupied) and its row pitch in 32-bit words */
-const uint32_t *mpp_map_occ_bits(const mpp_map *map, int *pitch_words);
-
-/* ---- batches of independent same-shape maps (BASELINE config 5: "batched sweep over independent maps") --------
- * Every MAACO entry point below works on a batch (one launch covers all maps: grid.y = map).  A single map is a
- * batch of one: mpp_map_as_batch(map) returns that view (owned by the map, no copy).
- * replaces: a Python loop `for grid in grids: MAACO(grid, ...)` around MAACO.py:11-53.
- * grids_host: n_maps x rows x cols bytes.  Synchronous. */
-typedef struct mpp_map_batch mpp_map_batch;
+ * (MAACO.py:15-41, helper.py:121-125, astar.py:17-22, pso.py:17-22, ga_solver.py:17-22, MPA.py:20-43), and a Python loop
+ * `for grid in grids: MAACO(grid, ...)` around MAACO.py:11-53.
+ * grids_host: n_maps x rows x cols bytes, row-major.  Start/target of a map = its first row-major 2 / 3.  Synchronous. */
+typedef struct mpp_map_batch mpp_map_batch; /* opaque: bit-packed occupancy grids + per-map tables on one device */
 int mpp_map_batch_create(const uint8_t *grids_host, int n_maps, int rows, int cols, int device, mpp_map_batch **out);
 void mpp_map_batch_destroy(mpp_map_batch *maps);
 int mpp_map_batch_size(const mpp_map_batch *maps);
 int mpp_map_batch_start(const mpp_map_batch *maps, int k);  /* cell id of map k's start or -1 */
 int mpp_map_batch_target(const mpp_map_batch *maps, int k);
-const mpp_map_batch *mpp_map_as_batch(const mpp_map *map);
 /* The same batch from grids already in device memory of `device`: grids_dev = n_maps x rows x cols contiguous cells of
  * elem_bytes bytes each (1 = uint8, 4 = int32, 8 = int64).  Cells are compared raw: 1 obstacle, 2 start candidate,
  * 3 target candidate, any other value free -- the classification the uint8 path gives after clipping to 0..255.
@@ -89,8 +73,9 @@ const mpp_map_batch *mpp_map_as_batch(const mpp_map *map);
  * the batch is ready. */
 int mpp_map_batch_create_device(const void *grids_dev, int elem_bytes, int n_maps, int rows, int cols, int device,
                                 void *stream, mpp_map_batch **out);
-/* the batch's occupancy, [n_maps][((rows+2) * pitch_words + 3) & ~3] words in mpp_map_occ_bits's layout, its static
- * move masks [n_maps][rows*cols] (MAACO move order) and its obstacle count over all maps */
+/* the batch's occupancy, [n_maps][((rows+2) * pitch_words + 3) & ~3] words: border-padded and bit-packed, bit (r+1, c+1)
+ * of map k in row r+1 of its slice (pitch_words 32-bit words per row), the border marked occupied; its static move masks
+ * [n_maps][rows*cols] (MAACO move order) and its obstacle count over all maps */
 const uint32_t *mpp_map_batch_occ_bits(const mpp_map_batch *maps, int *pitch_words);
 const uint8_t *mpp_map_batch_svalid(const mpp_map_batch *maps);
 long long mpp_map_batch_obstacles(const mpp_map_batch *maps);
@@ -294,52 +279,40 @@ typedef struct {
 
 /* replaces calculate_path_safety_penalty's O(len x n_obstacles) scan (helper.py:67-80) by a per-cell class
  * table (u16: min squared distance to an obstacle within floor(msd)) + a LUT of (msd - d)**2 per class, evaluated
- * with libm on the host.  0 <= msd <= 180 (u16 classes).  Cached in the map for one msd at a time; called
- * implicitly by the stats entry points. */
-int mpp_map_safety_table(mpp_map *map, double min_safe_distance, void *stream);
-/* the same tables for every map of a batch (one launch, grid.y = map): [n_maps][rows*cols] classes and one LUT shared
- * by all maps (it depends on msd only).  Cached in the batch for one msd at a time; called implicitly by
- * mpp_astar_batch_maps.  Not for the view mpp_map_as_batch returns (its map has its own table). */
+ * with libm on the host.  0 <= msd <= 180 (u16 classes).  One launch (grid.y = map) builds [n_maps][rows*cols] classes;
+ * one LUT is shared by all maps (it depends on msd only).  Cached in the batch for one msd at a time; called implicitly
+ * by every entry point that computes statistics in mode 0. */
 int mpp_map_batch_safety_table(mpp_map_batch *maps, double min_safe_distance, void *stream);
 
 /* replaces helper.calculate_path_stats (helper.py:98-113; count_turns :58-65, safety :67-80, diagonal
- * penalty :82-96) and MPA._calculate_path_stats (MPA.py:215-229) for n_paths paths, one warp each.
- * length uses CPython 3.12's Neumaier-compensated sum().  stats_dev: n_paths x 5 doubles =
- * (length, turns, safety_penalty, diag_penalty, fitness); empty path -> (inf, 0, 0, 0, inf). */
-int mpp_path_stats(mpp_map *map, const int32_t *cells_dev, int max_cells, const int32_t *n_cells_dev, int n_paths,
-                   const mpp_policy *policy, double *stats_dev, void *stream);
+ * penalty :82-96) and MPA._calculate_path_stats (MPA.py:215-229) for n_paths paths, one warp each; path i lies on map
+ * map_dev[i].  length uses CPython 3.12's Neumaier-compensated sum().  stats_dev: n_paths x 5 doubles =
+ * (length, turns, safety_penalty, diag_penalty, fitness); an empty path, or one whose map index lies outside the batch
+ * -> (inf, 0, 0, 0, inf). */
+int mpp_path_stats(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *cells_dev, int max_cells,
+                   const int32_t *n_cells_dev, int n_paths, const mpp_policy *policy, double *stats_dev, void *stream);
 
-/* scratch sizing for the search entry points: n_slots concurrent searches (one warp each; mpp_astar_max_slots
- * = the number that are resident at once), each with a heap of heap_cap entries.  The scratch buffer must be
- * zero-filled once before its first use (search stamps live in it). */
-size_t mpp_astar_scratch_bytes(const mpp_map *map, int n_slots, int heap_cap);
-int mpp_astar_max_slots(const mpp_map *map);
+/* search slots (one lane group each) of a batch that are resident at once; the scratch of the search entry points is
+ * 256 + n_slots * mpp_astar_slot_bytes(rows, cols, heap_cap) bytes for n_slots concurrent searches with a heap of
+ * heap_cap entries each, zero-filled once before its first use (search stamps live in it). */
+int mpp_map_batch_max_slots(const mpp_map_batch *maps);
 
 /* replaces n independent calls of AStarSolver.solve (variant 0, astar.py:33-101, with get_valid_neighbors
  * helper.py:18-53), MPA._a_star (variant 1, MPA.py:106-151) or DijkstraSolver.solve (variant 2,
- * dijkstra.py:32-97 = variant 0 with a zero heuristic).  avoid_bits_dev: optional n x ceil(rows*cols/32)
- * bitmaps (nodes_to_avoid).  cells_dev: n x max_cells; n_cells_dev[i] = path length (0 = no path / invalid
- * endpoint, -1 = heap_cap overflow, > max_cells = truncated); g_dev[i] = g of the popped target (nullable).
- * counters_dev: optional [4] = (node expansions, successful relaxations, ring-bucket pushes, overflow-heap
- * pushes), accumulated. */
-int mpp_astar_batch(mpp_map *map, int variant, const int32_t *src_dev, const int32_t *dst_dev,
-                    const uint32_t *avoid_bits_dev, int n, int allow_diagonal, int restrict_corner,
-                    int32_t *cells_dev, int max_cells, int32_t *n_cells_dev, double *g_dev, void *scratch_dev,
-                    size_t scratch_bytes, int n_slots, int heap_cap, unsigned long long *counters_dev, void *stream);
-
-/* search slots of a batch that are resident at once (mpp_astar_max_slots for a batch); the scratch of
- * mpp_astar_batch_maps is 256 + n_slots * mpp_astar_slot_bytes(rows, cols, heap_cap) bytes, zero-filled once. */
-int mpp_map_batch_max_slots(const mpp_map_batch *maps);
-
-/* replaces one AStarSolver(grid).solve() (astar.py:33-101) / DijkstraSolver(grid).solve() (dijkstra.py:32-97) per map
- * of a sweep over independent maps, statistics (helper.py:98-113) included: mpp_astar_batch over a batch of same-shape
- * maps in one launch.  Query i runs on map map_dev[i] (any number of queries per map, each with its own endpoints and
- * avoid set); a query whose map index or endpoint lies outside the batch / map gets n_cells = 0 without a search.
- * Result conventions, avoid_bits_dev and counters_dev as mpp_astar_batch.  stats_policy (nullable): the lane group
- * computes the statistics of its own path right after the search into stats_dev (n x 5, as mpp_path_stats; mode 0
- * uses that map's safety table, mpp_map_batch_safety_table); a query with n_cells <= 0 or > max_cells gets the empty
- * path's (inf, 0, 0, 0, inf).  order_dev: optional permutation of 0..n-1 = the order in which free slots take the
- * queries (start the long ones first); results stay indexed by query.  n_slots <= mpp_map_batch_max_slots is useful. */
+ * dijkstra.py:32-97 = variant 0 with a zero heuristic), on a batch of same-shape maps in one launch -- with map
+ * indices, also one AStarSolver(grid).solve() / DijkstraSolver(grid).solve() per map of a sweep over independent maps.
+ * Query i runs on map map_dev[i] (any number of queries per map, each with its own endpoints and avoid set); a query
+ * whose map index or endpoint lies outside the batch / map gets n_cells = 0 without a search.  avoid_bits_dev:
+ * optional n x ceil(rows*cols/32) bitmaps (nodes_to_avoid).  cells_dev: n x max_cells; n_cells_dev[i] = path length
+ * (0 = no path / invalid endpoint, -1 = heap_cap overflow, > max_cells = truncated); g_dev[i] = g of the popped
+ * target (nullable).  counters_dev: optional [4] = (node expansions, successful relaxations, ring-bucket pushes,
+ * overflow-heap pushes), accumulated.  stats_policy (nullable): the lane group computes the statistics of its own path
+ * right after the search into stats_dev (n x 5, as mpp_path_stats; mode 0 uses that map's safety table,
+ * mpp_map_batch_safety_table); a query with n_cells <= 0 or > max_cells gets the empty path's (inf, 0, 0, 0, inf).
+ * order_dev: optional permutation of 0..n-1 = the order in which free slots take the queries (start the long ones
+ * first); results stay indexed by query.  n_slots <= mpp_map_batch_max_slots is useful.  A one-map batch whose
+ * occupancy fits is staged in shared memory by every block; larger maps and batches of several maps read it through
+ * L2. */
 int mpp_astar_batch_maps(mpp_map_batch *maps, int variant, const int32_t *map_dev, const int32_t *src_dev,
                          const int32_t *dst_dev, const uint32_t *avoid_bits_dev, int n, int allow_diagonal,
                          int restrict_corner, const mpp_policy *stats_policy, int32_t *cells_dev, int max_cells,
@@ -350,7 +323,7 @@ int mpp_astar_batch_maps(mpp_map_batch *maps, int variant, const int32_t *map_de
 /* ---- exact Dijkstra distance fields (dijkstra.py) -----------------------------------------------------------------
  * replaces DijkstraSolver.solve's search (dijkstra.py:32-97, with get_valid_neighbors helper.py:18-53) when one source
  * serves many targets, or a whole map's costs are wanted: ONE field per map gives every target's popped g and path.
- * mpp_dijkstra_fields: for every map k of the batch (a single map: mpp_map_as_batch), the complete field from cell
+ * mpp_dijkstra_fields: for every map k of the batch (a single map: a batch of one), the complete field from cell
  *   src_dev[k]: g_dev [n_maps][rows*cols] = the g with which dijkstra.py pops each cell (+inf: obstacle or unreachable),
  *   parent_dev [n_maps][rows*cols] = the move parent -> cell in the move order of helper.py:30-36 ((0,1), (0,-1), (1,0),
  *   (-1,0), (1,1), (1,-1), (-1,1), (-1,-1)), 0xFF = none (source, obstacle, unreachable).  Both are bit for bit what the
@@ -372,133 +345,85 @@ int mpp_dijkstra_field_paths(mpp_map_batch *maps, const double *g_dev, const uin
 
 /* replaces PSOSolver._reconstruct_path_from_position (pso.py:56-94, after rounding/clamping) /
  * GASolver._reconstruct_path_from_chromosome (ga_solver.py:58-93) followed by
- * BasePathfinder._calculate_stats_for_path (helper.py:138-147) for a whole population: one lane group (a warp)
- * per individual runs its W+1 connector searches with the growing avoid set and the statistics of the
- * joined path.  waypoints_dev: N x W cells.  visited_dev: N x ceil(rows*cols/32) words of scratch.
- * n_cells_dev[i]: 0 = invalid individual ([]), -1 = heap overflow, > max_cells = truncated.
+ * BasePathfinder._calculate_stats_for_path (helper.py:138-147) for whole populations, on a batch of same-shape maps in
+ * one launch: one lane group (a warp) per individual runs its W+1 connector searches with the growing avoid set and the
+ * statistics of the joined path.  Individual i runs on map map_dev[i] from that map's start, through its waypoints
+ * (waypoints_dev: N x W cells), to that map's target; mode 0 uses that map's safety table (mpp_map_batch_safety_table).
+ * An individual whose map index lies outside the batch (or whose map has no start / target) gets n_cells = 0 without a
+ * search.  visited_dev: n_slots x ceil(rows*cols/32) words of scratch (one bitmap per search slot).  Scratch as
+ * mpp_astar_batch_maps.  n_cells_dev[i]: 0 = invalid individual ([]), -1 = heap overflow, > max_cells = truncated.
  * order_dev: optional permutation of 0..N-1 = the order in which free search slots take individuals (the evaluation
- * lasts as long as its longest chain of searches: start the long ones first); results stay indexed by individual. */
-int mpp_waypoint_fitness(mpp_map *map, const int32_t *waypoints_dev, int n_individuals, int n_waypoints,
-                         const mpp_policy *policy, int32_t *cells_dev, int max_cells, int32_t *n_cells_dev,
-                         double *stats_dev, uint32_t *visited_dev, void *scratch_dev, size_t scratch_bytes,
-                         int n_slots, int heap_cap, unsigned long long *counters_dev, const int32_t *order_dev,
-                         void *stream);
-
-/* replaces one PSOSolver / GASolver fitness evaluation per (map, individual) of a sweep over independent maps:
- * _reconstruct_path_from_position (pso.py:56-94) / _reconstruct_path_from_chromosome (ga_solver.py:58-93) followed by
- * helper.calculate_path_stats (helper.py:98-113) -- mpp_waypoint_fitness over a batch of same-shape maps in one launch.
- * Individual i runs on map map_dev[i] from that map's start, through its waypoints, to that map's target; mode 0 uses
- * that map's safety table (mpp_map_batch_safety_table).  An individual whose map index lies outside the batch (or whose
- * map has no start / target) gets n_cells = 0 without a search.  visited_dev: n_slots x ceil(rows*cols/32) words of
- * scratch (one bitmap per search slot).  Scratch as mpp_astar_batch_maps; result conventions and order_dev as
- * mpp_waypoint_fitness. */
+ * lasts as long as its longest chain of searches: start the long ones first); results stay indexed by individual.
+ * Occupancy staging as mpp_astar_batch_maps. */
 int mpp_waypoint_fitness_maps(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *waypoints_dev,
                               int n_individuals, int n_waypoints, const mpp_policy *policy, int32_t *cells_dev,
                               int max_cells, int32_t *n_cells_dev, double *stats_dev, uint32_t *visited_dev,
                               void *scratch_dev, size_t scratch_bytes, int n_slots, int heap_cap,
                               unsigned long long *counters_dev, const int32_t *order_dev, void *stream);
 
-/* ---- PSO / GA population updates (pso.py, ga_solver.py) ------------------------------------------- */
-
-/* replaces the velocity/position update of the particle loop (pso.py:183-206) for particles
- * [particle_offset, particle_offset + n_particles) (device arrays start at that particle; a suffix is
- * re-run when an earlier particle improved gbest -- the reference's loop is asynchronous, pso.py:222-229).
- * pos/vel/pbest: n x W x 2 doubles (row, col); gbest: W x 2.  Exactly 4W uniforms per particle, stream
- * (seed, PSO_UPDATE, iteration, particle).  Also writes the integer waypoints pso.py:61,69-70
- * (round-half-even, clamped) as cells into waypoint_cells_dev (n x W). */
-int mpp_pso_update(const mpp_map *map, double *pos_dev, double *vel_dev, const double *pbest_pos_dev,
-                   const double *gbest_pos_dev, int n_particles, int particle_offset, int n_waypoints, double w,
-                   double c1, double c2, double max_vel, uint64_t seed, int iteration, int32_t *waypoint_cells_dev,
-                   void *stream);
-/* pso.py:61,69-70 alone (used for the initial particles) */
-int mpp_pso_round(const mpp_map *map, const double *pos_dev, int n_particles, int n_waypoints,
-                  int32_t *waypoint_cells_dev, void *stream);
-
-/* replaces GASolver._selection (ga_solver.py:136-142): n tournaments of min(tournament_size, n) individuals
- * drawn with CPython's random.sample algorithm (randbelow(n) = floor(u*n)); winner = first minimum in sample
- * order.  fitness_dev is in population (sorted) order; parents_dev receives n population indices.
- * Stream (seed, GA_SELECT, generation, tournament). */
-int mpp_ga_select(const double *fitness_dev, int n, int tournament_size, uint64_t seed, int generation,
-                  int32_t *parents_dev, void *stream);
-
-/* replaces the breeding loop ga_solver.py:186-194 (_crossover :144-152, _mutate :154-160,
- * _generate_random_waypoint :48-53): pair p = (parents[2p % n], parents[(2p+1) % n]) -> children 2p, 2p+1.
- * chrom_dev: n x W cells in population order; children_dev: n x W.  Stream (seed, GA_BREED, generation, pair). */
-int mpp_ga_breed(const mpp_map *map, const int32_t *chrom_dev, const int32_t *parents_dev, int n, int n_waypoints,
-                 double crossover_rate, double mutation_rate, uint64_t seed, int generation, int32_t *children_dev,
-                 void *stream);
-
 /* ---- MPA (MPA.py) ------------------------------------------------------------------------------- */
 
-/* replaces one iteration of MPA.solve_path_planning for the whole population (MPA.py:339-410): the
- * phase loop (:340-377: start index + gate draw, Levy :250-264 / Brownian :266-282 target,
- * _reconstruct_path_segment :284-318 with the private A* :106-151 and stats :215-229), the
- * marine-memory step (:380-384) and the FADs step (:387-410).  The old population (cells/n_cells/stats,
- * N x max_cells) must be sorted by fitness (row 0 = elite, :333-334); the next population is written
- * unsorted to out_*.  phase = 1/2/3 (:339,:348,:365), CF as computed at :336, levy_sigma as at :251-253.
- * tmp_cells_dev: n_slots x max_cells, avoid_dev: n_slots x ceil(rows*cols/32) words of scratch.
- * Only predators [pred_begin, pred_end) are processed (a rank's shard of the population; their rows of out_* are
- * written).  status_dev[0] (zero it first): 1 = heap overflow, 2 = a path exceeded max_cells (repeat with larger
- * buffers).  Streams (seed, MPA_PHASE, iteration, i) and (seed, MPA_FADS, iteration, i). */
-int mpp_mpa_iteration(mpp_map *map, const mpp_policy *policy, int n_predators, int pred_begin, int pred_end,
-                      int iteration, int phase,
-                      double P_const, double CF, double FADs_rate, double levy_sigma, double levy_beta, uint64_t seed,
-                      const int32_t *cells_dev, const int32_t *n_cells_dev, const double *stats_dev, int max_cells,
-                      int32_t *out_cells_dev, int32_t *out_n_dev, double *out_stats_dev, int32_t *tmp_cells_dev,
-                      uint32_t *avoid_dev, void *scratch_dev, size_t scratch_bytes, int n_slots, int heap_cap,
-                      int32_t *status_dev, unsigned long long *counters_dev, void *stream);
-
-/* MPA over a batch of independent same-shape maps (BASELINE config 5), one launch per iteration for every map.
- * Population buffers are [n_maps][n_predators][...] (cells: max_cells int32 per predator; stats: 5 doubles).
+/* MPA over a batch of independent same-shape maps (BASELINE config 5; a single map is a batch of one), one launch per
+ * iteration for every map.  Population buffers are [n_maps][n_predators][...] (cells: max_cells int32 per predator;
+ * stats: 5 doubles).
  * mpp_mpa_init_batch: MPA._initialize_population_with_safety (MPA.py:231-245) -- ONE private-A* search start -> target
  *   per map (the reference runs N identical ones); writes row 0 of every map (path, n_cells, stats); the caller
- *   replicates it.  scratch: 256 + n_maps * slot bytes (mpp_astar_scratch_bytes of a same-shape map with n_maps slots).
- * mpp_mpa_iteration_batch: mpp_mpa_iteration for every map at once.  order_dev [n_maps][n_predators] = stable argsort of
- *   the old population's fitness column (the sorts of MPA.py:333,412 as an index, no path is moved): predator i reads row
- *   order[i], the elite is row order[0]; results go to row i of the out buffers.  seeds_dev: one Philox seed per map;
- *   queue_dev: n_maps uint32 scratch; scratch: 256 + n_maps * warps_per_map slots. */
+ *   replicates it.  scratch: 256 + n_maps * mpp_astar_slot_bytes(rows, cols, heap_cap).
+ * mpp_mpa_iteration_batch: replaces one iteration of MPA.solve_path_planning for the whole population (MPA.py:339-410)
+ *   of every map: the phase loop (:340-377: start index + gate draw, Levy :250-264 / Brownian :266-282 target,
+ *   _reconstruct_path_segment :284-318 with the private A* :106-151 and stats :215-229), the marine-memory step
+ *   (:380-384) and the FADs step (:387-410).  The old population must be sorted by fitness (row 0 = elite, :333-334)
+ *   -- or order_dev [n_maps][n_predators] is the stable argsort of its fitness column (the sorts of MPA.py:333,412 as an
+ *   index, no path is moved): predator i reads row order[i], the elite is row order[0] (null: the identity).  The next
+ *   population is written unsorted to row i of the out buffers.  phase = 1/2/3 (:339,:348,:365), CF as computed at
+ *   :336, levy_sigma as at :251-253.  Only predators [pred_begin, pred_end) of every map are processed (a rank's shard
+ *   of the population; their rows of out_* are written).  seeds_dev: one Philox seed per map; streams (seed, MPA_PHASE,
+ *   iteration, i) and (seed, MPA_FADS, iteration, i).  tmp_cells_dev: n_maps * warps_per_map x max_cells, avoid_dev:
+ *   n_maps * warps_per_map x ceil(rows*cols/32) words of scratch; queue_dev: n_maps uint32 scratch; scratch:
+ *   256 + n_maps * warps_per_map slots.  status_dev[0] (zero it first): 1 = heap overflow, 2 = a path exceeded
+ *   max_cells (repeat with larger buffers).  The occupancy is staged in shared memory when it fits. */
 int mpp_mpa_init_batch(const mpp_map_batch *maps, const mpp_policy *policy, int n_predators, int max_cells,
                        int32_t *cells_dev, int32_t *n_cells_dev, double *stats_dev, void *scratch_dev,
                        size_t scratch_bytes, int heap_cap, int32_t *status_dev, unsigned long long *counters_dev,
                        void *stream);
-int mpp_mpa_iteration_batch(const mpp_map_batch *maps, const mpp_policy *policy, int n_predators, int iteration, int phase,
+int mpp_mpa_iteration_batch(const mpp_map_batch *maps, const mpp_policy *policy, int n_predators, int pred_begin,
+                            int pred_end, int iteration, int phase,
                             double P_const, double CF, double FADs_rate, double levy_sigma, double levy_beta,
                             const uint64_t *seeds_dev, const int32_t *order_dev, const int32_t *cells_dev,
                             const int32_t *n_cells_dev, const double *stats_dev, int max_cells, int32_t *out_cells_dev,
                             int32_t *out_n_dev, double *out_stats_dev, int32_t *tmp_cells_dev, uint32_t *avoid_dev,
                             void *scratch_dev, size_t scratch_bytes, int warps_per_map, int heap_cap, uint32_t *queue_dev,
                             int32_t *status_dev, unsigned long long *counters_dev, void *stream);
-/* bytes of one search slot's scratch for a rows x cols map (the per-slot term of mpp_astar_scratch_bytes) */
+/* bytes of one search slot's scratch for a rows x cols map */
 size_t mpp_astar_slot_bytes(int rows, int cols, int heap_cap);
 
-/* replaces the attempt generation of PSOSolver._initialize_particles (pso.py:97-105: W uniform waypoints + W x 2
- * uniform velocities per attempt) for attempts [attempt_offset, attempt_offset + n_attempts): pos_dev / vel_dev are
- * n_attempts x W x 2 doubles, waypoint_cells_dev the rounded, clamped cells (pso.py:61,69-70).  Stream (seed, PSO_INIT, 0,
- * attempt).  The accept / pad bookkeeping (pso.py:107-160) stays with the caller. */
-int mpp_pso_init(const mpp_map *map, int n_attempts, int attempt_offset, int n_waypoints, double max_vel, uint64_t seed,
-                 double *pos_dev, double *vel_dev, int32_t *waypoint_cells_dev, void *stream);
-
-/* replaces GASolver._create_chromosome (ga_solver.py:48-56: integer genes redrawn until the cell is free) for attempts
- * [attempt_offset, attempt_offset + n_attempts) of _initialize_population (:95-104).  chrom_dev: n_attempts x W cells.
- * Stream (seed, GA_INIT, 0, attempt). */
-int mpp_ga_init(const mpp_map *map, int n_attempts, int attempt_offset, int n_waypoints, uint64_t seed, int32_t *chrom_dev,
-                void *stream);
-
-/* ---- PSO / GA over a batch of independent same-shape maps (one launch per step for every map) -------------------
- * The same kernels as the single-map entry points above, with grid.y = map: map m's arrays are row m of
- * [n_maps][...] buffers, and it draws from the streams of seeds_dev[m] -- exactly what a per-map solver with
- * rng_seed = seeds[m] draws.  Replace a Python loop `for grid in grids: PSOSolver(grid, ...).solve()` /
- * `GASolver(grid, ...).solve()`.
- * mpp_pso_init_batch: pso.py:97-105, :50-51, :61, :69-70 -- attempts [off[m], off[m] + n_attempts) of every map with
- *   attempt_offset_dev[m] >= 0 (a negative offset: the map is done, its rows are not written).  pos / vel: [n_maps]
- *   [n_attempts][W][2], waypoint cells [n_maps][n_attempts][W].
- * mpp_ga_init_batch: ga_solver.py:48-56, :95-104 -- the same for chromosomes [n_maps][n_attempts][W].
- * mpp_pso_update_batch: pso.py:183-206 -- particles [start_dev[m], n_particles) of map m (start = n_particles: the map
- *   is idle; the particles below start are not touched).  pos / vel / pbest: [n_maps][n_particles][W][2], gbest
- *   [n_maps][W][2], waypoint cells [n_maps][n_particles][W].
- * mpp_ga_select_batch: ga_solver.py:136-142 over fitness [n_maps][n] -> parents [n_maps][n].
- * mpp_ga_breed_batch: ga_solver.py:144-160, :186-194 over chromosomes / children [n_maps][n][W]; mutated genes are
- *   free cells of the map's own grid. */
+/* ---- PSO / GA population updates (pso.py, ga_solver.py) ------------------------------------------------------------
+ * One launch per step for every map of a batch (grid.y = map): map m's arrays are row m of [n_maps][...] buffers, and
+ * it draws from the streams of seeds_dev[m] -- exactly what a per-map solver with rng_seed = seeds[m] draws (a single
+ * solver passes a one-map batch and one seed).  With several maps they replace a Python loop
+ * `for grid in grids: PSOSolver(grid, ...).solve()` / `GASolver(grid, ...).solve()`.
+ * mpp_pso_init_batch: replaces the attempt generation of PSOSolver._initialize_particles (pso.py:97-105: W uniform
+ *   waypoints + W x 2 uniform velocities per attempt, :50-51, the rounded, clamped cells :61, :69-70) for attempts
+ *   [off[m], off[m] + n_attempts) of every map with attempt_offset_dev[m] >= 0 (a negative offset: the map is done, its
+ *   rows are not written).  pos / vel: [n_maps][n_attempts][W][2], waypoint cells [n_maps][n_attempts][W].  Stream
+ *   (seed, PSO_INIT, 0, attempt).  The accept / pad bookkeeping (pso.py:107-160) stays with the caller.
+ * mpp_ga_init_batch: replaces GASolver._create_chromosome (ga_solver.py:48-56: integer genes redrawn until the cell is
+ *   free) for the attempts of _initialize_population (:95-104) -- the same for chromosomes [n_maps][n_attempts][W].
+ *   Stream (seed, GA_INIT, 0, attempt).
+ * mpp_pso_update_batch: replaces the velocity/position update of the particle loop (pso.py:183-206) for particles
+ *   [start_dev[m], n_particles) of map m (start = n_particles: the map is idle; the particles below start are not
+ *   touched; a suffix is re-run when an earlier particle improved gbest -- the reference's loop is asynchronous,
+ *   pso.py:222-229).  pos / vel / pbest: [n_maps][n_particles][W][2] doubles (row, col), gbest [n_maps][W][2].  Exactly
+ *   4W uniforms per particle, stream (seed, PSO_UPDATE, iteration, particle).  Also writes the integer waypoints
+ *   pso.py:61,69-70 (round-half-even, clamped) as cells into waypoint cells [n_maps][n_particles][W].
+ * mpp_ga_select_batch: replaces GASolver._selection (ga_solver.py:136-142) over fitness [n_maps][n] (population,
+ *   i.e. sorted, order) -> parents [n_maps][n] population indices: n tournaments of min(tournament_size, n)
+ *   individuals drawn with CPython's random.sample algorithm (randbelow(n) = floor(u*n)); winner = first minimum in
+ *   sample order.  Stream (seed, GA_SELECT, generation, tournament).
+ * mpp_ga_breed_batch: replaces the breeding loop ga_solver.py:186-194 (_crossover :144-152, _mutate :154-160,
+ *   _generate_random_waypoint :48-53) over chromosomes / children [n_maps][n][W] in population order: pair
+ *   p = (parents[2p % n], parents[(2p+1) % n]) -> children 2p, 2p+1; mutated genes are free cells of the map's own
+ *   grid.  Stream (seed, GA_BREED, generation, pair). */
 int mpp_pso_init_batch(const mpp_map_batch *maps, int n_attempts, const int32_t *attempt_offset_dev, int n_waypoints,
                        double max_vel, const uint64_t *seeds_dev, double *pos_dev, double *vel_dev,
                        int32_t *waypoint_cells_dev, void *stream);

@@ -50,20 +50,11 @@ _SIGS = {
     "mpp_abi_version": (c_int, []),
     "mpp_last_error": (C.c_char_p, []),
     "mpp_device_count": (c_int, []),
-    "mpp_map_create": (c_int, [c_void_p, c_int, c_int, c_int, C.POINTER(c_void_p)]),
-    "mpp_map_destroy": (None, [c_void_p]),
-    "mpp_map_rows": (c_int, [c_void_p]),
-    "mpp_map_cols": (c_int, [c_void_p]),
-    "mpp_map_start": (c_int, [c_void_p]),
-    "mpp_map_target": (c_int, [c_void_p]),
-    "mpp_map_device": (c_int, [c_void_p]),
-    "mpp_map_occ_bits": (c_void_p, [c_void_p, C.POINTER(c_int)]),
     "mpp_map_batch_create": (c_int, [c_void_p, c_int, c_int, c_int, c_int, C.POINTER(c_void_p)]),
     "mpp_map_batch_destroy": (None, [c_void_p]),
     "mpp_map_batch_size": (c_int, [c_void_p]),
     "mpp_map_batch_start": (c_int, [c_void_p, c_int]),
     "mpp_map_batch_target": (c_int, [c_void_p, c_int]),
-    "mpp_map_as_batch": (c_void_p, [c_void_p]),
     "mpp_map_batch_create_device": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, C.POINTER(c_void_p)]),
     "mpp_map_batch_occ_bits": (c_void_p, [c_void_p, C.POINTER(c_int)]),
     "mpp_map_batch_svalid": (c_void_p, [c_void_p]),
@@ -94,39 +85,24 @@ _SIGS = {
                                 c_void_p, c_int, c_int, c_void_p]),
     "mpp_maaco_xunpack": (c_int, [c_void_p, C.POINTER(Colony), c_void_p, C.c_longlong, c_int, c_int, c_int, c_void_p,
                                   c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
-    "mpp_map_safety_table": (c_int, [c_void_p, c_double, c_void_p]),
-    "mpp_path_stats": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, C.POINTER(Policy), c_void_p, c_void_p]),
-    "mpp_astar_scratch_bytes": (C.c_size_t, [c_void_p, c_int, c_int]),
-    "mpp_astar_max_slots": (c_int, [c_void_p]),
+    "mpp_path_stats": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, C.POINTER(Policy), c_void_p,
+                               c_void_p]),
     "mpp_map_batch_safety_table": (c_int, [c_void_p, c_double, c_void_p]),
     "mpp_map_batch_max_slots": (c_int, [c_void_p]),
     "mpp_astar_batch_maps": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                      C.POINTER(Policy), c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                                      C.c_size_t, c_int, c_int, c_void_p, c_void_p, c_void_p]),
-    "mpp_astar_batch": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int,
-                                c_void_p, c_void_p, c_void_p, C.c_size_t, c_int, c_int, c_void_p, c_void_p]),
-    "mpp_waypoint_fitness": (c_int, [c_void_p, c_void_p, c_int, c_int, C.POINTER(Policy), c_void_p, c_int, c_void_p,
-                                     c_void_p, c_void_p, c_void_p, C.c_size_t, c_int, c_int, c_void_p, c_void_p,
-                                     c_void_p]),
     "mpp_dijkstra_field_scratch_bytes": (C.c_size_t, [c_void_p]),
     "mpp_dijkstra_fields": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, C.c_size_t, c_void_p]),
     "mpp_dijkstra_field_paths": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, C.POINTER(Policy),
                                          c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
-    "mpp_pso_update": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_double,
-                               c_double, c_double, c_double, c_u64, c_int, c_void_p, c_void_p]),
-    "mpp_pso_round": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
-    "mpp_ga_select": (c_int, [c_void_p, c_int, c_int, c_u64, c_int, c_void_p, c_void_p]),
-    "mpp_ga_breed": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_double, c_double, c_u64, c_int, c_void_p,
-                             c_void_p]),
     "mpp_astar_slot_bytes": (C.c_size_t, [c_int, c_int, c_int]),
     "mpp_mpa_init_batch": (c_int, [c_void_p, C.POINTER(Policy), c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                                    C.c_size_t, c_int, c_void_p, c_void_p, c_void_p]),
-    "mpp_mpa_iteration_batch": (c_int, [c_void_p, C.POINTER(Policy), c_int, c_int, c_int, c_double, c_double, c_double,
-                                        c_double, c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+    "mpp_mpa_iteration_batch": (c_int, [c_void_p, C.POINTER(Policy), c_int, c_int, c_int, c_int, c_int, c_double, c_double,
+                                        c_double, c_double, c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
                                         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, C.c_size_t, c_int,
                                         c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
-    "mpp_pso_init": (c_int, [c_void_p, c_int, c_int, c_int, c_double, c_u64, c_void_p, c_void_p, c_void_p, c_void_p]),
-    "mpp_ga_init": (c_int, [c_void_p, c_int, c_int, c_int, c_u64, c_void_p, c_void_p]),
     "mpp_waypoint_fitness_maps": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, C.POINTER(Policy), c_void_p, c_int,
                                           c_void_p, c_void_p, c_void_p, c_void_p, C.c_size_t, c_int, c_int, c_void_p,
                                           c_void_p, c_void_p]),
@@ -138,10 +114,6 @@ _SIGS = {
     "mpp_ga_select_batch": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p]),
     "mpp_ga_breed_batch": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_double, c_double, c_void_p, c_int,
                                    c_void_p, c_void_p]),
-    "mpp_mpa_iteration": (c_int, [c_void_p, C.POINTER(Policy), c_int, c_int, c_int, c_int, c_int, c_double, c_double, c_double,
-                                  c_double, c_double, c_u64, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p,
-                                  c_void_p, c_void_p, c_void_p, c_void_p, C.c_size_t, c_int, c_int, c_void_p, c_void_p,
-                                  c_void_p]),
 }
 
 _lib = None

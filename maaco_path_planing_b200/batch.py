@@ -619,7 +619,7 @@ class MPABatch:
             phase = 1 if it <= K / 3 else (2 if it <= 2 * K / 3 else 3)
             nxt = cur ^ 1
             _lib.check(L.mpp_mpa_iteration_batch(
-                self._maps, C.byref(self.policy), N, it, phase, self.P_const, CF, self.FADs_rate, self._levy_sigma,
+                self._maps, C.byref(self.policy), N, 0, N, it, phase, self.P_const, CF, self.FADs_rate, self._levy_sigma,
                 self.levy_beta, _lib.ptr(seeds), _lib.ptr(order), _lib.ptr(cells[cur]), _lib.ptr(ncell[cur]),
                 _lib.ptr(stats[cur]), mc, _lib.ptr(cells[nxt]), _lib.ptr(ncell[nxt]), _lib.ptr(stats[nxt]), _lib.ptr(tmp),
                 _lib.ptr(avoid), _lib.ptr(scratch), scratch.numel(), self.warps_per_map, self.heap_cap, _lib.ptr(queue),
@@ -778,7 +778,9 @@ class SearchBatch:
                                   allow_diagonal_moves, mode=0)
         self.n = self.rows * self.cols
         self.words = (self.n + 31) // 32
-        self.heap_cap = int(heap_cap or min(8 * self.n, max(4096, self.n // 4)))        # SearchEngine's sizes
+        # a search's open set is a frontier: a few thousand entries on the largest maps; overflow is reported
+        # (n_cells = -1) and the search is repeated with a larger heap
+        self.heap_cap = int(heap_cap or min(8 * self.n, max(4096, self.n // 4)))
         self.max_cells = int(max_cells or min(self.n, max(4096, 16 * (self.rows + self.cols))))
         self.max_slots = L.mpp_map_batch_max_slots(self._maps)
         self.n_slots = int(n_slots or self.max_slots)
@@ -806,6 +808,23 @@ class SearchBatch:
             return a.to(device=self.device, dtype=torch.int32).contiguous()
         return torch.as_tensor(np.ascontiguousarray(a, dtype=np.int32), device=self.device)
 
+    def _stream(self):
+        import torch
+        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _grow_from(self, mn, mx):
+        """Heap overflow (mn < 0) or truncated paths (mx > max_cells) -> enlarge; True: the caller repeats."""
+        grew = False
+        if mn < 0:
+            if self.heap_cap >= 8 * self.n:
+                raise _lib.MppError("A* heap overflow at maximum capacity")
+            self.heap_cap = min(8 * self.n, self.heap_cap * 4)
+            grew = True
+        if mx > self.max_cells:
+            self.max_cells = min(2 * self.n, max(mx, 2 * self.max_cells))
+            grew = True
+        return grew
+
     def _scratch_for(self, n):
         """(scratch, search slots) for a launch over n queries / individuals with the current heap_cap."""
         import torch as t
@@ -816,8 +835,9 @@ class SearchBatch:
             self._scratch_key = (slots, self.heap_cap)
         return self._scratch, slots
 
-    def _launch(self, variant, mi, src, dst, avoid, longest_first):
-        """One mpp_astar_batch_maps launch over the given (valid) queries with the current sizes."""
+    def _launch(self, variant, mi, src, dst, avoid, longest_first, allow_diagonal, restrict_corner, policy):
+        """One mpp_astar_batch_maps launch over the given (valid) queries with the current sizes; stats is None when
+        policy is."""
         import torch as t
         n, mc = mi.numel(), self.max_cells
         _, slots = self._scratch_for(n)
@@ -830,17 +850,29 @@ class SearchBatch:
         cells = t.empty((n, mc), dtype=t.int32, device=self.device)
         ncell = t.empty(n, dtype=t.int32, device=self.device)
         g = t.empty(n, dtype=t.float64, device=self.device)
-        stats = t.empty((n, 5), dtype=t.float64, device=self.device)
-        stream = C.c_void_p(t.cuda.current_stream(self.device).cuda_stream)
+        stats = None if policy is None else t.empty((n, 5), dtype=t.float64, device=self.device)
         _lib.check(_lib.lib().mpp_astar_batch_maps(
             self._maps, int(variant), _lib.ptr(mi), _lib.ptr(src), _lib.ptr(dst), _lib.ptr(avoid), n,
-            int(self.allow_diagonal_moves), int(self.restrict_corners), C.byref(self.policy), _lib.ptr(cells), mc,
-            _lib.ptr(ncell), _lib.ptr(g), _lib.ptr(stats), _lib.ptr(self._scratch), self._scratch.numel(), slots,
-            self.heap_cap, _lib.ptr(self.counters), _lib.ptr(order), stream), "mpp_astar_batch_maps")
+            int(bool(allow_diagonal)), int(bool(restrict_corner)), None if policy is None else C.byref(policy),
+            _lib.ptr(cells), mc, _lib.ptr(ncell), _lib.ptr(g), _lib.ptr(stats), _lib.ptr(self._scratch),
+            self._scratch.numel(), slots, self.heap_cap, _lib.ptr(self.counters), _lib.ptr(order), self._stream()),
+            "mpp_astar_batch_maps")
         self.launches += 1
         return cells, ncell, g, stats
 
-    def _chain_launch(self, mi, wps):
+    def _chain_order(self, mi, wps):
+        """Individuals ordered by the Euclidean length of their waypoint chain, longest first (those outside the batch
+        last): a chain costs roughly the sum of its squared hop lengths, and the launch ends with its slowest
+        individual."""
+        import torch as t
+        ok = (mi >= 0) & (mi < self.n_maps)
+        m = mi.clamp(0, self.n_maps - 1).long()
+        chain = t.cat([self._start_dev[m][:, None], wps, self._target_dev[m][:, None]], dim=1).to(t.float64)
+        r, c = t.div(chain, self.cols, rounding_mode="floor"), chain % self.cols
+        d = ((r[:, 1:] - r[:, :-1]) ** 2 + (c[:, 1:] - c[:, :-1]) ** 2).sqrt().sum(dim=1)
+        return t.argsort(t.where(ok, d, -1.0), descending=True).to(t.int32).contiguous()
+
+    def _chain_launch(self, mi, wps, policy):
         """One mpp_waypoint_fitness_maps launch over individuals mi [n] (map index, -1 = not searched), wps [n, W] with the
         current sizes, longest chains first."""
         import torch as t
@@ -849,23 +881,14 @@ class SearchBatch:
         scratch, slots = self._scratch_for(n)
         if self._visited is None or self._visited.shape[0] < slots:
             self._visited = t.empty((slots, self.words), dtype=t.int32, device=self.device)
-        order = None
-        if n > slots // 2:
-            # a chain costs roughly the sum of its squared hop lengths; the launch ends with its slowest individual
-            ok = (mi >= 0) & (mi < self.n_maps)
-            m = mi.clamp(0, self.n_maps - 1).long()
-            chain = t.cat([self._start_dev[m][:, None], wps, self._target_dev[m][:, None]], dim=1).to(t.float64)
-            r, c = t.div(chain, self.cols, rounding_mode="floor"), chain % self.cols
-            d = ((r[:, 1:] - r[:, :-1]) ** 2 + (c[:, 1:] - c[:, :-1]) ** 2).sqrt().sum(dim=1)
-            order = t.argsort(t.where(ok, d, -1.0), descending=True).to(t.int32).contiguous()
+        order = self._chain_order(mi, wps) if n > slots // 2 else None
         cells = t.empty((n, mc), dtype=t.int32, device=self.device)
         ncell = t.empty(n, dtype=t.int32, device=self.device)
         stats = t.empty((n, 5), dtype=t.float64, device=self.device)
-        stream = C.c_void_p(t.cuda.current_stream(self.device).cuda_stream)
         _lib.check(_lib.lib().mpp_waypoint_fitness_maps(
-            self._maps, _lib.ptr(mi), _lib.ptr(wps), n, W, C.byref(self.policy), _lib.ptr(cells), mc, _lib.ptr(ncell),
+            self._maps, _lib.ptr(mi), _lib.ptr(wps), n, W, C.byref(policy), _lib.ptr(cells), mc, _lib.ptr(ncell),
             _lib.ptr(stats), _lib.ptr(self._visited), _lib.ptr(scratch), scratch.numel(), slots, self.heap_cap,
-            _lib.ptr(self.counters), _lib.ptr(order), stream), "mpp_waypoint_fitness_maps")
+            _lib.ptr(self.counters), _lib.ptr(order), self._stream()), "mpp_waypoint_fitness_maps")
         self.launches += 1
         return cells, ncell, stats
 
@@ -873,15 +896,15 @@ class SearchBatch:
         """After _grow_from enlarged the buffers: repeats the individuals whose heap overflowed or whose path was truncated
         (the searches are deterministic) until none is; returns the patched (cells, n_cells, stats)."""
         import torch as t
-        from .engine import SearchEngine
         while True:
             bad = ((ncell < 0) | (ncell > cells.shape[1])).nonzero().squeeze(1)
-            c, nc, st = self._chain_launch(mi.index_select(0, bad).contiguous(), wps.index_select(0, bad).contiguous())
+            c, nc, st = self._chain_launch(mi.index_select(0, bad).contiguous(), wps.index_select(0, bad).contiguous(),
+                                           self.policy)
             if c.shape[1] > cells.shape[1]:                                  # max_cells grew: widen the earlier rows
                 cells = t.nn.functional.pad(cells, (0, c.shape[1] - cells.shape[1]))
             cells[bad, :c.shape[1]] = c
             ncell[bad], stats[bad] = nc, st
-            if not SearchEngine._grow_from(self, *t.stack([nc.min(), nc.max()]).tolist()):
+            if not self._grow_from(*t.stack([nc.min(), nc.max()]).tolist()):
                 return cells, ncell, stats
 
     def chains(self, map_index, waypoints):
@@ -890,11 +913,10 @@ class SearchBatch:
         (cells [n, max_cells] int32, n_cells [n] int32, stats [n, 5] float64).  n_cells = 0: an invalid chain, or a map
         index outside the batch (not searched).  A heap overflow or a truncated path grows the buffers and repeats only
         those individuals."""
-        from .engine import SearchEngine
         import torch as t
         mi, wps = self._i32(map_index), self._i32(waypoints)
-        cells, ncell, stats = self._chain_launch(mi, wps)
-        if SearchEngine._grow_from(self, *t.stack([ncell.min(), ncell.max()]).tolist()):
+        cells, ncell, stats = self._chain_launch(mi, wps, self.policy)
+        if self._grow_from(*t.stack([ncell.min(), ncell.max()]).tolist()):
             cells, ncell, stats = self._chain_repeat(mi, wps, cells, ncell, stats)
         return cells, ncell, stats
 
@@ -906,7 +928,6 @@ class SearchBatch:
         path, or an endpoint / map index outside the batch (not searched).  A heap overflow or a truncated path grows
         the buffers and repeats only those queries (the searches are deterministic)."""
         import torch as t
-        from .engine import SearchEngine
         mi, src, dst = self._i32(map_index), self._i32(src), self._i32(dst)
         valid = _valid_queries(mi, src, dst, self.n_maps, self.n)
         n = mi.numel()
@@ -925,7 +946,8 @@ class SearchBatch:
         idx = valid.nonzero().squeeze(1)
         while idx.numel():
             sub = lambda x: None if x is None else x.index_select(0, idx).contiguous()
-            c, nc, gg, st = self._launch(variant, sub(mi), sub(src), sub(dst), sub(avoid), longest_first)
+            c, nc, gg, st = self._launch(variant, sub(mi), sub(src), sub(dst), sub(avoid), longest_first,
+                                         self.allow_diagonal_moves, self.restrict_corners, self.policy)
             if c.shape[1] > cells.shape[1]:                                  # max_cells grew: widen the earlier rows
                 wide = t.zeros((n, c.shape[1]), dtype=t.int32, device=self.device)
                 wide[:, :cells.shape[1]] = cells
@@ -933,7 +955,7 @@ class SearchBatch:
             cells[idx, :c.shape[1]] = c
             ncell[idx], g[idx], stats[idx] = nc, gg, st
             bad = (nc < 0) | (nc > c.shape[1])
-            if not SearchEngine._grow_from(self, int(nc.min().item()), int(nc.max().item())):
+            if not self._grow_from(int(nc.min().item()), int(nc.max().item())):
                 break
             idx = idx[bad]
         return cells, ncell, g, stats
@@ -1224,7 +1246,7 @@ class PSOBatch(_WaypointBatch):
                 act = ar[None, :] >= st_d[:, None]
                 mi = t.where(act, rows[:, None], -1).to(t.int32).reshape(-1)
                 wp = wp.reshape(M * N, W)
-                c_r, nc_r, s_r = self._search._chain_launch(mi, wp)
+                c_r, nc_r, s_r = self._search._chain_launch(mi, wp, self._search.policy)
                 for m in np.flatnonzero(start < N):
                     self.fitness_evaluations[m] += N - int(start[m])
                 while True:
@@ -1237,8 +1259,7 @@ class PSOBatch(_WaypointBatch):
                     nxt = t.where(hit, q + 1, N)
                     # the round's one host synchronise: buffer growth flags and the next round's start of every map
                     flags = t.cat([t.stack([nc_r.min(), nc_r.max()]).to(t.int64), nxt.to(t.int64)]).tolist()
-                    from .engine import SearchEngine
-                    if not SearchEngine._grow_from(self._search, flags[0], flags[1]):
+                    if not self._search._grow_from(flags[0], flags[1]):
                         break
                     c_r, nc_r, s_r = self._search._chain_repeat(mi, wp, c_r, nc_r, s_r)
                 upd = imp_p & (ar[None, :] <= q[:, None])                     # pso.py:217-220 for the final particles
@@ -1300,7 +1321,6 @@ class GABatch(_WaypointBatch):
         convergence_curve.  After it, chrom / fitness hold every map's final population in sorted order ([M, N, W],
         [M, N]; meaningful for maps whose initialisation found a valid chain)."""
         import torch as t
-        from .engine import SearchEngine
         if self.num_waypoints == 0:
             return self._solve_direct()
         M, N, W, K, dev = self.n_maps, self.population_size, self.num_waypoints, self.num_generations, self.device

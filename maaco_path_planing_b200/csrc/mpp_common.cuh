@@ -47,50 +47,26 @@ struct MppMapMeta {         // per-map scalars the MAACO kernels read from devic
 };
 MppMapMeta mpp_make_meta(int rows, int cols, int start, int target);
 
-// A batch of same-shape maps: what every MAACO launcher takes (grid.y / blockIdx.y = map).  A single mpp_map
-// owns a batch of one (`self_batch`) over its own buffers.
+// A batch of same-shape maps: what every launcher takes (grid.y / blockIdx.y = map); a single map is a batch of one.
 struct mpp_map_batch {
     int n_maps, rows, cols, device, sm_count;
-    int pitch_words, occ_words;
-    uint32_t *occ_dev;      // [n_maps][occ_words]
-    uint8_t *svalid_dev;    // [n_maps][rows*cols]
+    int pitch_words;        // padded occupancy row pitch (32-bit words)
+    int occ_words;          // (rows+2)*pitch_words, rounded up to a multiple of 4 words (16 B bulk copies)
+    uint32_t *occ_dev;      // [n_maps][occ_words] border-padded bit-packed occupancy; bit (r+1, c+1); border = 1
+    uint8_t *svalid_dev;    // [n_maps][rows*cols] static move masks, MAACO move order (bounds/obstacle/corner-cut)
     MppMapMeta *meta_dev;   // [n_maps]
     MppMapMeta *meta_host;  // [n_maps]
-    uint8_t *grid_host;     // [n_maps][rows*cols] (host copy for host-side table builds), may be null for views
-    int owns;               // 1 = buffers are freed by mpp_map_batch_destroy
+    uint8_t *grid_host;     // [n_maps][rows*cols] (host copy for host-side table builds), null for device-built batches
     long long n_obstacles;  // over all maps (0 = no map needs a safety table)
-    // safety-class cache of every map (helper.py:67-80, see mpp_map below); built by mpp_map_batch_safety_table
+    // safety-class cache of every map (helper.py:67-80); built by mpp_map_batch_safety_table
     double safety_msd;      // msd the tables were built for (<0 = none)
-    uint16_t *safety_d2_dev; // [n_maps][rows*cols]
+    uint16_t *safety_d2_dev; // [n_maps][rows*cols]: min d^2 to an obstacle inside the (2*floor(msd)+1)^2 stencil, 0 = none
     double *safety_lut_dev; // safety_lut_n doubles, shared by every map (the LUT depends on msd only)
     int safety_lut_n;
 };
 
-struct mpp_map {
-    int rows, cols, device;
-    int start, target;      // cell ids or -1
-    int pitch_words;        // padded occupancy row pitch (32-bit words)
-    int occ_words;          // (rows+2)*pitch_words, rounded up to a multiple of 4 words (16 B bulk copies)
-    uint32_t *occ_dev;      // border-padded bit-packed occupancy; bit (r+1, c+1); border = 1
-    uint8_t *svalid_dev;    // per-cell static move mask, MAACO move order (bounds/obstacle/corner-cut)
-    uint8_t *grid_host;     // host copy of the caller's grid (rows*cols) for host-side table builds
-    int n_obstacles;
-    int sm_count;
-    // safety-class cache (helper.py:67-80): per cell min d^2 to an obstacle inside the (2*floor(msd)+1)^2 stencil, 0 = none
-    double safety_msd;      // msd the table was built for (<0 = none)
-    uint16_t *safety_d2_dev; // rows*cols
-    double *safety_lut_dev; // safety_lut_n doubles: penalty contribution for class d^2
-    int safety_lut_n;
-    mpp_map_batch self_batch; // this map as a batch of one (view; meta_dev / meta_host owned by the map)
-};
-
 int mpp_check_device(int device);
 
-// Builds the safety-class tables of n_maps maps whose occupancy is laid out [n_maps][occ_words] (mpp_astar.cu): one
-// kernel launch (grid.y = map) into *d2 ([n_maps][rows*cols] u16) and one LUT for msd into *lut, (re)allocating both
-// as needed and recording msd in *cached_msd.  Shared by mpp_map_safety_table and mpp_map_batch_safety_table.
-int mpp_build_safety(int device, const uint32_t *occ, int occ_words, int pitch_words, int rows, int cols, int n_maps,
-                     double msd, cudaStream_t s, double *cached_msd, uint16_t **d2, double **lut, int *lut_n);
 
 // ---------------------------------------------------------------------------------------------
 // Philox4x32-10 streams (RNG contract)

@@ -16,7 +16,6 @@
 //     field.
 // (A* is another matter: with a floating-point heuristic it can pop a cell one ulp above g*, so it has no field form.)
 #include <cooperative_groups.h>
-#include <cstddef>
 
 #include "mpp_astar.cuh"
 #include "mpp_stats.cuh"
@@ -260,20 +259,8 @@ extern "C" int mpp_dijkstra_field_paths(mpp_map_batch *maps, const double *g_dev
     FieldPathArgs A;
     memset(&A, 0, sizeof(A));
     if (stats_policy) {
-        A.X.occ = maps->occ_dev; A.X.pitch = maps->pitch_words; A.X.R = maps->rows; A.X.C = maps->cols;
-        A.X.pol = *stats_policy;
-        if (stats_policy->mode == 0 && maps->n_obstacles > 0) {  // an obstacle-free map's classes are all 0 (penalty 0.0)
-            if (maps->owns) {
-                const int rc = mpp_map_batch_safety_table(maps, stats_policy->min_safe_distance, stream);
-                if (rc) return rc;
-                A.X.cls = maps->safety_d2_dev; A.X.lut = maps->safety_lut_dev;
-            } else {                                             // mpp_map_as_batch: the map keeps its own table
-                mpp_map *map = (mpp_map *)((char *)maps - offsetof(mpp_map, self_batch));
-                const int rc = mpp_map_safety_table(map, stats_policy->min_safe_distance, stream);
-                if (rc) return rc;
-                A.X.cls = map->safety_d2_dev; A.X.lut = map->safety_lut_dev;
-            }
-        }
+        const int rc = mpp_stats_ctx(maps, stats_policy, stream, &A.X);
+        if (rc) return rc;
         A.stats = stats_dev;
     }
     A.C = maps->cols; A.rc = maps->rows * maps->cols; A.n_maps = maps->n_maps; A.n = n;

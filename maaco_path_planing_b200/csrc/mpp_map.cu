@@ -1,5 +1,5 @@
-// mpp_map.cu -- grid-map handle: env.py grid (list-of-lists of 0/1/2/3) -> border-padded,
-// bit-packed occupancy tensor in HBM + the per-map safety-class table (helper.py:67-80).
+// mpp_map.cu -- map-batch handle: env.py grids (list-of-lists of 0/1/2/3) -> border-padded,
+// bit-packed occupancy tensors in HBM + per-map metadata (the safety-class tables, helper.py:67-80, are in mpp_astar.cu).
 #include <stdarg.h>
 #include <stdlib.h>
 
@@ -95,55 +95,6 @@ __global__ void mpp_svalid_kernel(const uint32_t *__restrict__ occ, int occ_word
     sv[i] = (uint8_t)mask;
 }
 
-extern "C" int mpp_map_create(const uint8_t *grid_host, int rows, int cols, int device, mpp_map **out) {
-    MPP_REQUIRE(grid_host && out, "mpp_map_create: null argument");
-    MPP_REQUIRE(rows > 0 && cols > 0 && (long long)rows * cols < (1ll << 30), "mpp_map_create: bad shape %dx%d", rows, cols);
-    int rc = mpp_check_device(device);
-    if (rc) return rc;
-    MPP_CUDA(cudaSetDevice(device));
-    mpp_map *m = (mpp_map *)calloc(1, sizeof(mpp_map));
-    if (!m) { mpp_set_error("out of host memory"); return MPP_ENOMEM; }
-    m->rows = rows; m->cols = cols; m->device = device;
-    m->start = m->target = -1;
-    m->safety_msd = -1.0;
-    size_t n = (size_t)rows * cols;
-    m->grid_host = (uint8_t *)malloc(n);
-    memcpy(m->grid_host, grid_host, n);
-    for (size_t i = 0; i < n; ++i) {
-        uint8_t v = grid_host[i];
-        if (v == 2 && m->start < 0) m->start = (int)i;   // first row-major hit, MAACO.py:32-41
-        if (v == 3 && m->target < 0) m->target = (int)i;
-        if (v == 1) m->n_obstacles++;
-    }
-    m->pitch_words = (cols + 2 + 31) / 32;
-    int words = (rows + 2) * m->pitch_words;
-    m->occ_words = (words + 3) & ~3;
-    MPP_CUDA(cudaDeviceGetAttribute(&m->sm_count, cudaDevAttrMultiProcessorCount, device));
-    uint8_t *gdev = nullptr;
-    MPP_CUDA(cudaMalloc(&gdev, n));
-    MPP_CUDA(cudaMalloc(&m->occ_dev, (size_t)m->occ_words * 4));
-    MPP_CUDA(cudaMemcpy(gdev, grid_host, n, cudaMemcpyHostToDevice));
-    mpp_pack_occ_kernel<<<(m->occ_words + 255) / 256, 256>>>(gdev, rows, cols, m->pitch_words, m->occ_words, m->occ_dev);
-    MPP_CUDA(cudaGetLastError());
-    MPP_CUDA(cudaMalloc(&m->svalid_dev, n));
-    mpp_svalid_kernel<<<((int)n + 255) / 256, 256>>>(m->occ_dev, m->occ_words, m->pitch_words, rows, cols, m->svalid_dev);
-    MPP_CUDA(cudaGetLastError());
-    // the map as a batch of one (what the MAACO entry points take)
-    mpp_map_batch &B = m->self_batch;
-    B.n_maps = 1; B.rows = rows; B.cols = cols; B.device = device; B.sm_count = m->sm_count;
-    B.pitch_words = m->pitch_words; B.occ_words = m->occ_words;
-    B.occ_dev = m->occ_dev; B.svalid_dev = m->svalid_dev; B.grid_host = m->grid_host; B.owns = 0;
-    B.n_obstacles = m->n_obstacles; B.safety_msd = -1.0;
-    B.meta_host = (MppMapMeta *)malloc(sizeof(MppMapMeta));
-    *B.meta_host = mpp_make_meta(rows, cols, m->start, m->target);
-    MPP_CUDA(cudaMalloc(&B.meta_dev, sizeof(MppMapMeta)));
-    MPP_CUDA(cudaMemcpy(B.meta_dev, B.meta_host, sizeof(MppMapMeta), cudaMemcpyHostToDevice));
-    MPP_CUDA(cudaDeviceSynchronize());
-    MPP_CUDA(cudaFree(gdev));
-    *out = m;
-    return MPP_OK;
-}
-
 static uint32_t host_orient_mask(int dR, int dC) {                // MAACO.py:146-157
     uint32_t k = 0xffu;
     if (dC > 0) k &= ~0x29u;
@@ -172,10 +123,8 @@ MppMapMeta mpp_make_meta(int rows, int cols, int start, int target) {
     return M;
 }
 
-extern "C" const mpp_map_batch *mpp_map_as_batch(const mpp_map *m) { return m ? &m->self_batch : nullptr; }
-
 // A batch of n_maps same-shape maps (BASELINE config 5: independent maps, one launch per colony pass of the
-// whole batch).  grids_host: n_maps * rows * cols bytes.
+// whole batch; a single map is a batch of one).  grids_host: n_maps * rows * cols bytes.
 extern "C" int mpp_map_batch_create(const uint8_t *grids_host, int n_maps, int rows, int cols, int device,
                                     mpp_map_batch **out) {
     MPP_REQUIRE(grids_host && out, "mpp_map_batch_create: null argument");
@@ -186,7 +135,7 @@ extern "C" int mpp_map_batch_create(const uint8_t *grids_host, int n_maps, int r
     MPP_CUDA(cudaSetDevice(device));
     mpp_map_batch *B = (mpp_map_batch *)calloc(1, sizeof(mpp_map_batch));
     if (!B) { mpp_set_error("out of host memory"); return MPP_ENOMEM; }
-    B->n_maps = n_maps; B->rows = rows; B->cols = cols; B->device = device; B->owns = 1;
+    B->n_maps = n_maps; B->rows = rows; B->cols = cols; B->device = device;
     B->safety_msd = -1.0;
     const size_t n = (size_t)rows * cols;
     B->grid_host = (uint8_t *)malloc(n * n_maps);
@@ -345,7 +294,7 @@ extern "C" int mpp_map_batch_create_device(const void *grids_dev, int elem_bytes
                 "mpp_map_batch_create_device: grids_dev is not memory of device %d", device);
     mpp_map_batch *B = (mpp_map_batch *)calloc(1, sizeof(mpp_map_batch));
     if (!B) { mpp_set_error("out of host memory"); return MPP_ENOMEM; }
-    B->n_maps = n_maps; B->rows = rows; B->cols = cols; B->device = device; B->owns = 1;
+    B->n_maps = n_maps; B->rows = rows; B->cols = cols; B->device = device;
     B->safety_msd = -1.0;
     rc = map_batch_ingest(B, grids_dev, elem_bytes, (cudaStream_t)stream);
     if (rc) {
@@ -357,7 +306,7 @@ extern "C" int mpp_map_batch_create_device(const void *grids_dev, int elem_bytes
 }
 
 extern "C" void mpp_map_batch_destroy(mpp_map_batch *B) {
-    if (!B || !B->owns) return;
+    if (!B) return;
     cudaSetDevice(B->device);
     if (B->occ_dev) cudaFree(B->occ_dev);
     if (B->svalid_dev) cudaFree(B->svalid_dev);
@@ -378,27 +327,3 @@ extern "C" const uint32_t *mpp_map_batch_occ_bits(const mpp_map_batch *B, int *p
 }
 extern "C" const uint8_t *mpp_map_batch_svalid(const mpp_map_batch *B) { return B ? B->svalid_dev : nullptr; }
 extern "C" long long mpp_map_batch_obstacles(const mpp_map_batch *B) { return B ? B->n_obstacles : -1; }
-
-extern "C" void mpp_map_destroy(mpp_map *m) {
-    if (!m) return;
-    cudaSetDevice(m->device);
-    if (m->occ_dev) cudaFree(m->occ_dev);
-    if (m->svalid_dev) cudaFree(m->svalid_dev);
-    if (m->safety_d2_dev) cudaFree(m->safety_d2_dev);
-    if (m->safety_lut_dev) cudaFree(m->safety_lut_dev);
-    if (m->self_batch.meta_dev) cudaFree(m->self_batch.meta_dev);
-    free(m->self_batch.meta_host);
-    free(m->grid_host);
-    free(m);
-}
-
-extern "C" int mpp_map_rows(const mpp_map *m) { return m ? m->rows : -1; }
-extern "C" int mpp_map_cols(const mpp_map *m) { return m ? m->cols : -1; }
-extern "C" int mpp_map_start(const mpp_map *m) { return m ? m->start : -1; }
-extern "C" int mpp_map_target(const mpp_map *m) { return m ? m->target : -1; }
-extern "C" int mpp_map_device(const mpp_map *m) { return m ? m->device : -1; }
-extern "C" const uint32_t *mpp_map_occ_bits(const mpp_map *m, int *pitch_words) {
-    if (!m) return nullptr;
-    if (pitch_words) *pitch_words = m->pitch_words;
-    return m->occ_dev;
-}

@@ -17,12 +17,10 @@ struct MpaArgs {
     AStarGrid G;
     int occ_words;
     StatsCtx X;
-    int start, target;
     int N, iteration, phase;          // phase 1/2/3 (MPA.py:339,348,365)
-    int pred_begin, pred_end;         // predators handled by this launch (a rank's shard)
+    int pred_begin, pred_end;         // predators of every map handled by this launch (a rank's shard)
     double P_const, CF, FADs_rate, levy_sigma, levy_inv_beta;
-    uint32_t k0, k1;
-    const int32_t *cells;             // old population, sorted: N x max_cells
+    const int32_t *cells;             // old population, sorted (or through `order`): N x max_cells
     const int32_t *n_cells;
     const double *stats;              // N x 5
     int max_cells;
@@ -37,8 +35,8 @@ struct MpaArgs {
     int32_t *status;                  // [0] = worst status seen (0 ok, 1 = heap overflow, 2 = path truncated)
     unsigned long long *counters;
     // ---- batches of independent same-shape maps (blockIdx.y = map; a single map is a batch of one) ----
-    const MppMapMeta *meta;           // per-map start / target (null: A.start / A.target)
-    const uint64_t *seeds;            // per-map Philox seed (null: k0 / k1)
+    const MppMapMeta *meta;           // per-map start / target
+    const uint64_t *seeds;            // per-map Philox seed
     const int32_t *order;             // [n_maps][N]: predator i of the (sorted) population is row order[i] (null: identity)
     unsigned int *queue;              // [n_maps] work counters
     int warps_per_map;                // search slots serving one map
@@ -142,8 +140,8 @@ __global__ void __launch_bounds__(MPP_MPA_THREADS, 3) mpp_mpa_iteration_kernel(M
     unsigned int *next = A.queue + map;
     uint32_t *avoid = A.avoid + (size_t)slot * A.words;
     int32_t *tmp = A.tmp_cells + (size_t)slot * A.max_cells;
-    if (A.meta) { A.start = A.meta[map].start; A.target = A.meta[map].target; }
-    if (A.seeds) { const uint64_t sd = A.seeds[map]; A.k0 = (uint32_t)sd; A.k1 = (uint32_t)(sd >> 32); }
+    const int start = A.meta[map].start, target = A.meta[map].target;
+    const uint64_t seed = A.seeds[map];
     {   // this map's slice of the population buffers
         const size_t pm = (size_t)map * A.N;
         A.cells += pm * A.max_cells; A.n_cells += pm; A.stats += pm * 5;
@@ -189,7 +187,7 @@ __global__ void __launch_bounds__(MPP_MPA_THREADS, 3) mpp_mpa_iteration_kernel(M
         int n_new = nP;            // candidate defaults to path_to_modify with its stats
         bool rebuilt = false;
         mpp_stream_rng rng;
-        rng.init(((uint64_t)A.k1 << 32) | A.k0, MPP_CLS_MPA_PHASE, (uint32_t)A.iteration, (uint32_t)i);
+        rng.init(seed, MPP_CLS_MPA_PHASE, (uint32_t)A.iteration, (uint32_t)i);
         if (nP > 1) {
             const int idx = rng.below(nP - 1);                                     // randint(0, len-2)
             if (rng.draw() < gate_p) {
@@ -218,15 +216,15 @@ __global__ void __launch_bounds__(MPP_MPA_THREADS, 3) mpp_mpa_iteration_kernel(M
                         a_start = inter;
                     }
                 }
-                if (a_start != A.target && st_flag == 0) {                         // :306-309
+                if (a_start != target && st_flag == 0) {                           // :306-309
                     const int cap = A.max_cells - (n - 1);
-                    const int sl = astar_search(L, G, S, 1, a_start, A.target, avoid, out + (n - 1), cap, nullptr, A.counters);
+                    const int sl = astar_search(L, G, S, 1, a_start, target, avoid, out + (n - 1), cap, nullptr, A.counters);
                     if (sl < 0) st_flag = 1;
                     else if (sl > cap) st_flag = 2;
                     else if (sl > 1) n += sl - 1;
                 }
                 // (consecutive duplicates cannot occur; :310-315 is a no-op)
-                if (st_flag == 0 && n > 0 && out[0] == A.start && out[n - 1] == A.target) {   // :316
+                if (st_flag == 0 && n > 0 && out[0] == start && out[n - 1] == target) {       // :316
                     n_new = n;
                     rebuilt = true;
                     path_stats_warp(L, X, out, n, ostats);
@@ -248,14 +246,14 @@ __global__ void __launch_bounds__(MPP_MPA_THREADS, 3) mpp_mpa_iteration_kernel(M
         }
         // ---------------- FADs MPA.py:387-410 ----------------
         mpp_stream_rng fr;
-        fr.init(((uint64_t)A.k1 << 32) | A.k0, MPP_CLS_MPA_FADS, (uint32_t)A.iteration, (uint32_t)i);
+        fr.init(seed, MPP_CLS_MPA_FADS, (uint32_t)A.iteration, (uint32_t)i);
         if (fr.draw() < A.FADs_rate && st_flag == 0) {
             int n2 = 0;
             if (fr.draw() < A.CF) {
                 const int r = fr.below(G.R), c = fr.below(G.C);                    // :391
                 const int node = r * C + c;
                 if (!occ_bit(G, r, c)) {
-                    const int sl1 = astar_search(L, G, S, 1, A.start, node, nullptr, tmp, A.max_cells, nullptr, A.counters);
+                    const int sl1 = astar_search(L, G, S, 1, start, node, nullptr, tmp, A.max_cells, nullptr, A.counters);
                     if (sl1 < 0) st_flag = 1;
                     else if (sl1 > A.max_cells) st_flag = 2;
                     else if (sl1 > 0) {
@@ -263,17 +261,17 @@ __global__ void __launch_bounds__(MPP_MPA_THREADS, 3) mpp_mpa_iteration_kernel(M
                         grp_sync(L);
                         warp_mark(L, avoid, tmp, sl1 - 1);                            // set(p1[:-1]) :396
                         const int cap = A.max_cells - (sl1 - 1);
-                        const int sl2 = astar_search(L, G, S, 1, node, A.target, avoid, tmp + (sl1 - 1), cap, nullptr, A.counters);
+                        const int sl2 = astar_search(L, G, S, 1, node, target, avoid, tmp + (sl1 - 1), cap, nullptr, A.counters);
                         if (sl2 < 0) st_flag = 1;
                         else if (sl2 > cap) st_flag = 2;
                         else if (sl2 > 0) {
                             const int nn = sl1 + sl2 - 1;                          // p1 + p2[1:]
-                            if (tmp[nn - 1] == A.target) n2 = nn;                  // :400
+                            if (tmp[nn - 1] == target) n2 = nn;                    // :400
                         }
                     }
                 }
             } else {
-                const int sl = astar_search(L, G, S, 1, A.start, A.target, nullptr, tmp, A.max_cells, nullptr, A.counters);  // :405
+                const int sl = astar_search(L, G, S, 1, start, target, nullptr, tmp, A.max_cells, nullptr, A.counters);  // :405
                 if (sl < 0) st_flag = 1;
                 else if (sl > A.max_cells) st_flag = 2;
                 else if (sl > 0) n2 = sl;
@@ -311,65 +309,28 @@ static int mpa_launch(MpaArgs &A, int n_maps, int device, size_t occ_bytes, cuda
     return MPP_OK;
 }
 
-extern "C" int mpp_mpa_iteration(mpp_map *map, const mpp_policy *policy, int n_predators, int pred_begin, int pred_end,
-                                 int iteration, int phase,
-                                 double P_const, double CF, double FADs_rate, double levy_sigma, double levy_beta,
-                                 uint64_t seed, const int32_t *cells_dev, const int32_t *n_cells_dev,
-                                 const double *stats_dev, int max_cells, int32_t *out_cells_dev, int32_t *out_n_dev,
-                                 double *out_stats_dev, int32_t *tmp_cells_dev, uint32_t *avoid_dev, void *scratch_dev,
-                                 size_t scratch_bytes, int n_slots, int heap_cap, int32_t *status_dev,
-                                 unsigned long long *counters_dev, void *stream) {
-    MPP_REQUIRE(map && policy && cells_dev && n_cells_dev && stats_dev && out_cells_dev && out_n_dev && out_stats_dev &&
-                    tmp_cells_dev && avoid_dev && scratch_dev && status_dev, "mpp_mpa_iteration: null argument");
-    MPP_REQUIRE(n_predators > 0 && max_cells > 1 && phase >= 1 && phase <= 3, "mpp_mpa_iteration: bad sizes");
-    MPP_REQUIRE(pred_begin >= 0 && pred_begin <= pred_end && pred_end <= n_predators, "mpp_mpa_iteration: bad predator range");
-    if (pred_begin == pred_end) return MPP_OK;
-    MPP_REQUIRE(map->start >= 0 && map->target >= 0, "mpp_mpa_iteration: map has no start/target");
-    MPP_REQUIRE(n_slots > 0 && heap_cap >= 64 && scratch_bytes >= mpp_astar_scratch_bytes(map, n_slots, heap_cap),
-                "mpp_mpa_iteration: scratch too small");
-    MPP_REQUIRE(map->rows < 32768 && map->cols < 65536, "mpp_mpa_iteration: map %dx%d exceeds the packed-node limit "
-                "(rows < 32768, cols < 65536)", map->rows, map->cols);
-    MPP_CUDA(cudaSetDevice(map->device));
-    cudaStream_t s = (cudaStream_t)stream;
-    MpaArgs A;
-    A.X.occ = map->occ_dev; A.X.pitch = map->pitch_words; A.X.R = map->rows; A.X.C = map->cols;
-    A.X.pol = *policy; A.X.pol.mode = 1; A.X.cls = nullptr; A.X.lut = nullptr;     // MPA.py:164-173: safety = 0.0
-    MPP_CUDA(cudaMemsetAsync(scratch_dev, 0, 256, s));
-    A.G.occ = map->occ_dev; A.G.pitch = map->pitch_words; A.G.R = map->rows; A.G.C = map->cols;
-    A.G.allow_diag = policy->allow_diagonal; A.G.restrict_corner = policy->restrict_policy;
-    A.occ_words = map->occ_words; A.start = map->start; A.target = map->target;
-    A.N = n_predators; A.iteration = iteration; A.phase = phase;
-    A.pred_begin = pred_begin; A.pred_end = pred_end;
-    A.P_const = P_const; A.CF = CF; A.FADs_rate = FADs_rate; A.levy_sigma = levy_sigma; A.levy_inv_beta = 1.0 / levy_beta;
-    A.k0 = (uint32_t)seed; A.k1 = (uint32_t)(seed >> 32);
-    A.cells = cells_dev; A.n_cells = n_cells_dev; A.stats = stats_dev; A.max_cells = max_cells;
-    A.out_cells = out_cells_dev; A.out_n = out_n_dev; A.out_stats = out_stats_dev;
-    A.tmp_cells = tmp_cells_dev; A.avoid = avoid_dev; A.words = (map->rows * map->cols + 31) / 32;
-    A.scratch = (char *)scratch_dev; A.n_slots = n_slots; A.heap_cap = heap_cap; A.status = status_dev;
-    A.counters = counters_dev;
-    A.meta = nullptr; A.seeds = nullptr; A.order = nullptr; A.queue = (unsigned int *)scratch_dev; A.warps_per_map = n_slots;
-    return mpa_launch(A, 1, map->device, (size_t)map->occ_words * 4, s);
-}
-
 // ---------------------------------------------------------------------------------------------
-// Batches of independent same-shape maps (BASELINE config 5): one launch serves the predators of every map
-// (blockIdx.y = map; `warps_per_map` search slots and one work queue per map).  The population buffers are
-// [n_maps][N][...]; the kernel reads the OLD population through `order` (the stable argsort of its fitness column,
-// computed on the device by the caller), so the sorts of MPA.py:333,412 never move a path.
+// Batches of independent same-shape maps (BASELINE config 5; a single map is a batch of one): one launch serves the
+// predators of every map (blockIdx.y = map; `warps_per_map` search slots and one work queue per map).  The population
+// buffers are [n_maps][N][...]; the kernel reads the OLD population through `order` when given (the stable argsort of
+// its fitness column, computed on the device by the caller), so the sorts of MPA.py:333,412 never move a path.
 // ---------------------------------------------------------------------------------------------
-extern "C" int mpp_mpa_iteration_batch(const mpp_map_batch *maps, const mpp_policy *policy, int n_predators, int iteration,
-                                       int phase, double P_const, double CF, double FADs_rate, double levy_sigma,
+extern "C" int mpp_mpa_iteration_batch(const mpp_map_batch *maps, const mpp_policy *policy, int n_predators,
+                                       int pred_begin, int pred_end, int iteration, int phase, double P_const, double CF, double FADs_rate, double levy_sigma,
                                        double levy_beta, const uint64_t *seeds_dev, const int32_t *order_dev,
                                        const int32_t *cells_dev, const int32_t *n_cells_dev, const double *stats_dev,
                                        int max_cells, int32_t *out_cells_dev, int32_t *out_n_dev, double *out_stats_dev,
                                        int32_t *tmp_cells_dev, uint32_t *avoid_dev, void *scratch_dev, size_t scratch_bytes,
                                        int warps_per_map, int heap_cap, uint32_t *queue_dev, int32_t *status_dev,
                                        unsigned long long *counters_dev, void *stream) {
-    MPP_REQUIRE(maps && policy && seeds_dev && order_dev && cells_dev && n_cells_dev && stats_dev && out_cells_dev &&
+    MPP_REQUIRE(maps && policy && seeds_dev && cells_dev && n_cells_dev && stats_dev && out_cells_dev &&
                     out_n_dev && out_stats_dev && tmp_cells_dev && avoid_dev && scratch_dev && queue_dev && status_dev,
                 "mpp_mpa_iteration_batch: null argument");
     MPP_REQUIRE(n_predators > 0 && max_cells > 1 && phase >= 1 && phase <= 3 && warps_per_map > 0 && heap_cap >= 64,
                 "mpp_mpa_iteration_batch: bad sizes");
+    MPP_REQUIRE(pred_begin >= 0 && pred_begin <= pred_end && pred_end <= n_predators,
+                "mpp_mpa_iteration_batch: bad predator range");
+    if (pred_begin == pred_end) return MPP_OK;
     MPP_REQUIRE(maps->rows < 32768 && maps->cols < 65536, "mpp_mpa_iteration_batch: map exceeds the packed-node limit");
     const int rc = maps->rows * maps->cols;
     const size_t need = 256 + (size_t)warps_per_map * maps->n_maps * astar_slot_bytes(rc, heap_cap);
@@ -379,16 +340,17 @@ extern "C" int mpp_mpa_iteration_batch(const mpp_map_batch *maps, const mpp_poli
     MPP_CUDA(cudaSetDevice(maps->device));
     cudaStream_t s = (cudaStream_t)stream;
     MpaArgs A;
-    A.X.occ = maps->occ_dev; A.X.pitch = maps->pitch_words; A.X.R = maps->rows; A.X.C = maps->cols;
-    A.X.pol = *policy; A.X.pol.mode = 1; A.X.cls = nullptr; A.X.lut = nullptr;     // MPA.py:164-173: safety = 0.0
+    mpp_policy pol = *policy;
+    pol.mode = 1;                                                      // MPA.py:164-173: safety = 0.0
+    int err = mpp_stats_ctx(const_cast<mpp_map_batch *>(maps), &pol, stream, &A.X);   // (mode 1 builds no tables)
+    if (err) return err;
     MPP_CUDA(cudaMemsetAsync(queue_dev, 0, sizeof(uint32_t) * maps->n_maps, s));
     A.G.occ = maps->occ_dev; A.G.pitch = maps->pitch_words; A.G.R = maps->rows; A.G.C = maps->cols;
     A.G.allow_diag = policy->allow_diagonal; A.G.restrict_corner = policy->restrict_policy;
-    A.occ_words = maps->occ_words; A.start = -1; A.target = -1;
+    A.occ_words = maps->occ_words;
     A.N = n_predators; A.iteration = iteration; A.phase = phase;
-    A.pred_begin = 0; A.pred_end = n_predators;
+    A.pred_begin = pred_begin; A.pred_end = pred_end;
     A.P_const = P_const; A.CF = CF; A.FADs_rate = FADs_rate; A.levy_sigma = levy_sigma; A.levy_inv_beta = 1.0 / levy_beta;
-    A.k0 = 0; A.k1 = 0;
     A.cells = cells_dev; A.n_cells = n_cells_dev; A.stats = stats_dev; A.max_cells = max_cells;
     A.out_cells = out_cells_dev; A.out_n = out_n_dev; A.out_stats = out_stats_dev;
     A.tmp_cells = tmp_cells_dev; A.avoid = avoid_dev; A.words = (rc + 31) / 32;
@@ -447,8 +409,10 @@ extern "C" int mpp_mpa_init_batch(const mpp_map_batch *maps, const mpp_policy *p
     MPP_CUDA(cudaSetDevice(maps->device));
     MpaArgs A;
     memset(&A, 0, sizeof(A));
-    A.X.occ = maps->occ_dev; A.X.pitch = maps->pitch_words; A.X.R = maps->rows; A.X.C = maps->cols;
-    A.X.pol = *policy; A.X.pol.mode = 1; A.X.cls = nullptr; A.X.lut = nullptr;
+    mpp_policy pol = *policy;
+    pol.mode = 1;                                                      // MPA.py:164-173: safety = 0.0
+    const int err = mpp_stats_ctx(const_cast<mpp_map_batch *>(maps), &pol, stream, &A.X);   // (mode 1 builds no tables)
+    if (err) return err;
     A.G.occ = maps->occ_dev; A.G.pitch = maps->pitch_words; A.G.R = maps->rows; A.G.C = maps->cols;
     A.G.allow_diag = policy->allow_diagonal; A.G.restrict_corner = policy->restrict_policy;
     A.occ_words = maps->occ_words; A.N = n_predators; A.max_cells = max_cells;

@@ -3,18 +3,11 @@
 // (particle, waypoint) / tournament / parent pair; every uniform comes from the Philox stream of the
 // RNG contract, so any rank can regenerate any individual's draws.
 // Every kernel runs over a batch of maps with grid.y = map: map m's arrays are row m of [n_maps][...] buffers and
-// its seed is seeds[m] (the same streams as a single-map solver with that seed).  A single map is the one-map case
-// (seeds = null: the scalar key k0, k1).
+// its seed is seeds[m] (the same streams as a single-map solver with that seed); a single map is a batch of one.
 #include "mpp_common.cuh"
 
 #define MPP_POP_MAX_MAPS 65535                                 // grid.y
 
-__device__ __forceinline__ void pop_key(const uint64_t *seeds, uint32_t &k0, uint32_t &k1) {
-    if (seeds) {
-        const uint64_t sd = seeds[blockIdx.y];
-        k0 = (uint32_t)sd; k1 = (uint32_t)(sd >> 32);
-    }
-}
 
 // ---------------------------------------------------------------------------------------------
 // K8: PSO update.  v = ((w*v) + ((c1*r1)*(pbest-x))) + ((c2*r2)*(gbest-x)); clip; x = clip(x+v).
@@ -22,24 +15,23 @@ __device__ __forceinline__ void pop_key(const uint64_t *seeds, uint32_t &k0, uin
 // => draws 4*dim+{0,1,2,3} of stream (seed, PSO_UPDATE, iteration, particle).
 // Also emits the integer waypoint pso.py:61,69-70: int(round(x)) (half-even) clamped to the grid.
 // ---------------------------------------------------------------------------------------------
-// Batch: particles [start[m], n) of map m (pid = particle index); start = null: all n, pid = particle_offset + p.
+// Particles [start[m], n) of map m (the stream index is the particle index).
 __global__ void mpp_pso_update_kernel(double *__restrict__ pos, double *__restrict__ vel,
                                       const double *__restrict__ pbest, const double *__restrict__ gbest, int n, int W,
-                                      int particle_offset, const int32_t *__restrict__ start, double w, double c1,
-                                      double c2, double max_vel, int R, int C, uint32_t k0, uint32_t k1,
-                                      const uint64_t *__restrict__ seeds, uint32_t iteration,
+                                      const int32_t *__restrict__ start, double w, double c1, double c2, double max_vel,
+                                      int R, int C, const uint64_t *__restrict__ seeds, uint32_t iteration,
                                       int32_t *__restrict__ wp_cells) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n * W) return;
     const int p = t / W, dim = t % W;
-    if (start && p < start[blockIdx.y]) return;
-    pop_key(seeds, k0, k1);
+    if (p < start[blockIdx.y]) return;
+    const uint64_t sd = seeds[blockIdx.y];
+    const uint32_t k0 = (uint32_t)sd, k1 = (uint32_t)(sd >> 32);
     const size_t row = (size_t)blockIdx.y * n * W;             // map m's particles
     pos += 2 * row; vel += 2 * row; pbest += 2 * row; wp_cells += row;
     gbest += (size_t)blockIdx.y * W * 2;
-    const uint32_t pid = (uint32_t)(particle_offset + p);
-    const mpp_u4 a = mpp_philox(2u * dim, pid, iteration, MPP_CLS_PSO_UPDATE, k0, k1);
-    const mpp_u4 b = mpp_philox(2u * dim + 1u, pid, iteration, MPP_CLS_PSO_UPDATE, k0, k1);
+    const mpp_u4 a = mpp_philox(2u * dim, (uint32_t)p, iteration, MPP_CLS_PSO_UPDATE, k0, k1);
+    const mpp_u4 b = mpp_philox(2u * dim + 1u, (uint32_t)p, iteration, MPP_CLS_PSO_UPDATE, k0, k1);
     const double r1 = mpp_u53(a.x, a.y), r2 = mpp_u53(a.z, a.w), r3 = mpp_u53(b.x, b.y), r4 = mpp_u53(b.z, b.w);
     const size_t i = ((size_t)p * W + dim) * 2;
     const double xr = pos[i], xc = pos[i + 1];
@@ -56,23 +48,6 @@ __global__ void mpp_pso_update_kernel(double *__restrict__ pos, double *__restri
     wp_cells[(size_t)p * W + dim] = ir * C + ic;
 }
 
-extern "C" int mpp_pso_update(const mpp_map *map, double *pos_dev, double *vel_dev, const double *pbest_pos_dev,
-                              const double *gbest_pos_dev, int n_particles, int particle_offset, int n_waypoints,
-                              double w, double c1, double c2, double max_vel, uint64_t seed, int iteration,
-                              int32_t *waypoint_cells_dev, void *stream) {
-    MPP_REQUIRE(map && pos_dev && vel_dev && pbest_pos_dev && gbest_pos_dev && waypoint_cells_dev,
-                "mpp_pso_update: null argument");
-    MPP_REQUIRE(n_particles > 0 && n_waypoints > 0, "mpp_pso_update: bad sizes");
-    MPP_CUDA(cudaSetDevice(map->device));
-    const int total = n_particles * n_waypoints;
-    mpp_pso_update_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
-        pos_dev, vel_dev, pbest_pos_dev, gbest_pos_dev, n_particles, n_waypoints, particle_offset, nullptr, w, c1, c2,
-        max_vel, map->rows, map->cols, (uint32_t)seed, (uint32_t)(seed >> 32), nullptr, (uint32_t)iteration,
-        waypoint_cells_dev);
-    MPP_CUDA(cudaGetLastError());
-    return MPP_OK;
-}
-
 extern "C" int mpp_pso_update_batch(const mpp_map_batch *maps, double *pos_dev, double *vel_dev,
                                     const double *pbest_pos_dev, const double *gbest_pos_dev, int n_particles,
                                     const int32_t *start_dev, int n_waypoints, double w, double c1, double c2,
@@ -84,28 +59,8 @@ extern "C" int mpp_pso_update_batch(const mpp_map_batch *maps, double *pos_dev, 
     MPP_CUDA(cudaSetDevice(maps->device));
     const int total = n_particles * n_waypoints;
     mpp_pso_update_kernel<<<dim3((total + 255) / 256, maps->n_maps), 256, 0, (cudaStream_t)stream>>>(
-        pos_dev, vel_dev, pbest_pos_dev, gbest_pos_dev, n_particles, n_waypoints, 0, start_dev, w, c1, c2, max_vel,
-        maps->rows, maps->cols, 0u, 0u, seeds_dev, (uint32_t)iteration, waypoint_cells_dev);
-    MPP_CUDA(cudaGetLastError());
-    return MPP_OK;
-}
-
-// Round float waypoints to cells (initialisation path: pso.py:61,69-70)
-__global__ void mpp_pso_round_kernel(const double *__restrict__ pos, int total, int R, int C, int32_t *__restrict__ wp) {
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= total) return;
-    int ir = (int)rint(pos[2 * (size_t)t]), ic = (int)rint(pos[2 * (size_t)t + 1]);
-    ir = max(0, min(R - 1, ir)); ic = max(0, min(C - 1, ic));
-    wp[t] = ir * C + ic;
-}
-
-extern "C" int mpp_pso_round(const mpp_map *map, const double *pos_dev, int n_particles, int n_waypoints,
-                             int32_t *waypoint_cells_dev, void *stream) {
-    MPP_REQUIRE(map && pos_dev && waypoint_cells_dev && n_particles > 0 && n_waypoints > 0, "mpp_pso_round: bad argument");
-    MPP_CUDA(cudaSetDevice(map->device));
-    const int total = n_particles * n_waypoints;
-    mpp_pso_round_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(pos_dev, total, map->rows, map->cols,
-                                                                               waypoint_cells_dev);
+        pos_dev, vel_dev, pbest_pos_dev, gbest_pos_dev, n_particles, n_waypoints, start_dev, w, c1, c2, max_vel,
+        maps->rows, maps->cols, seeds_dev, (uint32_t)iteration, waypoint_cells_dev);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }
@@ -116,16 +71,14 @@ extern "C" int mpp_pso_round(const mpp_map *map, const double *pos_dev, int n_pa
 // winner = first minimum fitness in sample order.  Stream (seed, GA_SELECT, generation, tournament).
 // ---------------------------------------------------------------------------------------------
 #define MPP_GA_MAX_K 16
-__global__ void mpp_ga_select_kernel(const double *__restrict__ fitness, int n, int k, uint32_t k0, uint32_t k1,
-                                     const uint64_t *__restrict__ seeds, uint32_t generation,
-                                     int32_t *__restrict__ parents) {
+__global__ void mpp_ga_select_kernel(const double *__restrict__ fitness, int n, int k, const uint64_t *__restrict__ seeds,
+                                     uint32_t generation, int32_t *__restrict__ parents) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n) return;
-    pop_key(seeds, k0, k1);
     fitness += (size_t)blockIdx.y * n;
     parents += (size_t)blockIdx.y * n;
     mpp_stream_rng rng;
-    rng.init(((uint64_t)k1 << 32) | k0, MPP_CLS_GA_SELECT, generation, (uint32_t)t);
+    rng.init(seeds[blockIdx.y], MPP_CLS_GA_SELECT, generation, (uint32_t)t);
     int setsize = 21;
     if (k > 5) {  // setsize += 4 ** ceil(log(k*3, 4))
         int e = 0, v = 1;
@@ -162,28 +115,18 @@ __global__ void mpp_ga_select_kernel(const double *__restrict__ fitness, int n, 
     parents[t] = best;
 }
 
-static int ga_select(int n_maps, const double *fitness_dev, int n, int tournament_size, uint64_t seed,
-                     const uint64_t *seeds_dev, int generation, int32_t *parents_dev, void *stream) {
-    MPP_REQUIRE(fitness_dev && parents_dev && n > 0, "mpp_ga_select: bad argument");
-    int k = tournament_size < n ? tournament_size : n;  // min(tournament_size, len(population))
-    MPP_REQUIRE(k >= 1 && k <= MPP_GA_MAX_K, "mpp_ga_select: tournament size %d unsupported (1..%d)", k, MPP_GA_MAX_K);
-    MPP_REQUIRE(k <= 5 || n > 21 + 64, "mpp_ga_select: tiny population with large tournament unsupported");
-    mpp_ga_select_kernel<<<dim3((n + 127) / 128, n_maps), 128, 0, (cudaStream_t)stream>>>(
-        fitness_dev, n, k, (uint32_t)seed, (uint32_t)(seed >> 32), seeds_dev, (uint32_t)generation, parents_dev);
-    MPP_CUDA(cudaGetLastError());
-    return MPP_OK;
-}
-
-extern "C" int mpp_ga_select(const double *fitness_dev, int n, int tournament_size, uint64_t seed, int generation,
-                             int32_t *parents_dev, void *stream) {
-    return ga_select(1, fitness_dev, n, tournament_size, seed, nullptr, generation, parents_dev, stream);
-}
-
 extern "C" int mpp_ga_select_batch(const mpp_map_batch *maps, const double *fitness_dev, int n, int tournament_size,
                                    const uint64_t *seeds_dev, int generation, int32_t *parents_dev, void *stream) {
-    MPP_REQUIRE(maps && seeds_dev && maps->n_maps <= MPP_POP_MAX_MAPS, "mpp_ga_select_batch: bad argument");
+    MPP_REQUIRE(maps && seeds_dev && fitness_dev && parents_dev && n > 0 && maps->n_maps <= MPP_POP_MAX_MAPS,
+                "mpp_ga_select_batch: bad argument");
+    int k = tournament_size < n ? tournament_size : n;  // min(tournament_size, len(population))
+    MPP_REQUIRE(k >= 1 && k <= MPP_GA_MAX_K, "mpp_ga_select_batch: tournament size %d unsupported (1..%d)", k, MPP_GA_MAX_K);
+    MPP_REQUIRE(k <= 5 || n > 21 + 64, "mpp_ga_select_batch: tiny population with large tournament unsupported");
     MPP_CUDA(cudaSetDevice(maps->device));
-    return ga_select(maps->n_maps, fitness_dev, n, tournament_size, 0, seeds_dev, generation, parents_dev, stream);
+    mpp_ga_select_kernel<<<dim3((n + 127) / 128, maps->n_maps), 128, 0, (cudaStream_t)stream>>>(
+        fitness_dev, n, k, seeds_dev, (uint32_t)generation, parents_dev);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -203,19 +146,17 @@ __device__ __forceinline__ int ga_random_free_cell(mpp_stream_rng &rng, const ui
 
 __global__ void mpp_ga_breed_kernel(const uint32_t *__restrict__ occ, int occ_words, int pitch, int R, int C,
                                     const int32_t *__restrict__ chrom, const int32_t *__restrict__ parents, int n, int W,
-                                    double cx_rate, double mut_rate, uint32_t k0, uint32_t k1,
-                                    const uint64_t *__restrict__ seeds, uint32_t generation,
-                                    int32_t *__restrict__ children) {
+                                    double cx_rate, double mut_rate, const uint64_t *__restrict__ seeds,
+                                    uint32_t generation, int32_t *__restrict__ children) {
     const int pair = blockIdx.x * blockDim.x + threadIdx.x;
     const int n_pairs = (n + 1) / 2;
     if (pair >= n_pairs) return;
-    pop_key(seeds, k0, k1);
     occ += (size_t)blockIdx.y * occ_words;                     // mutated genes are free cells of the map's own grid
     chrom += (size_t)blockIdx.y * n * W;
     parents += (size_t)blockIdx.y * n;
     children += (size_t)blockIdx.y * n * W;
     mpp_stream_rng rng;
-    rng.init(((uint64_t)k1 << 32) | k0, MPP_CLS_GA_BREED, generation, (uint32_t)pair);
+    rng.init(seeds[blockIdx.y], MPP_CLS_GA_BREED, generation, (uint32_t)pair);
     const int32_t *p1 = chrom + (size_t)parents[(2 * pair) % n] * W;
     const int32_t *p2 = chrom + (size_t)parents[(2 * pair + 1) % n] * W;
     int32_t c1[MPP_GA_MAX_W], c2[MPP_GA_MAX_W];
@@ -237,23 +178,6 @@ __global__ void mpp_ga_breed_kernel(const uint32_t *__restrict__ occ, int occ_wo
         for (int i = 0; i < W; ++i) children[(size_t)(2 * pair + 1) * W + i] = c2[i];
 }
 
-extern "C" int mpp_ga_breed(const mpp_map *map, const int32_t *chrom_dev, const int32_t *parents_dev, int n,
-                            int n_waypoints, double crossover_rate, double mutation_rate, uint64_t seed, int generation,
-                            int32_t *children_dev, void *stream) {
-    MPP_REQUIRE(map && chrom_dev && parents_dev && children_dev && n > 0, "mpp_ga_breed: bad argument");
-    MPP_REQUIRE(n_waypoints >= 1 && n_waypoints <= MPP_GA_MAX_W, "mpp_ga_breed: %d waypoints unsupported (1..%d)",
-                n_waypoints, MPP_GA_MAX_W);
-    MPP_REQUIRE(map->n_obstacles < map->rows * map->cols, "mpp_ga_breed: map has no free cell");
-    MPP_CUDA(cudaSetDevice(map->device));
-    const int n_pairs = (n + 1) / 2;
-    mpp_ga_breed_kernel<<<(n_pairs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        map->occ_dev, map->occ_words, map->pitch_words, map->rows, map->cols, chrom_dev, parents_dev, n, n_waypoints,
-        crossover_rate, mutation_rate, (uint32_t)seed, (uint32_t)(seed >> 32), nullptr, (uint32_t)generation,
-        children_dev);
-    MPP_CUDA(cudaGetLastError());
-    return MPP_OK;
-}
-
 extern "C" int mpp_ga_breed_batch(const mpp_map_batch *maps, const int32_t *chrom_dev, const int32_t *parents_dev, int n,
                                   int n_waypoints, double crossover_rate, double mutation_rate, const uint64_t *seeds_dev,
                                   int generation, int32_t *children_dev, void *stream) {
@@ -267,7 +191,7 @@ extern "C" int mpp_ga_breed_batch(const mpp_map_batch *maps, const int32_t *chro
     const int n_pairs = (n + 1) / 2;
     mpp_ga_breed_kernel<<<dim3((n_pairs + 127) / 128, maps->n_maps), 128, 0, (cudaStream_t)stream>>>(
         maps->occ_dev, maps->occ_words, maps->pitch_words, maps->rows, maps->cols, chrom_dev, parents_dev, n, n_waypoints,
-        crossover_rate, mutation_rate, 0u, 0u, seeds_dev, (uint32_t)generation, children_dev);
+        crossover_rate, mutation_rate, seeds_dev, (uint32_t)generation, children_dev);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }
@@ -279,14 +203,16 @@ extern "C" int mpp_ga_breed_batch(const mpp_map_batch *maps, const int32_t *chro
 // ---------------------------------------------------------------------------------------------
 // PSO attempt: W waypoints [uniform(0, R-1), uniform(0, C-1)] (pso.py:50-51, draws 0..2W-1), then W velocities
 // [uniform(-max_vel/5, max_vel/5)] x 2 (pso.py:105, draws 2W..4W-1); also the rounded, clamped cells (pso.py:61,69-70).
-// Batch: attempts [offsets[m], offsets[m] + n) of map m (offsets[m] < 0: the map is done, nothing is written).
-__global__ void mpp_pso_init_kernel(int n, int W, int attempt0, const int32_t *__restrict__ offsets, int R, int C,
-                                    double max_vel, uint32_t k0, uint32_t k1, const uint64_t *__restrict__ seeds,
-                                    double *__restrict__ pos, double *__restrict__ vel, int32_t *__restrict__ wp_cells) {
+// Attempts [offsets[m], offsets[m] + n) of map m (offsets[m] < 0: the map is done, nothing is written).
+__global__ void mpp_pso_init_kernel(int n, int W, const int32_t *__restrict__ offsets, int R, int C, double max_vel,
+                                    const uint64_t *__restrict__ seeds, double *__restrict__ pos,
+                                    double *__restrict__ vel, int32_t *__restrict__ wp_cells) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n * W) return;
-    if (offsets && (attempt0 = offsets[blockIdx.y]) < 0) return;
-    pop_key(seeds, k0, k1);
+    const int attempt0 = offsets[blockIdx.y];
+    if (attempt0 < 0) return;
+    const uint64_t sd = seeds[blockIdx.y];
+    const uint32_t k0 = (uint32_t)sd, k1 = (uint32_t)(sd >> 32);
     const size_t row = (size_t)blockIdx.y * n * W;
     pos += 2 * row; vel += 2 * row; wp_cells += row;
     const int p = t / W, dim = t % W;
@@ -306,19 +232,6 @@ __global__ void mpp_pso_init_kernel(int n, int W, int attempt0, const int32_t *_
     wp_cells[(size_t)p * W + dim] = ir * C + ic;
 }
 
-extern "C" int mpp_pso_init(const mpp_map *map, int n_attempts, int attempt_offset, int n_waypoints, double max_vel,
-                            uint64_t seed, double *pos_dev, double *vel_dev, int32_t *waypoint_cells_dev, void *stream) {
-    MPP_REQUIRE(map && pos_dev && vel_dev && waypoint_cells_dev && n_attempts > 0 && n_waypoints > 0 && attempt_offset >= 0,
-                "mpp_pso_init: bad argument");
-    MPP_CUDA(cudaSetDevice(map->device));
-    const int total = n_attempts * n_waypoints;
-    mpp_pso_init_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
-        n_attempts, n_waypoints, attempt_offset, nullptr, map->rows, map->cols, max_vel, (uint32_t)seed,
-        (uint32_t)(seed >> 32), nullptr, pos_dev, vel_dev, waypoint_cells_dev);
-    MPP_CUDA(cudaGetLastError());
-    return MPP_OK;
-}
-
 extern "C" int mpp_pso_init_batch(const mpp_map_batch *maps, int n_attempts, const int32_t *attempt_offset_dev,
                                   int n_waypoints, double max_vel, const uint64_t *seeds_dev, double *pos_dev,
                                   double *vel_dev, int32_t *waypoint_cells_dev, void *stream) {
@@ -327,37 +240,25 @@ extern "C" int mpp_pso_init_batch(const mpp_map_batch *maps, int n_attempts, con
     MPP_CUDA(cudaSetDevice(maps->device));
     const int total = n_attempts * n_waypoints;
     mpp_pso_init_kernel<<<dim3((total + 255) / 256, maps->n_maps), 256, 0, (cudaStream_t)stream>>>(
-        n_attempts, n_waypoints, 0, attempt_offset_dev, maps->rows, maps->cols, max_vel, 0u, 0u, seeds_dev, pos_dev,
-        vel_dev, waypoint_cells_dev);
+        n_attempts, n_waypoints, attempt_offset_dev, maps->rows, maps->cols, max_vel, seeds_dev, pos_dev, vel_dev,
+        waypoint_cells_dev);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }
 
 // GA attempt: W genes, each (randint(0, R-1), randint(0, C-1)) redrawn until the cell is free (ga_solver.py:48-56)
 __global__ void mpp_ga_init_kernel(const uint32_t *__restrict__ occ, int occ_words, int pitch, int R, int C, int n, int W,
-                                   int attempt0, const int32_t *__restrict__ offsets, uint32_t k0, uint32_t k1,
-                                   const uint64_t *__restrict__ seeds, int32_t *__restrict__ chrom) {
+                                   const int32_t *__restrict__ offsets, const uint64_t *__restrict__ seeds,
+                                   int32_t *__restrict__ chrom) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n) return;
-    if (offsets && (attempt0 = offsets[blockIdx.y]) < 0) return;   // the map is done
-    pop_key(seeds, k0, k1);
+    const int attempt0 = offsets[blockIdx.y];
+    if (attempt0 < 0) return;                                          // the map is done
     occ += (size_t)blockIdx.y * occ_words;
     chrom += (size_t)blockIdx.y * n * W;
     mpp_stream_rng rng;
-    rng.init(((uint64_t)k1 << 32) | k0, MPP_CLS_GA_INIT, 0u, (uint32_t)(attempt0 + p));
+    rng.init(seeds[blockIdx.y], MPP_CLS_GA_INIT, 0u, (uint32_t)(attempt0 + p));
     for (int k = 0; k < W; ++k) chrom[(size_t)p * W + k] = ga_random_free_cell(rng, occ, pitch, R, C);
-}
-
-extern "C" int mpp_ga_init(const mpp_map *map, int n_attempts, int attempt_offset, int n_waypoints, uint64_t seed,
-                           int32_t *chrom_dev, void *stream) {
-    MPP_REQUIRE(map && chrom_dev && n_attempts > 0 && n_waypoints > 0 && attempt_offset >= 0, "mpp_ga_init: bad argument");
-    MPP_REQUIRE(map->n_obstacles < map->rows * map->cols, "mpp_ga_init: map has no free cell");
-    MPP_CUDA(cudaSetDevice(map->device));
-    mpp_ga_init_kernel<<<(n_attempts + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        map->occ_dev, map->occ_words, map->pitch_words, map->rows, map->cols, n_attempts, n_waypoints, attempt_offset,
-        nullptr, (uint32_t)seed, (uint32_t)(seed >> 32), nullptr, chrom_dev);
-    MPP_CUDA(cudaGetLastError());
-    return MPP_OK;
 }
 
 extern "C" int mpp_ga_init_batch(const mpp_map_batch *maps, int n_attempts, const int32_t *attempt_offset_dev,
@@ -368,8 +269,8 @@ extern "C" int mpp_ga_init_batch(const mpp_map_batch *maps, int n_attempts, cons
         MPP_REQUIRE(maps->meta_host[k].start >= 0, "mpp_ga_init_batch: map %d has no start", k);
     MPP_CUDA(cudaSetDevice(maps->device));
     mpp_ga_init_kernel<<<dim3((n_attempts + 127) / 128, maps->n_maps), 128, 0, (cudaStream_t)stream>>>(
-        maps->occ_dev, maps->occ_words, maps->pitch_words, maps->rows, maps->cols, n_attempts, n_waypoints, 0,
-        attempt_offset_dev, 0u, 0u, seeds_dev, chrom_dev);
+        maps->occ_dev, maps->occ_words, maps->pitch_words, maps->rows, maps->cols, n_attempts, n_waypoints,
+        attempt_offset_dev, seeds_dev, chrom_dev);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }

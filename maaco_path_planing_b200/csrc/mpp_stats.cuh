@@ -14,6 +14,10 @@ struct StatsCtx {
     mpp_policy pol;
 };
 
+// X for the maps of a batch (mpp_astar.cu): their occupancy, the policy and -- mode 0 on a batch with obstacles -- the
+// batch's safety tables (mpp_map_batch_safety_table).  A kernel offsets occ / cls to the map a path lies on.
+int mpp_stats_ctx(mpp_map_batch *maps, const mpp_policy *pol, void *stream, StatsCtx *X);
+
 static __device__ void path_stats_warp(const LaneGroup &L, const StatsCtx &X, const int32_t *cells, int n, double *out) {
     const int lane = L.gl;
     const double INF = __longlong_as_double(MPP_INF_BITS);

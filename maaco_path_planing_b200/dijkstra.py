@@ -5,7 +5,6 @@ from __future__ import annotations
 
 import numpy as np
 
-from . import _lib
 from .astar import AStarSolver
 from .field import dijkstra_fields, field_paths
 from .gridmap import START_NODE_VAL, TARGET_NODE_VAL
@@ -35,11 +34,11 @@ class DijkstraSolver(AStarSolver):
         return 0 <= n[0] < self.rows and 0 <= n[1] < self.cols
 
     def _field(self, start_node):
-        """(mpp_map_batch view of the map, g, parent) of the field from start_node (None: the grid's start)."""
+        """(the map's one-map batch, g, parent) of the field from start_node (None: the grid's start)."""
         s = start_node if start_node else self.start_node                     # (as solve() reads its override)
         src = self._cell(s) if self._inb(s) else -1                           # -1: an all-inf field
-        batch = _lib.lib().mpp_map_as_batch(self.map.handle)
-        g, parent = dijkstra_fields(self.engine, batch, (1, self.rows, self.cols), self.engine._dev_i32([src]),
+        batch = self.map.handle
+        g, parent = dijkstra_fields(self.engine, batch, (1, self.rows, self.cols), self.engine._i32([src]),
                                     self.allow_diagonal_moves, self.dijkstra_strictly_restricts_corners)
         return batch, g, parent
 
@@ -58,8 +57,8 @@ class DijkstraSolver(AStarSolver):
         res = {}
         if q:
             batch, g, parent = self._field(s)
-            mi = self.engine._dev_i32(np.zeros(len(q)))
-            dst = self.engine._dev_i32([self._cell(targets[i]) for i in q])
+            mi = self.engine._i32(np.zeros(len(q)))
+            dst = self.engine._i32([self._cell(targets[i]) for i in q])
             cells, ncell, gout, stats = field_paths(self.engine, batch, g, parent, mi, dst, self.policy)
             cells, ncell, gout, stats = cells.cpu().numpy(), ncell.cpu().numpy(), gout.cpu().numpy(), stats.cpu().numpy()
             res = {i: (cells[j, :ncell[j]], float(gout[j]), stats[j]) for j, i in enumerate(q)}

@@ -1,6 +1,6 @@
-"""SearchEngine -- host-side owner of the device buffers behind the connector / fitness entry points
-(mpp_astar_batch, mpp_waypoint_fitness, mpp_path_stats).  Populations are torch tensors in HBM; the
-engine only moves pointers across the C ABI.  No CPU fallback."""
+"""SearchEngine -- the connector / fitness / statistics entry points (mpp_astar_batch_maps, mpp_waypoint_fitness_maps,
+mpp_path_stats) on one map: a SearchBatch over a GridMap's one-map batch, with the reference's single-map arguments.
+Populations are torch tensors in HBM; the engine only moves pointers across the C ABI.  No CPU fallback."""
 from __future__ import annotations
 
 import ctypes as C
@@ -8,6 +8,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
+from .batch import SearchBatch
 from .gridmap import GridMap
 
 INF = float("inf")
@@ -20,48 +21,26 @@ def make_policy(turn_penalty_factor, safety_penalty_factor, min_safe_distance, d
                        int(mode))
 
 
-class SearchEngine:
+class SearchEngine(SearchBatch):
+    """The searches of one map (every launch on map 0 of its batch).  Buffer sizes, their growth, the scratch and the
+    longest-first order are SearchBatch's; a launch whose heap overflowed or whose paths were truncated is repeated
+    whole, and `counters` adds up every launch."""
+
     def __init__(self, gridmap: GridMap, max_cells=None, heap_cap=None, n_slots=None, group=None):
         import torch
+        super().__init__(gridmap._maps, max_cells=max_cells, heap_cap=heap_cap, n_slots=n_slots)
         self.group = group            # torch.distributed group: population batches are sharded over its ranks
         self.torch = torch
         self.map = gridmap
-        self.rows, self.cols = gridmap.rows, gridmap.cols
-        self.n = self.rows * self.cols
-        self.words = (self.n + 31) // 32
-        self.device = torch.device("cuda", gridmap.device)
-        L = _lib.lib()
-        self.max_slots = L.mpp_astar_max_slots(gridmap.handle)
-        self.n_slots = int(n_slots or self.max_slots)
-        # a search's open set is a frontier: a few thousand entries on the largest maps; overflow is
-        # reported (n_cells = -1) and the call is repeated with a larger heap
-        self.heap_cap = int(heap_cap or min(8 * self.n, max(4096, self.n // 4)))
-        self.max_cells = int(max_cells or min(self.n, max(4096, 16 * (self.rows + self.cols))))
-        self._scratch = None
-        self._scratch_key = None
-        self.counters = torch.zeros(4, dtype=torch.int64, device=self.device)  # expansions, relaxations, ring / heap pushes
-        self.launches = 0
 
-    # -- buffers ---------------------------------------------------------------------------------
-    def _scratch_for(self, n_work):
-        slots = max(1, min(self.n_slots, n_work))
-        key = (slots, self.heap_cap)
-        if self._scratch_key != key:
-            nbytes = _lib.lib().mpp_astar_scratch_bytes(self.map.handle, slots, self.heap_cap)
-            self._scratch = self.torch.zeros(nbytes, dtype=self.torch.uint8, device=self.device)
-            self._scratch_key = key
-        return self._scratch, slots
+    def _map0(self, n):
+        return self.torch.zeros(n, dtype=self.torch.int32, device=self.device)
 
-    def _stream(self):
-        return C.c_void_p(self.torch.cuda.current_stream(self.device).cuda_stream)
-
-    def _dev_i32(self, a):
-        t = self.torch
-        if isinstance(a, t.Tensor):
-            return a.to(device=self.device, dtype=t.int32).contiguous()
-        return t.as_tensor(np.ascontiguousarray(a, dtype=np.int32), device=self.device)
+    def _grown(self, ncell):
+        return self._grow_from(*self.torch.stack([ncell.min(), ncell.max()]).tolist())
 
     def expansions(self):
+        """(node expansions, successful relaxations) of the searches so far."""
         c = self.counters.cpu().numpy()
         return int(c[0]), int(c[1])
 
@@ -74,23 +53,16 @@ class SearchEngine:
     def astar_batch(self, variant, src, dst, avoid_bits=None, allow_diagonal=True, restrict_corner=True):
         """n independent searches.  Returns (cells[n,max_cells], n_cells[n], g[n]) as device tensors."""
         t = self.torch
-        src, dst = self._dev_i32(src), self._dev_i32(dst)
+        src, dst = self._i32(src), self._i32(dst)
         n = src.numel()
         if avoid_bits is not None:
             avoid_bits = t.as_tensor(avoid_bits, device=self.device).contiguous()
             assert avoid_bits.numel() == n * self.words
+        mi = self._map0(n)
         while True:
-            scratch, slots = self._scratch_for(n)
-            cells = t.empty((n, self.max_cells), dtype=t.int32, device=self.device)
-            ncell = t.empty(n, dtype=t.int32, device=self.device)
-            g = t.empty(n, dtype=t.float64, device=self.device)
-            _lib.check(_lib.lib().mpp_astar_batch(
-                self.map.handle, int(variant), _lib.ptr(src), _lib.ptr(dst), _lib.ptr(avoid_bits), n,
-                int(bool(allow_diagonal)), int(bool(restrict_corner)), _lib.ptr(cells), self.max_cells, _lib.ptr(ncell),
-                _lib.ptr(g), _lib.ptr(scratch), scratch.numel(), slots, self.heap_cap, _lib.ptr(self.counters),
-                self._stream()), "mpp_astar_batch")
-            self.launches += 1
-            if not self._grow_if_needed(ncell):
+            cells, ncell, g, _ = self._launch(variant, mi, src, dst, avoid_bits, False, allow_diagonal, restrict_corner,
+                                              None)
+            if not self._grown(ncell):
                 return cells, ncell, g
 
     # -- K6 + K7 ----------------------------------------------------------------------------------
@@ -100,7 +72,9 @@ class SearchEngine:
         With a process group, individuals are independent units: rank g evaluates rows
         [g*per, (g+1)*per) and the results are all-gathered (no other data-path collective)."""
         t = self.torch
-        wps = self._dev_i32(waypoints)
+        if self.map.start_cell < 0 or self.map.target_cell < 0:
+            raise _lib.MppError("waypoint_fitness: the map has no start / target")
+        wps = self._i32(waypoints)
         N, W = wps.shape
         world = 1
         if self.group is not None:
@@ -127,58 +101,22 @@ class SearchEngine:
             return a_cells[:N], a_ncell[:N], a_stats[:N]
 
     def _waypoint_fitness_local(self, wps, policy, retry=True):
-        t = self.torch
-        N, W = wps.shape
+        mi = self._map0(wps.shape[0])
         while True:
-            scratch, slots = self._scratch_for(N)
-            cells = t.empty((N, self.max_cells), dtype=t.int32, device=self.device)
-            ncell = t.empty(N, dtype=t.int32, device=self.device)
-            stats = t.empty((N, 5), dtype=t.float64, device=self.device)
-            visited = t.empty((N, self.words), dtype=t.int32, device=self.device)
-            order = self._longest_first(wps) if N > slots // 2 and W > 0 else None
-            _lib.check(_lib.lib().mpp_waypoint_fitness(
-                self.map.handle, _lib.ptr(wps), N, W, C.byref(policy), _lib.ptr(cells), self.max_cells,
-                _lib.ptr(ncell), _lib.ptr(stats), _lib.ptr(visited), _lib.ptr(scratch), scratch.numel(), slots,
-                self.heap_cap, _lib.ptr(self.counters), _lib.ptr(order), self._stream()), "mpp_waypoint_fitness")
-            self.launches += 1
-            if not retry or not self._grow_if_needed(ncell):
+            cells, ncell, stats = self._chain_launch(mi, wps, policy)
+            if not retry or not self._grown(ncell):
                 return cells, ncell, stats
-
-    def _longest_first(self, wps):
-        """Individuals ordered by the Euclidean length of their waypoint chain, longest first: the searches of a chain
-        cost roughly its length squared, and the evaluation ends with its slowest individual."""
-        t = self.torch
-        s, g = self.map.start_cell, self.map.target_cell
-        chain = t.cat([t.full_like(wps[:, :1], s), wps, t.full_like(wps[:, :1], g)], dim=1).to(t.float64)
-        r, c = t.div(chain, self.cols, rounding_mode="floor"), chain % self.cols
-        d = ((r[:, 1:] - r[:, :-1]) ** 2 + (c[:, 1:] - c[:, :-1]) ** 2).sqrt().sum(dim=1)
-        return t.argsort(d, descending=True).to(t.int32).contiguous()
-
-    def _grow_if_needed(self, ncell):
-        """Heap overflow (-1) or truncated paths (> max_cells) -> enlarge and tell the caller to repeat."""
-        return self._grow_from(int(ncell.min().item()), int(ncell.max().item()))
-
-    def _grow_from(self, mn, mx):
-        grew = False
-        if mn < 0:
-            if self.heap_cap >= 8 * self.n:
-                raise _lib.MppError("A* heap overflow at maximum capacity")
-            self.heap_cap = min(8 * self.n, self.heap_cap * 4)
-            grew = True
-        if mx > self.max_cells:
-            self.max_cells = min(2 * self.n, max(mx, 2 * self.max_cells))
-            grew = True
-        return grew
 
     # -- K7 ---------------------------------------------------------------------------------------
     def path_stats(self, cells, n_cells, policy):
         """cells [P, max_cells] int32, n_cells [P] -> stats [P,5] device tensor."""
         t = self.torch
         cells = cells if isinstance(cells, t.Tensor) else t.as_tensor(np.ascontiguousarray(cells, np.int32), device=self.device)
-        ncell = self._dev_i32(n_cells)
+        cells = cells.contiguous()
+        ncell = self._i32(n_cells)
         P, mc = cells.shape
         stats = t.empty((P, 5), dtype=t.float64, device=self.device)
-        _lib.check(_lib.lib().mpp_path_stats(self.map.handle, _lib.ptr(cells.contiguous()), mc, _lib.ptr(ncell), P,
+        _lib.check(_lib.lib().mpp_path_stats(self._maps, _lib.ptr(self._map0(P)), _lib.ptr(cells), mc, _lib.ptr(ncell), P,
                                              C.byref(policy), _lib.ptr(stats), self._stream()), "mpp_path_stats")
         self.launches += 1
         return stats

@@ -52,14 +52,13 @@ def field_paths(owner, batch, g, parent, mi, dst, policy):
     stats [n, 5] float64) with SearchBatch.search's conventions.  A truncated path grows owner.max_cells and repeats only
     the truncated queries."""
     import torch as t
-    from .engine import SearchEngine
     n = mi.numel()
     if n == 0:
         return (t.zeros((0, owner.max_cells), dtype=t.int32, device=owner.device),
                 t.zeros(0, dtype=t.int32, device=owner.device), t.zeros(0, dtype=t.float64, device=owner.device),
                 t.zeros((0, 5), dtype=t.float64, device=owner.device))
     cells, ncell, gout, stats = _paths_launch(owner, batch, g, parent, mi, dst, policy)
-    while SearchEngine._grow_from(owner, 0, int(ncell.max().item())):
+    while owner._grow_from(0, int(ncell.max().item())):
         bad = (ncell > cells.shape[1]).nonzero().squeeze(1)
         c, nc, gg, st = _paths_launch(owner, batch, g, parent, mi.index_select(0, bad).contiguous(),
                                       dst.index_select(0, bad).contiguous(), policy)

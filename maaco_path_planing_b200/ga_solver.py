@@ -1,10 +1,8 @@
 """GASolver -- drop-in for ga_solver.GASolver (ga_solver.py:8-223).  Chromosomes (integer waypoints)
-live in HBM; tournament selection, crossover + mutation (mpp_ga_select / mpp_ga_breed) and the
-A*-connector fitness (mpp_waypoint_fitness) are sm_100a kernels.  Breeding consumes RNG but evaluation
+live in HBM; tournament selection, crossover + mutation (mpp_ga_select_batch / mpp_ga_breed_batch) and the
+A*-connector fitness (mpp_waypoint_fitness_maps) are sm_100a kernels, launched on the map as a batch of one.  Breeding consumes RNG but evaluation
 does not, so a whole generation is bred first and evaluated in one batch (ga_solver.py:186-205)."""
 from __future__ import annotations
-
-import ctypes as C
 
 import numpy as np
 
@@ -43,6 +41,8 @@ class GASolver(BasePathfinder):
                                           restrict_diagonal_near_obstacle_policy=self.restrict_diagonal_near_obstacle_policy,
                                           diagonal_obstacle_penalty_value=0, gridmap=self.map, engine=self.engine)
         self.rng_seed = _fresh_seed() if rng_seed is None else int(rng_seed)
+        self._seeds = self.engine.torch.from_numpy(np.array([self.rng_seed & (2 ** 64 - 1)], np.uint64).view(np.int64)
+                                                   ).to(self.engine.device)
         self.engine.group = group   # fitness evaluation is sharded over the group's ranks (individuals are independent)
         self.verbose = verbose
         self.best_solution_overall = {'fitness': INF, 'path': []}
@@ -73,8 +73,9 @@ class GASolver(BasePathfinder):
         while n_acc < N and attempts < max_total:
             batch = min(max_total - attempts, max(32, int(1.25 * (N - n_acc)) + 8))
             chrom_d = t.empty((batch, W), dtype=t.int32, device=dev)             # _create_chromosome :55-56 on the device
-            _lib.check(_lib.lib().mpp_ga_init(self.map.handle, batch, attempts, W, C.c_uint64(self.rng_seed),
-                                              _lib.ptr(chrom_d), self.engine._stream()), "mpp_ga_init")
+            offs = t.tensor([attempts], dtype=t.int32, device=dev)
+            _lib.check(_lib.lib().mpp_ga_init_batch(self.map.handle, batch, _lib.ptr(offs), W, _lib.ptr(self._seeds),
+                                                    _lib.ptr(chrom_d), self.engine._stream()), "mpp_ga_init_batch")
             cells, ncell, stats = self._evaluate(chrom_d)
             take = np.flatnonzero((ncell > 0).cpu().numpy())
             room = N - n_acc
@@ -148,12 +149,12 @@ class GASolver(BasePathfinder):
         dev = self.engine.device
         parents = t.empty(N, dtype=t.int32, device=dev)
         fit = P["stats"][:, 4].contiguous()
-        _lib.check(L.mpp_ga_select(_lib.ptr(fit), N, self.tournament_size, C.c_uint64(self.rng_seed), gen,
-                                   _lib.ptr(parents), self.engine._stream()), "mpp_ga_select")
+        _lib.check(L.mpp_ga_select_batch(self.map.handle, _lib.ptr(fit), N, self.tournament_size, _lib.ptr(self._seeds),
+                                         gen, _lib.ptr(parents), self.engine._stream()), "mpp_ga_select_batch")
         children = t.empty((N, W), dtype=t.int32, device=dev)
-        _lib.check(L.mpp_ga_breed(self.map.handle, _lib.ptr(P["chrom"]), _lib.ptr(parents), N, W, self.crossover_rate,
-                                  self.mutation_rate, C.c_uint64(self.rng_seed), gen, _lib.ptr(children),
-                                  self.engine._stream()), "mpp_ga_breed")
+        _lib.check(L.mpp_ga_breed_batch(self.map.handle, _lib.ptr(P["chrom"]), _lib.ptr(parents), N, W,
+                                        self.crossover_rate, self.mutation_rate, _lib.ptr(self._seeds), gen,
+                                        _lib.ptr(children), self.engine._stream()), "mpp_ga_breed_batch")
         cells, ncell, stats = self._evaluate(children)
         # invalid child -> the parent object: p1 for even slots, p2 for odd (:204-205)
         bad = (ncell <= 0).nonzero().flatten()

@@ -1,4 +1,4 @@
-"""GridMap -- env.py's occupancy grid as a bit-packed HBM tensor (mpp_map handle).
+"""GridMap -- env.py's occupancy grid as a bit-packed HBM tensor: a one-map mpp_map_batch.
 
 Grid convention (env.py:4-7): 0 free, 1 obstacle, 2 start, 3 target; start/target are the
 first row-major cells equal to 2 / 3 (MAACO.py:32-41) and are traversable.
@@ -21,38 +21,32 @@ def _current_device():
 
 
 class GridMap:
+    """`handle` is the batch of one map every entry point takes; the batch is freed by close() or with the last
+    object (GridMap, SearchEngine) holding it."""
+
     def __init__(self, grid, device=None):
+        from .batch import _map_set
         g = np.array(grid, dtype=int)  # same coercion as the reference constructors
         if g.ndim != 2:
             raise ValueError("grid must be 2-D")
         self.grid = g
         self.rows, self.cols = g.shape
-        self.device = _current_device() if device is None else int(device)
-        g8 = np.ascontiguousarray(np.clip(g, 0, 255), dtype=np.uint8)
-        h = C.c_void_p()
-        _lib.check(_lib.lib().mpp_map_create(g8.ctypes.data_as(C.c_void_p), self.rows, self.cols, self.device,
-                                             C.byref(h)), "mpp_map_create")
-        self.handle = h
-        s, t = _lib.lib().mpp_map_start(h), _lib.lib().mpp_map_target(h)
+        self._maps = _map_set(g[None], _current_device() if device is None else int(device))
+        self.handle = self._maps.handle
+        self.device = self._maps.device_index
+        s, t = int(self._maps.start[0]), int(self._maps.target[0])
         self.start_cell, self.target_cell = s, t
         self.start_node = divmod(s, self.cols) if s >= 0 else None
         self.target_node = divmod(t, self.cols) if t >= 0 else None
 
     def close(self):
-        h, self.handle = getattr(self, "handle", None), None
-        if h:
-            _lib.lib().mpp_map_destroy(h)
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
+        self.handle = None
+        self._maps.close()
 
     def occ_bits(self):
         """(device pointer, pitch in words) of the padded bit-packed occupancy tensor."""
         pitch = C.c_int()
-        p = _lib.lib().mpp_map_occ_bits(self.handle, C.byref(pitch))
+        p = _lib.lib().mpp_map_batch_occ_bits(self.handle, C.byref(pitch))
         return p, pitch.value
 
 

@@ -94,7 +94,7 @@ class MAACO:
 
         L = _lib.lib()
         self.map = GridMap(self.grid, device=device)
-        self._maps = C.c_void_p(L.mpp_map_as_batch(self.map.handle))
+        self._maps = self.map.handle
         self.device = torch.device("cuda", self.map.device)
         n = self.rows * self.cols
         R, Cc = self.rows, self.cols

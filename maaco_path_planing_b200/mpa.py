@@ -1,6 +1,6 @@
 """MPA -- drop-in for MPA.MPA (MPA.py:9-464).  The predator population (variable-length paths) lives
-in HBM; each iteration's phase move + memory + FADs step is one kernel launch (mpp_mpa_iteration), the
-stable sorts and the best-so-far cascade (MPA.py:412-437) stay on the host."""
+in HBM; each iteration's phase move + memory + FADs step is one kernel launch (mpp_mpa_iteration_batch on the map
+as a batch of one), the stable sorts and the best-so-far cascade (MPA.py:412-437) stay on the host."""
 from __future__ import annotations
 
 import ctypes as C
@@ -53,6 +53,9 @@ class MPA:
         self.group = group          # predators are independent given the sorted old population: sharded over ranks
         self.map = GridMap(self.grid, device=device)
         self.engine = SearchEngine(self.map)
+        self._seeds = self.engine.torch.from_numpy(np.array([self.rng_seed & (2 ** 64 - 1)], np.uint64).view(np.int64)
+                                                   ).to(self.engine.device)
+        self._queue = self.engine.torch.zeros(1, dtype=self.engine.torch.int32, device=self.engine.device)
         self.policy = make_policy(turn_penalty_factor, safety_penalty_factor, min_safe_distance,
                                   diagonal_obstacle_penalty, restrict_diagonal_near_obstacle, allow_diagonal_moves, mode=1)
         # Levy sigma MPA.py:251-253 (constant per solver; evaluated with the reference's own expression)
@@ -149,12 +152,12 @@ class MPA:
             tmp = t.empty((slots, mc), dtype=t.int32, device=eng.device)
             avoid = t.empty((slots, eng.words), dtype=t.int32, device=eng.device)
             status = t.zeros(1, dtype=t.int32, device=eng.device)
-            _lib.check(_lib.lib().mpp_mpa_iteration(
+            _lib.check(_lib.lib().mpp_mpa_iteration_batch(
                 self.map.handle, C.byref(self.policy), N, lo, hi, it, phase, self.P_const, CF, self.FADs_rate,
-                self._levy_sigma, self.levy_beta, C.c_uint64(self.rng_seed), _lib.ptr(P["cells"]), _lib.ptr(P["ncell"]),
+                self._levy_sigma, self.levy_beta, _lib.ptr(self._seeds), None, _lib.ptr(P["cells"]), _lib.ptr(P["ncell"]),
                 _lib.ptr(P["stats"]), mc, _lib.ptr(out_cells), _lib.ptr(out_n), _lib.ptr(out_stats), _lib.ptr(tmp),
-                _lib.ptr(avoid), _lib.ptr(scratch), scratch.numel(), slots, eng.heap_cap, _lib.ptr(status),
-                _lib.ptr(eng.counters), eng._stream()), "mpp_mpa_iteration")
+                _lib.ptr(avoid), _lib.ptr(scratch), scratch.numel(), slots, eng.heap_cap, _lib.ptr(self._queue),
+                _lib.ptr(status), _lib.ptr(eng.counters), eng._stream()), "mpp_mpa_iteration_batch")
             eng.launches += 1
             if world > 1:
                 dist.all_reduce(status, op=dist.ReduceOp.MAX, group=self.group)

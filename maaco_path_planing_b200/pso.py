@@ -1,13 +1,11 @@
 """PSOSolver -- drop-in for pso.PSOSolver (pso.py:8-240).  Particles live in HBM as torch tensors;
-the velocity/position update (mpp_pso_update) and the A*-connector fitness (mpp_waypoint_fitness) are
-sm_100a kernels.  The reference's particle loop is *asynchronous* (a particle sees the gbest already
+the velocity/position update (mpp_pso_update_batch) and the A*-connector fitness (mpp_waypoint_fitness_maps) are
+sm_100a kernels, launched on the map as a batch of one.  The reference's particle loop is *asynchronous* (a particle sees the gbest already
 improved by earlier particles of the same iteration, pso.py:187,190 vs :222-229); this is reproduced
 exactly by speculating with the current gbest and re-running only the particles after the first
 improver.  RNG: Philox streams of the RNG contract (rng_seed=None -> fresh entropy, like the reference).
 """
 from __future__ import annotations
-
-import ctypes as C
 
 import numpy as np
 
@@ -45,6 +43,8 @@ class PSOSolver(BasePathfinder):
                                           restrict_diagonal_near_obstacle_policy=self.restrict_diagonal_near_obstacle_policy,
                                           diagonal_obstacle_penalty_value=0, gridmap=self.map, engine=self.engine)
         self.rng_seed = _fresh_seed() if rng_seed is None else int(rng_seed)
+        self._seeds = self.engine.torch.from_numpy(np.array([self.rng_seed & (2 ** 64 - 1)], np.uint64).view(np.int64)
+                                                   ).to(self.engine.device)
         self.engine.group = group   # fitness evaluation is sharded over the group's ranks (individuals are independent)
         self.verbose = verbose
         self.gbest_particle_data = {'fitness': INF, 'path': [], 'position': []}
@@ -62,17 +62,6 @@ class PSOSolver(BasePathfinder):
         n = int(nc[0])
         return self._nodes(pc[0, :n].cpu().numpy()) if n > 0 else []
 
-    # ---- batched evaluation --------------------------------------------------------------------
-    def _evaluate_positions(self, pos):
-        """pos: device tensor [n, W, 2] -> (cells, n_cells, stats)."""
-        t = self.engine.torch
-        n = pos.shape[0]
-        wp = t.empty((n, self.num_waypoints), dtype=t.int32, device=pos.device)
-        _lib.check(_lib.lib().mpp_pso_round(self.map.handle, _lib.ptr(pos), n, self.num_waypoints, _lib.ptr(wp),
-                                            self.engine._stream()), "mpp_pso_round")
-        self.fitness_evaluations += n
-        return self.engine.waypoint_fitness(wp, self.policy)
-
     def _initialize_particles(self):                                        # pso.py:97-161
         t = self.engine.torch
         dev = self.engine.device
@@ -82,14 +71,15 @@ class PSOSolver(BasePathfinder):
         n_acc, attempts = 0, 0
         while n_acc < N and attempts < max_total:
             batch = min(max_total - attempts, max(32, int(1.25 * (N - n_acc)) + 8))
-            # the attempts of this batch are generated on the device (mpp_pso_init: same Philox streams as the reference
-            # harness, pso.py:50-51,105) and evaluated in one launch
+            # the attempts of this batch are generated on the device (mpp_pso_init_batch: same Philox streams as the
+            # reference harness, pso.py:50-51,105) and evaluated in one launch
             pos_d = t.empty((batch, W, 2), dtype=t.float64, device=dev)
             vel_d = t.empty((batch, W, 2), dtype=t.float64, device=dev)
             wp = t.empty((batch, W), dtype=t.int32, device=dev)
-            _lib.check(_lib.lib().mpp_pso_init(self.map.handle, batch, attempts, W, self.max_vel, C.c_uint64(self.rng_seed),
-                                               _lib.ptr(pos_d), _lib.ptr(vel_d), _lib.ptr(wp), self.engine._stream()),
-                       "mpp_pso_init")
+            offs = t.tensor([attempts], dtype=t.int32, device=dev)
+            _lib.check(_lib.lib().mpp_pso_init_batch(self.map.handle, batch, _lib.ptr(offs), W, self.max_vel,
+                                                     _lib.ptr(self._seeds), _lib.ptr(pos_d), _lib.ptr(vel_d), _lib.ptr(wp),
+                                                     self.engine._stream()), "mpp_pso_init_batch")
             self.fitness_evaluations += batch
             cells, ncell, stats = self.engine.waypoint_fitness(wp, self.policy)
             valid = (ncell > 0).cpu().numpy()
@@ -179,14 +169,14 @@ class PSOSolver(BasePathfinder):
             if rounds:
                 S["pos"][start:] = pos0[start:]
                 S["vel"][start:] = vel0[start:]
-            wp = t.empty((n, W), dtype=t.int32, device=S["pos"].device)
-            off = start * W * 2 * 8
-            _lib.check(L.mpp_pso_update(self.map.handle, C.c_void_p(S["pos"].data_ptr() + off),
-                                        C.c_void_p(S["vel"].data_ptr() + off),
-                                        C.c_void_p(S["pbest_pos"].data_ptr() + off), _lib.ptr(self._gbest_pos), n, start,
-                                        W, self.w, self.c1, self.c2, self.max_vel, C.c_uint64(self.rng_seed),
-                                        iteration, _lib.ptr(wp), self.engine._stream()), "mpp_pso_update")
-            cells, ncell, stats = self.engine.waypoint_fitness(wp, self.policy)
+            # particles [start, N) are updated; their waypoint cells are rows [start, N) of wp
+            wp = t.empty((N, W), dtype=t.int32, device=S["pos"].device)
+            first = t.tensor([start], dtype=t.int32, device=S["pos"].device)
+            _lib.check(L.mpp_pso_update_batch(self.map.handle, _lib.ptr(S["pos"]), _lib.ptr(S["vel"]),
+                                              _lib.ptr(S["pbest_pos"]), _lib.ptr(self._gbest_pos), N, _lib.ptr(first), W,
+                                              self.w, self.c1, self.c2, self.max_vel, _lib.ptr(self._seeds), iteration,
+                                              _lib.ptr(wp), self.engine._stream()), "mpp_pso_update_batch")
+            cells, ncell, stats = self.engine.waypoint_fitness(wp[start:], self.policy)
             self.fitness_evaluations += n
             rounds += 1
             valid = ncell > 0

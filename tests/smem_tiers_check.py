@@ -1,7 +1,8 @@
 """The search, fitness and MPA kernels on both sides of their shared-memory staging limits, against the oracle.
 
-mpp_astar_batch, mpp_waypoint_fitness and mpp_mpa_iteration[_batch] stage a map's packed occupancy in dynamic shared
-memory up to 32 KB without the opt-in attribute, up to 40 KB with it, and read it through L2 above that.  The kernels
+mpp_astar_batch_maps and mpp_waypoint_fitness_maps on a one-map batch, and mpp_mpa_iteration_batch on any batch, stage
+a map's packed occupancy in dynamic shared memory up to 32 KB without the opt-in attribute, up to 40 KB with it, and
+read it through L2 above that.  The kernels
 also declare ~16 KB of static shared memory, so a map of exactly 32 KB of occupancy needs the opt-in too.  Raising
 the attribute lasts for the rest of the process, so the 32 KB maps are only tested honestly in a process in which no
 larger map ran before: run as a script, this file checks the 32 KB shapes first and only then a larger one, and prints

@@ -48,10 +48,10 @@ def test_ctypes_signatures_match_header_arity():
     assert not bad, f"(ctypes argtypes, header parameters) differ: {bad}"
 
 
-def test_abi_version_and_error_string():
+def test_abi_version_3_and_error_string():
     from maaco_path_planing_b200 import _lib
     L = _lib.lib()
-    assert L.mpp_abi_version() == 2
+    assert L.mpp_abi_version() == 3
     assert isinstance(L.mpp_last_error(), bytes)
 
 

@@ -249,9 +249,9 @@ def test_pso_ga_medium_vs_oracle_mirrors():
     assert np.array_equal(ga._pop["chrom"].cpu().numpy(), np.array([ind[0] for ind in go.pop], np.int32))
 
 
-def test_population_kernels_full_size_vs_oracle():
+def test_population_kernels_one_map_batch_full_size_vs_oracle():
     """K8 / K9 at BASELINE config-3 population (4096 x 5 waypoints, 512x512): update, selection and breeding
-    kernels vs the C oracle, bit-exact."""
+    kernels on a one-map batch vs the C oracle, bit-exact."""
     import ctypes as C
     import torch
     import pyoracle as O
@@ -271,8 +271,11 @@ def test_population_kernels_full_size_vs_oracle():
     wp = torch.empty((N, W), dtype=torch.int32, device=dev)
     stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
     max_vel = max(1.0, 0.15 * 512)
-    _lib.check(L.mpp_pso_update(gm.handle, _lib.ptr(d_pos), _lib.ptr(d_vel), _lib.ptr(d_pb), _lib.ptr(d_gb), N, 0, W, 0.7,
-                                1.5, 1.5, max_vel, C.c_uint64(seed), it, _lib.ptr(wp), stream), "mpp_pso_update")
+    seeds = torch.tensor([seed], dtype=torch.int64, device=dev)
+    first = torch.zeros(1, dtype=torch.int32, device=dev)                  # every particle
+    _lib.check(L.mpp_pso_update_batch(gm.handle, _lib.ptr(d_pos), _lib.ptr(d_vel), _lib.ptr(d_pb), _lib.ptr(d_gb), N,
+                                      _lib.ptr(first), W, 0.7, 1.5, 1.5, max_vel, _lib.ptr(seeds), it, _lib.ptr(wp),
+                                      stream), "mpp_pso_update_batch")
     torch.cuda.synchronize()
     owp = np.zeros(W, np.int32)
     gpos, gvel, gwp = d_pos.cpu().numpy(), d_vel.cpu().numpy(), wp.cpu().numpy()
@@ -287,13 +290,14 @@ def test_population_kernels_full_size_vs_oracle():
     fit = np.sort(rng.random(N) * 100 + 700)
     d_fit = torch.as_tensor(fit, device=dev)
     parents = torch.empty(N, dtype=torch.int32, device=dev)
-    _lib.check(L.mpp_ga_select(_lib.ptr(d_fit), N, 3, C.c_uint64(seed), it, _lib.ptr(parents), stream), "mpp_ga_select")
+    _lib.check(L.mpp_ga_select_batch(gm.handle, _lib.ptr(d_fit), N, 3, _lib.ptr(seeds), it, _lib.ptr(parents), stream),
+               "mpp_ga_select_batch")
     free = np.flatnonzero(g.ravel() != 1)
     chrom = free[rng.integers(0, len(free), (N, W))].astype(np.int32)
     d_chrom = torch.as_tensor(chrom, device=dev)
     children = torch.empty((N, W), dtype=torch.int32, device=dev)
-    _lib.check(L.mpp_ga_breed(gm.handle, _lib.ptr(d_chrom), _lib.ptr(parents), N, W, 0.8, 0.1, C.c_uint64(seed), it,
-                              _lib.ptr(children), stream), "mpp_ga_breed")
+    _lib.check(L.mpp_ga_breed_batch(gm.handle, _lib.ptr(d_chrom), _lib.ptr(parents), N, W, 0.8, 0.1, _lib.ptr(seeds), it,
+                                    _lib.ptr(children), stream), "mpp_ga_breed_batch")
     torch.cuda.synchronize()
     par, ch = parents.cpu().numpy(), children.cpu().numpy()
     want = np.array([O.lib().orc_ga_select(p(fit), N, 3, C.c_uint64(seed), it, t) for t in range(N)], np.int32)

@@ -15,7 +15,7 @@ k = int(N * pso_frac)
 wps[k:] = free[rng.integers(0, len(free), (N - k, W))]
 eng = SearchEngine(GridMap(grid))
 if not use_order:
-    eng._longest_first = lambda w: None
+    eng._chain_order = lambda mi, w: None
 cells, ncell, stats = eng.waypoint_fitness(wps, make_policy(0.3, 0.8, 1.8, 100.0))
 torch.cuda.synchronize()
 ocells, oncell, ostats, oexp = O.waypoint_fitness(grid, wps, 0.3, 0.8, 1.8, 100.0, threads=0)

@@ -104,7 +104,7 @@ def main():
             x0 = sb.expansions()
             e0.record()
             for _ in range(args.reps):
-                sb._launch(variant, mi, src, dst, None, True)
+                sb._launch(variant, mi, src, dst, None, True, sb.allow_diagonal_moves, sb.restrict_corners, sb.policy)
             e1.record()
             torch.cuda.synchronize()
             ms = e0.elapsed_time(e1) / args.reps
