@@ -175,6 +175,19 @@ int mpp_maaco_e01_maps(const mpp_map_batch *maps, const mpp_maaco_params *p, dou
                        void *stream);
 int mpp_libm_exp_pow(int n, const double *e, const double *x, const double *y, double *out, int device, void *stream);
 
+/* The same two per-map tables for a batch whose maps also have their own colony parameters: params_dev is a DEVICE array
+ * of n_maps mpp_maaco_params, map k's entry read by the blocks of grid row k.
+ * mpp_maaco_tau0_maps_p: mpp_maaco_tau0_maps with C0_initial_pheromone of params_dev[k] for map k (MAACO.py:58-84);
+ *   bit for bit what mpp_maaco_tables writes for that map alone with those parameters.
+ * mpp_maaco_e01_maps_p: mpp_maaco_e01_maps with beta, a_turn_coef, wh_max, wh_min and k_h_adaptive of params_dev[k]
+ *   (MAACO.py:197-210, :238); bit for bit mpp_maaco_e01_host's table of map k under its parameters where the host's
+ *   libm is the build mpp_exp / mpp_pow reproduce.
+ * A null params_dev or a map without start or target is an MPP_EINVAL.  Asynchronous on `stream`. */
+int mpp_maaco_tau0_maps_p(const mpp_map_batch *maps, const mpp_maaco_params *params_dev, double *tau0_dev,
+                          long long tau_stride, void *stream);
+int mpp_maaco_e01_maps_p(const mpp_map_batch *maps, const mpp_maaco_params *params_dev, double *E01_dev,
+                         long long E01_stride, void *stream);
+
 /* replaces MAACO._calculate_adaptive_q0 (MAACO.py:212-226); pure host function */
 double mpp_maaco_q0(int num_iterations, int iteration, double q0_initial);
 
@@ -234,6 +247,18 @@ int mpp_maaco_pheromone(const mpp_map_batch *maps, const mpp_colony *colony, uin
 /* one whole pass of a non-sharded colony: rank + tours + best + pheromone, enqueued on `stream` (asynchronous) */
 int mpp_maaco_pass(const mpp_map_batch *maps, const mpp_colony *colony, const mpp_maaco_params *p, int iteration,
                    int n_ants, int ants_per_warp, void *stream);
+
+/* mpp_maaco_pass with per-map colony parameters -- one iteration of MAACO.solve_path_planning's loop
+ * (MAACO.py:336-359) for every map under ITS parameters, as if each map were solved alone with them.  params_dev: DEVICE
+ * array of n_maps mpp_maaco_params (alpha, Q and rho are read here; num_iterations is not); q0_dev: DEVICE table
+ * [num_iterations][n_maps] with q0_dev[(k-1) * n_maps + m] = mpp_maaco_q0(num_iterations, k, q0_initial of map m)
+ * (MAACO.py:212-226), row iteration-1 is read.  The four kernels are per-map instantiations of mpp_maaco_pass's and
+ * give map m the bits mpp_maaco_pass gives a one-map batch with map m's parameters (alpha != 1 included: both run CUDA's
+ * pow for tau**alpha, see mpp_maaco_rank).  colony->E01 may be shared (E01_stride 0) when every map shares its endpoints
+ * and table parameters, or per map (mpp_maaco_e01_maps_p).  A null params_dev / q0_dev, iteration < 1 or a map without
+ * start or target is an MPP_EINVAL.  Asynchronous on `stream`. */
+int mpp_maaco_pass_maps(const mpp_map_batch *maps, const mpp_colony *colony, const mpp_maaco_params *params_dev,
+                        const double *q0_dev, int iteration, int n_ants, int ants_per_warp, void *stream);
 
 /* the same pass with HOST buffers -- what a caller holding NumPy arrays binds: copies the pheromone field in
  * (tau_in_host: n_maps x rows*cols doubles, or NULL to keep the device field), runs the pass, copies out the updated

@@ -63,6 +63,8 @@ _SIGS = {
     "mpp_maaco_e01_host": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, C.POINTER(MaacoParams), c_void_p, c_int]),
     "mpp_maaco_tau0_maps": (c_int, [c_void_p, C.POINTER(MaacoParams), c_void_p, C.c_longlong, c_void_p]),
     "mpp_maaco_e01_maps": (c_int, [c_void_p, C.POINTER(MaacoParams), c_void_p, C.c_longlong, c_void_p]),
+    "mpp_maaco_tau0_maps_p": (c_int, [c_void_p, c_void_p, c_void_p, C.c_longlong, c_void_p]),
+    "mpp_maaco_e01_maps_p": (c_int, [c_void_p, c_void_p, c_void_p, C.c_longlong, c_void_p]),
     "mpp_libm_exp_pow": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "mpp_maaco_q0": (c_double, [c_int, c_int, c_double]),
     "mpp_maaco_rank_words": (C.c_longlong, [c_int, c_int]),
@@ -77,6 +79,7 @@ _SIGS = {
     "mpp_maaco_pheromone": (c_int, [c_void_p, C.POINTER(Colony), c_void_p, c_void_p, c_int, c_int, c_int, c_double,
                                     c_int, c_int, c_void_p, c_int, c_void_p]),
     "mpp_maaco_pass": (c_int, [c_void_p, C.POINTER(Colony), C.POINTER(MaacoParams), c_int, c_int, c_int, c_void_p]),
+    "mpp_maaco_pass_maps": (c_int, [c_void_p, C.POINTER(Colony), c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "mpp_maaco_pass_host": (c_int, [c_void_p, C.POINTER(Colony), C.POINTER(MaacoParams), c_int, c_int, c_int, c_void_p,
                                     c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "mpp_maaco_max_peers": (c_int, []),

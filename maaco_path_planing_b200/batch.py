@@ -9,7 +9,8 @@ holds maps of one (start, target) pair and shares ONE table computed on the host
 reference), and tau0 of each map is that shared table with the map's obstacles masked on the device
 (mpp_maaco_tables).  With per_map_endpoints=True a wave may mix endpoints: it then holds one eta'**beta table per map,
 built on the device with replicas of the host libm's exp / pow (mpp_maaco_e01_maps, bit for bit mpp_maaco_e01_host's),
-and tau0 is computed per map on the device (mpp_maaco_tau0_maps).
+and tau0 is computed per map on the device (mpp_maaco_tau0_maps).  With map_params each map of a wave also has its own
+colony parameters (a parameter sweep in one launch per pass): the pass kernels read them per map (mpp_maaco_pass_maps).
 
 Every batch class takes `grids` either on the host ([M, rows, cols] cell codes, anything np.asarray takes) or as an
 [M, rows, cols] CUDA tensor of bool, uint8, int8, int16, int32 or int64 cells; every sweep also takes a sequence of 2-D
@@ -171,6 +172,46 @@ def _maaco_params(num_iterations, alpha, beta, rho, Q, a_turn_coef, wh_max, wh_m
                             C0_initial_pheromone, num_iterations)
 
 
+MAP_PARAM_KEYS = ("alpha", "beta", "rho", "Q", "a_turn_coef", "wh_max", "wh_min", "k_h_adaptive", "q0_initial",
+                  "C0_initial_pheromone")
+_TABLE_KEYS = ("beta", "a_turn_coef", "wh_max", "wh_min", "k_h_adaptive")     # what eta'**beta depends on
+
+
+def resolve_map_params(defaults, map_params, n_maps):
+    """One dict of the ten MAP_PARAM_KEYS per map: map k's mapping of `map_params` over `defaults` (which holds at least
+    those keys).  ValueError for a length other than n_maps, an entry that is not a mapping, an unknown key or
+    num_iterations / num_ants (common to a wave: the pass count and the buffer layouts depend on them)."""
+    if isinstance(map_params, (str, bytes)) or not hasattr(map_params, "__len__"):
+        raise ValueError("map_params must be a sequence of one mapping per map")
+    if len(map_params) != n_maps:
+        raise ValueError(f"map_params has {len(map_params)} entries for {n_maps} maps")
+    defaults = {"C0_initial_pheromone": 0.1, **defaults}                      # (MAACO's default, MAACO.py:14)
+    base = {k: float(defaults[k]) for k in MAP_PARAM_KEYS}
+    out = []
+    for i, mp in enumerate(map_params):
+        if not hasattr(mp, "keys"):
+            raise ValueError(f"map_params[{i}] is not a mapping")
+        for k in mp.keys():
+            if k in ("num_iterations", "num_ants"):
+                raise ValueError(f"map_params[{i}]: {k} is common to all maps of a wave and cannot be set per map")
+            if k not in base:
+                raise ValueError(f"map_params[{i}]: unknown parameter {k!r} (per-map keys: {', '.join(MAP_PARAM_KEYS)})")
+        out.append({**base, **{k: float(v) for k, v in mp.items()}})
+    return out
+
+
+def q0_table(num_iterations, q0_initial):
+    """[max(1, num_iterations), len(q0_initial)] float64: row k-1 holds every map's q0 of pass k,
+    mpp_maaco_q0(num_iterations, k, q0_initial[m]) -- the value solo MAACO passes to its k-th pass (MAACO.py:212-226)."""
+    L = _lib.lib()
+    K = max(1, int(num_iterations))
+    q = np.asarray(q0_initial, np.float64)
+    out = np.empty((K, len(q)), np.float64)
+    for v in np.unique(q):                                       # one column per distinct q0_initial
+        out[:, q == v] = np.array([L.mpp_maaco_q0(int(num_iterations), k, float(v)) for k in range(1, K + 1)])[:, None]
+    return out
+
+
 def _e01_host(rows, cols, start, target, params, out, threads=0):
     """eta'**beta tables of the endpoint pairs (start[k], target[k]) of a rows x cols map into `out` (a contiguous
     float64 host tensor or array of at least len(start) * 2 * rows * cols values): mpp_maaco_e01_host."""
@@ -236,11 +277,18 @@ class MAACOBatch:
     device on the wave's stream by mpp_maaco_e01_maps -- or on the host by mpp_maaco_e01_host where _device_e01 says the
     device's exp / pow do not match the host libm), and tau0 is computed on the device from each map's own endpoints
     (mpp_maaco_tau0_maps).  A wave whose maps all share their endpoints takes the shared table
-    either way.  Results are those of solo MAACO with the same seed in both modes."""
+    either way.  Results are those of solo MAACO with the same seed in both modes.
+
+    map_params (None or one mapping per map) gives each map its own colony parameters: a mapping overrides any of
+    MAP_PARAM_KEYS, and the keys it leaves out take the constructor's values (`b.map_params` holds the resolved dicts).
+    The passes then run the per-map instantiations of the kernels (mpp_maaco_pass_maps), tau0 comes from
+    mpp_maaco_tau0_maps_p, and E01 is one table per map (mpp_maaco_e01_maps_p, or mpp_maaco_e01_host once per distinct
+    parameter set) unless every map shares its endpoints and the five parameters eta'**beta depends on.  Map k's results
+    are those of solo MAACO with map k's parameters and seed."""
 
     def __init__(self, grids, num_ants, num_iterations, alpha, beta, rho, Q, a_turn_coef, wh_max, wh_min, k_h_adaptive,
                  q0_initial, C0_initial_pheromone=0.1, *, seeds=None, device=None, max_cells=None, ants_per_warp=0,
-                 reuse=None, per_map_endpoints=False, _e01=None):
+                 reuse=None, per_map_endpoints=False, map_params=None, _e01=None):
         # _e01 (the max_cells repeat): this wave's per-map tables, already built -- an [M, 2 * rows * cols] CUDA tensor
         # on the wave's device, used as it is
         import torch
@@ -257,9 +305,20 @@ class MAACOBatch:
                                      q0_initial, C0_initial_pheromone)
         M, R, Cc, N = self.n_maps, self.rows, self.cols, self.num_ants
         start, target = self._map_set.start, self._map_set.target
-        # one table per map only where the endpoints differ: a wave that shares them keeps the shared table
-        self.per_map_tables = bool(per_map_endpoints) and M > 0 and not (
-            (start == start[0]).all() and (target == target[0]).all())
+        self.map_params = None
+        if map_params is not None:
+            self.map_params = resolve_map_params(
+                dict(alpha=alpha, beta=beta, rho=rho, Q=Q, a_turn_coef=a_turn_coef, wh_max=wh_max, wh_min=wh_min,
+                     k_h_adaptive=k_h_adaptive, q0_initial=q0_initial, C0_initial_pheromone=C0_initial_pheromone),
+                map_params, M)
+        shared_ends = M == 0 or ((start == start[0]).all() and (target == target[0]).all())
+        if self.map_params is not None and not per_map_endpoints and not shared_ends:
+            raise _lib.MppError("MAACOBatch: the maps of a wave must share start and target unless "
+                                "per_map_endpoints=True; group them")
+        # the eta'**beta parameter set of every map (map_params: each its own, else the constructor's)
+        table_keys = [tuple(p[k] for k in _TABLE_KEYS) for p in self.map_params] if self.map_params is not None else []
+        # one table per map only where the endpoints or the table parameters differ: otherwise the shared table
+        self.per_map_tables = M > 0 and ((bool(per_map_endpoints) and not shared_ends) or len(set(table_keys)) > 1)
         n = R * Cc
         TR = (R + 31) // 32
         self._auto_cells = max_cells is None
@@ -273,11 +332,12 @@ class MAACOBatch:
         self._ctor = dict(num_ants=num_ants, num_iterations=num_iterations, alpha=alpha, beta=beta, rho=rho, Q=Q,
                           a_turn_coef=a_turn_coef, wh_max=wh_max, wh_min=wh_min, k_h_adaptive=k_h_adaptive,
                           q0_initial=q0_initial, C0_initial_pheromone=C0_initial_pheromone, seeds=self.seeds,
-                          ants_per_warp=ants_per_warp, per_map_endpoints=per_map_endpoints)
+                          ants_per_warp=ants_per_warp, per_map_endpoints=per_map_endpoints, map_params=self.map_params)
         dev = self.device
         f64, i32, i64, u8 = torch.float64, torch.int32, torch.int64, torch.uint8
         K = max(1, self.num_iterations)
-        key = (M, R, Cc, N, self.max_cells, K, self.device_index, self.per_map_tables)   # (the E01 layout)
+        key = (M, R, Cc, N, self.max_cells, K, self.device_index, self.per_map_tables,   # (the E01 layout)
+               self.map_params is not None)
         if reuse is not None and getattr(reuse, "_key", None) == key:
             # the previous wave's device buffers (same shapes): nothing to allocate, only `touched` / counters to clear
             for name in ("_tau", "_E01", "_dist_t", "_rank", "_slabs", "_touched", "_moves", "_result", "_deposit", "_okbits",
@@ -305,23 +365,48 @@ class MAACOBatch:
             self._log = torch.zeros((M, K, 4), dtype=f64, device=dev)
         self._key = key
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        self._params_dev = self._q0_dev = None
+        if self.map_params is not None:
+            host = (_lib.MaacoParams * M)(*[_maaco_params(num_iterations, **p) for p in self.map_params])
+            self._params_dev = torch.frombuffer(bytearray(bytes(host)), dtype=u8).to(dev)
+            self._q0_dev = torch.from_numpy(q0_table(num_iterations, [p["q0_initial"] for p in self.map_params])).to(dev)
         if self.per_map_tables:
             if _e01 is not None:
                 if tuple(_e01.shape) != (M, 2 * n) or _e01.device != dev or _e01.dtype != f64:
                     raise ValueError(f"_e01 must be a float64 [{M}, {2 * n}] tensor on {dev}")
                 self._E01 = _e01
             elif _device_e01(self.device_index):
-                _lib.check(L.mpp_maaco_e01_maps(self._maps, C.byref(self._params), _lib.ptr(self._E01), 2 * n, stream),
-                           "mpp_maaco_e01_maps")
+                if self._params_dev is not None:
+                    _lib.check(L.mpp_maaco_e01_maps_p(self._maps, _lib.ptr(self._params_dev), _lib.ptr(self._E01), 2 * n,
+                                                      stream), "mpp_maaco_e01_maps_p")
+                else:
+                    _lib.check(L.mpp_maaco_e01_maps(self._maps, C.byref(self._params), _lib.ptr(self._E01), 2 * n,
+                                                    stream), "mpp_maaco_e01_maps")
             else:
-                host = _e01_host(R, Cc, start, target, self._params, torch.empty(M * 2 * n, dtype=f64, pin_memory=True))
+                host = torch.empty((M, 2 * n), dtype=f64, pin_memory=True)
+                if self.map_params is None:
+                    _e01_host(R, Cc, start, target, self._params, host)
+                else:
+                    for tk in dict.fromkeys(table_keys):                 # once per distinct parameter set
+                        idx = [k for k in range(M) if table_keys[k] == tk]
+                        pk = _maaco_params(num_iterations, **self.map_params[idx[0]])
+                        host[idx] = torch.from_numpy(_e01_host(R, Cc, start[idx], target[idx], pk,
+                                                               np.empty(len(idx) * 2 * n)).reshape(len(idx), 2 * n))
                 # (a pinned tensor of torch's host allocator is not reused before this copy has run)
-                self._E01.view(-1).copy_(host, non_blocking=True)
-            _lib.check(L.mpp_maaco_tau0_maps(self._maps, C.byref(self._params), _lib.ptr(self._tau), n, stream),
-                       "mpp_maaco_tau0_maps")
-        else:
+                self._E01.view(-1).copy_(host.view(-1), non_blocking=True)
+        elif self.map_params is None:
             _lib.check(L.mpp_maaco_tables(self._maps, C.byref(self._params), _lib.ptr(self._tau), n,
                                           _lib.ptr(self._E01), _lib.ptr(self._dist_t), stream), "mpp_maaco_tables")
+        else:                                                            # the table of map 0's (shared) table parameters
+            _lib.check(L.mpp_maaco_tables(self._maps, C.byref(_maaco_params(num_iterations, **self.map_params[0])),
+                                          _lib.ptr(self._tau), n, _lib.ptr(self._E01), _lib.ptr(self._dist_t), stream),
+                       "mpp_maaco_tables")
+        if self.map_params is not None:
+            _lib.check(L.mpp_maaco_tau0_maps_p(self._maps, _lib.ptr(self._params_dev), _lib.ptr(self._tau), n, stream),
+                       "mpp_maaco_tau0_maps_p")
+        elif self.per_map_tables:
+            _lib.check(L.mpp_maaco_tau0_maps(self._maps, C.byref(self._params), _lib.ptr(self._tau), n, stream),
+                       "mpp_maaco_tau0_maps")
         self._seeds = torch.from_numpy(np.array(self.seeds, np.uint64).view(np.int64)).to(dev)
         st = bytes(_lib.MaacoState(INF, -1, 0, 0, -1, INF, -1, -1))
         self._state = torch.frombuffer(bytearray(st * M), dtype=u8).to(dev)
@@ -349,8 +434,13 @@ class MAACOBatch:
         if not 1 <= it <= max(1, self.num_iterations):
             raise ValueError(f"iteration {it} outside 1..{self.num_iterations}")
         stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        _lib.check(_lib.lib().mpp_maaco_pass(self._maps, C.byref(self._colony), C.byref(self._params), it, self.num_ants,
-                                             self._apw, stream), "mpp_maaco_pass")
+        if self._params_dev is not None:
+            _lib.check(_lib.lib().mpp_maaco_pass_maps(self._maps, C.byref(self._colony), _lib.ptr(self._params_dev),
+                                                      _lib.ptr(self._q0_dev), it, self.num_ants, self._apw, stream),
+                       "mpp_maaco_pass_maps")
+        else:
+            _lib.check(_lib.lib().mpp_maaco_pass(self._maps, C.byref(self._colony), C.byref(self._params), it,
+                                                 self.num_ants, self._apw, stream), "mpp_maaco_pass")
         self.kernel_launches += 4
         self._iter_done = max(self._iter_done, it)
 
@@ -480,7 +570,7 @@ def _waves(keys, wave):
 
 
 def solve_maaco_batch(grids, num_ants, num_iterations, params, seeds=None, wave=256, group=None, device=None,
-                      max_cells=None, per_map_endpoints=False):
+                      max_cells=None, per_map_endpoints=False, map_params=None):
     """Run MAACO on every grid of `grids` (this rank's shard when `group` is given), `wave` maps per launch.  `grids`:
     host maps, a [n_maps, rows, cols] CUDA tensor or a sequence of 2-D CUDA tensors (which never leave the GPU).
 
@@ -489,8 +579,14 @@ def solve_maaco_batch(grids, num_ants, num_iterations, params, seeds=None, wave=
     (MAACOBatch(per_map_endpoints=True), whose per-map eta'**beta tables are built on the device).  A map without a
     start or target then raises before any wave runs.
 
+    map_params (None or one mapping per map of `grids`, by global index) gives map i its own colony parameters, as
+    MAACOBatch(map_params=...) takes them: map i is solved as MAACO(grids[i], ..., **{**params, **map_params[i]}).
+    Parameters never split waves; invalid map_params raise ValueError before any wave runs.
+
     Returns a list of (map_index, path, length, turns, convergence_curve) for the maps of this rank; results
     are identical to solving each map alone (same seeds => same Philox streams)."""
+    if map_params is not None:
+        map_params = resolve_map_params(params, map_params, len(grids))
     lo, hi = shard_maps(len(grids), group)
     maps = _sweep_maps(grids, lo, hi)
     start, target = maps.first_cells()
@@ -504,7 +600,8 @@ def solve_maaco_batch(grids, num_ants, num_iterations, params, seeds=None, wave=
     for idx in waves:
         b = MAACOBatch(maps.wave(idx), num_ants, num_iterations,
                        seeds=None if seeds is None else [seeds[i] for i in idx], device=device, max_cells=max_cells,
-                       reuse=prev, per_map_endpoints=per_map_endpoints, **params)
+                       reuse=prev, per_map_endpoints=per_map_endpoints,
+                       map_params=None if map_params is None else [map_params[i] for i in idx], **params)
         for i, (path, length, turns, curve) in zip(idx, b.solve()):
             out.append((i, path, length, turns, curve))
         b.close()

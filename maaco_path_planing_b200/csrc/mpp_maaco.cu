@@ -185,12 +185,16 @@ extern "C" int mpp_maaco_tables(const mpp_map_batch *maps, const mpp_maaco_param
 // tau0 of every map from its OWN start / target (MAACO.py:58-84, dsT floored as :43-45), obstacles at 1e-9 (:62-63):
 // host_table_rows' expression with the same integer dr^2 + dc^2, correctly rounded sqrt and division and no FMA
 // (-fmad=false), so each value is bit for bit what the host writes.
-__global__ void mpp_maaco_tau0_maps_kernel(const MppMapMeta *__restrict__ meta, const uint32_t *__restrict__ occ,
-                                           int occ_words, int pitch, int R, int C, double C0, double *__restrict__ tau,
-                                           long long tau_stride) {
+// MP (per-map parameters): C0 is params[k].C0_initial_pheromone instead of the launch's scalar.
+template <bool MP>
+__device__ __forceinline__ void tau0_maps_body(const MppMapMeta *__restrict__ meta, const uint32_t *__restrict__ occ,
+                                               int occ_words, int pitch, int R, int C, double C0,
+                                               const mpp_maaco_params *__restrict__ params, double *__restrict__ tau,
+                                               long long tau_stride) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= R * C) return;
     const int k = blockIdx.y;
+    if constexpr (MP) C0 = params[k].C0_initial_pheromone;
     occ += (size_t)k * occ_words;
     const int r = i / C, c = i % C, pb = c + 1;
     const int start = meta[k].start, target = meta[k].target;
@@ -210,34 +214,67 @@ __global__ void mpp_maaco_tau0_maps_kernel(const MppMapMeta *__restrict__ meta, 
     const bool obst = (occ[(r + 1) * pitch + (pb >> 5)] >> (pb & 31)) & 1u;
     tau[(size_t)k * tau_stride + i] = obst || v < 1e-9 ? 1e-9 : v;
 }
+__global__ void mpp_maaco_tau0_maps_kernel(const MppMapMeta *__restrict__ meta, const uint32_t *__restrict__ occ,
+                                           int occ_words, int pitch, int R, int C, double C0, double *__restrict__ tau,
+                                           long long tau_stride) {
+    tau0_maps_body<false>(meta, occ, occ_words, pitch, R, C, C0, nullptr, tau, tau_stride);
+}
+__global__ void mpp_maaco_tau0_maps_p_kernel(const MppMapMeta *__restrict__ meta, const uint32_t *__restrict__ occ,
+                                             int occ_words, int pitch, int R, int C,
+                                             const mpp_maaco_params *__restrict__ params, double *__restrict__ tau,
+                                             long long tau_stride) {
+    tau0_maps_body<true>(meta, occ, occ_words, pitch, R, C, 0.0, params, tau, tau_stride);
+}
+
+// one of p (the launch's scalars) / params_dev (per map) is given; `who` names the entry point in errors
+static int tau0_maps_launch(const mpp_map_batch *maps, const mpp_maaco_params *p, const mpp_maaco_params *params_dev,
+                            double *tau0_dev, long long tau_stride, void *stream, const char *who) {
+    MPP_REQUIRE(maps && (p || params_dev) && tau0_dev, "%s: null argument", who);
+    const int R = maps->rows, C = maps->cols;
+    const long long n = (long long)R * C;
+    MPP_REQUIRE(tau_stride >= n, "%s: tau_stride < rows*cols", who);
+    for (int k = 0; k < maps->n_maps; ++k)
+        MPP_REQUIRE(maps->meta_host[k].start >= 0 && maps->meta_host[k].target >= 0, "%s: map %d has no start/target", who, k);
+    if (maps->n_maps == 0) return MPP_OK;
+    MPP_CUDA(cudaSetDevice(maps->device));
+    const dim3 grid((unsigned)((n + 255) / 256), maps->n_maps);
+    if (params_dev)
+        mpp_maaco_tau0_maps_p_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(
+            maps->meta_dev, maps->occ_dev, maps->occ_words, maps->pitch_words, R, C, params_dev, tau0_dev, tau_stride);
+    else
+        mpp_maaco_tau0_maps_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(
+            maps->meta_dev, maps->occ_dev, maps->occ_words, maps->pitch_words, R, C, p->C0_initial_pheromone, tau0_dev,
+            tau_stride);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
 
 extern "C" int mpp_maaco_tau0_maps(const mpp_map_batch *maps, const mpp_maaco_params *p, double *tau0_dev,
                                    long long tau_stride, void *stream) {
-    MPP_REQUIRE(maps && p && tau0_dev, "mpp_maaco_tau0_maps: null argument");
-    const int R = maps->rows, C = maps->cols;
-    const long long n = (long long)R * C;
-    MPP_REQUIRE(tau_stride >= n, "mpp_maaco_tau0_maps: tau_stride < rows*cols");
-    for (int k = 0; k < maps->n_maps; ++k)
-        MPP_REQUIRE(maps->meta_host[k].start >= 0 && maps->meta_host[k].target >= 0,
-                    "mpp_maaco_tau0_maps: map %d has no start/target", k);
-    if (maps->n_maps == 0) return MPP_OK;
-    MPP_CUDA(cudaSetDevice(maps->device));
-    mpp_maaco_tau0_maps_kernel<<<dim3((unsigned)((n + 255) / 256), maps->n_maps), 256, 0, (cudaStream_t)stream>>>(
-        maps->meta_dev, maps->occ_dev, maps->occ_words, maps->pitch_words, R, C, p->C0_initial_pheromone, tau0_dev,
-        tau_stride);
-    MPP_CUDA(cudaGetLastError());
-    return MPP_OK;
+    return tau0_maps_launch(maps, p, nullptr, tau0_dev, tau_stride, stream, "mpp_maaco_tau0_maps");
+}
+
+extern "C" int mpp_maaco_tau0_maps_p(const mpp_map_batch *maps, const mpp_maaco_params *params_dev, double *tau0_dev,
+                                     long long tau_stride, void *stream) {
+    MPP_REQUIRE(params_dev, "mpp_maaco_tau0_maps_p: null params_dev");
+    return tau0_maps_launch(maps, nullptr, params_dev, tau0_dev, tau_stride, stream, "mpp_maaco_tau0_maps_p");
 }
 
 // E01 of every map from its OWN start / target (MAACO.py:197-210, dsT floored as :43-45): host_table_rows' expression
 // in its order -- integer dr^2 + dc^2, correctly rounded sqrt and division, no FMA (-fmad=false) -- with mpp_exp /
 // mpp_pow for libm's exp / pow, so each value is bit for bit what mpp_maaco_e01_host writes.
-__global__ void mpp_maaco_e01_maps_kernel(const MppMapMeta *__restrict__ meta, int R, int C, double beta, double wh_max,
-                                          double wh_min, double k_h, double a_turn, double *__restrict__ E01,
-                                          long long E01_stride) {
+template <bool MP>
+__device__ __forceinline__ void e01_maps_body(const MppMapMeta *__restrict__ meta, int R, int C, double beta,
+                                              double wh_max, double wh_min, double k_h, double a_turn,
+                                              const mpp_maaco_params *__restrict__ params, double *__restrict__ E01,
+                                              long long E01_stride) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= R * C) return;
     const int k = blockIdx.y;
+    if constexpr (MP) {
+        const mpp_maaco_params &P = params[k];
+        beta = P.beta; wh_max = P.wh_max; wh_min = P.wh_min; k_h = P.k_h_adaptive; a_turn = P.a_turn_coef;
+    }
     const int r = i / C, c = i % C;
     const int start = meta[k].start, target = meta[k].target;
     const int sr = start / C, sc = start % C, tr = target / C, tc = target % C;
@@ -256,24 +293,49 @@ __global__ void mpp_maaco_e01_maps_kernel(const MppMapMeta *__restrict__ meta, i
     d1 = d1 > 1e-9 ? d1 : 1e-9;
     *(double2 *)(E01 + (size_t)k * E01_stride + 2 * (size_t)i) = make_double2(mpp_pow(1.0 / d0, beta), mpp_pow(1.0 / d1, beta));
 }
+__global__ void mpp_maaco_e01_maps_kernel(const MppMapMeta *__restrict__ meta, int R, int C, double beta, double wh_max,
+                                          double wh_min, double k_h, double a_turn, double *__restrict__ E01,
+                                          long long E01_stride) {
+    e01_maps_body<false>(meta, R, C, beta, wh_max, wh_min, k_h, a_turn, nullptr, E01, E01_stride);
+}
+// MP: beta, a_turn_coef, wh_max, wh_min, k_h_adaptive of params[k]
+__global__ void mpp_maaco_e01_maps_p_kernel(const MppMapMeta *__restrict__ meta, int R, int C,
+                                            const mpp_maaco_params *__restrict__ params, double *__restrict__ E01,
+                                            long long E01_stride) {
+    e01_maps_body<true>(meta, R, C, 0.0, 0.0, 0.0, 0.0, 0.0, params, E01, E01_stride);
+}
+
+static int e01_maps_launch(const mpp_map_batch *maps, const mpp_maaco_params *p, const mpp_maaco_params *params_dev,
+                           double *E01_dev, long long E01_stride, void *stream, const char *who) {
+    MPP_REQUIRE(maps && (p || params_dev) && E01_dev, "%s: null argument", who);
+    const int R = maps->rows, C = maps->cols;
+    const long long n = (long long)R * C;
+    MPP_REQUIRE(E01_stride >= 2 * n && E01_stride % 2 == 0, "%s: E01_stride %lld is odd or < 2*rows*cols", who, E01_stride);
+    MPP_REQUIRE(((uintptr_t)E01_dev & 15) == 0, "%s: E01_dev is not 16-byte aligned", who);
+    for (int k = 0; k < maps->n_maps; ++k)
+        MPP_REQUIRE(maps->meta_host[k].start >= 0 && maps->meta_host[k].target >= 0, "%s: map %d has no start/target", who, k);
+    if (maps->n_maps == 0) return MPP_OK;
+    MPP_CUDA(cudaSetDevice(maps->device));
+    const dim3 grid((unsigned)((n + 255) / 256), maps->n_maps);
+    if (params_dev)
+        mpp_maaco_e01_maps_p_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(maps->meta_dev, R, C, params_dev, E01_dev,
+                                                                             E01_stride);
+    else
+        mpp_maaco_e01_maps_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(
+            maps->meta_dev, R, C, p->beta, p->wh_max, p->wh_min, p->k_h_adaptive, p->a_turn_coef, E01_dev, E01_stride);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
 
 extern "C" int mpp_maaco_e01_maps(const mpp_map_batch *maps, const mpp_maaco_params *p, double *E01_dev,
                                   long long E01_stride, void *stream) {
-    MPP_REQUIRE(maps && p && E01_dev, "mpp_maaco_e01_maps: null argument");
-    const int R = maps->rows, C = maps->cols;
-    const long long n = (long long)R * C;
-    MPP_REQUIRE(E01_stride >= 2 * n && E01_stride % 2 == 0, "mpp_maaco_e01_maps: E01_stride %lld is odd or < 2*rows*cols",
-                E01_stride);
-    MPP_REQUIRE(((uintptr_t)E01_dev & 15) == 0, "mpp_maaco_e01_maps: E01_dev is not 16-byte aligned");
-    for (int k = 0; k < maps->n_maps; ++k)
-        MPP_REQUIRE(maps->meta_host[k].start >= 0 && maps->meta_host[k].target >= 0,
-                    "mpp_maaco_e01_maps: map %d has no start/target", k);
-    if (maps->n_maps == 0) return MPP_OK;
-    MPP_CUDA(cudaSetDevice(maps->device));
-    mpp_maaco_e01_maps_kernel<<<dim3((unsigned)((n + 255) / 256), maps->n_maps), 256, 0, (cudaStream_t)stream>>>(
-        maps->meta_dev, R, C, p->beta, p->wh_max, p->wh_min, p->k_h_adaptive, p->a_turn_coef, E01_dev, E01_stride);
-    MPP_CUDA(cudaGetLastError());
-    return MPP_OK;
+    return e01_maps_launch(maps, p, nullptr, E01_dev, E01_stride, stream, "mpp_maaco_e01_maps");
+}
+
+extern "C" int mpp_maaco_e01_maps_p(const mpp_map_batch *maps, const mpp_maaco_params *params_dev, double *E01_dev,
+                                    long long E01_stride, void *stream) {
+    MPP_REQUIRE(params_dev, "mpp_maaco_e01_maps_p: null params_dev");
+    return e01_maps_launch(maps, nullptr, params_dev, E01_dev, E01_stride, stream, "mpp_maaco_e01_maps_p");
 }
 
 __global__ void mpp_libm_exp_pow_kernel(int n, const double *__restrict__ e, const double *__restrict__ x,
@@ -578,14 +640,30 @@ __device__ __forceinline__ uint32_t ldg32_nc_pinned(const uint32_t *p) {
 #define MPP_TOUR1_MINB 4
 #endif
 struct TourNoPeers {};
-template <bool P2P>
+// per-map colony parameters (the kernel's MP instantiation, mpp_maaco_pass_maps): alpha of params[map] and q0 of the
+// pass's row of the q0 table instead of TourArgs' scalars; they travel in the third parameter, which P2P never combines with
+struct TourMapParams {
+    const mpp_maaco_params *params;  // [n_maps]
+    const double *q0;                // [n_maps] this pass's q0 of every map
+};
+template <bool P2P, bool MP>
+using TourExtra = typename std::conditional<P2P, TourPeers, typename std::conditional<MP, TourMapParams, TourNoPeers>::type>::type;
+template <bool P2P, bool MP>
 __global__ void __launch_bounds__(MPP_TOUR1_THREADS, MPP_TOUR1_MINB)
-mpp_maaco_tour1_kernel(const TourArgs A, const int apw, const typename std::conditional<P2P, TourPeers, TourNoPeers>::type PA) {
+mpp_maaco_tour1_kernel(const TourArgs A, const int apw, const TourExtra<P2P, MP> PA) {
+    static_assert(!(P2P && MP), "a sharded colony has one parameter set");
     extern __shared__ __align__(16) uint8_t t1_smem[];
     if (A.latch && *A.latch) return;
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int R = A.R, C = A.C, TC = (C + 31) >> 5;
     const int map = blockIdx.y;
+    // MP: the same for the whole CTA (grid.y = map), loaded once and held in registers through the step loop.  (Read as
+    // `MP ? k_q0 : A.q0`: the other instantiations keep reading TourArgs' scalars exactly as before.)
+    double k_q0 = 0.0, k_alpha = 0.0;
+    if constexpr (MP) {
+        k_q0 = __shfl_sync(0xffffffffu, PA.q0[map], 0);
+        k_alpha = __shfl_sync(0xffffffffu, PA.params[map].alpha, 0);
+    }
     const MppMapMeta &MM = A.meta[map];
     const MppS1 s1 = MM.s1;
     const int target = MM.target;
@@ -744,7 +822,7 @@ mpp_maaco_tour1_kernel(const TourArgs A, const int apw, const typename std::cond
                 const mpp_u4 rb = mpp_philox(step + (uint32_t)(lane / apw), (uint32_t)(A.ant_offset + a0 + la), A.it,
                                              MPP_CLS_MAACO_TOUR, key0, key1);
                 const double u0 = mpp_u53(rb.x, rb.y), u1 = mpp_u53(rb.z, rb.w);
-                const bool greedy = u0 <= A.q0;
+                const bool greedy = u0 <= (MP ? k_q0 : A.q0);
                 uint32_t pack = greedy ? (1u << 24) : 0u;
 #pragma unroll
                 for (int n = 2; n <= 8; ++n) {
@@ -890,7 +968,8 @@ mpp_maaco_tour1_kernel(const TourArgs A, const int apw, const typename std::cond
                         m = __ffs(cand) - 1;                          // one candidate: every rule picks it
                     } else if ((fw & 7u) != 0u) {                     // some attractiveness >= 1e-10: literal rules
                         const double2 uu = rngu[(slot >> 2) + lane];
-                        m = tour_select_slow(cand, cur / C, cur % C, C, n_path >= 2, prev_m, tau_m, E01_m, A.alpha, A.q0, uu.x, uu.y);
+                        m = tour_select_slow(cand, cur / C, cur % C, C, n_path >= 2, prev_m, tau_m, E01_m, MP ? k_alpha : A.alpha,
+                                         MP ? k_q0 : A.q0, uu.x, uu.y);
                     } else {
                         uint32_t pool = cand;                         // roulette over tiny values: uniform (:253-254)
                         if (pack & (1u << 24)) {
@@ -982,7 +1061,7 @@ static int colony_check(const mpp_map_batch *maps, const mpp_colony *c, const ch
 static int tours_launch(const mpp_map_batch *maps, const mpp_colony *c, int iteration, double q0, double alpha,
                         int n_ants, int ant_offset, int n_ants_total, int ants_per_warp,
                         uint32_t *const *peer_slabs, uint32_t *const *peer_touched, mpp_ant_result *const *peer_result,
-                        int n_peers, int rows_per_rank, void *stream) {
+                        int n_peers, int rows_per_rank, void *stream, const TourMapParams *mp = nullptr) {
     int rc = colony_check(maps, c, "mpp_maaco_tours");
     if (rc) return rc;
     MPP_REQUIRE(n_ants > 0 && ant_offset >= 0 && ant_offset + n_ants <= n_ants_total, "mpp_maaco_tours: bad ant range");
@@ -1028,14 +1107,16 @@ static int tours_launch(const mpp_map_batch *maps, const mpp_colony *c, int iter
         static size_t smem_set[64] = {0};
         const int dv = maps->device & 63;
         if (smem > smem_set[dv]) {
-            MPP_CUDA(cudaFuncSetAttribute(mpp_maaco_tour1_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            MPP_CUDA(cudaFuncSetAttribute(mpp_maaco_tour1_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            MPP_CUDA(cudaFuncSetAttribute(mpp_maaco_tour1_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            MPP_CUDA(cudaFuncSetAttribute(mpp_maaco_tour1_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            MPP_CUDA(cudaFuncSetAttribute(mpp_maaco_tour1_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             smem_set[dv] = smem;
         }
     }
     const dim3 grid((warps + wpb - 1) / wpb, maps->n_maps);
-    if (n_peers > 0) mpp_maaco_tour1_kernel<true><<<grid, MPP_TOUR1_THREADS, smem, (cudaStream_t)stream>>>(A, apw, PA);
-    else mpp_maaco_tour1_kernel<false><<<grid, MPP_TOUR1_THREADS, smem, (cudaStream_t)stream>>>(A, apw, TourNoPeers());
+    if (mp) mpp_maaco_tour1_kernel<false, true><<<grid, MPP_TOUR1_THREADS, smem, (cudaStream_t)stream>>>(A, apw, *mp);
+    else if (n_peers > 0) mpp_maaco_tour1_kernel<true, false><<<grid, MPP_TOUR1_THREADS, smem, (cudaStream_t)stream>>>(A, apw, PA);
+    else mpp_maaco_tour1_kernel<false, false><<<grid, MPP_TOUR1_THREADS, smem, (cudaStream_t)stream>>>(A, apw, TourNoPeers());
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }
@@ -1072,19 +1153,21 @@ extern "C" int mpp_maaco_tours_p2p(const mpp_map_batch *maps, const mpp_colony *
 // field 0 = 0 when the ranking applies (all attractiveness < 1e-10), 7 when it does not; fields 1..7 are only
 // filled when P1 has exactly three moves.
 // ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) mpp_maaco_rank_kernel(const uint8_t *__restrict__ svalid_all,
-                                                             const double *__restrict__ tau_all, size_t tau_stride,
-                                                             const double *__restrict__ E01_all, size_t E01_stride,
-                                                             double alpha, int R, int C,
-                                                             const MppMapMeta *__restrict__ meta, uint32_t *__restrict__ rank_all,
-                                                             size_t rank_stride, size_t rank_margin, size_t rank_fast_words,
-                                                             size_t rank_bundle_words, size_t rank_nb8_words,
-                                                             const int32_t *__restrict__ latch) {
+// MP (per-map parameters): alpha of params[map] instead of the launch's scalar
+template <bool MP>
+__device__ __forceinline__ void rank_body(const uint8_t *__restrict__ svalid_all, const double *__restrict__ tau_all,
+                                          size_t tau_stride, const double *__restrict__ E01_all, size_t E01_stride,
+                                          double alpha, const mpp_maaco_params *__restrict__ params, int R, int C,
+                                          const MppMapMeta *__restrict__ meta, uint32_t *__restrict__ rank_all,
+                                          size_t rank_stride, size_t rank_margin, size_t rank_fast_words,
+                                          size_t rank_bundle_words, size_t rank_nb8_words,
+                                          const int32_t *__restrict__ latch, const unsigned tid) {
     // one thread per cell: the eight neighbours' tau / eta' are read once and serve all nine contexts
-    const int cell = blockIdx.x * 128 + threadIdx.x;
+    const int cell = blockIdx.x * 128 + tid;
     if (cell >= R * C) return;
     if (latch && *latch) return;
     const int map = blockIdx.y;
+    if constexpr (MP) alpha = params[map].alpha;
     const uint8_t *svalid = svalid_all + (size_t)map * R * C;
     const double *tau = tau_all + (size_t)map * tau_stride;
     const double *E01 = E01_all + (size_t)map * E01_stride;
@@ -1160,18 +1243,53 @@ __global__ void __launch_bounds__(128) mpp_maaco_rank_kernel(const uint8_t *__re
         }
     }
 }
+__global__ void __launch_bounds__(128) mpp_maaco_rank_kernel(const uint8_t *__restrict__ svalid_all,
+                                                             const double *__restrict__ tau_all, size_t tau_stride,
+                                                             const double *__restrict__ E01_all, size_t E01_stride,
+                                                             double alpha, int R, int C,
+                                                             const MppMapMeta *__restrict__ meta, uint32_t *__restrict__ rank_all,
+                                                             size_t rank_stride, size_t rank_margin, size_t rank_fast_words,
+                                                             size_t rank_bundle_words, size_t rank_nb8_words,
+                                                             const int32_t *__restrict__ latch) {
+    rank_body<false>(svalid_all, tau_all, tau_stride, E01_all, E01_stride, alpha, nullptr, R, C, meta, rank_all, rank_stride,
+                     rank_margin, rank_fast_words, rank_bundle_words, rank_nb8_words, latch, threadIdx.x);
+}
+__global__ void __launch_bounds__(128) mpp_maaco_rank_p_kernel(const uint8_t *__restrict__ svalid_all,
+                                                               const double *__restrict__ tau_all, size_t tau_stride,
+                                                               const double *__restrict__ E01_all, size_t E01_stride,
+                                                               const mpp_maaco_params *__restrict__ params, int R, int C,
+                                                               const MppMapMeta *__restrict__ meta,
+                                                               uint32_t *__restrict__ rank_all, size_t rank_stride,
+                                                               size_t rank_margin, size_t rank_fast_words,
+                                                               size_t rank_bundle_words, size_t rank_nb8_words,
+                                                               const int32_t *__restrict__ latch) {
+    rank_body<true>(svalid_all, tau_all, tau_stride, E01_all, E01_stride, 0.0, params, R, C, meta, rank_all, rank_stride,
+                    rank_margin, rank_fast_words, rank_bundle_words, rank_nb8_words, latch, threadIdx.x);
+}
 
-extern "C" int mpp_maaco_rank(const mpp_map_batch *maps, const mpp_colony *c, double alpha, void *stream) {
+// params_dev != null: the per-map instantiation (alpha of each map's params)
+static int rank_launch(const mpp_map_batch *maps, const mpp_colony *c, double alpha, const mpp_maaco_params *params_dev,
+                       void *stream) {
     int rc = colony_check(maps, c, "mpp_maaco_rank");
     if (rc) return rc;
     MPP_CUDA(cudaSetDevice(maps->device));
     const int total = maps->rows * maps->cols;
     const RankLayout L = rank_layout(maps->rows, maps->cols);
-    mpp_maaco_rank_kernel<<<dim3((total + 127) / 128, maps->n_maps), 128, 0, (cudaStream_t)stream>>>(
-        maps->svalid_dev, c->tau, (size_t)c->tau_stride, c->E01, (size_t)c->E01_stride, alpha, maps->rows, maps->cols,
-        maps->meta_dev, c->rank, L.total_words, L.margin, L.fast_words, L.bundle_words, L.nb8_words, c->latch);
+    const dim3 grid((total + 127) / 128, maps->n_maps);
+    if (params_dev)
+        mpp_maaco_rank_p_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(
+            maps->svalid_dev, c->tau, (size_t)c->tau_stride, c->E01, (size_t)c->E01_stride, params_dev, maps->rows,
+            maps->cols, maps->meta_dev, c->rank, L.total_words, L.margin, L.fast_words, L.bundle_words, L.nb8_words, c->latch);
+    else
+        mpp_maaco_rank_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(
+            maps->svalid_dev, c->tau, (size_t)c->tau_stride, c->E01, (size_t)c->E01_stride, alpha, maps->rows, maps->cols,
+            maps->meta_dev, c->rank, L.total_words, L.margin, L.fast_words, L.bundle_words, L.nb8_words, c->latch);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
+}
+
+extern "C" int mpp_maaco_rank(const mpp_map_batch *maps, const mpp_colony *c, double alpha, void *stream) {
+    return rank_launch(maps, c, alpha, nullptr, stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1186,12 +1304,14 @@ __device__ __forceinline__ int move_delta(uint32_t m, int C) {
     return ((int)((0xA940u >> (2 * m)) & 3u) - 1) * C + ((int)((0x9224u >> (2 * m)) & 3u) - 1);
 }
 
-__global__ void __launch_bounds__(MPP_BEST_THREADS)
-mpp_maaco_best_kernel(const mpp_ant_result *__restrict__ res_all, const uint8_t *__restrict__ moves_all, int max_cells,
-                      int moves_ant_offset, int moves_n_ants, int n, double Q, int iteration, int C,
-                      const MppMapMeta *__restrict__ meta, mpp_maaco_state *state_all, int32_t *best_cells_all,
-                      double *deposit_all, uint32_t *okbits_all, double *log_all, int log_rows,
-                      const int32_t *__restrict__ latch) {
+// MP (per-map parameters): Q of params[map] instead of the launch's scalar
+template <bool MP>
+__device__ __forceinline__ void best_body(const mpp_ant_result *__restrict__ res_all, const uint8_t *__restrict__ moves_all,
+                                          int max_cells, int moves_ant_offset, int moves_n_ants, int n, double Q,
+                                          const mpp_maaco_params *__restrict__ params, int iteration, int C,
+                                          const MppMapMeta *__restrict__ meta, mpp_maaco_state *state_all,
+                                          int32_t *best_cells_all, double *deposit_all, uint32_t *okbits_all,
+                                          double *log_all, int log_rows, const int32_t *__restrict__ latch) {
     __shared__ double s_len[32];
     __shared__ int s_idx[32];
     __shared__ int s_t[32];
@@ -1199,6 +1319,7 @@ mpp_maaco_best_kernel(const mpp_ant_result *__restrict__ res_all, const uint8_t 
     __shared__ int b_r, b_ant, b_turns, b_copy, s_base;
     if (latch && *latch) return;
     const int map = blockIdx.x;
+    if constexpr (MP) Q = params[map].Q;
     const mpp_ant_result *res = res_all + (size_t)map * n;
     double *deposit = deposit_all + (size_t)map * n;
     uint32_t *okbits = okbits_all + (size_t)map * ((n + 31) >> 5);
@@ -1327,18 +1448,46 @@ mpp_maaco_best_kernel(const mpp_ant_result *__restrict__ res_all, const uint8_t 
         }
     }
 }
+__global__ void __launch_bounds__(MPP_BEST_THREADS)
+mpp_maaco_best_kernel(const mpp_ant_result *__restrict__ res_all, const uint8_t *__restrict__ moves_all, int max_cells,
+                      int moves_ant_offset, int moves_n_ants, int n, double Q, int iteration, int C,
+                      const MppMapMeta *__restrict__ meta, mpp_maaco_state *state_all, int32_t *best_cells_all,
+                      double *deposit_all, uint32_t *okbits_all, double *log_all, int log_rows,
+                      const int32_t *__restrict__ latch) {
+    best_body<false>(res_all, moves_all, max_cells, moves_ant_offset, moves_n_ants, n, Q, nullptr, iteration, C, meta,
+                     state_all, best_cells_all, deposit_all, okbits_all, log_all, log_rows, latch);
+}
+__global__ void __launch_bounds__(MPP_BEST_THREADS)
+mpp_maaco_best_p_kernel(const mpp_ant_result *__restrict__ res_all, const uint8_t *__restrict__ moves_all, int max_cells,
+                        int moves_ant_offset, int moves_n_ants, int n, const mpp_maaco_params *__restrict__ params,
+                        int iteration, int C, const MppMapMeta *__restrict__ meta, mpp_maaco_state *state_all,
+                        int32_t *best_cells_all, double *deposit_all, uint32_t *okbits_all, double *log_all, int log_rows,
+                        const int32_t *__restrict__ latch) {
+    best_body<true>(res_all, moves_all, max_cells, moves_ant_offset, moves_n_ants, n, 0.0, params, iteration, C, meta,
+                    state_all, best_cells_all, deposit_all, okbits_all, log_all, log_rows, latch);
+}
 
-extern "C" int mpp_maaco_best(const mpp_map_batch *maps, const mpp_colony *c, int moves_ant_offset, int moves_n_ants,
-                              int n_ants_total, double Q, int iteration, void *stream) {
+static int best_launch(const mpp_map_batch *maps, const mpp_colony *c, int moves_ant_offset, int moves_n_ants,
+                       int n_ants_total, double Q, const mpp_maaco_params *params_dev, int iteration, void *stream) {
     int rc = colony_check(maps, c, "mpp_maaco_best");
     if (rc) return rc;
     MPP_REQUIRE(n_ants_total > 0 && iteration >= 1, "mpp_maaco_best: n_ants=%d iteration=%d", n_ants_total, iteration);
     MPP_CUDA(cudaSetDevice(maps->device));
-    mpp_maaco_best_kernel<<<maps->n_maps, MPP_BEST_THREADS, 0, (cudaStream_t)stream>>>(
-        c->result, c->moves, c->max_cells, moves_ant_offset, moves_n_ants, n_ants_total, Q, iteration, maps->cols,
-        maps->meta_dev, c->state, c->best_cells, c->deposit, c->okbits, c->log, c->log_rows, c->latch);
+    if (params_dev)
+        mpp_maaco_best_p_kernel<<<maps->n_maps, MPP_BEST_THREADS, 0, (cudaStream_t)stream>>>(
+            c->result, c->moves, c->max_cells, moves_ant_offset, moves_n_ants, n_ants_total, params_dev, iteration,
+            maps->cols, maps->meta_dev, c->state, c->best_cells, c->deposit, c->okbits, c->log, c->log_rows, c->latch);
+    else
+        mpp_maaco_best_kernel<<<maps->n_maps, MPP_BEST_THREADS, 0, (cudaStream_t)stream>>>(
+            c->result, c->moves, c->max_cells, moves_ant_offset, moves_n_ants, n_ants_total, Q, iteration, maps->cols,
+            maps->meta_dev, c->state, c->best_cells, c->deposit, c->okbits, c->log, c->log_rows, c->latch);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
+}
+
+extern "C" int mpp_maaco_best(const mpp_map_batch *maps, const mpp_colony *c, int moves_ant_offset, int moves_n_ants,
+                              int n_ants_total, double Q, int iteration, void *stream) {
+    return best_launch(maps, c, moves_ant_offset, moves_n_ants, n_ants_total, Q, nullptr, iteration, stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1402,7 +1551,9 @@ __device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; a
 #ifndef MPP_PHER_MINB
 #define MPP_PHER_MINB 7
 #endif
-__global__ void __launch_bounds__(MPP_PHER_THREADS, MPP_PHER_MINB) mpp_maaco_pheromone_kernel(const PherArgs A) {
+// MP (per-map parameters): rho of params[map] instead of PherArgs' scalar
+template <bool MP>
+__device__ __forceinline__ void pheromone_body(const PherArgs &A, const mpp_maaco_params *__restrict__ params) {
     __shared__ int s_list[MPP_PHER_CHUNK];
 #ifdef MPP_PHER_PROF
     const unsigned long long prof_t0 = gtimer();
@@ -1416,6 +1567,8 @@ __global__ void __launch_bounds__(MPP_PHER_THREADS, MPP_PHER_MINB) mpp_maaco_phe
     if ((blockIdx.x >> 2) != MPP_PHER_ONLY) return;
 #endif
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, map = blockIdx.y;
+    double rho = A.rho;
+    if constexpr (MP) rho = params[map].rho;
     const int TC = (A.C + 31) >> 5;
     // the start and the target tile carry the longest chains (every depositing ant): their CTAs go first
     int tile_l = blockIdx.x >> 2;                                     // tile index inside the buffers
@@ -1449,7 +1602,7 @@ __global__ void __launch_bounds__(MPP_PHER_THREADS, MPP_PHER_MINB) mpp_maaco_phe
     uint32_t *slab_t = A.slabs + (size_t)map * A.slab_stride + (size_t)tile_l * A.n_ants * 32 + row_in_tile;
     const double *dep = A.deposit + (size_t)map * A.n_ants;
     double t = 0.0;
-    if (live) t = tau[(size_t)r * A.C + c] * (1.0 - A.rho);            // :305
+    if (live) t = tau[(size_t)r * A.C + c] * (1.0 - rho);              // :305
     for (int w0 = 0; w0 < NW; w0 += MPP_PHER_CHUNK / 32) {
         // ---- the ants of this chunk that have a slab here and deposit, in index order ----
 #ifdef MPP_PHER_PROF
@@ -1557,7 +1710,7 @@ __global__ void __launch_bounds__(MPP_PHER_THREADS, MPP_PHER_MINB) mpp_maaco_phe
         __syncthreads();                                               // s_list is rebuilt by the next chunk
     }
     if (live) {
-        const double v = pher_finalize(t, r, c, A.occ + (size_t)map * A.occ_words, A.pitch, A.R, A.C, A.rho, A.state + map);
+        const double v = pher_finalize(t, r, c, A.occ + (size_t)map * A.occ_words, A.pitch, A.R, A.C, rho, A.state + map);
         if (A.tau_peers) {
             // fused with the "all-gather" of the tau slices: the value goes straight into every rank's field (NVLink stores)
             for (int k = 0; k < A.n_peers; ++k) A.tau_peers[k][(size_t)r * A.C + c] = v;
@@ -1578,10 +1731,18 @@ __global__ void __launch_bounds__(MPP_PHER_THREADS, MPP_PHER_MINB) mpp_maaco_phe
         for (int w = rg * MPP_PHER_THREADS + threadIdx.x; w < NW; w += 4 * MPP_PHER_THREADS) tn[w] = 0u;
     }
 }
+__global__ void __launch_bounds__(MPP_PHER_THREADS, MPP_PHER_MINB) mpp_maaco_pheromone_kernel(const PherArgs A) {
+    pheromone_body<false>(A, nullptr);
+}
+__global__ void __launch_bounds__(MPP_PHER_THREADS, MPP_PHER_MINB)
+mpp_maaco_pheromone_p_kernel(const PherArgs A, const mpp_maaco_params *__restrict__ params) {
+    pheromone_body<true>(A, params);
+}
 
-extern "C" int mpp_maaco_pheromone(const mpp_map_batch *maps, const mpp_colony *c, uint32_t *slabs_dev, uint32_t *touched_dev,
-                                   int n_ants_total, int tile_row0, int buf_tile_rows, double rho, int iteration,
-                                   int clear_slabs, double *const *tau_peers_dev, int n_peers, void *stream) {
+static int pheromone_launch(const mpp_map_batch *maps, const mpp_colony *c, uint32_t *slabs_dev, uint32_t *touched_dev,
+                            int n_ants_total, int tile_row0, int buf_tile_rows, double rho, int iteration, int clear_slabs,
+                            double *const *tau_peers_dev, int n_peers, void *stream,
+                            const mpp_maaco_params *params_dev = nullptr) {
     int rc = colony_check(maps, c, "mpp_maaco_pheromone");
     if (rc) return rc;
     const int TR = tiles_r(maps->rows), TC = tiles_c(maps->cols);
@@ -1607,9 +1768,18 @@ extern "C" int mpp_maaco_pheromone(const mpp_map_batch *maps, const mpp_colony *
     A.tau_peers = tau_peers_dev; A.n_peers = n_peers;
     A.meta = maps->meta_dev;
     MPP_REQUIRE(!tau_peers_dev || (n_peers > 0 && maps->n_maps == 1), "mpp_maaco_pheromone: peer tau needs n_peers > 0 and one map");
-    mpp_maaco_pheromone_kernel<<<dim3(n_tile_rows * TC * 4, maps->n_maps), MPP_PHER_THREADS, 0, (cudaStream_t)stream>>>(A);
+    const dim3 grid(n_tile_rows * TC * 4, maps->n_maps);
+    if (params_dev) mpp_maaco_pheromone_p_kernel<<<grid, MPP_PHER_THREADS, 0, (cudaStream_t)stream>>>(A, params_dev);
+    else mpp_maaco_pheromone_kernel<<<grid, MPP_PHER_THREADS, 0, (cudaStream_t)stream>>>(A);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
+}
+
+extern "C" int mpp_maaco_pheromone(const mpp_map_batch *maps, const mpp_colony *c, uint32_t *slabs_dev, uint32_t *touched_dev,
+                                   int n_ants_total, int tile_row0, int buf_tile_rows, double rho, int iteration,
+                                   int clear_slabs, double *const *tau_peers_dev, int n_peers, void *stream) {
+    return pheromone_launch(maps, c, slabs_dev, touched_dev, n_ants_total, tile_row0, buf_tile_rows, rho, iteration,
+                            clear_slabs, tau_peers_dev, n_peers, stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1839,6 +2009,25 @@ extern "C" int mpp_maaco_pass(const mpp_map_batch *maps, const mpp_colony *c, co
     rc = mpp_maaco_best(maps, c, 0, n_ants, n_ants, p->Q, iteration, stream);
     if (rc) return rc;
     return mpp_maaco_pheromone(maps, c, c->slabs, c->touched, n_ants, 0, tiles_r(maps->rows), p->rho, iteration, 0, nullptr, 0, stream);
+}
+
+// The same pass with per-map colony parameters: params_dev [n_maps] on the device, q0_dev the [num_iterations][n_maps]
+// q0 table (row iteration-1 is this pass's); the per-map instantiations of the four kernels read their scalars from them.
+extern "C" int mpp_maaco_pass_maps(const mpp_map_batch *maps, const mpp_colony *c, const mpp_maaco_params *params_dev,
+                                   const double *q0_dev, int iteration, int n_ants, int ants_per_warp, void *stream) {
+    MPP_REQUIRE(maps && c, "mpp_maaco_pass_maps: null argument");
+    MPP_REQUIRE(params_dev && q0_dev, "mpp_maaco_pass_maps: null params_dev / q0_dev");
+    MPP_REQUIRE(iteration >= 1, "mpp_maaco_pass_maps: iteration %d < 1", iteration);
+    int rc = rank_launch(maps, c, 0.0, params_dev, stream);
+    if (rc) return rc;
+    const TourMapParams mp{params_dev, q0_dev + (size_t)(iteration - 1) * maps->n_maps};
+    rc = tours_launch(maps, c, iteration, 0.0, 0.0, n_ants, 0, n_ants, ants_per_warp, nullptr, nullptr, nullptr, 0, 1, stream,
+                      &mp);
+    if (rc) return rc;
+    rc = best_launch(maps, c, 0, n_ants, n_ants, 0.0, params_dev, iteration, stream);
+    if (rc) return rc;
+    return pheromone_launch(maps, c, c->slabs, c->touched, n_ants, 0, tiles_r(maps->rows), 0.0, iteration, 0, nullptr, 0,
+                            stream, params_dev);
 }
 
 extern "C" int mpp_maaco_pass_host(const mpp_map_batch *maps, const mpp_colony *c, const mpp_maaco_params *p, int iteration,
