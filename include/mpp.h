@@ -386,6 +386,37 @@ int mpp_waypoint_fitness_maps(mpp_map_batch *maps, const int32_t *map_dev, const
                               void *scratch_dev, size_t scratch_bytes, int n_slots, int heap_cap,
                               unsigned long long *counters_dev, const int32_t *order_dev, void *stream);
 
+/* ---- per-map parameters of the population planners (a parameter sweep as one batch) --------------------------------
+ * One entry per map of a batch, kept by the caller in a DEVICE array params_dev[n_maps]; map m's entry is read by the
+ * blocks (or lane groups) that work on map m.  Each planner reads its own fields and the three statistics weights:
+ *   PSO: w, c1, c2 (pso.py:185-190); GA: crossover_rate, mutation_rate, tournament_size (ga_solver.py:136-160);
+ *   MPA: P_const, FADs_rate, levy_sigma (MPA.py:251-253, computed by the caller), levy_beta (MPA.py:10-18);
+ *   the statistics: turn_penalty_factor, safety_penalty_factor, diagonal_obstacle_penalty_value (helper.py:98-113,
+ *   MPA.py:215-229) in place of the mpp_policy fields of those names.
+ * What changes the search or the safety tables -- min_safe_distance, allow_diagonal, restrict_policy, mode -- stays in
+ * the mpp_policy argument and is common to the batch. */
+typedef struct {
+    double w, c1, c2;
+    double crossover_rate, mutation_rate;
+    int tournament_size;
+    double P_const, FADs_rate, levy_sigma, levy_beta;
+    double turn_penalty_factor, safety_penalty_factor, diagonal_obstacle_penalty_value;
+} mpp_pop_params;
+
+/* mpp_waypoint_fitness_maps / mpp_path_stats with the statistics weights of params_dev[m] for an individual / path on
+ * map m (an individual or path outside the batch gets the empty path's statistics, as there); the searches are those of
+ * the functions without _p.  For map m the results are bit for bit what the function without _p gives with a policy
+ * carrying params_dev[m]'s weights.  A null params_dev is an MPP_EINVAL. */
+int mpp_waypoint_fitness_maps_p(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *waypoints_dev,
+                                int n_individuals, int n_waypoints, const mpp_policy *policy,
+                                const mpp_pop_params *params_dev, int32_t *cells_dev, int max_cells,
+                                int32_t *n_cells_dev, double *stats_dev, uint32_t *visited_dev, void *scratch_dev,
+                                size_t scratch_bytes, int n_slots, int heap_cap, unsigned long long *counters_dev,
+                                const int32_t *order_dev, void *stream);
+int mpp_path_stats_p(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *cells_dev, int max_cells,
+                     const int32_t *n_cells_dev, int n_paths, const mpp_policy *policy,
+                     const mpp_pop_params *params_dev, double *stats_dev, void *stream);
+
 /* ---- MPA (MPA.py) ------------------------------------------------------------------------------- */
 
 /* MPA over a batch of independent same-shape maps (BASELINE config 5; a single map is a batch of one), one launch per
@@ -419,6 +450,21 @@ int mpp_mpa_iteration_batch(const mpp_map_batch *maps, const mpp_policy *policy,
                             int32_t *out_n_dev, double *out_stats_dev, int32_t *tmp_cells_dev, uint32_t *avoid_dev,
                             void *scratch_dev, size_t scratch_bytes, int warps_per_map, int heap_cap, uint32_t *queue_dev,
                             int32_t *status_dev, unsigned long long *counters_dev, void *stream);
+/* The same two steps for a batch whose maps have their own MPA parameters (mpp_pop_params above): map m reads P_const,
+ * FADs_rate, levy_sigma and levy_beta (1 / levy_beta is an IEEE division, as mpp_mpa_iteration_batch computes it) and
+ * the three statistics weights from params_dev[m] in place of the scalars and the policy's weights; map m's results are
+ * bit for bit those of the functions without _p given map m's values.  A null params_dev is an MPP_EINVAL. */
+int mpp_mpa_init_batch_p(const mpp_map_batch *maps, const mpp_policy *policy, const mpp_pop_params *params_dev,
+                         int n_predators, int max_cells, int32_t *cells_dev, int32_t *n_cells_dev, double *stats_dev,
+                         void *scratch_dev, size_t scratch_bytes, int heap_cap, int32_t *status_dev,
+                         unsigned long long *counters_dev, void *stream);
+int mpp_mpa_iteration_batch_p(const mpp_map_batch *maps, const mpp_policy *policy, int n_predators, int pred_begin,
+                              int pred_end, int iteration, int phase, const mpp_pop_params *params_dev, double CF,
+                              const uint64_t *seeds_dev, const int32_t *order_dev, const int32_t *cells_dev,
+                              const int32_t *n_cells_dev, const double *stats_dev, int max_cells, int32_t *out_cells_dev,
+                              int32_t *out_n_dev, double *out_stats_dev, int32_t *tmp_cells_dev, uint32_t *avoid_dev,
+                              void *scratch_dev, size_t scratch_bytes, int warps_per_map, int heap_cap,
+                              uint32_t *queue_dev, int32_t *status_dev, unsigned long long *counters_dev, void *stream);
 /* bytes of one search slot's scratch for a rows x cols map */
 size_t mpp_astar_slot_bytes(int rows, int cols, int heap_cap);
 
@@ -463,6 +509,22 @@ int mpp_ga_select_batch(const mpp_map_batch *maps, const double *fitness_dev, in
 int mpp_ga_breed_batch(const mpp_map_batch *maps, const int32_t *chrom_dev, const int32_t *parents_dev, int n,
                        int n_waypoints, double crossover_rate, double mutation_rate, const uint64_t *seeds_dev,
                        int generation, int32_t *children_dev, void *stream);
+
+/* The three update steps with per-map parameters: map m reads w, c1, c2 / tournament_size / crossover_rate,
+ * mutation_rate from params_dev[m] (mpp_pop_params) in place of the scalars; everything else as above, and map m's
+ * results are bit for bit those of the functions without _p given map m's values.  A map whose
+ * k = min(tournament_size, n) the selection cannot take (k outside 1..16, or k > 5 with n <= 85: the scalar function
+ * refuses such a launch) gets parents -1 in every slot; the breeding reads a parent index outside 0..n-1 as 0.  Neither
+ * kernel reads or writes outside its buffers for any parameter value.  A null params_dev is an MPP_EINVAL. */
+int mpp_pso_update_batch_p(const mpp_map_batch *maps, double *pos_dev, double *vel_dev, const double *pbest_pos_dev,
+                           const double *gbest_pos_dev, int n_particles, const int32_t *start_dev, int n_waypoints,
+                           const mpp_pop_params *params_dev, double max_vel, const uint64_t *seeds_dev, int iteration,
+                           int32_t *waypoint_cells_dev, void *stream);
+int mpp_ga_select_batch_p(const mpp_map_batch *maps, const double *fitness_dev, int n, const mpp_pop_params *params_dev,
+                          const uint64_t *seeds_dev, int generation, int32_t *parents_dev, void *stream);
+int mpp_ga_breed_batch_p(const mpp_map_batch *maps, const int32_t *chrom_dev, const int32_t *parents_dev, int n,
+                         int n_waypoints, const mpp_pop_params *params_dev, const uint64_t *seeds_dev, int generation,
+                         int32_t *children_dev, void *stream);
 
 #ifdef __cplusplus
 }

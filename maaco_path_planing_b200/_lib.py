@@ -46,6 +46,14 @@ class Policy(C.Structure):
                 ("restrict_policy", c_int), ("allow_diagonal", c_int), ("mode", c_int)]
 
 
+class PopParams(C.Structure):
+    """mpp_pop_params (include/mpp.h): one map's PSO / GA / MPA parameters and statistics weights."""
+    _fields_ = [("w", c_double), ("c1", c_double), ("c2", c_double), ("crossover_rate", c_double),
+                ("mutation_rate", c_double), ("tournament_size", c_int), ("P_const", c_double), ("FADs_rate", c_double),
+                ("levy_sigma", c_double), ("levy_beta", c_double), ("turn_penalty_factor", c_double),
+                ("safety_penalty_factor", c_double), ("diagonal_obstacle_penalty_value", c_double)]
+
+
 _SIGS = {
     "mpp_abi_version": (c_int, []),
     "mpp_last_error": (C.c_char_p, []),
@@ -109,6 +117,17 @@ _SIGS = {
     "mpp_waypoint_fitness_maps": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, C.POINTER(Policy), c_void_p, c_int,
                                           c_void_p, c_void_p, c_void_p, c_void_p, C.c_size_t, c_int, c_int, c_void_p,
                                           c_void_p, c_void_p]),
+    "mpp_waypoint_fitness_maps_p": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, C.POINTER(Policy), c_void_p,
+                                            c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, C.c_size_t, c_int,
+                                            c_int, c_void_p, c_void_p, c_void_p]),
+    "mpp_path_stats_p": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, C.POINTER(Policy), c_void_p,
+                                 c_void_p, c_void_p]),
+    "mpp_mpa_init_batch_p": (c_int, [c_void_p, C.POINTER(Policy), c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, C.c_size_t, c_int, c_void_p, c_void_p, c_void_p]),
+    "mpp_mpa_iteration_batch_p": (c_int, [c_void_p, C.POINTER(Policy), c_int, c_int, c_int, c_int, c_int, c_void_p,
+                                          c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
+                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, C.c_size_t, c_int, c_int,
+                                          c_void_p, c_void_p, c_void_p, c_void_p]),
     "mpp_pso_init_batch": (c_int, [c_void_p, c_int, c_void_p, c_int, c_double, c_void_p, c_void_p, c_void_p, c_void_p,
                                    c_void_p]),
     "mpp_ga_init_batch": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
@@ -117,6 +136,11 @@ _SIGS = {
     "mpp_ga_select_batch": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p]),
     "mpp_ga_breed_batch": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_double, c_double, c_void_p, c_int,
                                    c_void_p, c_void_p]),
+    "mpp_pso_update_batch_p": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int,
+                                       c_void_p, c_double, c_void_p, c_int, c_void_p, c_void_p]),
+    "mpp_ga_select_batch_p": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
+    "mpp_ga_breed_batch_p": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p,
+                                     c_void_p]),
 }
 
 _lib = None

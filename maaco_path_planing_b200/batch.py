@@ -176,28 +176,130 @@ MAP_PARAM_KEYS = ("alpha", "beta", "rho", "Q", "a_turn_coef", "wh_max", "wh_min"
                   "C0_initial_pheromone")
 _TABLE_KEYS = ("beta", "a_turn_coef", "wh_max", "wh_min", "k_h_adaptive")     # what eta'**beta depends on
 
+_WEIGHT_KEYS = ("turn_penalty_factor", "safety_penalty_factor", "diagonal_obstacle_penalty_value")
+_WAYPOINT_WAVE_KEYS = ("min_safe_distance", "allow_diagonal_moves", "restrict_diagonal_near_obstacle_policy")
+_WAYPOINT_DEFAULTS = dict(turn_penalty_factor=0.1, safety_penalty_factor=0.05, min_safe_distance=1.5,   # pso.py:22-25,
+                          allow_diagonal_moves=True, restrict_diagonal_near_obstacle_policy=True,      # ga_solver.py:19-22
+                          diagonal_obstacle_penalty_value=1000.0)
+# planner -> (keys a map may set, keys a map may set only to its wave's value (they change the searches or the safety
+# tables; the sweeps group waves by them), keys common to a wave (sizes), the constructor's defaults)
+PLANNER_MAP_PARAMS = {
+    "maaco": (MAP_PARAM_KEYS, (), ("num_iterations", "num_ants"),
+              {"C0_initial_pheromone": 0.1}),                                 # (MAACO's default, MAACO.py:14)
+    "pso": (("w", "c1", "c2") + _WEIGHT_KEYS, _WAYPOINT_WAVE_KEYS,
+            ("num_iterations", "num_particles", "num_waypoints_per_particle"), _WAYPOINT_DEFAULTS),
+    "ga": (("mutation_rate", "crossover_rate", "tournament_size") + _WEIGHT_KEYS, _WAYPOINT_WAVE_KEYS,
+           ("num_generations", "population_size", "num_waypoints_per_chromosome"),
+           dict(_WAYPOINT_DEFAULTS, tournament_size=3)),
+    "mpa": (("FADs_rate", "P_const", "levy_beta", "turn_penalty_factor", "safety_penalty_factor",
+             "diagonal_obstacle_penalty", "min_safe_distance"),               # (min_safe_distance: never read, MPA.py:173)
+            ("allow_diagonal_moves", "restrict_diagonal_near_obstacle"), ("num_predators", "num_iterations"),
+            dict(FADs_rate=0.2, P_const=0.5, levy_beta=1.5, turn_penalty_factor=0.1, safety_penalty_factor=0.05,
+                 min_safe_distance=1.5, allow_diagonal_moves=True, restrict_diagonal_near_obstacle=True,
+                 diagonal_obstacle_penalty=1000.0)),                          # MPA.py:10-18
+}
+_GA_MAX_K = 16                                     # the sample buffers of the selection kernel (mpp_pop.cu)
 
-def resolve_map_params(defaults, map_params, n_maps):
-    """One dict of the ten MAP_PARAM_KEYS per map: map k's mapping of `map_params` over `defaults` (which holds at least
-    those keys).  ValueError for a length other than n_maps, an entry that is not a mapping, an unknown key or
-    num_iterations / num_ants (common to a wave: the pass count and the buffer layouts depend on them)."""
+
+def levy_sigma(levy_beta):
+    """The Levy sigma of MPA.py:251-253; ValueError where the reference expression is complex."""
+    import math
+    b = levy_beta
+    num = math.gamma(1 + b) * math.sin(math.pi * b / 2)
+    den = math.gamma((1 + b) / 2) * b * (2 ** ((b - 1) / 2))
+    sig = (num / den) ** (1 / b) if den > 1e-9 else 1.0
+    if isinstance(sig, complex):
+        raise ValueError("levy_beta gives a complex Levy sigma in the reference expression (MPA.py:253)")
+    return float(sig)
+
+
+def _map_param_value(planner, i, k, v):
+    """Map i's value of key k as the planner's kernels take it: tournament_size an integer, the two move switches
+    booleans, everything else a float."""
+    if k in ("allow_diagonal_moves", "restrict_diagonal_near_obstacle_policy", "restrict_diagonal_near_obstacle"):
+        return bool(v)
+    if planner == "ga" and k == "tournament_size":
+        if isinstance(v, bool) or int(v) != v:
+            raise ValueError(f"map_params[{i}]: tournament_size must be an integer, not {v!r}")
+        return int(v)
+    return float(v)
+
+
+def resolve_map_params(defaults, map_params, n_maps, planner="maaco", population=None):
+    """One dict per map of the keys `planner` may set per map and per wave (PLANNER_MAP_PARAMS; MAACO: the ten
+    MAP_PARAM_KEYS): map k's mapping of `map_params` over `defaults` (the constructor's arguments; keys it leaves out
+    take the constructor's defaults).  ValueError for a length other than n_maps, an entry that is not a mapping, an
+    unknown key or a size common to a wave (MAACO: num_iterations / num_ants -- the pass count and the buffer layouts
+    depend on them), and for values the kernels cannot take: GA's tournament_size where min(tournament_size,
+    population) lies outside 1..16 or exceeds 5 with a population of 85 or less (mpp_ga_select_batch's limits), MPA's
+    levy_beta where the Levy sigma is complex.  Whether the per-wave keys agree is the caller's matter
+    (_wave_params)."""
+    per_map, per_wave, sizes, ctor_defaults = PLANNER_MAP_PARAMS[planner]
     if isinstance(map_params, (str, bytes)) or not hasattr(map_params, "__len__"):
         raise ValueError("map_params must be a sequence of one mapping per map")
     if len(map_params) != n_maps:
         raise ValueError(f"map_params has {len(map_params)} entries for {n_maps} maps")
-    defaults = {"C0_initial_pheromone": 0.1, **defaults}                      # (MAACO's default, MAACO.py:14)
-    base = {k: float(defaults[k]) for k in MAP_PARAM_KEYS}
+    defaults = {**ctor_defaults, **defaults}
+    base = {k: _map_param_value(planner, "defaults", k, defaults[k]) for k in per_map + per_wave}
+    known = f"per-map keys: {', '.join(per_map)}" + (f"; per-wave keys: {', '.join(per_wave)}" if per_wave else "")
     out = []
     for i, mp in enumerate(map_params):
         if not hasattr(mp, "keys"):
             raise ValueError(f"map_params[{i}] is not a mapping")
         for k in mp.keys():
-            if k in ("num_iterations", "num_ants"):
+            if k in sizes:
                 raise ValueError(f"map_params[{i}]: {k} is common to all maps of a wave and cannot be set per map")
             if k not in base:
-                raise ValueError(f"map_params[{i}]: unknown parameter {k!r} (per-map keys: {', '.join(MAP_PARAM_KEYS)})")
-        out.append({**base, **{k: float(v) for k, v in mp.items()}})
+                raise ValueError(f"map_params[{i}]: unknown parameter {k!r} ({known})")
+        p = {**base, **{k: _map_param_value(planner, i, k, v) for k, v in mp.items()}}
+        if planner == "ga":
+            k = min(p["tournament_size"], population)
+            if not (1 <= k <= _GA_MAX_K and (k <= 5 or population > 21 + 64)):
+                raise ValueError(f"map_params[{i}]: tournament_size {p['tournament_size']} unsupported with a population "
+                                 f"of {population} (min(tournament_size, population) must lie in 1..{_GA_MAX_K}, and "
+                                 f"be at most 5 for a population of 85 or less)")
+        if planner == "mpa":
+            try:
+                levy_sigma(p["levy_beta"])
+            except ValueError as e:
+                raise ValueError(f"map_params[{i}]: {e}") from None
+        out.append(p)
     return out
+
+
+def _wave_params(planner, resolved):
+    """The per-wave values (PLANNER_MAP_PARAMS) every map of `resolved` shares; ValueError naming the first map whose
+    value differs from map 0's."""
+    keys = PLANNER_MAP_PARAMS[planner][1]
+    first = {k: resolved[0][k] for k in keys} if resolved else {}
+    for i, p in enumerate(resolved):
+        for k in keys:
+            if p[k] != first[k]:
+                raise ValueError(f"map_params[{i}]: {k}={p[k]!r} differs from map 0's {first[k]!r}; it is common to the "
+                                 f"maps of a wave (the sweeps group maps by it)")
+    return first
+
+
+def _pop_params_dev(planner, resolved, device):
+    """[M] mpp_pop_params of the resolved per-map parameters (_pop_params_host) as a uint8 CUDA tensor on `device`."""
+    import torch
+    return torch.frombuffer(bytearray(_pop_params_host(planner, resolved)), dtype=torch.uint8).to(device)
+
+
+def _pop_params_host(planner, resolved):
+    """The bytes of [M] mpp_pop_params holding the resolved per-map parameters (the kernels read the fields of their
+    planner and the statistics weights; MPA's Levy sigma is computed here, as MPA.py:251-253 does)."""
+    rows = []
+    for p in resolved:
+        q = _lib.PopParams()
+        for f, _ in _lib.PopParams._fields_:
+            if f in p:
+                setattr(q, f, p[f])
+        if planner == "mpa":
+            q.diagonal_obstacle_penalty_value = p["diagonal_obstacle_penalty"]
+            q.levy_sigma = levy_sigma(p["levy_beta"])
+        rows.append(bytes(q))
+    return b"".join(rows)
 
 
 def q0_table(num_iterations, q0_initial):
@@ -614,15 +716,33 @@ class MPABatch:
     """M same-shape maps, one MPA population of `num_predators` paths per map, every iteration of every map in one
     launch (mpp_mpa_iteration_batch); the stable sorts (MPA.py:333,412) are a batched device argsort whose index
     the kernel reads through, and the best-so-far cascade (MPA.py:415-437) is a few vector operations over the maps --
-    no host round trip inside the solve.  Same parameters as MPA (MPA.py:10-18); `seeds` = one Philox seed per map."""
+    no host round trip inside the solve.  Same parameters as MPA (MPA.py:10-18); `seeds` = one Philox seed per map.
+
+    map_params (None or one mapping per map) gives each map its own FADs_rate, P_const, levy_beta, statistics weights
+    and min_safe_distance (which MPA never reads): keys left out take the constructor's values, and `b.map_params` holds
+    the resolved dicts.  allow_diagonal_moves and restrict_diagonal_near_obstacle may appear only with one value for
+    every map; num_predators and num_iterations cannot appear.  Invalid map_params (a levy_beta whose Levy sigma is
+    complex among them) raise ValueError before any device work.  The launches then read the parameters per map
+    (mpp_mpa_init_batch_p, mpp_mpa_iteration_batch_p); map k's results are those of MPA with map k's parameters and
+    seed."""
 
     def __init__(self, grids, num_predators, num_iterations, FADs_rate=0.2, P_const=0.5, levy_beta=1.5,
                  turn_penalty_factor=0.1, safety_penalty_factor=0.05, min_safe_distance=1.5, allow_diagonal_moves=True,
                  restrict_diagonal_near_obstacle=True, diagonal_obstacle_penalty=1000.0, *, seeds=None, device=None,
-                 max_cells=None, heap_cap=None, warps_per_map=None):
-        import math
+                 max_cells=None, heap_cap=None, warps_per_map=None, map_params=None):
         import torch
         from .engine import make_policy
+        self.map_params = None
+        if map_params is not None:
+            self.map_params = resolve_map_params(
+                dict(FADs_rate=FADs_rate, P_const=P_const, levy_beta=levy_beta, turn_penalty_factor=turn_penalty_factor,
+                     safety_penalty_factor=safety_penalty_factor, min_safe_distance=min_safe_distance,
+                     allow_diagonal_moves=allow_diagonal_moves,
+                     restrict_diagonal_near_obstacle=restrict_diagonal_near_obstacle,
+                     diagonal_obstacle_penalty=diagonal_obstacle_penalty), map_params, _grid_count(grids), "mpa")
+            wave = _wave_params("mpa", self.map_params)
+            allow_diagonal_moves = wave["allow_diagonal_moves"]
+            restrict_diagonal_near_obstacle = wave["restrict_diagonal_near_obstacle"]
         self._map_set = _map_set(grids, device, _all_endpoints("MPA: Start node not found in grid.",      # MPA.py:36-37
                                                                "MPA: Target node not found in grid."))    # MPA.py:38-39
         self._maps = self._map_set.handle
@@ -633,13 +753,8 @@ class MPABatch:
         self.FADs_rate, self.P_const, self.levy_beta = FADs_rate, P_const, levy_beta
         self.policy = make_policy(turn_penalty_factor, safety_penalty_factor, min_safe_distance, diagonal_obstacle_penalty,
                                   restrict_diagonal_near_obstacle, allow_diagonal_moves, mode=1)
-        b = levy_beta                                                         # Levy sigma MPA.py:251-253
-        num = math.gamma(1 + b) * math.sin(math.pi * b / 2)
-        den = math.gamma((1 + b) / 2) * b * (2 ** ((b - 1) / 2))
-        sig = (num / den) ** (1 / b) if den > 1e-9 else 1.0
-        if isinstance(sig, complex):
-            raise ValueError("levy_beta gives a complex Levy sigma in the reference expression (MPA.py:253)")
-        self._levy_sigma = float(sig)
+        self._levy_sigma = levy_sigma(levy_beta)                              # MPA.py:251-253
+        self._params_dev = None if self.map_params is None else _pop_params_dev("mpa", self.map_params, self.device)
         n = self.rows * self.cols
         self.max_cells = int(max_cells or min(n, max(1024, 4 * (self.rows + self.cols))))
         self.heap_cap = int(heap_cap or min(8 * n, max(4096, n // 4)))
@@ -655,7 +770,7 @@ class MPABatch:
                           allow_diagonal_moves=allow_diagonal_moves,
                           restrict_diagonal_near_obstacle=restrict_diagonal_near_obstacle,
                           diagonal_obstacle_penalty=diagonal_obstacle_penalty, seeds=self.seeds,
-                          warps_per_map=warps_per_map)
+                          warps_per_map=warps_per_map, map_params=self.map_params)
         self.predator_evaluations = 0
         self.kernel_launches = 0
 
@@ -691,9 +806,16 @@ class MPABatch:
         seeds = t.from_numpy(np.array(self.seeds, np.uint64).view(np.int64)).to(dev)
         stream = C.c_void_p(t.cuda.current_stream(dev).cuda_stream)
         # ---- initial population: one search per map, replicated (MPA.py:231-245) ----
-        _lib.check(L.mpp_mpa_init_batch(self._maps, C.byref(self.policy), N, mc, _lib.ptr(cells[0]), _lib.ptr(ncell[0]),
-                                        _lib.ptr(stats[0]), _lib.ptr(scratch), scratch.numel(), self.heap_cap,
-                                        _lib.ptr(status), _lib.ptr(counters), stream), "mpp_mpa_init_batch")
+        if self._params_dev is None:
+            _lib.check(L.mpp_mpa_init_batch(self._maps, C.byref(self.policy), N, mc, _lib.ptr(cells[0]),
+                                            _lib.ptr(ncell[0]), _lib.ptr(stats[0]), _lib.ptr(scratch), scratch.numel(),
+                                            self.heap_cap, _lib.ptr(status), _lib.ptr(counters), stream),
+                       "mpp_mpa_init_batch")
+        else:
+            _lib.check(L.mpp_mpa_init_batch_p(self._maps, C.byref(self.policy), _lib.ptr(self._params_dev), N, mc,
+                                              _lib.ptr(cells[0]), _lib.ptr(ncell[0]), _lib.ptr(stats[0]),
+                                              _lib.ptr(scratch), scratch.numel(), self.heap_cap, _lib.ptr(status),
+                                              _lib.ptr(counters), stream), "mpp_mpa_init_batch_p")
         cells[0][:, 1:] = cells[0][:, :1]
         ncell[0][:, 1:] = ncell[0][:, :1]
         stats[0][:, 1:] = stats[0][:, :1]
@@ -715,12 +837,18 @@ class MPABatch:
             CF = 0.0 if ratio >= 1.0 else ((1.0 - ratio) ** (2.0 * ratio) if ratio > 0 else 1.0)   # MPA.py:336
             phase = 1 if it <= K / 3 else (2 if it <= 2 * K / 3 else 3)
             nxt = cur ^ 1
-            _lib.check(L.mpp_mpa_iteration_batch(
-                self._maps, C.byref(self.policy), N, 0, N, it, phase, self.P_const, CF, self.FADs_rate, self._levy_sigma,
-                self.levy_beta, _lib.ptr(seeds), _lib.ptr(order), _lib.ptr(cells[cur]), _lib.ptr(ncell[cur]),
-                _lib.ptr(stats[cur]), mc, _lib.ptr(cells[nxt]), _lib.ptr(ncell[nxt]), _lib.ptr(stats[nxt]), _lib.ptr(tmp),
-                _lib.ptr(avoid), _lib.ptr(scratch), scratch.numel(), self.warps_per_map, self.heap_cap, _lib.ptr(queue),
-                _lib.ptr(status), _lib.ptr(counters), stream), "mpp_mpa_iteration_batch")
+            bufs = (_lib.ptr(seeds), _lib.ptr(order), _lib.ptr(cells[cur]), _lib.ptr(ncell[cur]), _lib.ptr(stats[cur]), mc,
+                    _lib.ptr(cells[nxt]), _lib.ptr(ncell[nxt]), _lib.ptr(stats[nxt]), _lib.ptr(tmp), _lib.ptr(avoid),
+                    _lib.ptr(scratch), scratch.numel(), self.warps_per_map, self.heap_cap, _lib.ptr(queue),
+                    _lib.ptr(status), _lib.ptr(counters), stream)
+            if self._params_dev is None:
+                _lib.check(L.mpp_mpa_iteration_batch(self._maps, C.byref(self.policy), N, 0, N, it, phase, self.P_const,
+                                                     CF, self.FADs_rate, self._levy_sigma, self.levy_beta, *bufs),
+                           "mpp_mpa_iteration_batch")
+            else:
+                _lib.check(L.mpp_mpa_iteration_batch_p(self._maps, C.byref(self.policy), N, 0, N, it, phase,
+                                                       _lib.ptr(self._params_dev), CF, *bufs),
+                           "mpp_mpa_iteration_batch_p")
             self.kernel_launches += 1
             self.predator_evaluations += M * N
             cur = nxt
@@ -767,16 +895,25 @@ class MPABatch:
         return out
 
 
-def solve_mpa_batch(grids, num_predators, num_iterations, params, seeds=None, wave=32, group=None, device=None):
+def solve_mpa_batch(grids, num_predators, num_iterations, params, seeds=None, wave=32, group=None, device=None,
+                    map_params=None):
     """MPA over this rank's shard of the maps (host maps or device grids, as solve_maaco_batch takes), `wave` maps per
     launch (grouped by shape).  Returns (map_index, path, length, turns, safety_p, diag_p, fitness, convergence_curve)
-    per map of this rank."""
+    per map of this rank.
+
+    map_params (None or one mapping per map of `grids`, by global index) gives map i its own parameters, as
+    MPABatch(map_params=...) takes them: map i is solved as MPA(grids[i], ..., **{**params, **map_params[i]}).  Waves
+    are formed by shape, allow_diagonal_moves and restrict_diagonal_near_obstacle, in index order; invalid map_params
+    raise ValueError before any grid is read."""
+    if map_params is not None:
+        map_params = resolve_map_params(params, map_params, len(grids), "mpa")
     lo, hi = shard_maps(len(grids), group)
     maps = _sweep_maps(grids, lo, hi)
     out = []
-    for idx in _shape_waves(grids, lo, hi, wave):
+    for idx in _shape_waves(grids, lo, hi, wave, _wave_key("mpa", map_params)):
         b = MPABatch(maps.wave(idx), num_predators, num_iterations,
-                     seeds=None if seeds is None else [seeds[i] for i in idx], device=device, **params)
+                     seeds=None if seeds is None else [seeds[i] for i in idx], device=device,
+                     map_params=None if map_params is None else [map_params[i] for i in idx], **params)
         for i, r in zip(idx, b.solve()):
             out.append((i,) + tuple(r))
         b.close()
@@ -838,11 +975,17 @@ def _map_shape(g):
     return tuple(g.shape) if hasattr(g, "shape") else np.shape(g)
 
 
-def _shape_waves(grids, lo, hi, wave=None):
-    """Maps lo..hi-1 grouped by shape (one mpp_map_batch each), `wave` maps per group at most (None: all of them)."""
+def _grid_count(grids):
+    """Maps in a batch class's `grids` (host maps, a CUDA tensor or a _MapSet) without reading them."""
+    return grids.shape[0] if isinstance(grids, _MapSet) else len(grids)
+
+
+def _shape_waves(grids, lo, hi, wave=None, key=None):
+    """Maps lo..hi-1 grouped by shape (one mpp_map_batch each) -- and by key(i) when given --, `wave` maps per group at
+    most (None: all of them)."""
     shapes = {}
     for i in range(lo, hi):
-        shapes.setdefault(_map_shape(grids[i]), []).append(i)
+        shapes.setdefault((_map_shape(grids[i]), None if key is None else key(i)), []).append(i)
     out = []
     for idx in shapes.values():
         step = wave or len(idx)
@@ -932,9 +1075,10 @@ class SearchBatch:
             self._scratch_key = (slots, self.heap_cap)
         return self._scratch, slots
 
-    def _launch(self, variant, mi, src, dst, avoid, longest_first, allow_diagonal, restrict_corner, policy):
+    def _launch(self, variant, mi, src, dst, avoid, longest_first, allow_diagonal, restrict_corner, policy, params=None):
         """One mpp_astar_batch_maps launch over the given (valid) queries with the current sizes; stats is None when
-        policy is."""
+        policy is.  params (a wave's per-map parameters, _pop_params_dev): the statistics of query i then take the
+        weights of map mi[i], computed after the searches by mpp_path_stats_p."""
         import torch as t
         n, mc = mi.numel(), self.max_cells
         _, slots = self._scratch_for(n)
@@ -948,13 +1092,19 @@ class SearchBatch:
         ncell = t.empty(n, dtype=t.int32, device=self.device)
         g = t.empty(n, dtype=t.float64, device=self.device)
         stats = None if policy is None else t.empty((n, 5), dtype=t.float64, device=self.device)
+        fused = policy is not None and params is None
         _lib.check(_lib.lib().mpp_astar_batch_maps(
             self._maps, int(variant), _lib.ptr(mi), _lib.ptr(src), _lib.ptr(dst), _lib.ptr(avoid), n,
-            int(bool(allow_diagonal)), int(bool(restrict_corner)), None if policy is None else C.byref(policy),
-            _lib.ptr(cells), mc, _lib.ptr(ncell), _lib.ptr(g), _lib.ptr(stats), _lib.ptr(self._scratch),
-            self._scratch.numel(), slots, self.heap_cap, _lib.ptr(self.counters), _lib.ptr(order), self._stream()),
-            "mpp_astar_batch_maps")
+            int(bool(allow_diagonal)), int(bool(restrict_corner)), C.byref(policy) if fused else None,
+            _lib.ptr(cells), mc, _lib.ptr(ncell), _lib.ptr(g), _lib.ptr(stats) if fused else None,
+            _lib.ptr(self._scratch), self._scratch.numel(), slots, self.heap_cap, _lib.ptr(self.counters),
+            _lib.ptr(order), self._stream()), "mpp_astar_batch_maps")
         self.launches += 1
+        if policy is not None and params is not None:
+            _lib.check(_lib.lib().mpp_path_stats_p(self._maps, _lib.ptr(mi), _lib.ptr(cells), mc, _lib.ptr(ncell), n,
+                                                   C.byref(policy), _lib.ptr(params), _lib.ptr(stats), self._stream()),
+                       "mpp_path_stats_p")
+            self.launches += 1
         return cells, ncell, g, stats
 
     def _chain_order(self, mi, wps):
@@ -969,9 +1119,10 @@ class SearchBatch:
         d = ((r[:, 1:] - r[:, :-1]) ** 2 + (c[:, 1:] - c[:, :-1]) ** 2).sqrt().sum(dim=1)
         return t.argsort(t.where(ok, d, -1.0), descending=True).to(t.int32).contiguous()
 
-    def _chain_launch(self, mi, wps, policy):
+    def _chain_launch(self, mi, wps, policy, params=None):
         """One mpp_waypoint_fitness_maps launch over individuals mi [n] (map index, -1 = not searched), wps [n, W] with the
-        current sizes, longest chains first."""
+        current sizes, longest chains first; with params (per-map parameters, _pop_params_dev) the statistics weights of
+        each individual's map (mpp_waypoint_fitness_maps_p)."""
         import torch as t
         n, W = wps.shape
         mc = self.max_cells
@@ -982,21 +1133,28 @@ class SearchBatch:
         cells = t.empty((n, mc), dtype=t.int32, device=self.device)
         ncell = t.empty(n, dtype=t.int32, device=self.device)
         stats = t.empty((n, 5), dtype=t.float64, device=self.device)
-        _lib.check(_lib.lib().mpp_waypoint_fitness_maps(
-            self._maps, _lib.ptr(mi), _lib.ptr(wps), n, W, C.byref(policy), _lib.ptr(cells), mc, _lib.ptr(ncell),
-            _lib.ptr(stats), _lib.ptr(self._visited), _lib.ptr(scratch), scratch.numel(), slots, self.heap_cap,
-            _lib.ptr(self.counters), _lib.ptr(order), self._stream()), "mpp_waypoint_fitness_maps")
+        L = _lib.lib()
+        if params is None:
+            _lib.check(L.mpp_waypoint_fitness_maps(
+                self._maps, _lib.ptr(mi), _lib.ptr(wps), n, W, C.byref(policy), _lib.ptr(cells), mc, _lib.ptr(ncell),
+                _lib.ptr(stats), _lib.ptr(self._visited), _lib.ptr(scratch), scratch.numel(), slots, self.heap_cap,
+                _lib.ptr(self.counters), _lib.ptr(order), self._stream()), "mpp_waypoint_fitness_maps")
+        else:
+            _lib.check(L.mpp_waypoint_fitness_maps_p(
+                self._maps, _lib.ptr(mi), _lib.ptr(wps), n, W, C.byref(policy), _lib.ptr(params), _lib.ptr(cells), mc,
+                _lib.ptr(ncell), _lib.ptr(stats), _lib.ptr(self._visited), _lib.ptr(scratch), scratch.numel(), slots,
+                self.heap_cap, _lib.ptr(self.counters), _lib.ptr(order), self._stream()), "mpp_waypoint_fitness_maps_p")
         self.launches += 1
         return cells, ncell, stats
 
-    def _chain_repeat(self, mi, wps, cells, ncell, stats):
+    def _chain_repeat(self, mi, wps, cells, ncell, stats, params=None):
         """After _grow_from enlarged the buffers: repeats the individuals whose heap overflowed or whose path was truncated
         (the searches are deterministic) until none is; returns the patched (cells, n_cells, stats)."""
         import torch as t
         while True:
             bad = ((ncell < 0) | (ncell > cells.shape[1])).nonzero().squeeze(1)
             c, nc, st = self._chain_launch(mi.index_select(0, bad).contiguous(), wps.index_select(0, bad).contiguous(),
-                                           self.policy)
+                                           self.policy, params)
             if c.shape[1] > cells.shape[1]:                                  # max_cells grew: widen the earlier rows
                 cells = t.nn.functional.pad(cells, (0, c.shape[1] - cells.shape[1]))
             cells[bad, :c.shape[1]] = c
@@ -1004,26 +1162,27 @@ class SearchBatch:
             if not self._grow_from(*t.stack([nc.min(), nc.max()]).tolist()):
                 return cells, ncell, stats
 
-    def chains(self, map_index, waypoints):
+    def chains(self, map_index, waypoints, params=None):
         """Waypoint-chain fitness (pso.py:56-94 / ga_solver.py:58-93 + helper.py:98-113): individual i runs on map
         map_index[i] from that map's start through the W cells waypoints[i] to its target.  Returns device tensors
         (cells [n, max_cells] int32, n_cells [n] int32, stats [n, 5] float64).  n_cells = 0: an invalid chain, or a map
         index outside the batch (not searched).  A heap overflow or a truncated path grows the buffers and repeats only
-        those individuals."""
+        those individuals.  params: per-map statistics weights (_pop_params_dev), as _chain_launch takes them."""
         import torch as t
         mi, wps = self._i32(map_index), self._i32(waypoints)
-        cells, ncell, stats = self._chain_launch(mi, wps, self.policy)
+        cells, ncell, stats = self._chain_launch(mi, wps, self.policy, params)
         if self._grow_from(*t.stack([ncell.min(), ncell.max()]).tolist()):
-            cells, ncell, stats = self._chain_repeat(mi, wps, cells, ncell, stats)
+            cells, ncell, stats = self._chain_repeat(mi, wps, cells, ncell, stats, params)
         return cells, ncell, stats
 
-    def search(self, variant, map_index, src, dst, avoid_bits=None, *, longest_first=True):
+    def search(self, variant, map_index, src, dst, avoid_bits=None, *, longest_first=True, params=None):
         """Query i: connector `variant` (0 = astar.py, 1 = MPA.py's private A*, 2 = dijkstra.py) from cell src[i] to
         cell dst[i] of map map_index[i], avoiding the cells set in avoid_bits[i] (n x ceil(rows*cols/32) bitmap words,
         or None).  Returns device tensors (cells [n, max_cells] int32, n_cells [n] int32, g [n] float64 = g of the
         popped target, stats [n, 5] float64 = (length, turns, safety, diag, fitness) of the path).  n_cells = 0: no
         path, or an endpoint / map index outside the batch (not searched).  A heap overflow or a truncated path grows
-        the buffers and repeats only those queries (the searches are deterministic)."""
+        the buffers and repeats only those queries (the searches are deterministic).  params: per-map statistics weights
+        (_pop_params_dev), as _launch takes them."""
         import torch as t
         mi, src, dst = self._i32(map_index), self._i32(src), self._i32(dst)
         valid = _valid_queries(mi, src, dst, self.n_maps, self.n)
@@ -1044,7 +1203,7 @@ class SearchBatch:
         while idx.numel():
             sub = lambda x: None if x is None else x.index_select(0, idx).contiguous()
             c, nc, gg, st = self._launch(variant, sub(mi), sub(src), sub(dst), sub(avoid), longest_first,
-                                         self.allow_diagonal_moves, self.restrict_corners, self.policy)
+                                         self.allow_diagonal_moves, self.restrict_corners, self.policy, params)
             if c.shape[1] > cells.shape[1]:                                  # max_cells grew: widen the earlier rows
                 wide = t.zeros((n, c.shape[1]), dtype=t.int32, device=self.device)
                 wide[:, :cells.shape[1]] = cells
@@ -1082,15 +1241,15 @@ class SearchBatch:
         g, parent = self._fields(src)
         return field_paths(self, self._maps, g, parent, mi, dst, self.policy)
 
-    def solve(self, algorithm="astar"):
+    def solve(self, algorithm="astar", params=None):
         """One start -> target query per map.  Returns, per map, what AStarSolver(grid, ...).solve() (algorithm
         "astar") or DijkstraSolver(grid, ...).solve() ("dijkstra") returns -- (path, length, turns, safety_p, diag_p,
         fitness) -- followed by the value that solver appends to its convergence_curve (g, or None when the path has
-        at most one cell)."""
+        at most one cell).  params: per-map statistics weights (_pop_params_dev), as search takes them."""
         variant = _search_algorithm(algorithm)[0]
         src, dst = self._map_set.start, self._map_set.target              # first row-major 2 / 3 (astar.py:17-18)
         _endpoint_check(algorithm)(src, dst)
-        cells, ncell, g, stats = self.search(variant, np.arange(self.n_maps), src, dst)
+        cells, ncell, g, stats = self.search(variant, np.arange(self.n_maps), src, dst, params=params)
         cells, ncell, g, stats = cells.cpu().numpy(), ncell.cpu().numpy(), g.cpu().numpy(), stats.cpu().numpy()
         out = []
         for k in range(self.n_maps):
@@ -1138,12 +1297,15 @@ def default_pop_wave(rows, cols, population):
 class _WaypointBatch:
     """What PSOBatch and GABatch share: M same-shape maps (start and target may differ from map to map) behind one
     SearchBatch (map batch, policy, buffer sizes and their growth), one Philox seed per map, and the population
-    initialisation of pso.py:97-161 / ga_solver.py:95-133 for every map at once."""
+    initialisation of pso.py:97-161 / ga_solver.py:95-133 for every map at once.  With per-map parameters (map_params,
+    resolved by the subclass) every statistic takes its map's weights: _params_dev goes to each SearchBatch call."""
     _planner = None        # "pso" / "ga"
     _pad_class = None      # RNG class of the padding draws
 
-    def __init__(self, grids, num_waypoints, policy, seeds, device, max_cells, heap_cap, n_slots):
+    def __init__(self, grids, num_waypoints, policy, seeds, device, max_cells, heap_cap, n_slots, map_params=None):
         import torch
+        if map_params is not None:                                           # the wave's value of every per-wave key
+            policy = {**policy, **_wave_params(self._planner, map_params)}
         endpoints = _endpoint_check(self._planner)
 
         def check(start, target):                                            # (host grids: before any device work)
@@ -1159,6 +1321,8 @@ class _WaypointBatch:
         self._search = SearchBatch(maps, max_cells=max_cells, heap_cap=heap_cap, n_slots=n_slots, **policy)
         self.device = self._search.device
         self._seeds = torch.from_numpy(np.array(self.seeds, np.uint64).view(np.int64)).to(self.device)
+        self.map_params = map_params
+        self._params_dev = None if map_params is None else _pop_params_dev(self._planner, map_params, self.device)
         self.fitness_evaluations = [0] * self.n_maps
         self.init_attempts = [0] * self.n_maps
         self.kernel_launches = 0
@@ -1178,7 +1342,7 @@ class _WaypointBatch:
     def _solve_direct(self):
         """num_waypoints == 0 (pso.py:165-170, ga_solver.py:163-168): one start -> target connector per map and the
         statistics of its path; the curve holds that fitness."""
-        return [r[:6] + ([r[5]],) for r in self._search.solve("astar")]
+        return [r[:6] + ([r[5]],) for r in self._search.solve("astar", self._params_dev)]
 
     def _initialize(self, generate, n):
         """pso.py:97-161 / ga_solver.py:95-133 for every map.  Each round generates one block of attempts for every map
@@ -1207,7 +1371,7 @@ class _WaypointBatch:
             k_r, wp = generate(offs, B)
             self.kernel_launches += 1
             mi = t.where(t.arange(B, device=dev)[None, :] < t.as_tensor(block, device=dev)[:, None], rows[:, None], -1)
-            c_r, nc_r, st_r = self._search.chains(mi.reshape(-1), wp.reshape(M * B, W))
+            c_r, nc_r, st_r = self._search.chains(mi.reshape(-1), wp.reshape(M * B, W), self._params_dev)
             valid = (nc_r > 0).reshape(M, B).cpu().numpy()
             src, dst = [], []
             for m in np.flatnonzero(need):
@@ -1240,7 +1404,7 @@ class _WaypointBatch:
         lost = np.flatnonzero(n_acc == 0)
         if lost.size:                                                        # the direct path as the one individual
             s, g = self._search._start_dev[lost], self._search._target_dev[lost]
-            c_d, nc_d, _, st_d = self._search.search(0, lost, s, g)
+            c_d, nc_d, _, st_d = self._search.search(0, lost, s, g, params=self._params_dev)
             found = (nc_d > 0).cpu().numpy()
             if found.any():
                 if c_d.shape[1] > cells.shape[1]:
@@ -1281,20 +1445,31 @@ class PSOBatch(_WaypointBatch):
     iteration is the speculative repair of PSOSolver._iterate for all maps at once: every map's active suffix is
     updated and evaluated in one update launch and one fitness launch (mpp_pso_update_batch, mpp_waypoint_fitness_maps),
     each map's first global-best improver is found on the device, and only the rest of that map's swarm is restored
-    and re-run in the next round; one host synchronise per round."""
+    and re-run in the next round; one host synchronise per round.
+
+    map_params (None or one mapping per map) gives each map its own w, c1, c2 and statistics weights (a parameter sweep
+    in one launch per step): keys left out take the constructor's values, and `b.map_params` holds the resolved dicts.
+    min_safe_distance, allow_diagonal_moves and restrict_diagonal_near_obstacle_policy may appear only with one value
+    for every map (they change the searches or the safety tables); the sizes cannot appear.  Invalid map_params raise
+    ValueError before any device work.  The update and fitness launches then read the parameters per map
+    (mpp_pso_update_batch_p, mpp_waypoint_fitness_maps_p); map k's results are those of PSOSolver with map k's
+    parameters and seed."""
     _planner = "pso"
 
     def __init__(self, grids, num_iterations, num_particles, num_waypoints_per_particle, w, c1, c2,
                  turn_penalty_factor=0.1, safety_penalty_factor=0.05, min_safe_distance=1.5, allow_diagonal_moves=True,
                  restrict_diagonal_near_obstacle_policy=True, diagonal_obstacle_penalty_value=1000.0, *, seeds=None,
-                 device=None, max_cells=None, heap_cap=None, n_slots=None):
+                 device=None, max_cells=None, heap_cap=None, n_slots=None, map_params=None):
         from . import rng
         self._pad_class = rng.CLS_PSO_PAD
         policy = dict(turn_penalty_factor=turn_penalty_factor, safety_penalty_factor=safety_penalty_factor,
                       min_safe_distance=min_safe_distance, allow_diagonal_moves=allow_diagonal_moves,
                       restrict_diagonal_near_obstacle_policy=restrict_diagonal_near_obstacle_policy,
                       diagonal_obstacle_penalty_value=diagonal_obstacle_penalty_value)
-        super().__init__(grids, num_waypoints_per_particle, policy, seeds, device, max_cells, heap_cap, n_slots)
+        if map_params is not None:
+            map_params = resolve_map_params(dict(policy, w=w, c1=c1, c2=c2), map_params, _grid_count(grids), "pso")
+        super().__init__(grids, num_waypoints_per_particle, policy, seeds, device, max_cells, heap_cap, n_slots,
+                         map_params)
         self.num_iterations, self.num_particles = int(num_iterations), int(num_particles)
         self.w, self.c1, self.c2 = w, c1, c2
         self.max_vel = max(1.0, 0.15 * max(self.rows, self.cols))            # pso.py:34
@@ -1335,15 +1510,21 @@ class PSOBatch(_WaypointBatch):
             while (start < N).any():
                 st_d = t.as_tensor(start.astype(np.int32), device=dev)
                 wp = t.empty((M, N, W), dtype=t.int32, device=dev)
-                _lib.check(L.mpp_pso_update_batch(self._search._maps, _lib.ptr(pos), _lib.ptr(vel), _lib.ptr(pbest_pos),
-                                                  _lib.ptr(g_pos), N, _lib.ptr(st_d), W, self.w, self.c1, self.c2,
-                                                  self.max_vel, _lib.ptr(self._seeds), it, _lib.ptr(wp), self._stream()),
-                           "mpp_pso_update_batch")
+                if self._params_dev is None:
+                    _lib.check(L.mpp_pso_update_batch(self._search._maps, _lib.ptr(pos), _lib.ptr(vel),
+                                                      _lib.ptr(pbest_pos), _lib.ptr(g_pos), N, _lib.ptr(st_d), W, self.w,
+                                                      self.c1, self.c2, self.max_vel, _lib.ptr(self._seeds), it,
+                                                      _lib.ptr(wp), self._stream()), "mpp_pso_update_batch")
+                else:
+                    _lib.check(L.mpp_pso_update_batch_p(self._search._maps, _lib.ptr(pos), _lib.ptr(vel),
+                                                        _lib.ptr(pbest_pos), _lib.ptr(g_pos), N, _lib.ptr(st_d), W,
+                                                        _lib.ptr(self._params_dev), self.max_vel, _lib.ptr(self._seeds),
+                                                        it, _lib.ptr(wp), self._stream()), "mpp_pso_update_batch_p")
                 self.kernel_launches += 1
                 act = ar[None, :] >= st_d[:, None]
                 mi = t.where(act, rows[:, None], -1).to(t.int32).reshape(-1)
                 wp = wp.reshape(M * N, W)
-                c_r, nc_r, s_r = self._search._chain_launch(mi, wp, self._search.policy)
+                c_r, nc_r, s_r = self._search._chain_launch(mi, wp, self._search.policy, self._params_dev)
                 for m in np.flatnonzero(start < N):
                     self.fitness_evaluations[m] += N - int(start[m])
                 while True:
@@ -1358,7 +1539,7 @@ class PSOBatch(_WaypointBatch):
                     flags = t.cat([t.stack([nc_r.min(), nc_r.max()]).to(t.int64), nxt.to(t.int64)]).tolist()
                     if not self._search._grow_from(flags[0], flags[1]):
                         break
-                    c_r, nc_r, s_r = self._search._chain_repeat(mi, wp, c_r, nc_r, s_r)
+                    c_r, nc_r, s_r = self._search._chain_repeat(mi, wp, c_r, nc_r, s_r, self._params_dev)
                 upd = imp_p & (ar[None, :] <= q[:, None])                     # pso.py:217-220 for the final particles
                 pbest_fit = t.where(upd, f, pbest_fit)
                 pbest_pos = t.where(upd[..., None, None], pos, pbest_pos)
@@ -1387,21 +1568,30 @@ class GABatch(_WaypointBatch):
     (row m draws what GASolver(grid, ..., rng_seed=seeds[m]) draws).  Start and target may differ from map to map.  A
     generation is one selection, one breeding and one fitness launch for every map (mpp_ga_select_batch,
     mpp_ga_breed_batch, mpp_waypoint_fitness_maps); the invalid-child replacement (:204-205), the stable sort
-    (:208-209) and the best-so-far update (:211-213) are torch operations over all maps."""
+    (:208-209) and the best-so-far update (:211-213) are torch operations over all maps.
+
+    map_params works as in PSOBatch, for mutation_rate, crossover_rate, tournament_size and the statistics weights
+    (mpp_ga_select_batch_p, mpp_ga_breed_batch_p, mpp_waypoint_fitness_maps_p); a tournament_size the selection kernel
+    cannot take raises ValueError naming the map."""
     _planner = "ga"
 
     def __init__(self, grids, num_generations, population_size, num_waypoints_per_chromosome, mutation_rate,
                  crossover_rate, tournament_size=3, turn_penalty_factor=0.1, safety_penalty_factor=0.05,
                  min_safe_distance=1.5, allow_diagonal_moves=True, restrict_diagonal_near_obstacle_policy=True,
                  diagonal_obstacle_penalty_value=1000.0, *, seeds=None, device=None, max_cells=None, heap_cap=None,
-                 n_slots=None):
+                 n_slots=None, map_params=None):
         from . import rng
         self._pad_class = rng.CLS_GA_PAD
         policy = dict(turn_penalty_factor=turn_penalty_factor, safety_penalty_factor=safety_penalty_factor,
                       min_safe_distance=min_safe_distance, allow_diagonal_moves=allow_diagonal_moves,
                       restrict_diagonal_near_obstacle_policy=restrict_diagonal_near_obstacle_policy,
                       diagonal_obstacle_penalty_value=diagonal_obstacle_penalty_value)
-        super().__init__(grids, num_waypoints_per_chromosome, policy, seeds, device, max_cells, heap_cap, n_slots)
+        if map_params is not None:
+            map_params = resolve_map_params(dict(policy, mutation_rate=mutation_rate, crossover_rate=crossover_rate,
+                                                 tournament_size=tournament_size), map_params, _grid_count(grids), "ga",
+                                            population=int(population_size))
+        super().__init__(grids, num_waypoints_per_chromosome, policy, seeds, device, max_cells, heap_cap, n_slots,
+                         map_params)
         self.num_generations, self.population_size = int(num_generations), int(population_size)
         self.mutation_rate, self.crossover_rate, self.tournament_size = mutation_rate, crossover_rate, tournament_size
         self.chrom = self.fitness = None
@@ -1439,15 +1629,23 @@ class GABatch(_WaypointBatch):
         for gen in range(K if evolving.any() else 0):
             parents = t.empty((M, N), dtype=t.int32, device=dev)
             fit = stats[..., 4].contiguous()
-            _lib.check(L.mpp_ga_select_batch(self._search._maps, _lib.ptr(fit), N, self.tournament_size,
-                                             _lib.ptr(self._seeds), gen, _lib.ptr(parents), self._stream()),
-                       "mpp_ga_select_batch")
             children = t.empty((M, N, W), dtype=t.int32, device=dev)
-            _lib.check(L.mpp_ga_breed_batch(self._search._maps, _lib.ptr(chrom.contiguous()), _lib.ptr(parents), N, W,
-                                            self.crossover_rate, self.mutation_rate, _lib.ptr(self._seeds), gen,
-                                            _lib.ptr(children), self._stream()), "mpp_ga_breed_batch")
+            if self._params_dev is None:
+                _lib.check(L.mpp_ga_select_batch(self._search._maps, _lib.ptr(fit), N, self.tournament_size,
+                                                 _lib.ptr(self._seeds), gen, _lib.ptr(parents), self._stream()),
+                           "mpp_ga_select_batch")
+                _lib.check(L.mpp_ga_breed_batch(self._search._maps, _lib.ptr(chrom.contiguous()), _lib.ptr(parents), N,
+                                                W, self.crossover_rate, self.mutation_rate, _lib.ptr(self._seeds), gen,
+                                                _lib.ptr(children), self._stream()), "mpp_ga_breed_batch")
+            else:
+                _lib.check(L.mpp_ga_select_batch_p(self._search._maps, _lib.ptr(fit), N, _lib.ptr(self._params_dev),
+                                                   _lib.ptr(self._seeds), gen, _lib.ptr(parents), self._stream()),
+                           "mpp_ga_select_batch_p")
+                _lib.check(L.mpp_ga_breed_batch_p(self._search._maps, _lib.ptr(chrom.contiguous()), _lib.ptr(parents),
+                                                  N, W, _lib.ptr(self._params_dev), _lib.ptr(self._seeds), gen,
+                                                  _lib.ptr(children), self._stream()), "mpp_ga_breed_batch_p")
             self.kernel_launches += 2
-            c_c, c_n, c_s = self._search.chains(mi, children.reshape(M * N, W))
+            c_c, c_n, c_s = self._search.chains(mi, children.reshape(M * N, W), self._params_dev)
             for m in np.flatnonzero(evolving):
                 self.fitness_evaluations[m] += N
             # an invalid child is replaced by its parent object (:204-205): child slot s of a map has parent parents[s]
@@ -1484,23 +1682,34 @@ class GABatch(_WaypointBatch):
         return out
 
 
-def _pop_waves(grids, lo, hi, population, wave=None):
-    """Maps lo..hi-1 grouped by shape, `wave` maps per wave at most (None: default_pop_wave of the shape)."""
+def _pop_waves(grids, lo, hi, population, wave=None, key=None):
+    """Maps lo..hi-1 grouped by shape (and key(i)), `wave` maps per wave at most (None: default_pop_wave of the
+    shape)."""
     out = []
-    for idx in _shape_waves(grids, lo, hi):
+    for idx in _shape_waves(grids, lo, hi, key=key):
         step = wave or default_pop_wave(*_map_shape(grids[idx[0]]), population)
         out += [idx[w0:w0 + step] for w0 in range(0, len(idx), step)]
     return out
 
 
-def _pop_sweep(cls, grids, sizes, params, seeds, wave, group, device):
+def _wave_key(planner, map_params):
+    """key(i) for _shape_waves: map i's per-wave values (None without map_params: waves by shape only)."""
+    if map_params is None:
+        return None
+    keys = PLANNER_MAP_PARAMS[planner][1]
+    return lambda i: tuple(map_params[i][k] for k in keys)
+
+
+def _pop_sweep(cls, grids, sizes, params, seeds, wave, group, device, map_params):
+    if map_params is not None:
+        map_params = resolve_map_params(params, map_params, len(grids), cls._planner, population=int(sizes[1]))
     lo, hi = shard_maps(len(grids), group)
     maps = _sweep_maps(grids, lo, hi)
     _endpoint_check(cls._planner)(*maps.first_cells())                      # before any search
     out = []
-    for idx in _pop_waves(grids, lo, hi, sizes[1], wave):
-        b = cls(maps.wave(idx), *sizes,
-                seeds=None if seeds is None else [seeds[i] for i in idx], device=device, **params)
+    for idx in _pop_waves(grids, lo, hi, sizes[1], wave, _wave_key(cls._planner, map_params)):
+        b = cls(maps.wave(idx), *sizes, seeds=None if seeds is None else [seeds[i] for i in idx], device=device,
+                map_params=None if map_params is None else [map_params[i] for i in idx], **params)
         for i, r in zip(idx, b.solve()):
             out.append((i,) + tuple(r))
         b.close()
@@ -1509,20 +1718,27 @@ def _pop_sweep(cls, grids, sizes, params, seeds, wave, group, device):
 
 
 def solve_pso_batch(grids, num_iterations, num_particles, num_waypoints_per_particle, params, seeds=None, wave=None,
-                    group=None, device=None):
+                    group=None, device=None, map_params=None):
     """PSO on every grid of `grids` (this rank's shard when `group` is given), grouped by shape, `wave` maps per
     PSOBatch (None: default_pop_wave, about 1 GiB of population paths per wave -- 32 maps of 1024 particles at
     256x256).  `params` = PSOBatch's other arguments (w, c1, c2, the policy, max_cells / heap_cap / n_slots).  Returns
     (map_index, path, length, turns, safety_p, diag_p, fitness, convergence_curve) per map of this rank, sorted by map
-    index; identical to PSOSolver(grid, ..., rng_seed=seeds[i]).solve() per map."""
+    index; identical to PSOSolver(grid, ..., rng_seed=seeds[i]).solve() per map.
+
+    map_params (None or one mapping per map of `grids`, by global index) gives map i its own parameters, as
+    PSOBatch(map_params=...) takes them: map i is solved as PSOSolver(grids[i], ..., **{**params, **map_params[i]}).
+    Waves are formed by shape and the per-wave keys (min_safe_distance, allow_diagonal_moves,
+    restrict_diagonal_near_obstacle_policy), in index order; invalid map_params raise ValueError before any grid is
+    read."""
     return _pop_sweep(PSOBatch, grids, (num_iterations, num_particles, num_waypoints_per_particle), params, seeds, wave,
-                      group, device)
+                      group, device, map_params)
 
 
 def solve_ga_batch(grids, num_generations, population_size, num_waypoints_per_chromosome, params, seeds=None, wave=None,
-                   group=None, device=None):
+                   group=None, device=None, map_params=None):
     """GA on every grid of `grids` (this rank's shard when `group` is given), like solve_pso_batch.  A wave keeps two
     [maps, population, max_cells] int32 path arrays (the population and its children): about 2 GiB with the default
-    wave.  `params` = GABatch's other arguments (mutation_rate, crossover_rate, tournament_size, the policy, ...)."""
+    wave.  `params` = GABatch's other arguments (mutation_rate, crossover_rate, tournament_size, the policy, ...);
+    map_params as solve_pso_batch takes it, with GASolver's per-map keys."""
     return _pop_sweep(GABatch, grids, (num_generations, population_size, num_waypoints_per_chromosome), params, seeds,
-                      wave, group, device)
+                      wave, group, device, map_params)

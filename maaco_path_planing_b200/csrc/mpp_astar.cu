@@ -85,10 +85,12 @@ int mpp_stats_ctx(mpp_map_batch *maps, const mpp_policy *pol, void *stream, Stat
     return MPP_OK;
 }
 
-__global__ void __launch_bounds__(MPP_AS_THREADS)
-mpp_path_stats_kernel(StatsCtx X, int occ_words, int n_maps, const int32_t *__restrict__ map,
-                      const int32_t *__restrict__ cells, int max_cells, const int32_t *__restrict__ n_cells, int n_paths,
-                      double *stats) {
+// MP (per-map parameters): the three statistics weights of params[m] in place of X.pol's
+template <bool MP>
+__device__ __forceinline__ void path_stats_body(StatsCtx &X, int occ_words, int n_maps, const int32_t *__restrict__ map,
+                                                const int32_t *__restrict__ cells, int max_cells,
+                                                const int32_t *__restrict__ n_cells, int n_paths,
+                                                const mpp_pop_params *__restrict__ params, double *stats) {
     const LaneGroup L = lane_group();
     const int w = (blockIdx.x * MPP_AS_THREADS + threadIdx.x) / MPP_GL;
     if (w >= n_paths) return;
@@ -98,27 +100,59 @@ mpp_path_stats_kernel(StatsCtx X, int occ_words, int n_maps, const int32_t *__re
     if ((unsigned)m < (unsigned)n_maps) {
         X.occ += (size_t)m * occ_words;
         if (X.cls) X.cls += (size_t)m * X.R * X.C;
+        if constexpr (MP) mpp_pop_weights(X.pol, params[m]);
     } else {
         n = 0;                                                  // outside the batch: the empty path's statistics
     }
     path_stats_warp(L, X, cells + (size_t)w * max_cells, n, stats + (size_t)w * 5);
 }
 
-extern "C" int mpp_path_stats(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *cells_dev, int max_cells,
-                              const int32_t *n_cells_dev, int n_paths, const mpp_policy *policy, double *stats_dev,
-                              void *stream) {
-    MPP_REQUIRE(maps && map_dev && cells_dev && n_cells_dev && policy && stats_dev, "mpp_path_stats: null argument");
-    MPP_REQUIRE(n_paths > 0 && max_cells > 0, "mpp_path_stats: bad sizes");
+__global__ void __launch_bounds__(MPP_AS_THREADS)
+mpp_path_stats_kernel(StatsCtx X, int occ_words, int n_maps, const int32_t *__restrict__ map,
+                      const int32_t *__restrict__ cells, int max_cells, const int32_t *__restrict__ n_cells, int n_paths,
+                      double *stats) {
+    path_stats_body<false>(X, occ_words, n_maps, map, cells, max_cells, n_cells, n_paths, nullptr, stats);
+}
+__global__ void __launch_bounds__(MPP_AS_THREADS)
+mpp_path_stats_p_kernel(StatsCtx X, int occ_words, int n_maps, const int32_t *__restrict__ map,
+                        const int32_t *__restrict__ cells, int max_cells, const int32_t *__restrict__ n_cells,
+                        int n_paths, const mpp_pop_params *__restrict__ params, double *stats) {
+    path_stats_body<true>(X, occ_words, n_maps, map, cells, max_cells, n_cells, n_paths, params, stats);
+}
+
+static int path_stats_launch(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *cells_dev, int max_cells,
+                             const int32_t *n_cells_dev, int n_paths, const mpp_policy *policy,
+                             const mpp_pop_params *params_dev, double *stats_dev, void *stream, const char *who) {
+    MPP_REQUIRE(maps && map_dev && cells_dev && n_cells_dev && policy && stats_dev, "%s: null argument", who);
+    MPP_REQUIRE(n_paths > 0 && max_cells > 0, "%s: bad sizes", who);
     MPP_CUDA(cudaSetDevice(maps->device));
     StatsCtx X;
     int rc = mpp_stats_ctx(maps, policy, stream, &X);
     if (rc) return rc;
     const int blocks = (n_paths + MPP_AS_GROUPS - 1) / MPP_AS_GROUPS;
-    mpp_path_stats_kernel<<<blocks, MPP_AS_THREADS, 0, (cudaStream_t)stream>>>(X, maps->occ_words, maps->n_maps, map_dev,
-                                                                             cells_dev, max_cells, n_cells_dev, n_paths,
-                                                                             stats_dev);
+    if (params_dev)
+        mpp_path_stats_p_kernel<<<blocks, MPP_AS_THREADS, 0, (cudaStream_t)stream>>>(
+            X, maps->occ_words, maps->n_maps, map_dev, cells_dev, max_cells, n_cells_dev, n_paths, params_dev, stats_dev);
+    else
+        mpp_path_stats_kernel<<<blocks, MPP_AS_THREADS, 0, (cudaStream_t)stream>>>(
+            X, maps->occ_words, maps->n_maps, map_dev, cells_dev, max_cells, n_cells_dev, n_paths, stats_dev);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
+}
+
+extern "C" int mpp_path_stats(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *cells_dev, int max_cells,
+                              const int32_t *n_cells_dev, int n_paths, const mpp_policy *policy, double *stats_dev,
+                              void *stream) {
+    return path_stats_launch(maps, map_dev, cells_dev, max_cells, n_cells_dev, n_paths, policy, nullptr, stats_dev,
+                             stream, "mpp_path_stats");
+}
+
+extern "C" int mpp_path_stats_p(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *cells_dev, int max_cells,
+                                const int32_t *n_cells_dev, int n_paths, const mpp_policy *policy,
+                                const mpp_pop_params *params_dev, double *stats_dev, void *stream) {
+    MPP_REQUIRE(params_dev, "mpp_path_stats_p: null params_dev");
+    return path_stats_launch(maps, map_dev, cells_dev, max_cells, n_cells_dev, n_paths, policy, params_dev, stats_dev,
+                             stream, "mpp_path_stats_p");
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -295,9 +329,11 @@ struct ChainArgs {
 };
 
 // Individual i on map A.map[i] from that map's start to its target, the occupancy read as mpp_astar_batch_kernel reads
-// it, its statistics from that map's safety classes.
-template <bool OCC_SMEM>
-__global__ void __launch_bounds__(MPP_AS_THREADS, 3) mpp_waypoint_fitness_kernel(ChainArgs A) {
+// it, its statistics from that map's safety classes.  MP (per-map parameters, mpp_waypoint_fitness_maps_p): the
+// statistics weights of params[map[i]] in place of A.X.pol's; the search is the same.
+template <bool OCC_SMEM, bool MP>
+__global__ void __launch_bounds__(MPP_AS_THREADS, 3)
+mpp_waypoint_fitness_kernel(ChainArgs A, const mpp_pop_params *__restrict__ params) {
     extern __shared__ __align__(16) uint32_t s_occ[];
     __shared__ __align__(8) uint64_t s_bar;
     __shared__ __align__(16) uint8_t s_cnt[MPP_AS_GROUPS][MPP_PQ_NB];
@@ -355,20 +391,36 @@ __global__ void __launch_bounds__(MPP_AS_THREADS, 3) mpp_waypoint_fitness_kernel
         StatsCtx Xm = A.X;
         Xm.occ = Gm.occ;
         if (Xm.cls) Xm.cls += (size_t)m * rc;
+        if constexpr (MP) mpp_pop_weights(Xm.pol, params[m]);
         path_stats_warp(L, Xm, path, status == 1 ? n : 0, A.stats + (size_t)i * 5);
     }
 }
 
-// Waypoint chains over a batch of same-shape maps (individual i on map map_dev[i], from that map's start to its target).
-extern "C" int mpp_waypoint_fitness_maps(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *waypoints_dev,
-                                         int n_individuals, int n_waypoints, const mpp_policy *policy, int32_t *cells_dev,
-                                         int max_cells, int32_t *n_cells_dev, double *stats_dev, uint32_t *visited_dev,
-                                         void *scratch_dev, size_t scratch_bytes, int n_slots, int heap_cap,
-                                         unsigned long long *counters_dev, const int32_t *order_dev, void *stream) {
+template <bool MP>
+static int fitness_launch(const ChainArgs &A, const mpp_pop_params *params_dev, const mpp_map_batch *maps, int blocks,
+                          cudaStream_t s) {
+    static MppStaging staging = {-1, {0}};
+    bool stage;
+    const int rc = stage_one_map((const void *)mpp_waypoint_fitness_kernel<true, MP>, staging, maps, &stage);
+    if (rc) return rc;
+    if (stage)
+        mpp_waypoint_fitness_kernel<true, MP><<<blocks, MPP_AS_THREADS, (size_t)maps->occ_words * 4, s>>>(A, params_dev);
+    else mpp_waypoint_fitness_kernel<false, MP><<<blocks, MPP_AS_THREADS, 0, s>>>(A, params_dev);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
+
+// Waypoint chains over a batch of same-shape maps (individual i on map map_dev[i], from that map's start to its target);
+// params_dev: per-map statistics weights (mpp_waypoint_fitness_maps_p) or null.
+static int waypoint_fitness(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *waypoints_dev, int n_individuals,
+                            int n_waypoints, const mpp_policy *policy, const mpp_pop_params *params_dev,
+                            int32_t *cells_dev, int max_cells, int32_t *n_cells_dev, double *stats_dev,
+                            uint32_t *visited_dev, void *scratch_dev, size_t scratch_bytes, int n_slots, int heap_cap,
+                            unsigned long long *counters_dev, const int32_t *order_dev, void *stream, const char *who) {
     MPP_REQUIRE(maps && map_dev && policy && cells_dev && n_cells_dev && stats_dev && visited_dev && scratch_dev,
-                "mpp_waypoint_fitness_maps: null argument");
-    MPP_REQUIRE(n_individuals > 0 && n_waypoints >= 0 && max_cells > 1, "mpp_waypoint_fitness_maps: bad sizes");
-    MPP_REQUIRE(n_waypoints == 0 || waypoints_dev, "mpp_waypoint_fitness_maps: null waypoints");
+                "%s: null argument", who);
+    MPP_REQUIRE(n_individuals > 0 && n_waypoints >= 0 && max_cells > 1, "%s: bad sizes", who);
+    MPP_REQUIRE(n_waypoints == 0 || waypoints_dev, "%s: null waypoints", who);
     int rc = check_search(maps, scratch_bytes, n_slots, heap_cap);
     if (rc) return rc;
     MPP_CUDA(cudaSetDevice(maps->device));
@@ -386,12 +438,28 @@ extern "C" int mpp_waypoint_fitness_maps(mpp_map_batch *maps, const int32_t *map
     A.scratch = (char *)scratch_dev; A.n_slots = n_slots; A.heap_cap = heap_cap; A.counters = counters_dev;
     A.order = order_dev;
     const int blocks = (n_slots + MPP_AS_GROUPS - 1) / MPP_AS_GROUPS;
-    static MppStaging staging = {-1, {0}};
-    bool stage;
-    rc = stage_one_map((const void *)mpp_waypoint_fitness_kernel<true>, staging, maps, &stage);
-    if (rc) return rc;
-    if (stage) mpp_waypoint_fitness_kernel<true><<<blocks, MPP_AS_THREADS, (size_t)maps->occ_words * 4, s>>>(A);
-    else mpp_waypoint_fitness_kernel<false><<<blocks, MPP_AS_THREADS, 0, s>>>(A);
-    MPP_CUDA(cudaGetLastError());
-    return MPP_OK;
+    return params_dev ? fitness_launch<true>(A, params_dev, maps, blocks, s)
+                      : fitness_launch<false>(A, nullptr, maps, blocks, s);
+}
+
+extern "C" int mpp_waypoint_fitness_maps(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *waypoints_dev,
+                                         int n_individuals, int n_waypoints, const mpp_policy *policy, int32_t *cells_dev,
+                                         int max_cells, int32_t *n_cells_dev, double *stats_dev, uint32_t *visited_dev,
+                                         void *scratch_dev, size_t scratch_bytes, int n_slots, int heap_cap,
+                                         unsigned long long *counters_dev, const int32_t *order_dev, void *stream) {
+    return waypoint_fitness(maps, map_dev, waypoints_dev, n_individuals, n_waypoints, policy, nullptr, cells_dev,
+                            max_cells, n_cells_dev, stats_dev, visited_dev, scratch_dev, scratch_bytes, n_slots, heap_cap,
+                            counters_dev, order_dev, stream, "mpp_waypoint_fitness_maps");
+}
+
+extern "C" int mpp_waypoint_fitness_maps_p(mpp_map_batch *maps, const int32_t *map_dev, const int32_t *waypoints_dev,
+                                           int n_individuals, int n_waypoints, const mpp_policy *policy,
+                                           const mpp_pop_params *params_dev, int32_t *cells_dev, int max_cells,
+                                           int32_t *n_cells_dev, double *stats_dev, uint32_t *visited_dev,
+                                           void *scratch_dev, size_t scratch_bytes, int n_slots, int heap_cap,
+                                           unsigned long long *counters_dev, const int32_t *order_dev, void *stream) {
+    MPP_REQUIRE(params_dev, "mpp_waypoint_fitness_maps_p: null params_dev");
+    return waypoint_fitness(maps, map_dev, waypoints_dev, n_individuals, n_waypoints, policy, params_dev, cells_dev,
+                            max_cells, n_cells_dev, stats_dev, visited_dev, scratch_dev, scratch_bytes, n_slots, heap_cap,
+                            counters_dev, order_dev, stream, "mpp_waypoint_fitness_maps_p");
 }

@@ -113,13 +113,22 @@ __device__ __forceinline__ void copy_stats(const LaneGroup &L, double *dst, cons
     grp_sync(L);
 }
 
-template <bool OCC_SMEM>
-__global__ void __launch_bounds__(MPP_MPA_THREADS, 3) mpp_mpa_iteration_kernel(MpaArgs A) {
+// MP (per-map parameters, mpp_mpa_iteration_batch_p): P_const, FADs_rate, levy_sigma, 1 / levy_beta and the statistics
+// weights of params[map] replace the launch's values in this kernel's copy of A; nothing downstream changes.
+template <bool OCC_SMEM, bool MP>
+__global__ void __launch_bounds__(MPP_MPA_THREADS, 3)
+mpp_mpa_iteration_kernel(MpaArgs A, const mpp_pop_params *__restrict__ params) {
     extern __shared__ __align__(16) uint32_t s_occ[];
     __shared__ __align__(8) uint64_t s_bar;
     __shared__ __align__(16) uint8_t s_cnt[MPP_MPA_GROUPS][MPP_PQ_NB];
     AStarGrid G = A.G;
     StatsCtx X = A.X;
+    if constexpr (MP) {
+        const mpp_pop_params &P = params[blockIdx.y];
+        A.P_const = P.P_const; A.FADs_rate = P.FADs_rate; A.levy_sigma = P.levy_sigma;
+        A.levy_inv_beta = __ddiv_rn(1.0, P.levy_beta);
+        mpp_pop_weights(X.pol, P);
+    }
     if (OCC_SMEM) {
         mpp_stage_bulk(s_occ, A.G.occ + (size_t)blockIdx.y * A.occ_words, (uint32_t)A.occ_words * 4u, &s_bar);
         G.occ = s_occ;
@@ -296,15 +305,17 @@ __global__ void __launch_bounds__(MPP_MPA_THREADS, 3) mpp_mpa_iteration_kernel(M
     }
 }
 
-static int mpa_launch(MpaArgs &A, int n_maps, int device, size_t occ_bytes, cudaStream_t s) {
+template <bool MP>
+static int mpa_launch(MpaArgs &A, const mpp_pop_params *params_dev, int n_maps, int device, size_t occ_bytes,
+                      cudaStream_t s) {
     const int blocks = (A.warps_per_map + MPP_MPA_GROUPS - 1) / MPP_MPA_GROUPS;
     const dim3 grid(blocks, n_maps);
     static MppStaging staging = {-1, {0}};
     bool stage = false;
-    const int rc = mpp_occ_staging((const void *)mpp_mpa_iteration_kernel<true>, staging, device, occ_bytes, &stage);
+    const int rc = mpp_occ_staging((const void *)mpp_mpa_iteration_kernel<true, MP>, staging, device, occ_bytes, &stage);
     if (rc) return rc;
-    if (stage) mpp_mpa_iteration_kernel<true><<<grid, MPP_MPA_THREADS, occ_bytes, s>>>(A);
-    else mpp_mpa_iteration_kernel<false><<<grid, MPP_MPA_THREADS, 0, s>>>(A);
+    if (stage) mpp_mpa_iteration_kernel<true, MP><<<grid, MPP_MPA_THREADS, occ_bytes, s>>>(A, params_dev);
+    else mpp_mpa_iteration_kernel<false, MP><<<grid, MPP_MPA_THREADS, 0, s>>>(A, params_dev);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }
@@ -315,28 +326,28 @@ static int mpa_launch(MpaArgs &A, int n_maps, int device, size_t occ_bytes, cuda
 // buffers are [n_maps][N][...]; the kernel reads the OLD population through `order` when given (the stable argsort of
 // its fitness column, computed on the device by the caller), so the sorts of MPA.py:333,412 never move a path.
 // ---------------------------------------------------------------------------------------------
-extern "C" int mpp_mpa_iteration_batch(const mpp_map_batch *maps, const mpp_policy *policy, int n_predators,
-                                       int pred_begin, int pred_end, int iteration, int phase, double P_const, double CF, double FADs_rate, double levy_sigma,
-                                       double levy_beta, const uint64_t *seeds_dev, const int32_t *order_dev,
-                                       const int32_t *cells_dev, const int32_t *n_cells_dev, const double *stats_dev,
-                                       int max_cells, int32_t *out_cells_dev, int32_t *out_n_dev, double *out_stats_dev,
-                                       int32_t *tmp_cells_dev, uint32_t *avoid_dev, void *scratch_dev, size_t scratch_bytes,
-                                       int warps_per_map, int heap_cap, uint32_t *queue_dev, int32_t *status_dev,
-                                       unsigned long long *counters_dev, void *stream) {
+// params_dev: per-map parameters (mpp_mpa_iteration_batch_p; the scalars are then unused) or null
+static int mpa_iteration(const mpp_map_batch *maps, const mpp_policy *policy, const mpp_pop_params *params_dev,
+                         int n_predators, int pred_begin, int pred_end, int iteration, int phase, double P_const,
+                         double CF, double FADs_rate, double levy_sigma, double levy_beta, const uint64_t *seeds_dev,
+                         const int32_t *order_dev, const int32_t *cells_dev, const int32_t *n_cells_dev,
+                         const double *stats_dev, int max_cells, int32_t *out_cells_dev, int32_t *out_n_dev,
+                         double *out_stats_dev, int32_t *tmp_cells_dev, uint32_t *avoid_dev, void *scratch_dev,
+                         size_t scratch_bytes, int warps_per_map, int heap_cap, uint32_t *queue_dev, int32_t *status_dev,
+                         unsigned long long *counters_dev, void *stream, const char *who) {
     MPP_REQUIRE(maps && policy && seeds_dev && cells_dev && n_cells_dev && stats_dev && out_cells_dev &&
                     out_n_dev && out_stats_dev && tmp_cells_dev && avoid_dev && scratch_dev && queue_dev && status_dev,
-                "mpp_mpa_iteration_batch: null argument");
+                "%s: null argument", who);
     MPP_REQUIRE(n_predators > 0 && max_cells > 1 && phase >= 1 && phase <= 3 && warps_per_map > 0 && heap_cap >= 64,
-                "mpp_mpa_iteration_batch: bad sizes");
-    MPP_REQUIRE(pred_begin >= 0 && pred_begin <= pred_end && pred_end <= n_predators,
-                "mpp_mpa_iteration_batch: bad predator range");
+                "%s: bad sizes", who);
+    MPP_REQUIRE(pred_begin >= 0 && pred_begin <= pred_end && pred_end <= n_predators, "%s: bad predator range", who);
     if (pred_begin == pred_end) return MPP_OK;
-    MPP_REQUIRE(maps->rows < 32768 && maps->cols < 65536, "mpp_mpa_iteration_batch: map exceeds the packed-node limit");
+    MPP_REQUIRE(maps->rows < 32768 && maps->cols < 65536, "%s: map exceeds the packed-node limit", who);
     const int rc = maps->rows * maps->cols;
     const size_t need = 256 + (size_t)warps_per_map * maps->n_maps * astar_slot_bytes(rc, heap_cap);
-    MPP_REQUIRE(scratch_bytes >= need, "mpp_mpa_iteration_batch: scratch too small (%zu < %zu)", scratch_bytes, need);
+    MPP_REQUIRE(scratch_bytes >= need, "%s: scratch too small (%zu < %zu)", who, scratch_bytes, need);
     for (int k = 0; k < maps->n_maps; ++k)
-        MPP_REQUIRE(maps->meta_host[k].start >= 0 && maps->meta_host[k].target >= 0, "mpp_mpa_iteration_batch: map %d has no start/target", k);
+        MPP_REQUIRE(maps->meta_host[k].start >= 0 && maps->meta_host[k].target >= 0, "%s: map %d has no start/target", who, k);
     MPP_CUDA(cudaSetDevice(maps->device));
     cudaStream_t s = (cudaStream_t)stream;
     MpaArgs A;
@@ -357,13 +368,49 @@ extern "C" int mpp_mpa_iteration_batch(const mpp_map_batch *maps, const mpp_poli
     A.scratch = (char *)scratch_dev; A.n_slots = warps_per_map * maps->n_maps; A.heap_cap = heap_cap; A.status = status_dev;
     A.counters = counters_dev;
     A.meta = maps->meta_dev; A.seeds = seeds_dev; A.order = order_dev; A.queue = queue_dev; A.warps_per_map = warps_per_map;
-    return mpa_launch(A, maps->n_maps, maps->device, (size_t)maps->occ_words * 4, s);
+    const size_t occ_bytes = (size_t)maps->occ_words * 4;
+    return params_dev ? mpa_launch<true>(A, params_dev, maps->n_maps, maps->device, occ_bytes, s)
+                      : mpa_launch<false>(A, nullptr, maps->n_maps, maps->device, occ_bytes, s);
+}
+
+extern "C" int mpp_mpa_iteration_batch(const mpp_map_batch *maps, const mpp_policy *policy, int n_predators,
+                                       int pred_begin, int pred_end, int iteration, int phase, double P_const, double CF, double FADs_rate, double levy_sigma,
+                                       double levy_beta, const uint64_t *seeds_dev, const int32_t *order_dev,
+                                       const int32_t *cells_dev, const int32_t *n_cells_dev, const double *stats_dev,
+                                       int max_cells, int32_t *out_cells_dev, int32_t *out_n_dev, double *out_stats_dev,
+                                       int32_t *tmp_cells_dev, uint32_t *avoid_dev, void *scratch_dev, size_t scratch_bytes,
+                                       int warps_per_map, int heap_cap, uint32_t *queue_dev, int32_t *status_dev,
+                                       unsigned long long *counters_dev, void *stream) {
+    return mpa_iteration(maps, policy, nullptr, n_predators, pred_begin, pred_end, iteration, phase, P_const, CF,
+                         FADs_rate, levy_sigma, levy_beta, seeds_dev, order_dev, cells_dev, n_cells_dev, stats_dev,
+                         max_cells, out_cells_dev, out_n_dev, out_stats_dev, tmp_cells_dev, avoid_dev, scratch_dev,
+                         scratch_bytes, warps_per_map, heap_cap, queue_dev, status_dev, counters_dev, stream,
+                         "mpp_mpa_iteration_batch");
+}
+
+extern "C" int mpp_mpa_iteration_batch_p(const mpp_map_batch *maps, const mpp_policy *policy, int n_predators,
+                                         int pred_begin, int pred_end, int iteration, int phase,
+                                         const mpp_pop_params *params_dev, double CF, const uint64_t *seeds_dev,
+                                         const int32_t *order_dev, const int32_t *cells_dev, const int32_t *n_cells_dev,
+                                         const double *stats_dev, int max_cells, int32_t *out_cells_dev,
+                                         int32_t *out_n_dev, double *out_stats_dev, int32_t *tmp_cells_dev,
+                                         uint32_t *avoid_dev, void *scratch_dev, size_t scratch_bytes,
+                                         int warps_per_map, int heap_cap, uint32_t *queue_dev, int32_t *status_dev,
+                                         unsigned long long *counters_dev, void *stream) {
+    MPP_REQUIRE(params_dev, "mpp_mpa_iteration_batch_p: null params_dev");
+    return mpa_iteration(maps, policy, params_dev, n_predators, pred_begin, pred_end, iteration, phase, 0.0, CF, 0.0,
+                         0.0, 1.0, seeds_dev, order_dev, cells_dev, n_cells_dev, stats_dev, max_cells, out_cells_dev,
+                         out_n_dev, out_stats_dev, tmp_cells_dev, avoid_dev, scratch_dev, scratch_bytes, warps_per_map,
+                         heap_cap, queue_dev, status_dev, counters_dev, stream, "mpp_mpa_iteration_batch_p");
 }
 
 // The initial population of every map (MPA.py:231-245): N identical runs of the private A* start -> target are ONE
 // search per map; row 0 of each map's buffers receives the path ([start, target] when there is none, :236) and its
 // statistics -- the caller replicates the row.  One warp per map.
-__global__ void __launch_bounds__(MPP_MPA_THREADS) mpp_mpa_init_kernel(MpaArgs A, int n_maps) {
+// MP (mpp_mpa_init_batch_p): the statistics weights of params[map] in place of A.X.pol's
+template <bool MP>
+__global__ void __launch_bounds__(MPP_MPA_THREADS)
+mpp_mpa_init_kernel(MpaArgs A, int n_maps, const mpp_pop_params *__restrict__ params) {
     __shared__ __align__(16) uint8_t s_cnt[MPP_MPA_GROUPS][MPP_PQ_NB];
     const LaneGroup L = lane_group();
     const int lane = L.gl;
@@ -387,6 +434,7 @@ __global__ void __launch_bounds__(MPP_MPA_THREADS) mpp_mpa_init_kernel(MpaArgs A
         sl = 2;
         grp_sync(L);
     }
+    if constexpr (MP) mpp_pop_weights(X.pol, params[map]);         // (loaded after the search: not live across it)
     path_stats_warp(L, X, out, sl, A.out_stats + (size_t)map * A.N * 5);
     if (lane == 0) {
         A.out_n[(size_t)map * A.N] = sl;
@@ -394,18 +442,18 @@ __global__ void __launch_bounds__(MPP_MPA_THREADS) mpp_mpa_init_kernel(MpaArgs A
     }
 }
 
-extern "C" int mpp_mpa_init_batch(const mpp_map_batch *maps, const mpp_policy *policy, int n_predators, int max_cells,
-                                  int32_t *cells_dev, int32_t *n_cells_dev, double *stats_dev, void *scratch_dev,
-                                  size_t scratch_bytes, int heap_cap, int32_t *status_dev, unsigned long long *counters_dev,
-                                  void *stream) {
+static int mpa_init(const mpp_map_batch *maps, const mpp_policy *policy, const mpp_pop_params *params_dev,
+                    int n_predators, int max_cells, int32_t *cells_dev, int32_t *n_cells_dev, double *stats_dev,
+                    void *scratch_dev, size_t scratch_bytes, int heap_cap, int32_t *status_dev,
+                    unsigned long long *counters_dev, void *stream, const char *who) {
     MPP_REQUIRE(maps && policy && cells_dev && n_cells_dev && stats_dev && scratch_dev && status_dev,
-                "mpp_mpa_init_batch: null argument");
-    MPP_REQUIRE(n_predators > 0 && max_cells > 1 && heap_cap >= 64, "mpp_mpa_init_batch: bad sizes");
-    MPP_REQUIRE(maps->rows < 32768 && maps->cols < 65536, "mpp_mpa_init_batch: map exceeds the packed-node limit");
+                "%s: null argument", who);
+    MPP_REQUIRE(n_predators > 0 && max_cells > 1 && heap_cap >= 64, "%s: bad sizes", who);
+    MPP_REQUIRE(maps->rows < 32768 && maps->cols < 65536, "%s: map exceeds the packed-node limit", who);
     const int rc = maps->rows * maps->cols;
-    MPP_REQUIRE(scratch_bytes >= 256 + (size_t)maps->n_maps * astar_slot_bytes(rc, heap_cap), "mpp_mpa_init_batch: scratch too small");
+    MPP_REQUIRE(scratch_bytes >= 256 + (size_t)maps->n_maps * astar_slot_bytes(rc, heap_cap), "%s: scratch too small", who);
     for (int k = 0; k < maps->n_maps; ++k)
-        MPP_REQUIRE(maps->meta_host[k].start >= 0 && maps->meta_host[k].target >= 0, "mpp_mpa_init_batch: map %d has no start/target", k);
+        MPP_REQUIRE(maps->meta_host[k].start >= 0 && maps->meta_host[k].target >= 0, "%s: map %d has no start/target", who, k);
     MPP_CUDA(cudaSetDevice(maps->device));
     MpaArgs A;
     memset(&A, 0, sizeof(A));
@@ -420,7 +468,26 @@ extern "C" int mpp_mpa_init_batch(const mpp_map_batch *maps, const mpp_policy *p
     A.scratch = (char *)scratch_dev; A.heap_cap = heap_cap; A.status = status_dev; A.counters = counters_dev;
     A.meta = maps->meta_dev;
     const int blocks = (maps->n_maps + MPP_MPA_GROUPS - 1) / MPP_MPA_GROUPS;
-    mpp_mpa_init_kernel<<<blocks, MPP_MPA_THREADS, 0, (cudaStream_t)stream>>>(A, maps->n_maps);
+    if (params_dev)
+        mpp_mpa_init_kernel<true><<<blocks, MPP_MPA_THREADS, 0, (cudaStream_t)stream>>>(A, maps->n_maps, params_dev);
+    else mpp_mpa_init_kernel<false><<<blocks, MPP_MPA_THREADS, 0, (cudaStream_t)stream>>>(A, maps->n_maps, nullptr);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
+}
+
+extern "C" int mpp_mpa_init_batch(const mpp_map_batch *maps, const mpp_policy *policy, int n_predators, int max_cells,
+                                  int32_t *cells_dev, int32_t *n_cells_dev, double *stats_dev, void *scratch_dev,
+                                  size_t scratch_bytes, int heap_cap, int32_t *status_dev, unsigned long long *counters_dev,
+                                  void *stream) {
+    return mpa_init(maps, policy, nullptr, n_predators, max_cells, cells_dev, n_cells_dev, stats_dev, scratch_dev,
+                    scratch_bytes, heap_cap, status_dev, counters_dev, stream, "mpp_mpa_init_batch");
+}
+
+extern "C" int mpp_mpa_init_batch_p(const mpp_map_batch *maps, const mpp_policy *policy, const mpp_pop_params *params_dev,
+                                    int n_predators, int max_cells, int32_t *cells_dev, int32_t *n_cells_dev,
+                                    double *stats_dev, void *scratch_dev, size_t scratch_bytes, int heap_cap,
+                                    int32_t *status_dev, unsigned long long *counters_dev, void *stream) {
+    MPP_REQUIRE(params_dev, "mpp_mpa_init_batch_p: null params_dev");
+    return mpa_init(maps, policy, params_dev, n_predators, max_cells, cells_dev, n_cells_dev, stats_dev, scratch_dev,
+                    scratch_bytes, heap_cap, status_dev, counters_dev, stream, "mpp_mpa_init_batch_p");
 }

@@ -8,23 +8,29 @@
 
 #define MPP_POP_MAX_MAPS 65535                                 // grid.y
 
-
 // ---------------------------------------------------------------------------------------------
 // K8: PSO update.  v = ((w*v) + ((c1*r1)*(pbest-x))) + ((c2*r2)*(gbest-x)); clip; x = clip(x+v).
 // Draw order per particle (pso.py:185-190): for each waypoint: r1,r2 (row) then r1',r2' (col)
 // => draws 4*dim+{0,1,2,3} of stream (seed, PSO_UPDATE, iteration, particle).
 // Also emits the integer waypoint pso.py:61,69-70: int(round(x)) (half-even) clamped to the grid.
 // ---------------------------------------------------------------------------------------------
-// Particles [start[m], n) of map m (the stream index is the particle index).
-__global__ void mpp_pso_update_kernel(double *__restrict__ pos, double *__restrict__ vel,
-                                      const double *__restrict__ pbest, const double *__restrict__ gbest, int n, int W,
-                                      const int32_t *__restrict__ start, double w, double c1, double c2, double max_vel,
-                                      int R, int C, const uint64_t *__restrict__ seeds, uint32_t iteration,
-                                      int32_t *__restrict__ wp_cells) {
+// Particles [start[m], n) of map m (the stream index is the particle index).  MP (per-map parameters): w, c1, c2 of
+// params[m] instead of the launch's scalars.
+template <bool MP>
+__device__ __forceinline__ void pso_update_body(double *__restrict__ pos, double *__restrict__ vel,
+                                                const double *__restrict__ pbest, const double *__restrict__ gbest, int n,
+                                                int W, const int32_t *__restrict__ start, double w, double c1, double c2,
+                                                const mpp_pop_params *__restrict__ params, double max_vel, int R, int C,
+                                                const uint64_t *__restrict__ seeds, uint32_t iteration,
+                                                int32_t *__restrict__ wp_cells) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n * W) return;
     const int p = t / W, dim = t % W;
     if (p < start[blockIdx.y]) return;
+    if constexpr (MP) {
+        const mpp_pop_params &P = params[blockIdx.y];
+        w = P.w; c1 = P.c1; c2 = P.c2;
+    }
     const uint64_t sd = seeds[blockIdx.y];
     const uint32_t k0 = (uint32_t)sd, k1 = (uint32_t)(sd >> 32);
     const size_t row = (size_t)blockIdx.y * n * W;             // map m's particles
@@ -46,6 +52,15 @@ __global__ void mpp_pso_update_kernel(double *__restrict__ pos, double *__restri
     int ir = (int)rint(nr), ic = (int)rint(nc);                                                       // :61 round-half-even
     ir = max(0, min(R - 1, ir)); ic = max(0, min(C - 1, ic));                                         // :69-70
     wp_cells[(size_t)p * W + dim] = ir * C + ic;
+}
+
+__global__ void mpp_pso_update_kernel(double *__restrict__ pos, double *__restrict__ vel,
+                                      const double *__restrict__ pbest, const double *__restrict__ gbest, int n, int W,
+                                      const int32_t *__restrict__ start, double w, double c1, double c2, double max_vel,
+                                      int R, int C, const uint64_t *__restrict__ seeds, uint32_t iteration,
+                                      int32_t *__restrict__ wp_cells) {
+    pso_update_body<false>(pos, vel, pbest, gbest, n, W, start, w, c1, c2, nullptr, max_vel, R, C, seeds, iteration,
+                           wp_cells);
 }
 
 extern "C" int mpp_pso_update_batch(const mpp_map_batch *maps, double *pos_dev, double *vel_dev,
@@ -144,10 +159,15 @@ __device__ __forceinline__ int ga_random_free_cell(mpp_stream_rng &rng, const ui
     }
 }
 
-__global__ void mpp_ga_breed_kernel(const uint32_t *__restrict__ occ, int occ_words, int pitch, int R, int C,
-                                    const int32_t *__restrict__ chrom, const int32_t *__restrict__ parents, int n, int W,
-                                    double cx_rate, double mut_rate, const uint64_t *__restrict__ seeds,
-                                    uint32_t generation, int32_t *__restrict__ children) {
+// MP: crossover and mutation rates of params[m]; a parent index outside 0..n-1 (mpp_ga_select_batch_p's -1) reads
+// individual 0.
+template <bool MP>
+__device__ __forceinline__ void ga_breed_body(const uint32_t *__restrict__ occ, int occ_words, int pitch, int R, int C,
+                                              const int32_t *__restrict__ chrom, const int32_t *__restrict__ parents,
+                                              int n, int W, double cx_rate, double mut_rate,
+                                              const mpp_pop_params *__restrict__ params,
+                                              const uint64_t *__restrict__ seeds, uint32_t generation,
+                                              int32_t *__restrict__ children) {
     const int pair = blockIdx.x * blockDim.x + threadIdx.x;
     const int n_pairs = (n + 1) / 2;
     if (pair >= n_pairs) return;
@@ -157,8 +177,15 @@ __global__ void mpp_ga_breed_kernel(const uint32_t *__restrict__ occ, int occ_wo
     children += (size_t)blockIdx.y * n * W;
     mpp_stream_rng rng;
     rng.init(seeds[blockIdx.y], MPP_CLS_GA_BREED, generation, (uint32_t)pair);
-    const int32_t *p1 = chrom + (size_t)parents[(2 * pair) % n] * W;
-    const int32_t *p2 = chrom + (size_t)parents[(2 * pair + 1) % n] * W;
+    int i1 = parents[(2 * pair) % n], i2 = parents[(2 * pair + 1) % n];
+    if constexpr (MP) {
+        const mpp_pop_params &P = params[blockIdx.y];
+        cx_rate = P.crossover_rate; mut_rate = P.mutation_rate;
+        if ((unsigned)i1 >= (unsigned)n) i1 = 0;
+        if ((unsigned)i2 >= (unsigned)n) i2 = 0;
+    }
+    const int32_t *p1 = chrom + (size_t)i1 * W;
+    const int32_t *p2 = chrom + (size_t)i2 * W;
     int32_t c1[MPP_GA_MAX_W], c2[MPP_GA_MAX_W];
     int point = 0;
     if (rng.draw() < cx_rate && W > 0) {                               // :145
@@ -176,6 +203,14 @@ __global__ void mpp_ga_breed_kernel(const uint32_t *__restrict__ occ, int occ_wo
     for (int i = 0; i < W; ++i) children[(size_t)(2 * pair) * W + i] = c1[i];
     if (2 * pair + 1 < n)
         for (int i = 0; i < W; ++i) children[(size_t)(2 * pair + 1) * W + i] = c2[i];
+}
+
+__global__ void mpp_ga_breed_kernel(const uint32_t *__restrict__ occ, int occ_words, int pitch, int R, int C,
+                                    const int32_t *__restrict__ chrom, const int32_t *__restrict__ parents, int n, int W,
+                                    double cx_rate, double mut_rate, const uint64_t *__restrict__ seeds,
+                                    uint32_t generation, int32_t *__restrict__ children) {
+    ga_breed_body<false>(occ, occ_words, pitch, R, C, chrom, parents, n, W, cx_rate, mut_rate, nullptr, seeds,
+                         generation, children);
 }
 
 extern "C" int mpp_ga_breed_batch(const mpp_map_batch *maps, const int32_t *chrom_dev, const int32_t *parents_dev, int n,
@@ -271,6 +306,125 @@ extern "C" int mpp_ga_init_batch(const mpp_map_batch *maps, int n_attempts, cons
     mpp_ga_init_kernel<<<dim3((n_attempts + 127) / 128, maps->n_maps), 128, 0, (cudaStream_t)stream>>>(
         maps->occ_dev, maps->occ_words, maps->pitch_words, maps->rows, maps->cols, n_attempts, n_waypoints,
         attempt_offset_dev, seeds_dev, chrom_dev);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// The same three steps with per-map parameters (mpp_pop_params, a parameter sweep as one batch).  Defined after every
+// kernel of the scalar API: placed among them, they change those kernels' code.
+// ---------------------------------------------------------------------------------------------
+__global__ void mpp_pso_update_p_kernel(double *__restrict__ pos, double *__restrict__ vel,
+                                        const double *__restrict__ pbest, const double *__restrict__ gbest, int n, int W,
+                                        const int32_t *__restrict__ start, const mpp_pop_params *__restrict__ params,
+                                        double max_vel, int R, int C, const uint64_t *__restrict__ seeds,
+                                        uint32_t iteration, int32_t *__restrict__ wp_cells) {
+    pso_update_body<true>(pos, vel, pbest, gbest, n, W, start, 0.0, 0.0, 0.0, params, max_vel, R, C, seeds, iteration,
+                          wp_cells);
+}
+// The sampling of mpp_ga_select_kernel (a copy: sharing it through an inline function changes that kernel's code) with
+// k = min(params[m].tournament_size, n), bounded here as mpp_ga_select_batch bounds the scalar on the host: a k the
+// sample buffers cannot hold makes every parent of the map -1.
+__global__ void mpp_ga_select_p_kernel(const double *__restrict__ fitness, int n,
+                                       const mpp_pop_params *__restrict__ params, const uint64_t *__restrict__ seeds,
+                                       uint32_t generation, int32_t *__restrict__ parents) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    fitness += (size_t)blockIdx.y * n;
+    parents += (size_t)blockIdx.y * n;
+    const int ts = params[blockIdx.y].tournament_size;
+    const int k = ts < n ? ts : n;                                     // min(tournament_size, len(population))
+    if (k < 1 || k > MPP_GA_MAX_K || (k > 5 && n <= 21 + 64)) { parents[t] = -1; return; }
+    mpp_stream_rng rng;
+    rng.init(seeds[blockIdx.y], MPP_CLS_GA_SELECT, generation, (uint32_t)t);
+    int setsize = 21;
+    if (k > 5) {  // setsize += 4 ** ceil(log(k*3, 4))
+        int e = 0, v = 1;
+        while (v < k * 3) { v *= 4; ++e; }
+        setsize += v;
+    }
+    int sel[MPP_GA_MAX_K];
+    if (n <= setsize) {
+        int pool[21 + 64];
+        for (int i = 0; i < n; ++i) pool[i] = i;
+        for (int i = 0; i < k; ++i) {
+            const int j = rng.below(n - i);
+            sel[i] = pool[j];
+            pool[j] = pool[n - i - 1];
+        }
+    } else {
+        for (int i = 0; i < k; ++i) {
+            int j;
+            bool dup;
+            do {
+                j = rng.below(n);
+                dup = false;
+                for (int q = 0; q < i; ++q) dup |= (sel[q] == j);
+            } while (dup);
+            sel[i] = j;
+        }
+    }
+    int best = sel[0];
+    double bf = fitness[best];
+    for (int i = 1; i < k; ++i) {
+        const double f = fitness[sel[i]];
+        if (f < bf) { bf = f; best = sel[i]; }
+    }
+    parents[t] = best;
+}
+__global__ void mpp_ga_breed_p_kernel(const uint32_t *__restrict__ occ, int occ_words, int pitch, int R, int C,
+                                      const int32_t *__restrict__ chrom, const int32_t *__restrict__ parents, int n,
+                                      int W, const mpp_pop_params *__restrict__ params,
+                                      const uint64_t *__restrict__ seeds, uint32_t generation,
+                                      int32_t *__restrict__ children) {
+    ga_breed_body<true>(occ, occ_words, pitch, R, C, chrom, parents, n, W, 0.0, 0.0, params, seeds, generation,
+                        children);
+}
+
+extern "C" int mpp_pso_update_batch_p(const mpp_map_batch *maps, double *pos_dev, double *vel_dev,
+                                      const double *pbest_pos_dev, const double *gbest_pos_dev, int n_particles,
+                                      const int32_t *start_dev, int n_waypoints, const mpp_pop_params *params_dev,
+                                      double max_vel, const uint64_t *seeds_dev, int iteration,
+                                      int32_t *waypoint_cells_dev, void *stream) {
+    MPP_REQUIRE(maps && pos_dev && vel_dev && pbest_pos_dev && gbest_pos_dev && start_dev && params_dev && seeds_dev &&
+                waypoint_cells_dev, "mpp_pso_update_batch_p: null argument");
+    MPP_REQUIRE(n_particles > 0 && n_waypoints > 0 && maps->n_maps <= MPP_POP_MAX_MAPS,
+                "mpp_pso_update_batch_p: bad sizes");
+    MPP_CUDA(cudaSetDevice(maps->device));
+    const int total = n_particles * n_waypoints;
+    mpp_pso_update_p_kernel<<<dim3((total + 255) / 256, maps->n_maps), 256, 0, (cudaStream_t)stream>>>(
+        pos_dev, vel_dev, pbest_pos_dev, gbest_pos_dev, n_particles, n_waypoints, start_dev, params_dev, max_vel,
+        maps->rows, maps->cols, seeds_dev, (uint32_t)iteration, waypoint_cells_dev);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
+
+extern "C" int mpp_ga_select_batch_p(const mpp_map_batch *maps, const double *fitness_dev, int n,
+                                     const mpp_pop_params *params_dev, const uint64_t *seeds_dev, int generation,
+                                     int32_t *parents_dev, void *stream) {
+    MPP_REQUIRE(maps && params_dev && seeds_dev && fitness_dev && parents_dev && n > 0 &&
+                maps->n_maps <= MPP_POP_MAX_MAPS, "mpp_ga_select_batch_p: bad argument");
+    MPP_CUDA(cudaSetDevice(maps->device));
+    mpp_ga_select_p_kernel<<<dim3((n + 127) / 128, maps->n_maps), 128, 0, (cudaStream_t)stream>>>(
+        fitness_dev, n, params_dev, seeds_dev, (uint32_t)generation, parents_dev);
+    MPP_CUDA(cudaGetLastError());
+    return MPP_OK;
+}
+
+extern "C" int mpp_ga_breed_batch_p(const mpp_map_batch *maps, const int32_t *chrom_dev, const int32_t *parents_dev,
+                                    int n, int n_waypoints, const mpp_pop_params *params_dev, const uint64_t *seeds_dev,
+                                    int generation, int32_t *children_dev, void *stream) {
+    MPP_REQUIRE(maps && chrom_dev && parents_dev && params_dev && seeds_dev && children_dev && n > 0 &&
+                maps->n_maps <= MPP_POP_MAX_MAPS, "mpp_ga_breed_batch_p: bad argument");
+    MPP_REQUIRE(n_waypoints >= 1 && n_waypoints <= MPP_GA_MAX_W, "mpp_ga_breed_batch_p: %d waypoints unsupported (1..%d)",
+                n_waypoints, MPP_GA_MAX_W);
+    for (int k = 0; k < maps->n_maps; ++k)                             // the start cell is free: mutation terminates
+        MPP_REQUIRE(maps->meta_host[k].start >= 0, "mpp_ga_breed_batch_p: map %d has no start", k);
+    MPP_CUDA(cudaSetDevice(maps->device));
+    const int n_pairs = (n + 1) / 2;
+    mpp_ga_breed_p_kernel<<<dim3((n_pairs + 127) / 128, maps->n_maps), 128, 0, (cudaStream_t)stream>>>(
+        maps->occ_dev, maps->occ_words, maps->pitch_words, maps->rows, maps->cols, chrom_dev, parents_dev, n, n_waypoints,
+        params_dev, seeds_dev, (uint32_t)generation, children_dev);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
 }

@@ -18,6 +18,13 @@ struct StatsCtx {
 // batch's safety tables (mpp_map_batch_safety_table).  A kernel offsets occ / cls to the map a path lies on.
 int mpp_stats_ctx(mpp_map_batch *maps, const mpp_policy *pol, void *stream, StatsCtx *X);
 
+// the statistics weights of a map's per-map parameters (mpp_pop_params) in place of the policy's
+static __device__ __forceinline__ void mpp_pop_weights(mpp_policy &pol, const mpp_pop_params &p) {
+    pol.turn_penalty_factor = p.turn_penalty_factor;
+    pol.safety_penalty_factor = p.safety_penalty_factor;
+    pol.diagonal_obstacle_penalty_value = p.diagonal_obstacle_penalty_value;
+}
+
 static __device__ void path_stats_warp(const LaneGroup &L, const StatsCtx &X, const int32_t *cells, int n, double *out) {
     const int lane = L.gl;
     const double INF = __longlong_as_double(MPP_INF_BITS);
