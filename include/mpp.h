@@ -260,6 +260,20 @@ int mpp_maaco_pass(const mpp_map_batch *maps, const mpp_colony *colony, const mp
 int mpp_maaco_pass_maps(const mpp_map_batch *maps, const mpp_colony *colony, const mpp_maaco_params *params_dev,
                         const double *q0_dev, int iteration, int n_ants, int ants_per_warp, void *stream);
 
+/* mpp_maaco_pass_maps with a colony size and a pass count per map: map m is solved as if alone with
+ * sizes_dev[m] = {num_ants, num_iterations} (DEVICE, [n_maps][2] int32).  n_ants is the colony's ant CAPACITY, the count
+ * the buffers are laid out for (slabs, touched, moves, result, deposit and okbits strides); q0_dev is [max K][n_maps]
+ * with column m = mpp_maaco_q0(K_m, k, q0_initial of map m) and must hold row iteration-1.  For map m:
+ *   - its colony is n_m = num_ants clamped to [0, n_ants]: ants [0, n_m) construct tours, take part in the best scans
+ *     and deposit; ants [n_m, n_ants) write no result, no slab, no `touched` bit and no step count, and get deposit 0.
+ *     n_m = 0 constructs no tour and deposits nothing (tau still evaporates);
+ *   - it takes part in pass `iteration` only if iteration <= num_iterations: past it (a negative count included) no
+ *     kernel touches the map, so its tau, state, best path, log and results stay as they are.
+ * sizes_dev = NULL is mpp_maaco_pass_maps (every map runs every pass with n_ants ants). */
+int mpp_maaco_pass_maps_sized(const mpp_map_batch *maps, const mpp_colony *colony, const mpp_maaco_params *params_dev,
+                              const double *q0_dev, const int32_t *sizes_dev, int iteration, int n_ants,
+                              int ants_per_warp, void *stream);
+
 /* the same pass with HOST buffers -- what a caller holding NumPy arrays binds: copies the pheromone field in
  * (tau_in_host: n_maps x rows*cols doubles, or NULL to keep the device field), runs the pass, copies out the updated
  * field, the per-ant results (n_maps x n_ants), the colony state(s) and the best path(s) so far

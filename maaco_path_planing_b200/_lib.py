@@ -88,6 +88,8 @@ _SIGS = {
                                     c_int, c_int, c_void_p, c_int, c_void_p]),
     "mpp_maaco_pass": (c_int, [c_void_p, C.POINTER(Colony), C.POINTER(MaacoParams), c_int, c_int, c_int, c_void_p]),
     "mpp_maaco_pass_maps": (c_int, [c_void_p, C.POINTER(Colony), c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
+    "mpp_maaco_pass_maps_sized": (c_int, [c_void_p, C.POINTER(Colony), c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                                          c_void_p]),
     "mpp_maaco_pass_host": (c_int, [c_void_p, C.POINTER(Colony), C.POINTER(MaacoParams), c_int, c_int, c_int, c_void_p,
                                     c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "mpp_maaco_max_peers": (c_int, []),

@@ -11,6 +11,8 @@ reference), and tau0 of each map is that shared table with the map's obstacles m
 built on the device with replicas of the host libm's exp / pow (mpp_maaco_e01_maps, bit for bit mpp_maaco_e01_host's),
 and tau0 is computed per map on the device (mpp_maaco_tau0_maps).  With map_params each map of a wave also has its own
 colony parameters (a parameter sweep in one launch per pass): the pass kernels read them per map (mpp_maaco_pass_maps).
+With map_sizes each map also has its own colony size and pass count inside buffers sized for the wave's largest
+(mpp_maaco_pass_maps_sized).
 
 Every batch class takes `grids` either on the host ([M, rows, cols] cell codes, anything np.asarray takes) or as an
 [M, rows, cols] CUDA tensor of bool, uint8, int8, int16, int32 or int64 cells; every sweep also takes a sequence of 2-D
@@ -19,6 +21,7 @@ through the host; results are the same as from the same grids on the host."""
 from __future__ import annotations
 
 import ctypes as C
+import numbers
 
 import numpy as np
 
@@ -182,7 +185,8 @@ _WAYPOINT_DEFAULTS = dict(turn_penalty_factor=0.1, safety_penalty_factor=0.05, m
                           allow_diagonal_moves=True, restrict_diagonal_near_obstacle_policy=True,      # ga_solver.py:19-22
                           diagonal_obstacle_penalty_value=1000.0)
 # planner -> (keys a map may set, keys a map may set only to its wave's value (they change the searches or the safety
-# tables; the sweeps group waves by them), keys common to a wave (sizes), the constructor's defaults)
+# tables; the sweeps group waves by them), sizes, which map_params never sets (MAACO takes them per map in map_sizes),
+# the constructor's defaults)
 PLANNER_MAP_PARAMS = {
     "maaco": (MAP_PARAM_KEYS, (), ("num_iterations", "num_ants"),
               {"C0_initial_pheromone": 0.1}),                                 # (MAACO's default, MAACO.py:14)
@@ -229,11 +233,10 @@ def resolve_map_params(defaults, map_params, n_maps, planner="maaco", population
     """One dict per map of the keys `planner` may set per map and per wave (PLANNER_MAP_PARAMS; MAACO: the ten
     MAP_PARAM_KEYS): map k's mapping of `map_params` over `defaults` (the constructor's arguments; keys it leaves out
     take the constructor's defaults).  ValueError for a length other than n_maps, an entry that is not a mapping, an
-    unknown key or a size common to a wave (MAACO: num_iterations / num_ants -- the pass count and the buffer layouts
-    depend on them), and for values the kernels cannot take: GA's tournament_size where min(tournament_size,
-    population) lies outside 1..16 or exceeds 5 with a population of 85 or less (mpp_ga_select_batch's limits), MPA's
-    levy_beta where the Levy sigma is complex.  Whether the per-wave keys agree is the caller's matter
-    (_wave_params)."""
+    unknown key or a size (MAACO: num_iterations / num_ants, which map_sizes sets per map), and for values the kernels
+    cannot take: GA's tournament_size where min(tournament_size, population) lies outside 1..16 or exceeds 5 with a
+    population of 85 or less (mpp_ga_select_batch's limits), MPA's levy_beta where the Levy sigma is complex.  Whether
+    the per-wave keys agree is the caller's matter (_wave_params)."""
     per_map, per_wave, sizes, ctor_defaults = PLANNER_MAP_PARAMS[planner]
     if isinstance(map_params, (str, bytes)) or not hasattr(map_params, "__len__"):
         raise ValueError("map_params must be a sequence of one mapping per map")
@@ -248,7 +251,8 @@ def resolve_map_params(defaults, map_params, n_maps, planner="maaco", population
             raise ValueError(f"map_params[{i}] is not a mapping")
         for k in mp.keys():
             if k in sizes:
-                raise ValueError(f"map_params[{i}]: {k} is common to all maps of a wave and cannot be set per map")
+                raise ValueError(f"map_params[{i}]: {k} is common to all maps of a wave and cannot be set per map"
+                                 + ("; MAACOBatch takes it per map in map_sizes" if planner == "maaco" else ""))
             if k not in base:
                 raise ValueError(f"map_params[{i}]: unknown parameter {k!r} ({known})")
         p = {**base, **{k: _map_param_value(planner, i, k, v) for k, v in mp.items()}}
@@ -303,14 +307,54 @@ def _pop_params_host(planner, resolved):
 
 
 def q0_table(num_iterations, q0_initial):
-    """[max(1, num_iterations), len(q0_initial)] float64: row k-1 holds every map's q0 of pass k,
-    mpp_maaco_q0(num_iterations, k, q0_initial[m]) -- the value solo MAACO passes to its k-th pass (MAACO.py:212-226)."""
+    """[max(1, K), len(q0_initial)] float64: row k-1 holds every map's q0 of pass k, mpp_maaco_q0(K_m, k, q0_initial[m])
+    -- the value solo MAACO with K_m iterations passes to its k-th pass (MAACO.py:212-226).  num_iterations is one count
+    for every map (K = it) or one per map (K = the largest; rows past a map's own count are never read)."""
     L = _lib.lib()
-    K = max(1, int(num_iterations))
     q = np.asarray(q0_initial, np.float64)
+    if np.ndim(num_iterations) == 0:
+        Ks = np.full(len(q), int(num_iterations), np.int64)
+        K = max(1, int(num_iterations))
+    else:
+        Ks = np.asarray(num_iterations, np.int64)
+        if Ks.shape != q.shape:
+            raise ValueError(f"q0_table: {len(Ks)} pass counts for {len(q)} maps")
+        K = max(1, int(Ks.max(initial=0)))
     out = np.empty((K, len(q)), np.float64)
-    for v in np.unique(q):                                       # one column per distinct q0_initial
-        out[:, q == v] = np.array([L.mpp_maaco_q0(int(num_iterations), k, float(v)) for k in range(1, K + 1)])[:, None]
+    for n, v in dict.fromkeys(zip(Ks.tolist(), q.tolist())):     # one column per distinct (K_m, q0_initial)
+        out[:, (Ks == n) & (q == v)] = np.array([L.mpp_maaco_q0(n, k, v) for k in range(1, K + 1)])[:, None]
+    return out
+
+
+MAP_SIZE_KEYS = ("num_ants", "num_iterations")
+
+
+def resolve_map_sizes(num_ants, num_iterations, map_sizes, n_maps):
+    """One {"num_ants", "num_iterations"} dict of ints per map: map k's mapping of `map_sizes` over the constructor's
+    num_ants / num_iterations.  ValueError for a length other than n_maps, an entry that is not a mapping, another key,
+    a value that is not an integer (bool included), num_ants < 1 or num_iterations < 0."""
+    if isinstance(map_sizes, (str, bytes)) or not hasattr(map_sizes, "__len__"):
+        raise ValueError("map_sizes must be a sequence of one mapping per map")
+    if len(map_sizes) != n_maps:
+        raise ValueError(f"map_sizes has {len(map_sizes)} entries for {n_maps} maps")
+    out = []
+    for i, ms in enumerate(map_sizes):
+        if not hasattr(ms, "keys"):
+            raise ValueError(f"map_sizes[{i}] is not a mapping")
+        for k in ms.keys():
+            if k not in MAP_SIZE_KEYS:
+                raise ValueError(f"map_sizes[{i}]: unknown key {k!r} (keys: {', '.join(MAP_SIZE_KEYS)})")
+        s = {"num_ants": num_ants, "num_iterations": num_iterations, **ms}
+        for k in MAP_SIZE_KEYS:
+            v = s[k]
+            if isinstance(v, (bool, np.bool_)) or not isinstance(v, numbers.Integral):
+                raise ValueError(f"map_sizes[{i}]: {k} must be an integer, not {v!r}")
+            s[k] = int(v)
+        if s["num_ants"] < 1:
+            raise ValueError(f"map_sizes[{i}]: num_ants {s['num_ants']} < 1")
+        if s["num_iterations"] < 0:
+            raise ValueError(f"map_sizes[{i}]: num_iterations {s['num_iterations']} < 0")
+        out.append({k: s[k] for k in MAP_SIZE_KEYS})
     return out
 
 
@@ -386,11 +430,21 @@ class MAACOBatch:
     The passes then run the per-map instantiations of the kernels (mpp_maaco_pass_maps), tau0 comes from
     mpp_maaco_tau0_maps_p, and E01 is one table per map (mpp_maaco_e01_maps_p, or mpp_maaco_e01_host once per distinct
     parameter set) unless every map shares its endpoints and the five parameters eta'**beta depends on.  Map k's results
-    are those of solo MAACO with map k's parameters and seed."""
+    are those of solo MAACO with map k's parameters and seed.
+
+    map_sizes (None or one mapping per map) gives each map its own colony size and pass count: a mapping sets
+    num_ants and / or num_iterations (resolve_map_sizes), the keys it leaves out take the constructor's values, and
+    `b.map_sizes` holds the resolved dicts.  The buffers are laid out for the wave's largest num_ants and the log for its
+    largest num_iterations; solve() runs passes up to the largest count, and map k takes part in its first
+    num_iterations_k passes with its first num_ants_k ants (mpp_maaco_pass_maps_sized).  Without map_params every map
+    carries the constructor's parameters through the per-map kernels (`b.map_params` then holds them).  Map k's
+    results are those of MAACO(grid_k, num_ants_k, num_iterations_k, ...) with map k's parameters and seed; its
+    convergence curve has num_iterations_k entries, and last_results() reads ants outside its colony, and every ant of
+    a map that has not run a pass yet, as failed ants (n_cells 0, length inf, turns -1)."""
 
     def __init__(self, grids, num_ants, num_iterations, alpha, beta, rho, Q, a_turn_coef, wh_max, wh_min, k_h_adaptive,
                  q0_initial, C0_initial_pheromone=0.1, *, seeds=None, device=None, max_cells=None, ants_per_warp=0,
-                 reuse=None, per_map_endpoints=False, map_params=None, _e01=None):
+                 reuse=None, per_map_endpoints=False, map_params=None, map_sizes=None, _e01=None):
         # _e01 (the max_cells repeat): this wave's per-map tables, already built -- an [M, 2 * rows * cols] CUDA tensor
         # on the wave's device, used as it is
         import torch
@@ -405,8 +459,17 @@ class MAACOBatch:
         self.alpha, self.rho, self.Q = alpha, rho, Q
         self._params = _maaco_params(num_iterations, alpha, beta, rho, Q, a_turn_coef, wh_max, wh_min, k_h_adaptive,
                                      q0_initial, C0_initial_pheromone)
-        M, R, Cc, N = self.n_maps, self.rows, self.cols, self.num_ants
+        M, R, Cc = self.n_maps, self.rows, self.cols
         start, target = self._map_set.start, self._map_set.target
+        self.map_sizes = None
+        if map_sizes is not None:
+            self.map_sizes = resolve_map_sizes(self.num_ants, self.num_iterations, map_sizes, M)
+            if map_params is None:                                       # the constructor's parameters, per map
+                map_params = [{}] * M
+        # the buffers' ant capacity and the passes solve() runs: the largest colony and pass count with map_sizes
+        sizes = self.map_sizes or [{"num_ants": self.num_ants, "num_iterations": self.num_iterations}]
+        self._ants = N = max(s["num_ants"] for s in sizes)
+        self._passes = max(s["num_iterations"] for s in sizes)
         self.map_params = None
         if map_params is not None:
             self.map_params = resolve_map_params(
@@ -434,10 +497,11 @@ class MAACOBatch:
         self._ctor = dict(num_ants=num_ants, num_iterations=num_iterations, alpha=alpha, beta=beta, rho=rho, Q=Q,
                           a_turn_coef=a_turn_coef, wh_max=wh_max, wh_min=wh_min, k_h_adaptive=k_h_adaptive,
                           q0_initial=q0_initial, C0_initial_pheromone=C0_initial_pheromone, seeds=self.seeds,
-                          ants_per_warp=ants_per_warp, per_map_endpoints=per_map_endpoints, map_params=self.map_params)
+                          ants_per_warp=ants_per_warp, per_map_endpoints=per_map_endpoints, map_params=self.map_params,
+                          map_sizes=self.map_sizes)
         dev = self.device
         f64, i32, i64, u8 = torch.float64, torch.int32, torch.int64, torch.uint8
-        K = max(1, self.num_iterations)
+        K = max(1, self._passes)
         key = (M, R, Cc, N, self.max_cells, K, self.device_index, self.per_map_tables,   # (the E01 layout)
                self.map_params is not None)
         if reuse is not None and getattr(reuse, "_key", None) == key:
@@ -467,11 +531,19 @@ class MAACOBatch:
             self._log = torch.zeros((M, K, 4), dtype=f64, device=dev)
         self._key = key
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        self._params_dev = self._q0_dev = None
+        self._params_dev = self._q0_dev = self._sizes_dev = None
         if self.map_params is not None:
-            host = (_lib.MaacoParams * M)(*[_maaco_params(num_iterations, **p) for p in self.map_params])
+            Ks = [s["num_iterations"] for s in self.map_sizes] if self.map_sizes is not None else num_iterations
+            host = (_lib.MaacoParams * M)(*[_maaco_params(Ks if np.ndim(Ks) == 0 else Ks[k], **p)
+                                            for k, p in enumerate(self.map_params)])
             self._params_dev = torch.frombuffer(bytearray(bytes(host)), dtype=u8).to(dev)
-            self._q0_dev = torch.from_numpy(q0_table(num_iterations, [p["q0_initial"] for p in self.map_params])).to(dev)
+            self._q0_dev = torch.from_numpy(q0_table(Ks, [p["q0_initial"] for p in self.map_params])).to(dev)
+        if self.map_sizes is not None:
+            self._sizes_dev = torch.tensor([[s["num_ants"], s["num_iterations"]] for s in self.map_sizes], dtype=i32,
+                                           device=dev)
+            # every record reads as a failed ant (length inf, n_cells 0, turns -1) until the map's own ants overwrite it
+            self._result[..., 0] = 0x7FF0000000000000
+            self._result[..., 1] = -(1 << 32)
         if self.per_map_tables:
             if _e01 is not None:
                 if tuple(_e01.shape) != (M, 2 * n) or _e01.device != dev or _e01.dtype != f64:
@@ -533,10 +605,14 @@ class MAACOBatch:
     def run_iteration(self, it):
         """Enqueue one colony pass of every map of the wave (asynchronous)."""
         import torch
-        if not 1 <= it <= max(1, self.num_iterations):
-            raise ValueError(f"iteration {it} outside 1..{self.num_iterations}")
+        if not 1 <= it <= max(1, self._passes):
+            raise ValueError(f"iteration {it} outside 1..{self._passes}")
         stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        if self._params_dev is not None:
+        if self._sizes_dev is not None:
+            _lib.check(_lib.lib().mpp_maaco_pass_maps_sized(
+                self._maps, C.byref(self._colony), _lib.ptr(self._params_dev), _lib.ptr(self._q0_dev),
+                _lib.ptr(self._sizes_dev), it, self._ants, self._apw, stream), "mpp_maaco_pass_maps_sized")
+        elif self._params_dev is not None:
             _lib.check(_lib.lib().mpp_maaco_pass_maps(self._maps, C.byref(self._colony), _lib.ptr(self._params_dev),
                                                       _lib.ptr(self._q0_dev), it, self.num_ants, self._apw, stream),
                        "mpp_maaco_pass_maps")
@@ -550,11 +626,12 @@ class MAACOBatch:
         return self._tau.cpu().numpy().reshape(self.n_maps, self.rows, self.cols)
 
     def last_results(self):
-        """(n_cells, length, turns), each [n_maps, num_ants], of the last pass."""
+        """(n_cells, length, turns), each [n_maps, num_ants], of the last pass (with map_sizes: [n_maps, largest
+        num_ants], and ants outside a map's colony read as failed ants)."""
         import torch
         torch.cuda.synchronize(self.device)
         rec = self._result.cpu().numpy().view(np.dtype([("length", "<f8"), ("n_cells", "<i4"), ("turns", "<i4")]))
-        rec = rec.reshape(self.n_maps, self.num_ants)
+        rec = rec.reshape(self.n_maps, self._ants)
         return rec["n_cells"].copy(), rec["length"].copy(), rec["turns"].copy()
 
     def total_steps(self):
@@ -564,10 +641,11 @@ class MAACOBatch:
         """Runs the remaining iterations; returns one (path, length, turns, convergence_curve) per map -- the values
         MAACO.solve_path_planning (MAACO.py:334-371) returns / stores for that map."""
         import torch
-        for it in range(self._iter_done + 1, self.num_iterations + 1):
+        for it in range(self._iter_done + 1, self._passes + 1):
             self.run_iteration(it)
         torch.cuda.synchronize(self.device)
-        M, K = self.n_maps, self.num_iterations
+        M = self.n_maps
+        Ks = [s["num_iterations"] for s in self.map_sizes] if self.map_sizes is not None else [self.num_iterations] * M
         st = np.frombuffer(self._state.cpu().numpy().tobytes(), dtype=np.dtype(
             [("best_len", "<f8"), ("best_turns", "<i4"), ("best_n_cells", "<i4"), ("best_iter", "<i4"), ("best_ant", "<i4"),
              ("iter_best_len", "<f8"), ("iter_best_turns", "<i4"), ("iter_best_ant", "<i4")]))
@@ -583,14 +661,14 @@ class MAACOBatch:
             self.__dict__.update(again.__dict__)
             return self.solve()
         best = self._best_cells.cpu().numpy()
-        log = self._log.cpu().numpy()[:, :K]
+        log = self._log.cpu().numpy()
         out = []
         for k in range(M):
             nb = int(st["best_n_cells"][k])
             pr, pc = np.divmod(best[k, :nb], self.cols)
             path = list(zip(pr.tolist(), pc.tolist()))
             turns = int(st["best_turns"][k]) if st["best_turns"][k] >= 0 else INF
-            curve = [float(v) if v != INF else None for v in log[k, :, 2]]
+            curve = [float(v) if v != INF else None for v in log[k, :Ks[k], 2]]
             out.append((path, float(st["best_len"][k]), turns, curve))
         return out
 
@@ -672,7 +750,7 @@ def _waves(keys, wave):
 
 
 def solve_maaco_batch(grids, num_ants, num_iterations, params, seeds=None, wave=256, group=None, device=None,
-                      max_cells=None, per_map_endpoints=False, map_params=None):
+                      max_cells=None, per_map_endpoints=False, map_params=None, map_sizes=None):
     """Run MAACO on every grid of `grids` (this rank's shard when `group` is given), `wave` maps per launch.  `grids`:
     host maps, a [n_maps, rows, cols] CUDA tensor or a sequence of 2-D CUDA tensors (which never leave the GPU).
 
@@ -685,10 +763,20 @@ def solve_maaco_batch(grids, num_ants, num_iterations, params, seeds=None, wave=
     MAACOBatch(map_params=...) takes them: map i is solved as MAACO(grids[i], ..., **{**params, **map_params[i]}).
     Parameters never split waves; invalid map_params raise ValueError before any wave runs.
 
+    map_sizes (None or one mapping per map of `grids`, by global index) gives map i its own num_ants and / or
+    num_iterations, as MAACOBatch(map_sizes=...) takes them: map i is solved as MAACO(grids[i], num_ants_i,
+    num_iterations_i, ...).  Sizes never split waves either, and invalid map_sizes raise ValueError before any wave runs
+    or any map is read.  A wave's buffers are sized by its largest colony: per map, 128 bytes of slabs per ant and
+    32 x 32 tile plus max_cells bytes of move codes per ant -- at 256 x 256 and 4 096 ants, 32 MiB of slabs and 16 MiB
+    of move codes (default max_cells 4 096) -- so a wave that mixes one large colony with small ones holds the large
+    one's memory for every map.
+
     Returns a list of (map_index, path, length, turns, convergence_curve) for the maps of this rank; results
     are identical to solving each map alone (same seeds => same Philox streams)."""
     if map_params is not None:
         map_params = resolve_map_params(params, map_params, len(grids))
+    if map_sizes is not None:
+        map_sizes = resolve_map_sizes(int(num_ants), int(num_iterations), map_sizes, len(grids))
     lo, hi = shard_maps(len(grids), group)
     maps = _sweep_maps(grids, lo, hi)
     start, target = maps.first_cells()
@@ -703,7 +791,8 @@ def solve_maaco_batch(grids, num_ants, num_iterations, params, seeds=None, wave=
         b = MAACOBatch(maps.wave(idx), num_ants, num_iterations,
                        seeds=None if seeds is None else [seeds[i] for i in idx], device=device, max_cells=max_cells,
                        reuse=prev, per_map_endpoints=per_map_endpoints,
-                       map_params=None if map_params is None else [map_params[i] for i in idx], **params)
+                       map_params=None if map_params is None else [map_params[i] for i in idx],
+                       map_sizes=None if map_sizes is None else [map_sizes[i] for i in idx], **params)
         for i, (path, length, turns, curve) in zip(idx, b.solve()):
             out.append((i, path, length, turns, curve))
         b.close()

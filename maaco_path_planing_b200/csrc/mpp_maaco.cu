@@ -645,7 +645,18 @@ struct TourNoPeers {};
 struct TourMapParams {
     const mpp_maaco_params *params;  // [n_maps]
     const double *q0;                // [n_maps] this pass's q0 of every map
+    const int32_t *sizes;            // [n_maps][2] {num_ants, num_iterations} of every map, or null (mpp_maaco_pass_maps_sized)
 };
+// Map m's colony under a sizes array (the MP instantiations): sizes[m].num_ants clamped to [0, cap], where cap is the
+// launch's n_ants (the buffers' ant capacity), so no value can index past them.  Map m takes part in pass k only
+// while k <= sizes[m].num_iterations.
+__device__ __forceinline__ int sized_ants(const int32_t *sizes, int map, int cap) {
+    const int n = sizes[2 * map];
+    return n < 0 ? 0 : (n < cap ? n : cap);
+}
+__device__ __forceinline__ bool sized_past(const int32_t *sizes, int map, int iteration) {
+    return iteration > sizes[2 * map + 1];
+}
 template <bool P2P, bool MP>
 using TourExtra = typename std::conditional<P2P, TourPeers, typename std::conditional<MP, TourMapParams, TourNoPeers>::type>::type;
 template <bool P2P, bool MP>
@@ -657,6 +668,16 @@ mpp_maaco_tour1_kernel(const TourArgs A, const int apw, const TourExtra<P2P, MP>
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int R = A.R, C = A.C, TC = (C + 31) >> 5;
     const int map = blockIdx.y;
+    // MP with sizes: a map past its pass count constructs nothing (the whole CTA: grid.y = map), and only the map's own
+    // colony of n_live ants runs, writes slabs and results and counts steps.  (Read as `MP ? n_live : A.n_ants`, like
+    // k_q0 below.)
+    int n_live = A.n_ants;
+    if constexpr (MP) {
+        if (PA.sizes) {
+            if (sized_past(PA.sizes, map, (int)A.it)) return;
+            n_live = sized_ants(PA.sizes, map, A.n_ants);
+        }
+    }
     // MP: the same for the whole CTA (grid.y = map), loaded once and held in registers through the step loop.  (Read as
     // `MP ? k_q0 : A.q0`: the other instantiations keep reading TourArgs' scalars exactly as before.)
     double k_q0 = 0.0, k_alpha = 0.0;
@@ -715,9 +736,9 @@ mpp_maaco_tour1_kernel(const TourArgs A, const int apw, const TourExtra<P2P, MP>
     __syncthreads();
     const int warp = (blockIdx.x * MPP_TOUR1_THREADS + threadIdx.x) >> 5;
     const int a0 = warp * apw;                                     // first ant of this warp
-    if (a0 >= A.n_ants) return;                                    // whole warp
+    if (a0 >= (MP ? n_live : A.n_ants)) return;                    // whole warp
     const int a = a0 + lane;
-    bool active = lane < apw && a < A.n_ants;
+    bool active = lane < apw && a < (MP ? n_live : A.n_ants);
     int cur = MM.start;
     auto orient_mask = [](int dR, int dC) -> uint32_t {           // MAACO.py:146-157
         uint32_t k = 0xffu;
@@ -1022,7 +1043,7 @@ mpp_maaco_tour1_kernel(const TourArgs A, const int apw, const TourExtra<P2P, MP>
         }
     }
     // ---- the windows still hold the marks of their four tiles: write them to the ants' slabs ----
-    for (int src = 0; src < apw && a0 + src < A.n_ants; ++src) {
+    for (int src = 0; src < apw && a0 + src < (MP ? n_live : A.n_ants); ++src) {
         const int s_wr = __shfl_sync(0xffffffffu, wr, src), s_wc = __shfl_sync(0xffffffffu, wc, src);
         const uint2 o0 = win_w[src * 64 + lane], o1 = win_w[src * 64 + lane + 32];
         tour_tile_store(V, a0 + src, s_wr, s_wc, lane, o0.x);
@@ -1030,7 +1051,7 @@ mpp_maaco_tour1_kernel(const TourArgs A, const int apw, const TourExtra<P2P, MP>
         tour_tile_store(V, a0 + src, s_wr + 1, s_wc, lane, o1.x);
         tour_tile_store(V, a0 + src, s_wr + 1, s_wc + 1, lane, o1.y);
     }
-    if (lane < apw && a < A.n_ants) {
+    if (lane < apw && a < (MP ? n_live : A.n_ants)) {
         const bool ok = !failed && cur == target;
         mpp_ant_result res;
         res.length = ok ? len : __longlong_as_double(0x7ff0000000000000ll);
@@ -1153,11 +1174,13 @@ extern "C" int mpp_maaco_tours_p2p(const mpp_map_batch *maps, const mpp_colony *
 // field 0 = 0 when the ranking applies (all attractiveness < 1e-10), 7 when it does not; fields 1..7 are only
 // filled when P1 has exactly three moves.
 // ---------------------------------------------------------------------------------------------
-// MP (per-map parameters): alpha of params[map] instead of the launch's scalar
+// MP (per-map parameters): alpha of params[map] instead of the launch's scalar; with sizes, a map past its pass count
+// is skipped (its tours return before they read the ranking)
 template <bool MP>
 __device__ __forceinline__ void rank_body(const uint8_t *__restrict__ svalid_all, const double *__restrict__ tau_all,
                                           size_t tau_stride, const double *__restrict__ E01_all, size_t E01_stride,
-                                          double alpha, const mpp_maaco_params *__restrict__ params, int R, int C,
+                                          double alpha, const mpp_maaco_params *__restrict__ params,
+                                          const int32_t *__restrict__ sizes, int iteration, int R, int C,
                                           const MppMapMeta *__restrict__ meta, uint32_t *__restrict__ rank_all,
                                           size_t rank_stride, size_t rank_margin, size_t rank_fast_words,
                                           size_t rank_bundle_words, size_t rank_nb8_words,
@@ -1167,7 +1190,10 @@ __device__ __forceinline__ void rank_body(const uint8_t *__restrict__ svalid_all
     if (cell >= R * C) return;
     if (latch && *latch) return;
     const int map = blockIdx.y;
-    if constexpr (MP) alpha = params[map].alpha;
+    if constexpr (MP) {
+        if (sizes && sized_past(sizes, map, iteration)) return;
+        alpha = params[map].alpha;
+    }
     const uint8_t *svalid = svalid_all + (size_t)map * R * C;
     const double *tau = tau_all + (size_t)map * tau_stride;
     const double *E01 = E01_all + (size_t)map * E01_stride;
@@ -1251,25 +1277,26 @@ __global__ void __launch_bounds__(128) mpp_maaco_rank_kernel(const uint8_t *__re
                                                              size_t rank_stride, size_t rank_margin, size_t rank_fast_words,
                                                              size_t rank_bundle_words, size_t rank_nb8_words,
                                                              const int32_t *__restrict__ latch) {
-    rank_body<false>(svalid_all, tau_all, tau_stride, E01_all, E01_stride, alpha, nullptr, R, C, meta, rank_all, rank_stride,
-                     rank_margin, rank_fast_words, rank_bundle_words, rank_nb8_words, latch, threadIdx.x);
+    rank_body<false>(svalid_all, tau_all, tau_stride, E01_all, E01_stride, alpha, nullptr, nullptr, 0, R, C, meta, rank_all,
+                     rank_stride, rank_margin, rank_fast_words, rank_bundle_words, rank_nb8_words, latch, threadIdx.x);
 }
 __global__ void __launch_bounds__(128) mpp_maaco_rank_p_kernel(const uint8_t *__restrict__ svalid_all,
                                                                const double *__restrict__ tau_all, size_t tau_stride,
                                                                const double *__restrict__ E01_all, size_t E01_stride,
-                                                               const mpp_maaco_params *__restrict__ params, int R, int C,
+                                                               const mpp_maaco_params *__restrict__ params,
+                                                               const int32_t *__restrict__ sizes, int iteration, int R, int C,
                                                                const MppMapMeta *__restrict__ meta,
                                                                uint32_t *__restrict__ rank_all, size_t rank_stride,
                                                                size_t rank_margin, size_t rank_fast_words,
                                                                size_t rank_bundle_words, size_t rank_nb8_words,
                                                                const int32_t *__restrict__ latch) {
-    rank_body<true>(svalid_all, tau_all, tau_stride, E01_all, E01_stride, 0.0, params, R, C, meta, rank_all, rank_stride,
-                    rank_margin, rank_fast_words, rank_bundle_words, rank_nb8_words, latch, threadIdx.x);
+    rank_body<true>(svalid_all, tau_all, tau_stride, E01_all, E01_stride, 0.0, params, sizes, iteration, R, C, meta, rank_all,
+                    rank_stride, rank_margin, rank_fast_words, rank_bundle_words, rank_nb8_words, latch, threadIdx.x);
 }
 
-// params_dev != null: the per-map instantiation (alpha of each map's params)
+// params_dev != null: the per-map instantiation (alpha of each map's params; sizes_dev: maps past their pass count skip)
 static int rank_launch(const mpp_map_batch *maps, const mpp_colony *c, double alpha, const mpp_maaco_params *params_dev,
-                       void *stream) {
+                       void *stream, const int32_t *sizes_dev = nullptr, int iteration = 0) {
     int rc = colony_check(maps, c, "mpp_maaco_rank");
     if (rc) return rc;
     MPP_CUDA(cudaSetDevice(maps->device));
@@ -1278,8 +1305,9 @@ static int rank_launch(const mpp_map_batch *maps, const mpp_colony *c, double al
     const dim3 grid((total + 127) / 128, maps->n_maps);
     if (params_dev)
         mpp_maaco_rank_p_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(
-            maps->svalid_dev, c->tau, (size_t)c->tau_stride, c->E01, (size_t)c->E01_stride, params_dev, maps->rows,
-            maps->cols, maps->meta_dev, c->rank, L.total_words, L.margin, L.fast_words, L.bundle_words, L.nb8_words, c->latch);
+            maps->svalid_dev, c->tau, (size_t)c->tau_stride, c->E01, (size_t)c->E01_stride, params_dev, sizes_dev, iteration,
+            maps->rows, maps->cols, maps->meta_dev, c->rank, L.total_words, L.margin, L.fast_words, L.bundle_words,
+            L.nb8_words, c->latch);
     else
         mpp_maaco_rank_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(
             maps->svalid_dev, c->tau, (size_t)c->tau_stride, c->E01, (size_t)c->E01_stride, alpha, maps->rows, maps->cols,
@@ -1304,11 +1332,13 @@ __device__ __forceinline__ int move_delta(uint32_t m, int C) {
     return ((int)((0xA940u >> (2 * m)) & 3u) - 1) * C + ((int)((0x9224u >> (2 * m)) & 3u) - 1);
 }
 
-// MP (per-map parameters): Q of params[map] instead of the launch's scalar
+// MP (per-map parameters): Q of params[map] instead of the launch's scalar; with sizes, a map past its pass count keeps
+// its state, best path and log, and the scans see only the map's own colony (ants [n_live, n) deposit nothing)
 template <bool MP>
 __device__ __forceinline__ void best_body(const mpp_ant_result *__restrict__ res_all, const uint8_t *__restrict__ moves_all,
                                           int max_cells, int moves_ant_offset, int moves_n_ants, int n, double Q,
-                                          const mpp_maaco_params *__restrict__ params, int iteration, int C,
+                                          const mpp_maaco_params *__restrict__ params, const int32_t *__restrict__ sizes,
+                                          int iteration, int C,
                                           const MppMapMeta *__restrict__ meta, mpp_maaco_state *state_all,
                                           int32_t *best_cells_all, double *deposit_all, uint32_t *okbits_all,
                                           double *log_all, int log_rows, const int32_t *__restrict__ latch) {
@@ -1319,7 +1349,14 @@ __device__ __forceinline__ void best_body(const mpp_ant_result *__restrict__ res
     __shared__ int b_r, b_ant, b_turns, b_copy, s_base;
     if (latch && *latch) return;
     const int map = blockIdx.x;
-    if constexpr (MP) Q = params[map].Q;
+    int n_live = n;
+    if constexpr (MP) {
+        if (sizes) {
+            if (sized_past(sizes, map, iteration)) return;              // the whole CTA (one block per map)
+            n_live = sized_ants(sizes, map, n);
+        }
+        Q = params[map].Q;
+    }
     const mpp_ant_result *res = res_all + (size_t)map * n;
     double *deposit = deposit_all + (size_t)map * n;
     uint32_t *okbits = okbits_all + (size_t)map * ((n + 31) >> 5);
@@ -1332,13 +1369,15 @@ __device__ __forceinline__ void best_body(const mpp_ant_result *__restrict__ res
     for (int i0 = 0; i0 < n; i0 += MPP_BEST_THREADS) {               // whole warps stay together for the ballot
         const int i = i0 + tid;
         bool dep = false;
-        if (i < n) {
+        if (i < n_live) {
             const mpp_ant_result ri = res[i];
             const double l = ri.length;
             if (lt_len_idx(l, i, ml, mi)) { ml = l; mi = i; }
             // deposit amount MAACO.py:307-308 (0.0 == "does not deposit"; x + 0.0 is exact anyway)
             dep = (l != INF && ri.n_cells > 0 && l > 1e-6);
             deposit[i] = dep ? Q / l : 0.0;
+        } else if (i < n) {
+            deposit[i] = 0.0;                                         // outside the map's colony (MP with sizes)
         }
         const uint32_t ok = __ballot_sync(0xffffffffu, dep);
         if (lane == 0 && i < n) okbits[i >> 5] = ok;
@@ -1367,7 +1406,7 @@ __device__ __forceinline__ void best_body(const mpp_ant_result *__restrict__ res
     // phase 2: among {r} U {i>r : |len_i - L| < 1e-9} the first index with the fewest turns
     int bt = 0x7fffffff, bi = 0x7fffffff;
     if (L != INF) {
-        for (int i = tid; i < n; i += MPP_BEST_THREADS) {
+        for (int i = tid; i < n_live; i += MPP_BEST_THREADS) {
             if (i < r) continue;
             const mpp_ant_result ri = res[i];
             const double l = ri.length;
@@ -1454,29 +1493,30 @@ mpp_maaco_best_kernel(const mpp_ant_result *__restrict__ res_all, const uint8_t 
                       const MppMapMeta *__restrict__ meta, mpp_maaco_state *state_all, int32_t *best_cells_all,
                       double *deposit_all, uint32_t *okbits_all, double *log_all, int log_rows,
                       const int32_t *__restrict__ latch) {
-    best_body<false>(res_all, moves_all, max_cells, moves_ant_offset, moves_n_ants, n, Q, nullptr, iteration, C, meta,
-                     state_all, best_cells_all, deposit_all, okbits_all, log_all, log_rows, latch);
+    best_body<false>(res_all, moves_all, max_cells, moves_ant_offset, moves_n_ants, n, Q, nullptr, nullptr, iteration, C,
+                     meta, state_all, best_cells_all, deposit_all, okbits_all, log_all, log_rows, latch);
 }
 __global__ void __launch_bounds__(MPP_BEST_THREADS)
 mpp_maaco_best_p_kernel(const mpp_ant_result *__restrict__ res_all, const uint8_t *__restrict__ moves_all, int max_cells,
                         int moves_ant_offset, int moves_n_ants, int n, const mpp_maaco_params *__restrict__ params,
-                        int iteration, int C, const MppMapMeta *__restrict__ meta, mpp_maaco_state *state_all,
-                        int32_t *best_cells_all, double *deposit_all, uint32_t *okbits_all, double *log_all, int log_rows,
-                        const int32_t *__restrict__ latch) {
-    best_body<true>(res_all, moves_all, max_cells, moves_ant_offset, moves_n_ants, n, 0.0, params, iteration, C, meta,
-                    state_all, best_cells_all, deposit_all, okbits_all, log_all, log_rows, latch);
+                        const int32_t *__restrict__ sizes, int iteration, int C, const MppMapMeta *__restrict__ meta,
+                        mpp_maaco_state *state_all, int32_t *best_cells_all, double *deposit_all, uint32_t *okbits_all,
+                        double *log_all, int log_rows, const int32_t *__restrict__ latch) {
+    best_body<true>(res_all, moves_all, max_cells, moves_ant_offset, moves_n_ants, n, 0.0, params, sizes, iteration, C,
+                    meta, state_all, best_cells_all, deposit_all, okbits_all, log_all, log_rows, latch);
 }
 
 static int best_launch(const mpp_map_batch *maps, const mpp_colony *c, int moves_ant_offset, int moves_n_ants,
-                       int n_ants_total, double Q, const mpp_maaco_params *params_dev, int iteration, void *stream) {
+                       int n_ants_total, double Q, const mpp_maaco_params *params_dev, int iteration, void *stream,
+                       const int32_t *sizes_dev = nullptr) {
     int rc = colony_check(maps, c, "mpp_maaco_best");
     if (rc) return rc;
     MPP_REQUIRE(n_ants_total > 0 && iteration >= 1, "mpp_maaco_best: n_ants=%d iteration=%d", n_ants_total, iteration);
     MPP_CUDA(cudaSetDevice(maps->device));
     if (params_dev)
         mpp_maaco_best_p_kernel<<<maps->n_maps, MPP_BEST_THREADS, 0, (cudaStream_t)stream>>>(
-            c->result, c->moves, c->max_cells, moves_ant_offset, moves_n_ants, n_ants_total, params_dev, iteration,
-            maps->cols, maps->meta_dev, c->state, c->best_cells, c->deposit, c->okbits, c->log, c->log_rows, c->latch);
+            c->result, c->moves, c->max_cells, moves_ant_offset, moves_n_ants, n_ants_total, params_dev, sizes_dev,
+            iteration, maps->cols, maps->meta_dev, c->state, c->best_cells, c->deposit, c->okbits, c->log, c->log_rows, c->latch);
     else
         mpp_maaco_best_kernel<<<maps->n_maps, MPP_BEST_THREADS, 0, (cudaStream_t)stream>>>(
             c->result, c->moves, c->max_cells, moves_ant_offset, moves_n_ants, n_ants_total, Q, iteration, maps->cols,
@@ -1551,9 +1591,11 @@ __device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; a
 #ifndef MPP_PHER_MINB
 #define MPP_PHER_MINB 7
 #endif
-// MP (per-map parameters): rho of params[map] instead of PherArgs' scalar
+// MP (per-map parameters): rho of params[map] instead of PherArgs' scalar; with sizes, a map past its pass count is left
+// as it is (no evaporation).  Ants outside a map's colony have no `touched` and no `okbits` bits: nothing else changes.
 template <bool MP>
-__device__ __forceinline__ void pheromone_body(const PherArgs &A, const mpp_maaco_params *__restrict__ params) {
+__device__ __forceinline__ void pheromone_body(const PherArgs &A, const mpp_maaco_params *__restrict__ params,
+                                               const int32_t *__restrict__ sizes, int iteration) {
     __shared__ int s_list[MPP_PHER_CHUNK];
 #ifdef MPP_PHER_PROF
     const unsigned long long prof_t0 = gtimer();
@@ -1568,7 +1610,10 @@ __device__ __forceinline__ void pheromone_body(const PherArgs &A, const mpp_maac
 #endif
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, map = blockIdx.y;
     double rho = A.rho;
-    if constexpr (MP) rho = params[map].rho;
+    if constexpr (MP) {
+        if (sizes && sized_past(sizes, map, iteration)) return;         // the whole CTA (grid.y = map)
+        rho = params[map].rho;
+    }
     const int TC = (A.C + 31) >> 5;
     // the start and the target tile carry the longest chains (every depositing ant): their CTAs go first
     int tile_l = blockIdx.x >> 2;                                     // tile index inside the buffers
@@ -1732,17 +1777,18 @@ __device__ __forceinline__ void pheromone_body(const PherArgs &A, const mpp_maac
     }
 }
 __global__ void __launch_bounds__(MPP_PHER_THREADS, MPP_PHER_MINB) mpp_maaco_pheromone_kernel(const PherArgs A) {
-    pheromone_body<false>(A, nullptr);
+    pheromone_body<false>(A, nullptr, nullptr, 0);
 }
 __global__ void __launch_bounds__(MPP_PHER_THREADS, MPP_PHER_MINB)
-mpp_maaco_pheromone_p_kernel(const PherArgs A, const mpp_maaco_params *__restrict__ params) {
-    pheromone_body<true>(A, params);
+mpp_maaco_pheromone_p_kernel(const PherArgs A, const mpp_maaco_params *__restrict__ params,
+                             const int32_t *__restrict__ sizes, int iteration) {
+    pheromone_body<true>(A, params, sizes, iteration);
 }
 
 static int pheromone_launch(const mpp_map_batch *maps, const mpp_colony *c, uint32_t *slabs_dev, uint32_t *touched_dev,
                             int n_ants_total, int tile_row0, int buf_tile_rows, double rho, int iteration, int clear_slabs,
                             double *const *tau_peers_dev, int n_peers, void *stream,
-                            const mpp_maaco_params *params_dev = nullptr) {
+                            const mpp_maaco_params *params_dev = nullptr, const int32_t *sizes_dev = nullptr) {
     int rc = colony_check(maps, c, "mpp_maaco_pheromone");
     if (rc) return rc;
     const int TR = tiles_r(maps->rows), TC = tiles_c(maps->cols);
@@ -1769,7 +1815,8 @@ static int pheromone_launch(const mpp_map_batch *maps, const mpp_colony *c, uint
     A.meta = maps->meta_dev;
     MPP_REQUIRE(!tau_peers_dev || (n_peers > 0 && maps->n_maps == 1), "mpp_maaco_pheromone: peer tau needs n_peers > 0 and one map");
     const dim3 grid(n_tile_rows * TC * 4, maps->n_maps);
-    if (params_dev) mpp_maaco_pheromone_p_kernel<<<grid, MPP_PHER_THREADS, 0, (cudaStream_t)stream>>>(A, params_dev);
+    if (params_dev)
+        mpp_maaco_pheromone_p_kernel<<<grid, MPP_PHER_THREADS, 0, (cudaStream_t)stream>>>(A, params_dev, sizes_dev, iteration);
     else mpp_maaco_pheromone_kernel<<<grid, MPP_PHER_THREADS, 0, (cudaStream_t)stream>>>(A);
     MPP_CUDA(cudaGetLastError());
     return MPP_OK;
@@ -2013,21 +2060,29 @@ extern "C" int mpp_maaco_pass(const mpp_map_batch *maps, const mpp_colony *c, co
 
 // The same pass with per-map colony parameters: params_dev [n_maps] on the device, q0_dev the [num_iterations][n_maps]
 // q0 table (row iteration-1 is this pass's); the per-map instantiations of the four kernels read their scalars from them.
-extern "C" int mpp_maaco_pass_maps(const mpp_map_batch *maps, const mpp_colony *c, const mpp_maaco_params *params_dev,
-                                   const double *q0_dev, int iteration, int n_ants, int ants_per_warp, void *stream) {
+// sizes_dev (null, or [n_maps] {num_ants, num_iterations} on the device) gives each map its own colony inside the
+// buffers' n_ants and its own pass count (sized_ants / sized_past).
+extern "C" int mpp_maaco_pass_maps_sized(const mpp_map_batch *maps, const mpp_colony *c, const mpp_maaco_params *params_dev,
+                                         const double *q0_dev, const int32_t *sizes_dev, int iteration, int n_ants,
+                                         int ants_per_warp, void *stream) {
     MPP_REQUIRE(maps && c, "mpp_maaco_pass_maps: null argument");
     MPP_REQUIRE(params_dev && q0_dev, "mpp_maaco_pass_maps: null params_dev / q0_dev");
     MPP_REQUIRE(iteration >= 1, "mpp_maaco_pass_maps: iteration %d < 1", iteration);
-    int rc = rank_launch(maps, c, 0.0, params_dev, stream);
+    int rc = rank_launch(maps, c, 0.0, params_dev, stream, sizes_dev, iteration);
     if (rc) return rc;
-    const TourMapParams mp{params_dev, q0_dev + (size_t)(iteration - 1) * maps->n_maps};
+    const TourMapParams mp{params_dev, q0_dev + (size_t)(iteration - 1) * maps->n_maps, sizes_dev};
     rc = tours_launch(maps, c, iteration, 0.0, 0.0, n_ants, 0, n_ants, ants_per_warp, nullptr, nullptr, nullptr, 0, 1, stream,
                       &mp);
     if (rc) return rc;
-    rc = best_launch(maps, c, 0, n_ants, n_ants, 0.0, params_dev, iteration, stream);
+    rc = best_launch(maps, c, 0, n_ants, n_ants, 0.0, params_dev, iteration, stream, sizes_dev);
     if (rc) return rc;
     return pheromone_launch(maps, c, c->slabs, c->touched, n_ants, 0, tiles_r(maps->rows), 0.0, iteration, 0, nullptr, 0,
-                            stream, params_dev);
+                            stream, params_dev, sizes_dev);
+}
+
+extern "C" int mpp_maaco_pass_maps(const mpp_map_batch *maps, const mpp_colony *c, const mpp_maaco_params *params_dev,
+                                   const double *q0_dev, int iteration, int n_ants, int ants_per_warp, void *stream) {
+    return mpp_maaco_pass_maps_sized(maps, c, params_dev, q0_dev, nullptr, iteration, n_ants, ants_per_warp, stream);
 }
 
 extern "C" int mpp_maaco_pass_host(const mpp_map_batch *maps, const mpp_colony *c, const mpp_maaco_params *p, int iteration,
